@@ -38,6 +38,7 @@ import time
 os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
 if os.environ.get("NCCL_DEBUG", "").upper() == "VERSION":      # the one level NCCL_DEBUG_FILE does not apply to
     os.environ["NCCL_DEBUG"] = "WARN"
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the (possibly read-only) tree, no __pycache__ either
 
 import numpy as np
 import torch
@@ -170,6 +171,20 @@ def _make_c2(seed):
     return tm_synth.make_design(seed=seed, **tm_synth.CONFIGS["c2"])
 
 
+def dump_outputs(out_dir, loss, pred, model, cnn):
+    """--dump-outputs: what one timed step hands its caller -- the loss, the predictions and every parameter gradient
+    -- as ``<out_dir>/<name>.npy`` in float32 (``grad.model.<param>``, ``grad.cnn.<param>``; 12 MB for config 2).
+    The design and the initial weights are seeded, so two builds given the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss, "pred": pred}
+    for prefix, mod in (("model", model), ("cnn", cnn)):
+        for k, p in mod.named_parameters():
+            if p.grad is not None:
+                arrays[f"grad.{prefix}.{k}"] = p.grad
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 # CUDA arm
 # ------------------------------------------------------------------------------------------------
@@ -186,6 +201,8 @@ def main():
     ap.add_argument("--no-sustained", action="store_true", help="skip the >= 3 s sustained repeat of the resident loop")
     ap.add_argument("--no-shuffled", action="store_true", help="skip the fresh-endpoint-batch-every-step end-to-end loop")
     ap.add_argument("--config5", type=int, default=64, help="designs of the config-5 run (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the last one's loss, predictions and parameter gradients to DIR/<name>.npy")
     ap.add_argument("--profile-step", action="store_true",
                     help="after the warm-up run ONE step between cudaProfilerStart/Stop and exit "
                          "(for `ncu --profile-from-start off`); prints no bench line")
@@ -267,7 +284,7 @@ def main():
     sync_all()
     e0.record()
     for _ in range(args.steps):
-        loss, _ = run_step()
+        loss, pred = run_step()
     e1.record()
     sync_all()
     launches = launches_per_step * args.steps
@@ -275,6 +292,8 @@ def main():
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms.item())
+    if args.dump_outputs and rank == 0:          # now: the loops below replay other graphs that rewrite param.grad
+        dump_outputs(args.dump_outputs, loss, pred, model, cnn)
 
     # ---- end to end from pinned host memory through the public API: every step copies its inputs
     # host -> device and reads its loss back.  The upload of step i+1 is issued on a copy stream before

@@ -19,8 +19,8 @@ Layout
 ``fake_dgl.py``   ~100-line stand-in for the DGL graph surface the reference
                   touches (``pull`` semantics per SURVEY.md Appendix A).
 ``dgl_stub/``     inert ``dgl.function`` so the reference's ``model.py`` imports.
-``ref_loader.py`` imports the UNMODIFIED reference modules from
-                  ``/root/reference/src`` (only possible in the dev container).
+``ref_loader.py`` imports the UNMODIFIED reference modules from the original
+                  project's ``src/`` (``TM_REFERENCE_SRC``; not in this repository).
 ``make_golden.py``runs the unmodified reference on seeded inputs and writes
                   ``tests/golden/*.npz`` -- the committed fixtures the oracle
                   restatement and the CUDA path are pinned against.

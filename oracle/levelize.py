@@ -10,7 +10,7 @@ numpy restatements of
   model.py:186-204)
 
 Pinned against the reference's own ``cal_topo_level`` / ``find_critical_path``
-source, executed from ``/root/reference`` on networkx graphs
+source, executed from the original project on networkx graphs
 (``oracle/make_golden.py`` -> ``tests/golden/levels_*.npz``,
 ``tests/test_oracle_pinning.py``).
 """

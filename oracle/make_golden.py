@@ -1,7 +1,7 @@
 """Generate ``tests/golden/*.npz`` by running the UNMODIFIED reference here.
 
-Oracle / test infrastructure only.  Run in the dev container (needs
-``/root/reference``):  ``python oracle/make_golden.py``.
+Oracle / test infrastructure only.  Needs a checkout of the original project:
+``TM_REFERENCE_SRC=<reference>/src python oracle/make_golden.py``.
 
 * ``step_<cfg>.npz``   one design step of the reference's own ``PathModel`` /
   ``PathConv`` / ``MLP`` (``src/model.py``) + ``UNet`` (``src/Unet.py``) driven
@@ -143,7 +143,7 @@ def dump_layoutnet(seed=0):
 
 
 if __name__ == "__main__":
-    assert ref_loader.available(), "needs /root/reference (dev container only)"
+    assert ref_loader.available(), "set TM_REFERENCE_SRC to the original project's src/ directory"
     os.makedirs(GOLD, exist_ok=True)
     dump_step("tiny")
     dump_levels("tiny")

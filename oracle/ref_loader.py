@@ -1,7 +1,9 @@
-"""Import the UNMODIFIED reference modules from ``/root/reference/src``.
+"""Import the UNMODIFIED reference modules from the original project's ``src/``
+directory, named by the environment variable ``TM_REFERENCE_SRC``.
 
-Oracle / test infrastructure only, and only usable in the dev container: the
-GPU box has no ``/root/reference``.  ``available()`` says whether it is there.
+Oracle / test infrastructure only, used by ``make_golden.py`` alone: the
+reference is not part of this repository, and the tests compare against the
+fixtures it generated.  ``available()`` says whether it is there.
 
 * ``ref_model()`` -> the reference ``model.py`` module (needs the inert
   ``dgl.function`` stub under ``oracle/dgl_stub``);
@@ -18,13 +20,13 @@ import importlib.util
 import os
 import sys
 
-REF_SRC = "/root/reference/src"
+REF_SRC = os.environ.get("TM_REFERENCE_SRC", "")
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _cache = {}
 
 
 def available():
-    return os.path.isfile(os.path.join(REF_SRC, "model.py"))
+    return bool(REF_SRC) and os.path.isfile(os.path.join(REF_SRC, "model.py"))
 
 
 def _load(name, filename):

@@ -1,5 +1,6 @@
 import sys, time, os
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/multimodal-fusion-based-pre-routing-timing-prediction-_b200')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'multimodal-fusion-based-pre-routing-timing-prediction-_b200'))
 import bench, torch
 print('cores', os.cpu_count())
 for scale in (10, 4, 2, 1):

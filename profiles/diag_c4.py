@@ -1,5 +1,5 @@
 import importlib, os, sys, torch
-ROOT="/root/repo"; sys.path.insert(0, ROOT); PKG="multimodal-fusion-based-pre-routing-timing-prediction-_b200"; sys.path.insert(0, os.path.join(ROOT, PKG))
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT); PKG="multimodal-fusion-based-pre-routing-timing-prediction-_b200"; sys.path.insert(0, os.path.join(ROOT, PKG))
 importlib.import_module(PKG)
 import Unet as U, tm_unet
 from oracle import restate

@@ -10,7 +10,7 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (run with `gpurun --gpus 2`)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (one rank per GPU)")
 def test_nccl_gradient_equivalence_world2():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", "29641", os.path.join(ROOT, "tests", "dp_equivalence.py")]

@@ -903,8 +903,8 @@ def test_mask_row_selection_on_device(mods):
 def test_loader_train_loop_shape(mods, tmp_path):
     """N3 + N1: a design written in the reference's per-design tuple format (generate_data.py:50-54, raw 42 / 3
     feature columns), read back by tm_loader.load_single_design (train.py:335-388: feat_reduce trim, oversampling)
-    and driven by a RESTATEMENT of the reference's batch loop (train.py:468-562; the file itself cannot run on the
-    GPU box: /root/reference is absent there and it imports tkinter / lib2to3 / dgl / torchmetrics): shuffled
+    and driven by a RESTATEMENT of the reference's batch loop (train.py:468-562; the file itself cannot run here:
+    it is not part of this repository and it imports tkinter / lib2to3 / dgl / torchmetrics): shuffled
     DataLoader batches, per-level model(graph, nodes, eids, targets, level_id, level_th, dense path_map) calls,
     MSELoss, backward(retain_graph=True), Adam, h rebinding, CNN forward again.  The SAME batches through the fused
     step (LoadedDesign.prepare: one CUDA-graph capture, endpoint batch refreshed in place) must give the same loss."""
