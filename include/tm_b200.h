@@ -56,12 +56,6 @@ typedef struct {
   /* device copies the persistent propagation kernels read (one launch loops over all levels) */
   const int32_t* level_ptr;  /* [num_levels+1] first schedule position of each level       */
   const int32_t* cell_base;  /* [num_levels+1] first compact cell row of each level        */
-  int32_t* sync_flags;       /* [n + n_cell_rows] scratch: per-pin / per-cell-row ready flags of the
-                              * dataflow-synchronised persistent kernels (zeroed by every call)   */
-  int32_t single_driver;     /* 1: every pin on an odd level has exactly one net in-edge and its source is on an
-                              * even level -- the persistent forward may then write net-level rows from their
-                              * driver's producer ("push" fusion) and skip the odd levels                */
-  int32_t reserved0;
 } tm_schedule;
 
 /* ------------------------------------------------------------------------------------
@@ -156,26 +150,19 @@ int tm_transpose(int64_t rows, int64_t cols, const float* in, float* out, void* 
  *   W1t[128,256], b1[256], W2t[256,128], b2[128]: fc_cell_neigh, weights TRANSPOSED;
  *   A[n_cell_rows,128], LSE[n_cell_rows,128], HID[n_cell_rows,256]: saved for backward
  *              (may be NULL for inference). */
-size_t tm_gnn_ws_bytes(void);   /* workspace of tm_gnn_forward / tm_gnn_backward: the grid-barrier counter of the
-                                 * persistent kernels (default) / the re-packed weights of the per-level kernels */
+size_t tm_gnn_ws_bytes(void);   /* workspace of tm_gnn_forward / tm_gnn_backward: the packed weights and the grid-barrier
+                                 * counter of the persistent kernels (default) / the re-packed weights of the per-level
+                                 * kernels */
 /* Implementation selector (process-wide; also env TM_GNN_IMPL=<bits>|persist|levels).  Bit 0 selects the forward
  * pass, bit 1 the backward pass; 4 (default) = auto: persistent forward, persistent backward only when the schedule
  * is wide (>= 6 000 pins per level on average) -- what measures fastest on config 2 and config 3:
  *   bit set   = ONE persistent kernel for the whole pass: 2-CTA clusters, fc_cell_neigh resident in shared memory,
  *               the tile MLP transposed on tcgen05 (fp16 two-term split, fp32 accumulate in TMEM), one grid-wide
- *               barrier per level (or, with TM_GNN_SYNC=flow, per-pin ready flags and no barrier);
+ *               barrier per level;
  *   bit clear = one launch per level (mma.sync 3xTF32 tile MLP, weights streamed per level, PDL-chained);
- *   8         = one launch per level with the CELL levels on the cluster tile kernel (tcgen05, fp16 split); measured
- *               slower than both (DESIGN.md section 4).
- * Returns the previous value; impl < 0 only queries. */
+ *   16        = the per-level cell kernels run the fp16 two-term split (mma.sync.m16n8k16) instead of 3xTF32.
+ * Other bits are ignored.  Returns the previous value; impl < 0 only queries. */
 int tm_gnn_set_impl(int impl);
-/* Level ordering inside the persistent kernels: 0 = grid barrier per level (default), 1 = per-pin ready flags
- * (dataflow; also env TM_GNN_SYNC=flow), 2 = grid barrier + net-level "push" fusion in the forward (rows of
- * single-driver net pins written by their driver's producer, odd levels skipped; also env TM_GNN_FUSE=1), 3 = sentinel
- * dataflow in the forward (H pre-filled with 0xFFFFFFFF words, every gathered 16-byte piece validates itself: no flag,
- * no fence; the backward uses the flags).  All alternatives measured slower than 0 on B200 (DESIGN.md section 4).
- * Returns the previous value; flow < 0 only queries. */
-int tm_gnn_set_sync(int flow);
 /* Grid-wide barriers inside the last tm_gnn_forward / tm_gnn_backward call of this thread (persistent kernel:
  * one per non-empty level; per-level kernels: 0, they synchronise by kernel boundaries). */
 int tm_gnn_last_barriers(void);

@@ -786,8 +786,7 @@ int launch_pdl(void (*kern)(KArgs...), unsigned grid, unsigned block, size_t sme
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  static const int pdl = getenv("TM_GNN_PDL") ? atoi(getenv("TM_GNN_PDL")) : 1;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
@@ -816,16 +815,15 @@ namespace tmk {
 size_t gnn_persist_ws_bytes();
 void gnn_persist_set_profile(long long* p);
 int gnn_persist_profile_slots();
-int gnn_persist_set_flow(int flow);
 int gnn_persist_forward(const tm_schedule* s, int lb, int le, float* H, const float* S, const float* W1t, const float* b1,
-                        const float* W2t, const float* b2, float* A, float* LSE, float* HIDb, void* ws, cudaStream_t st,
-                        bool begin, bool per_level);
+                        const float* W2t, const float* b2, float* A, float* LSE, float* HIDb, void* ws, cudaStream_t st);
 int gnn_persist_backward(const tm_schedule* s, const float* H, float* G, const float* W1, const float* W2, const float* A,
                          const float* LSE, const float* HIDb, float* GA, float* GHID, float* GZC, void* ws, cudaStream_t st,
-                         int lb, int le, bool begin, bool per_level);
+                         int lb, int le);
 }  // namespace tmk
 
 namespace {
+constexpr int IMPL_BITS = 1 | 2 | 4 | 16;     // the tm_gnn_set_impl bits that select something
 std::atomic<int> g_impl{-1};
 thread_local int g_last_barriers = 0;
 int gnn_impl() {
@@ -838,7 +836,7 @@ int gnn_impl() {
     //   persistent backward only on wide schedules (>= 6 000 pins per level on average).
     const char* e = getenv("TM_GNN_IMPL");
     //   Bit 4 (16): the per-level cell kernels run the fp16 two-term split (mma.sync.m16n8k16) instead of 3xTF32.
-    v = !e ? 20 : (e[0] == 'l' ? 0 : (e[0] == 'p' ? 3 : (atoi(e) & 31)));
+    v = !e ? 20 : (e[0] == 'l' ? 0 : (e[0] == 'p' ? 3 : (atoi(e) & IMPL_BITS)));
     g_impl.store(v, std::memory_order_relaxed);
   }
   return v;
@@ -852,11 +850,10 @@ int count_levels(const tm_schedule* s, int lb, int le) {
 
 extern "C" int tm_gnn_set_impl(int impl) {
   const int prev = gnn_impl();
-  if (impl >= 0) g_impl.store(impl & 31, std::memory_order_relaxed);
+  if (impl >= 0) g_impl.store(impl & IMPL_BITS, std::memory_order_relaxed);
   return prev;
 }
 extern "C" int tm_gnn_last_barriers() { return g_last_barriers; }
-extern "C" int tm_gnn_set_sync(int flow) { return tmk::gnn_persist_set_flow(flow); }
 extern "C" int tm_gnn_set_profile(void* clocks) {
   tmk::gnn_persist_set_profile(reinterpret_cast<long long*>(clocks));
   return 0;
@@ -898,25 +895,19 @@ extern "C" int tm_gnn_forward(const tm_schedule* s, int32_t lb, int32_t le, floa
   if (gnn_impl() & 5) {
     TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_forward: workspace too small (tm_gnn_ws_bytes)");
     g_last_barriers = count_levels(s, lb, le);
-    return tmk::gnn_persist_forward(s, lb, le, H, S, W1t_in, b1, W2t_in, b2, A, LSE, HIDb, ws, st, true, false);
+    return tmk::gnn_persist_forward(s, lb, le, H, S, W1t_in, b1, W2t_in, b2, A, LSE, HIDb, ws, st);
   }
   g_last_barriers = 0;
-  const bool tc_levels = (gnn_impl() & 8) && s->level_ptr && s->cell_base && s->sync_flags;   // cell levels on the tcgen05 cluster tile kernel
   TM_TRY(cell_smem_optin());
   const float *W1t = nullptr, *W2t = nullptr;
   const bool h16 = gnn_impl() & 16;
-  if (!tc_levels) TM_TRY(pack_pair(W1t_in, W2t_in, ws, ws_bytes, &W1t, &W2t, st, h16));
+  TM_TRY(pack_pair(W1t_in, W2t_in, ws, ws_bytes, &W1t, &W2t, st, h16));
   int crow0 = cell_base_of(s, lb + (lb & 1));
-  bool tc_begun = false;
   for (int l = lb; l < le; ++l) {
     const int p0 = s->h_level_ptr[l], cnt = s->h_level_ptr[l + 1] - p0;
     const bool cell = (l > 0) && !(l & 1);
     if (cnt > 0) {
-      if (cell && tc_levels) {
-        TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_forward: workspace too small (tm_gnn_ws_bytes)");
-        TM_TRY(tmk::gnn_persist_forward(s, l, l + 1, H, S, W1t_in, b1, W2t_in, b2, A, LSE, HIDb, ws, st, !tc_begun, true));
-        tc_begun = true;
-      } else if (!cell) {
+      if (!cell) {
         TM_TRY(launch_pdl(gnn_net_fwd_kernel, (unsigned)cdiv(cnt, 8), 256, 0, st, "gnn_net_fwd", s->order, p0, cnt, s->f_ptr,
                           s->f_src, S, H));
       } else {
@@ -938,16 +929,14 @@ extern "C" int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, c
   if ((gnn_impl() & 2) || ((gnn_impl() & 4) && wide)) {
     TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_backward: workspace too small (tm_gnn_ws_bytes)");
     g_last_barriers = count_levels(s, 0, s->num_levels);
-    return tmk::gnn_persist_backward(s, H, G, W1_in, W2_in, A, LSE, HIDb, GA, GHID, GZC, ws, st, 0, s->num_levels, true, false);
+    return tmk::gnn_persist_backward(s, H, G, W1_in, W2_in, A, LSE, HIDb, GA, GHID, GZC, ws, st, 0, s->num_levels);
   }
   g_last_barriers = 0;
-  const bool tc_levels = (gnn_impl() & 8) && s->level_ptr && s->cell_base && s->sync_flags;
   TM_TRY(cell_smem_optin());
   // backward products: g_hid = g_z @ W2 (W2 [128][256] is "Wa"), g_a = g_hid @ W1 (W1 [256][128] is "Wb")
   const float *W2 = nullptr, *W1 = nullptr;
   const bool h16 = gnn_impl() & 16;
-  if (!tc_levels) TM_TRY(pack_pair(W2_in, W1_in, ws, ws_bytes, &W2, &W1, st, h16));
-  bool tc_begun = false;
+  TM_TRY(pack_pair(W2_in, W1_in, ws, ws_bytes, &W2, &W1, st, h16));
   SchedDev d{s->order, s->bn_ptr, s->bn_dst, s->bn_w, s->bc_ptr, s->bc_row};
   int crow_end = cell_base_of(s, s->num_levels + (s->num_levels & 1));  // total cell rows
   for (int l = s->num_levels - 1; l >= 0; --l) {
@@ -955,11 +944,7 @@ extern "C" int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, c
     const bool cell = (l > 0) && !(l & 1);
     if (cell) crow_end -= cnt;
     if (cnt <= 0) continue;
-    if (cell && tc_levels) {
-      TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_backward: workspace too small (tm_gnn_ws_bytes)");
-      TM_TRY(tmk::gnn_persist_backward(s, H, G, W1_in, W2_in, A, LSE, HIDb, GA, GHID, GZC, ws, st, l, l + 1, !tc_begun, true));
-      tc_begun = true;
-    } else if (!cell) {
+    if (!cell) {
       TM_TRY(launch_pdl(gnn_net_bwd_kernel, (unsigned)cdiv(cnt, 8), 256, 0, st, "gnn_net_bwd", d, p0, cnt, H, G, (const float*)GA, A, LSE));
     } else {
       TM_TRY(launch_pdl(h16 ? gnn_cell_bwd_kernel<true> : gnn_cell_bwd_kernel<false>, (unsigned)cdiv(cnt, TILE), CT, CELL_SMEM, st, "gnn_cell_bwd", d, p0, cnt, crow_end, H,

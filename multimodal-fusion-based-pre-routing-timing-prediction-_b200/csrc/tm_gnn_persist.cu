@@ -1,13 +1,11 @@
 // G2/G3, persistent form: the WHOLE level-wise propagation (forward) or its reverse sweep (backward)
 // is ONE kernel -- 74 two-CTA clusters, one CTA per SM, each looping over the levels -- instead of
-// one launch per level.  Two ways of ordering the levels are compiled (template FLOW):
-//   * barrier (default): a grid-wide barrier per level on a monotonic counter (one release-add per
-//     CTA, one warp polls), static prefetches between arrive and wait;
-//   * dataflow (TM_GNN_SYNC=flow): no grid barrier; every pin has a ready flag (zeroed by the host), a
-//     producer publishes a row with a release store, a consumer polls the flags of exactly the rows it
-//     gathers.  Measured SLOWER on B200 (config 2 forward 1.32 ms against 0.93 ms): a release fence
-//     per produced row and a flag round trip before every gather cost more than one barrier per level.  Replaces PathConv.forward and its UDFs (src/model.py:88-116,138-153,158-213, one DGL `pull`
-// + cuBLAS calls + an (N,128) index_copy PER LEVEL) and the autograd backward (src/train.py:553).
+// one launch per level.  Levels are ordered by a grid-wide barrier per level on a monotonic counter
+// (one release-add per CTA, one warp polls), with the next level's static inputs prefetched into L2
+// between arrive and wait.  (Dataflow orderings without a barrier, net-level push fusion and one launch
+// per cell level were all measured slower on B200: DESIGN.md section 4.)  Replaces PathConv.forward
+// and its UDFs (src/model.py:88-116,138-153,158-213, one DGL `pull` + cuBLAS calls + an (N,128)
+// index_copy PER LEVEL) and the autograd backward (src/train.py:553).
 //
 // Why a cluster pair: the 128->256->128 MLP of fc_cell_neigh (model.py:48,138-146) sits inside the
 // level recurrence and every cell pin needs all of its weights.  They stay RESIDENT in shared
@@ -27,9 +25,8 @@
 //
 // Net levels / level 0 (mean over net in-edges) are processed by sub-warp groups (8 / 16 / 32 lanes
 // per pin, chosen per level so that every pin gets its own group when the level fits).
-// Everything static (schedule pointers, edge indices, S rows) is fetched BEFORE the flags are polled.
+// Everything static (schedule pointers, edge indices, S rows) is fetched BEFORE the barrier wait.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "tm_common.cuh"
 
@@ -106,39 +103,6 @@ struct GridBar {
     __syncthreads();
   }
 };
-
-// Ready flags (one uint32 per pin / per compact cell row, zeroed by the host before the launch).
-// Rows are read with ld.global.cg (L2, the coherence point) strictly after the flag was seen set;
-// the producer's release store orders its row stores (and, through bar.sync / __syncwarp, those of
-// the other threads that wrote the row) before the flag.  Bounded: a lost producer traps.
-__device__ __forceinline__ unsigned int ld_flag(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void wait_flag(const unsigned int* p) {
-  for (uint32_t spin = 0; ld_flag(p) == 0u; ++spin)
-    if (spin > (1u << 22)) __trap();
-}
-// Sentinel dataflow (forward, sync mode 3): H is pre-filled with the bit pattern 0xFFFFFFFF (a NaN no arithmetic
-// produces); a row needs no flag and no fence -- every 16-byte piece a consumer lane loads validates itself, and a
-// piece that still holds a sentinel word (not yet written, or torn) is simply loaded again.
-__device__ __forceinline__ float4 ld_poll4(const float* p) {       // re-load that the compiler may neither hoist nor fold
-  float4 r;
-  asm volatile("ld.relaxed.gpu.global.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p) : "memory");
-  return r;
-}
-__device__ __forceinline__ bool f4_pending(float4 v) {
-  return __float_as_uint(v.x) == 0xFFFFFFFFu || __float_as_uint(v.y) == 0xFFFFFFFFu ||
-         __float_as_uint(v.z) == 0xFFFFFFFFu || __float_as_uint(v.w) == 0xFFFFFFFFu;
-}
-__device__ __forceinline__ void set_flag(unsigned int* p) {
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(1u) : "memory");
-}
-
-// programmatic dependent launch (per-level launches of the same kernels, tm_gnn_set_impl bit 3)
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
@@ -518,44 +482,15 @@ struct FwdArgs {
   const float* S; float* H;
   const uint8_t* planes; const float* b1; const float* b2;                // packed fc_cell_neigh weights (gnn_pack_planes_kernel)
   float* A; float* LSE; float* HIDb;
-  unsigned int* ready;             // [n] by pin id: H[v] is final
+  unsigned int* bar;               // grid-barrier counter (zeroed by gnn_persist_begin)
   long long* prof;
-  int lb, le, prefetch;
-  // net-level fusion ("push"): when every net-level pin has exactly ONE driver, its row
-  //   h[s] = relu(S[s] + h[driver])                         (model.py:103-108 with a mean over one edge)
-  // is written by whoever produces h[driver] -- level 0 for primary inputs, the cell tile's epilogue for cell
-  // outputs -- over the driver's net out-edge list.  Odd levels then need no pass and no barrier: 51 barriers
-  // instead of 101 for config 2.
-  const int* bn_ptr; const int* bn_dst;
-  int fuse;
-  int pdl;                         // one launch per cell level: wait for the previous grid (griddepcontrol) instead of a grid barrier
-  int sentinel;                    // FLOW kernels: validate the gathered data itself instead of per-pin flags
+  int lb, le;
 };
-
-// rows of the sinks driven by one pin; lane layout of the caller: `cols` = this lane's float4 columns (NV of them)
-template <int NV>
-__device__ __forceinline__ void push_sinks(const FwdArgs& a, int pos, const float4 (&h)[NV], int col0, int colstride) {
-  const int e0 = __ldg(a.bn_ptr + pos), e1 = __ldg(a.bn_ptr + pos + 1);
-  for (int i = e0; i < e1; i += 2) {
-    const int s0 = __ldg(a.bn_dst + i), s1 = (i + 1 < e1) ? __ldg(a.bn_dst + i + 1) : -1;
-    float4 v0[NV], v1[NV];
-#pragma unroll
-    for (int j = 0; j < NV; ++j) {
-      v0[j] = ldg4(a.S + (int64_t)s0 * D + col0 + j * colstride);
-      if (s1 >= 0) v1[j] = ldg4(a.S + (int64_t)s1 * D + col0 + j * colstride);
-    }
-#pragma unroll
-    for (int j = 0; j < NV; ++j) {
-      *reinterpret_cast<float4*>(a.H + (int64_t)s0 * D + col0 + j * colstride) = f4relu(f4add(v0[j], h[j]));
-      if (s1 >= 0) *reinterpret_cast<float4*>(a.H + (int64_t)s1 * D + col0 + j * colstride) = f4relu(f4add(v1[j], h[j]));
-    }
-  }
-}
 
 // issue the loads the prefetch of level l1 depends on (pass k); consumed by pf_end_fwd
 __device__ __forceinline__ PfState pf_begin_fwd(const FwdArgs& a, int l1, int k) {
   PfState st{};
-  if (!a.prefetch || l1 >= a.le) return st;
+  if (l1 >= a.le) return st;
   const int p0 = __ldg(a.level_ptr + l1), cnt = __ldg(a.level_ptr + l1 + 1) - p0;
   int q0, qn;
   cta_range(l1, cnt, k, q0, qn);
@@ -565,7 +500,7 @@ __device__ __forceinline__ PfState pf_begin_fwd(const FwdArgs& a, int l1, int k)
     st.e1 = __ldg(a.f_ptr + p0 + q0 + qn);
     st.qn = qn;
   }
-  const int l2 = a.fuse ? l1 + 2 : l1 + 1;
+  const int l2 = l1 + 1;
   if (k == 0 && l2 < a.le) {                   // pointer lines of the level after
     const int p2 = __ldg(a.level_ptr + l2), cnt2 = __ldg(a.level_ptr + l2 + 1) - p2;
     int r0, rn;
@@ -586,12 +521,11 @@ __device__ __forceinline__ void pf_end_fwd(const FwdArgs& a, const PfState& st) 
 
 // level 0 and odd levels: h[v] = relu(S[v] + mean_{u->v in net} h[u])  (model.py:103-108,148-153,186-187)
 // NV float4 per lane, 32/NV lanes per pin.
-template <int NV, bool FLOW>
+template <int NV>
 __device__ __forceinline__ void fwd_net_level(const FwdArgs& a, int p0, int cnt, Ctx& c, const GridBar& gb) {
   constexpr int G = 32 / NV, UN = (NV == 4) ? 2 : 4;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int lg = lane % G, grp = lane / G;
-  const unsigned int gmask = (G == 32) ? 0xffffffffu : (((1u << G) - 1u) << (grp * G));
   const int ngroups = gridDim.x * WARPS * NV;
   int p = (blockIdx.x * WARPS + warp) * NV + grp;
   int s = 0, e = 0, v = 0, idx[UN];
@@ -606,7 +540,7 @@ __device__ __forceinline__ void fwd_net_level(const FwdArgs& a, int p0, int cnt,
     for (int j = 0; j < NV; ++j) sv[j] = ldg4(a.S + (int64_t)v * D + (j * G + lg) * 4);
   };
   if (p < cnt) fetch();
-  if (!FLOW) gb.wait();
+  gb.wait();
   c.stamp(PH_NPRE);
   while (p < cnt) {
     float4 acc[NV];
@@ -617,61 +551,34 @@ __device__ __forceinline__ void fwd_net_level(const FwdArgs& a, int p0, int cnt,
 #pragma unroll
         for (int q = 0; q < UN; ++q) idx[q] = (i + q < e) ? __ldg(a.f_src + i + q) : 0;
       }
-#pragma unroll
-      for (int q = 0; q < UN; ++q)
-        if (FLOW && !a.sentinel && i + q < e) wait_flag(a.ready + idx[q]);
       float4 m[UN][NV];
 #pragma unroll
       for (int q = 0; q < UN; ++q)
 #pragma unroll
         for (int j = 0; j < NV; ++j)
           m[q][j] = (i + q < e) ? ldcg4(a.H + (int64_t)idx[q] * D + (j * G + lg) * 4) : f4zero();
-      if (FLOW && a.sentinel) {
-        for (uint32_t spin = 0;; ++spin) {
-          bool pending = false;
-#pragma unroll
-          for (int q = 0; q < UN; ++q)
-#pragma unroll
-            for (int j = 0; j < NV; ++j)
-              if (i + q < e && f4_pending(m[q][j])) {
-                m[q][j] = ld_poll4(a.H + (int64_t)idx[q] * D + (j * G + lg) * 4);
-                pending = true;
-              }
-          if (!pending) break;
-          if (spin > (1u << 22)) __trap();
-        }
-      }
 #pragma unroll
       for (int q = 0; q < UN; ++q)
 #pragma unroll
         for (int j = 0; j < NV; ++j) acc[j] = f4add(acc[j], m[q][j]);
     }
     const float rdeg = (e > s) ? 1.f / (float)(e - s) : 0.f;
-    float4 hv[NV];
 #pragma unroll
-    for (int j = 0; j < NV; ++j) {
-      hv[j] = f4relu(f4fma(acc[j], rdeg, sv[j]));
-      *reinterpret_cast<float4*>(a.H + (int64_t)v * D + (j * G + lg) * 4) = hv[j];
-    }
-    if (!FLOW && a.fuse) push_sinks<NV>(a, p0 + p, hv, lg * 4, G * 4);
-    if (FLOW && !a.sentinel) {
-      __syncwarp(gmask);
-      if (lg == 0) set_flag(a.ready + v);
-    }
+    for (int j = 0; j < NV; ++j)
+      *reinterpret_cast<float4*>(a.H + (int64_t)v * D + (j * G + lg) * 4) = f4relu(f4fma(acc[j], rdeg, sv[j]));
     p += ngroups;
     if (p < cnt) fetch();
   }
   c.stamp(PH_NBODY);
 }
 
-template <bool FLOW>
 __global__ void __launch_bounds__(THREADS, 1) gnn_persist_fwd_kernel(const FwdArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   Ctx c;
   ctx_setup(c, smem, a.planes, a.prof);
   const int cluster_id = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
-  GridBar gb{a.ready, gridDim.x, 0u};                      // barrier mode: the first flag word is the counter
+  GridBar gb{a.bar, gridDim.x, 0u};
   const bool save = a.A != nullptr;
   const int qd = warp & 3;
   const float b1m = __ldg(a.b1 + c.rank * 128 + qd * 32 + lane), b2m = __ldg(a.b2 + qd * 32 + lane);
@@ -679,27 +586,24 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_fwd_kernel(const FwdAr
   for (int l = a.lb; l < a.le; ++l) {
     const int p0 = __ldg(a.level_ptr + l), cnt = __ldg(a.level_ptr + l + 1) - p0;
     if (cnt <= 0) continue;
-    const bool fused = !FLOW && a.fuse;
-    if (fused && (l & 1)) continue;                          // written by their drivers' producers
     {
-      const int ln = fused ? (l == 0 ? 2 : l + 2) : l + 1;    // the next level this kernel processes
-      const PfState pf0 = pf_begin_fwd(a, ln, 0), pf1 = pf_begin_fwd(a, ln, 1);
+      const PfState pf0 = pf_begin_fwd(a, l + 1, 0), pf1 = pf_begin_fwd(a, l + 1, 1);
       pf_end_fwd(a, pf0);
       pf_end_fwd(a, pf1);
     }
     if (l == 0 || (l & 1)) {
       const int nw = gridDim.x * WARPS;
-      if (cnt <= nw) fwd_net_level<1, FLOW>(a, p0, cnt, c, gb);
-      else if (cnt <= 2 * nw) fwd_net_level<2, FLOW>(a, p0, cnt, c, gb);
-      else fwd_net_level<4, FLOW>(a, p0, cnt, c, gb);
-      if (!FLOW) gb.arrive();
+      if (cnt <= nw) fwd_net_level<1>(a, p0, cnt, c, gb);
+      else if (cnt <= 2 * nw) fwd_net_level<2>(a, p0, cnt, c, gb);
+      else fwd_net_level<4>(a, p0, cnt, c, gb);
+      gb.arrive();
       continue;
     }
     // even level > 0:  a = sum_e m_e softmax_e(m)_e per channel (model.py:113-116);
     //                  h = relu(S + W2 relu(W1 a + b1) + b2)     (model.py:138-146)
     const int crow0 = __ldg(a.cell_base + l);
     const int N = tile_width(cnt, nclusters), ntiles = (cnt + N - 1) / N;
-    const int PPW = N >> 4, half = N >> 1;
+    const int PPW = N >> 4;
     bool waited = false;
     for (int tile = cluster_id; tile < ntiles; tile += nclusters) {
       const int t0 = tile * N;
@@ -714,12 +618,8 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_fwd_kernel(const FwdAr
       }
       const int E0 = __shfl_sync(0xffffffffu, ptrs, 0), E1 = __shfl_sync(0xffffffffu, ptrs, max(npin, 0));
       int idx = (E0 + (lane & 7) < E1) ? __ldg(a.f_src + E0 + (lane & 7)) : 0;
-      if (!FLOW && !waited) {
-        if (a.pdl) pdl_wait();                               // per-level launch: the previous level's grid has completed
-        gb.wait();                                           // (ends with a CTA barrier; no-op for a launch's first level)
-        if (a.pdl) __syncthreads();
-      }
-      else __syncthreads();                                  // the previous tile's epilogue / publication still reads pin_s
+      if (!waited) gb.wait();                                // ends with a CTA barrier
+      else __syncthreads();                                  // the previous tile's epilogue still reads pin_s
       waited = true;
       c.stamp(PH_CPRE);
 
@@ -747,30 +647,11 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_fwd_kernel(const FwdAr
         int bnd = __shfl_sync(0xffffffffu, ptrs, 1);
         for (int i = E0; i < E1; i += 8) {
           if (i > E0) idx = (i + (lane & 7) < E1) ? __ldg(a.f_src + i + (lane & 7)) : 0;
-          if (FLOW && !a.sentinel) {
-            if (i + (lane & 7) < E1) wait_flag(a.ready + idx);     // every source row of the batch is final
-            __syncwarp();
-          }
           float4 m[8];
-          int srcs[8];
 #pragma unroll
           for (int u = 0; u < 8; ++u) {
-            srcs[u] = __shfl_sync(0xffffffffu, idx, u);
-            m[u] = (i + u < E1) ? ldcg4(a.H + (int64_t)srcs[u] * D + lane * 4) : f4zero();
-          }
-          if (FLOW && a.sentinel) {
-            for (uint32_t spin = 0;; ++spin) {
-              bool pending = false;
-#pragma unroll
-              for (int u = 0; u < 8; ++u)
-                if (i + u < E1 && f4_pending(m[u])) {
-                  m[u] = ld_poll4(a.H + (int64_t)srcs[u] * D + lane * 4);
-                  pending = true;
-                }
-              if (!pending) break;
-              if (spin > (1u << 22)) __trap();
-            }
-            __syncwarp();
+            const int src = __shfl_sync(0xffffffffu, idx, u);
+            m[u] = (i + u < E1) ? ldcg4(a.H + (int64_t)src * D + lane * 4) : f4zero();
           }
 #pragma unroll
           for (int u = 0; u < 8; ++u) {
@@ -817,43 +698,15 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_fwd_kernel(const FwdAr
         }
       };
       mlp_tile(c, N, [] {}, epi1, pre2);
-      if (a.pdl) pdl_launch_dependents();                    // the next level's launch may start its prologue (weights, TMEM)
       auto fin = [&](int n, int m, int slot, float val) {
         const int v = c.pin_s[n];
-        if (v >= 0) {
-          const float h = fmaxf(val + b2m + sreg[slot], 0.f);
-          a.H[(int64_t)v * D + m] = h;
-          if (fused) {                                       // the sinks this pin drives (warp-uniform edge range)
-            const int pos = p0 + t0 + n;
-            const int e0 = __ldg(a.bn_ptr + pos), e1 = __ldg(a.bn_ptr + pos + 1);
-            for (int i = e0; i < e1; i += 4) {
-              int sk[4];
-              float sv[4];
-#pragma unroll
-              for (int u = 0; u < 4; ++u) sk[u] = (i + u < e1) ? __ldg(a.bn_dst + i + u) : -1;
-#pragma unroll
-              for (int u = 0; u < 4; ++u) sv[u] = sk[u] >= 0 ? __ldg(a.S + (int64_t)sk[u] * D + m) : 0.f;
-#pragma unroll
-              for (int u = 0; u < 4; ++u)
-                if (sk[u] >= 0) a.H[(int64_t)sk[u] * D + m] = fmaxf(sv[u] + h, 0.f);
-            }
-          }
-        }
+        if (v >= 0) a.H[(int64_t)v * D + m] = fmaxf(val + b2m + sreg[slot], 0.f);
       };
       exchange_tile(c, N, fin);
-      if (FLOW && !a.sentinel) {
-        __syncthreads();                                     // every warp's H stores precede the publication
-        if (tid < half) {
-          const int v = c.pin_s[(int)c.rank * half + tid];
-          if (v >= 0) set_flag(a.ready + v);
-        }
-      }
       c.stamp(PH_CPUB);
     }
-    if (!FLOW) {
-      if (!waited) gb.wait();
-      gb.arrive();
-    }
+    if (!waited) gb.wait();
+    gb.arrive();
   }
   ctx_teardown(c);
 }
@@ -871,17 +724,14 @@ struct BwdArgs {
   const uint8_t* planes;                                 // packed W2 [128][256], W1 [256][128] (gnn_pack_planes_kernel)
   const float* A; const float* LSE; const float* HIDb;
   float* GA; float* GHID; float* GZC;
-  unsigned int* ready_n;           // [n] by pin id: G[v] = g_z[v] is final (net-level pins, level 0)
-  unsigned int* ready_c;           // [n_cell_rows] by compact row: GA[row] is final
+  unsigned int* bar;               // grid-barrier counter (zeroed by gnn_persist_begin)
   long long* prof;
-  int num_levels, prefetch;
   int lb, le;                      // levels [lb, le) are processed (downwards)
-  int pdl;
 };
 
 __device__ __forceinline__ PfState pf_begin_bwd(const BwdArgs& a, int l1, int k) {
   PfState st{};
-  if (!a.prefetch || l1 < 0) return st;
+  if (l1 < 0) return st;
   const int p0 = __ldg(a.level_ptr + l1), cnt = __ldg(a.level_ptr + l1 + 1) - p0;
   int q0, qn;
   cta_range(l1, cnt, k, q0, qn);
@@ -927,12 +777,11 @@ __device__ __forceinline__ float hsel(const float (&h)[NMAX / 4], int k) {
   return r;
 }
 
-template <int NV, bool FLOW>
+template <int NV>
 __device__ __forceinline__ void bwd_net_level(const BwdArgs& a, int p0, int cnt, Ctx& c, const GridBar& gb) {
   constexpr int G = 32 / NV, UN = (NV == 4) ? 2 : 4;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int lg = lane % G, grp = lane / G;
-  const unsigned int gmask = (G == 32) ? 0xffffffffu : (((1u << G) - 1u) << (grp * G));
   const int ngroups = gridDim.x * WARPS * NV;
   int p = (blockIdx.x * WARPS + warp) * NV + grp;
   int ns = 0, ne = 0, cs = 0, ce = 0, v = 0, ndst[UN], crow[2];
@@ -956,7 +805,7 @@ __device__ __forceinline__ void bwd_net_level(const BwdArgs& a, int p0, int cnt,
     }
   };
   if (p < cnt) fetch();
-  if (!FLOW) gb.wait();
+  gb.wait();
   c.stamp(PH_NPRE);
   while (p < cnt) {
     for (int i = ns; i < ne; i += UN) {
@@ -967,9 +816,6 @@ __device__ __forceinline__ void bwd_net_level(const BwdArgs& a, int p0, int cnt,
           nw[q] = (i + q < ne) ? __ldg(a.bn_w + i + q) : 0.f;
         }
       }
-#pragma unroll
-      for (int q = 0; q < UN; ++q)
-        if (FLOW && i + q < ne) wait_flag(a.ready_n + ndst[q]);
       float4 m[UN][NV];
 #pragma unroll
       for (int q = 0; q < UN; ++q)
@@ -991,12 +837,11 @@ __device__ __forceinline__ void bwd_net_level(const BwdArgs& a, int p0, int cnt,
         if (i + q < ce) {
           float4 ls[NV], aa[NV];
 #pragma unroll
-          for (int j = 0; j < NV; ++j) {                           // static rows first, then the flag
+          for (int j = 0; j < NV; ++j) {
             const int64_t co = (int64_t)crow[q] * D + (j * G + lg) * 4;
             ls[j] = ldg4(a.LSE + co);
             aa[j] = ldg4(a.A + co);
           }
-          if (FLOW) wait_flag(a.ready_c + crow[q]);
 #pragma unroll
           for (int j = 0; j < NV; ++j)
             g[j] = f4add(g[j], cell_edge_grad(hv[j], ldcg4(a.GA + (int64_t)crow[q] * D + (j * G + lg) * 4), ls[j], aa[j]));
@@ -1006,17 +851,12 @@ __device__ __forceinline__ void bwd_net_level(const BwdArgs& a, int p0, int cnt,
 #pragma unroll
     for (int j = 0; j < NV; ++j)
       *reinterpret_cast<float4*>(a.G + (int64_t)v * D + (j * G + lg) * 4) = relu_mask(hv[j], g[j]);
-    if (FLOW) {
-      __syncwarp(gmask);
-      if (lg == 0) set_flag(a.ready_n + v);
-    }
     p += ngroups;
     if (p < cnt) fetch();
   }
   c.stamp(PH_NBODY);
 }
 
-template <bool FLOW>
 __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1024,7 +864,7 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
   ctx_setup(c, smem, a.planes, a.prof);
   const int cluster_id = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
   float* scratch = reinterpret_cast<float*>(smem + OFF_B);      // [N][128] fp32 gradient accumulators during the gather
-  GridBar gb{a.ready_n, gridDim.x, 0u};                    // barrier mode: the first flag word is the counter
+  GridBar gb{a.bar, gridDim.x, 0u};
 
   for (int l = a.le - 1; l >= a.lb; --l) {
     const int p0 = __ldg(a.level_ptr + l), cnt = __ldg(a.level_ptr + l + 1) - p0;
@@ -1036,15 +876,15 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
     }
     if (l == 0 || (l & 1)) {
       const int nw = gridDim.x * WARPS;
-      if (cnt <= nw) bwd_net_level<1, FLOW>(a, p0, cnt, c, gb);
-      else if (cnt <= 2 * nw) bwd_net_level<2, FLOW>(a, p0, cnt, c, gb);
-      else bwd_net_level<4, FLOW>(a, p0, cnt, c, gb);
-      if (!FLOW) gb.arrive();
+      if (cnt <= nw) bwd_net_level<1>(a, p0, cnt, c, gb);
+      else if (cnt <= 2 * nw) bwd_net_level<2>(a, p0, cnt, c, gb);
+      else bwd_net_level<4>(a, p0, cnt, c, gb);
+      gb.arrive();
       continue;
     }
     const int crow0 = __ldg(a.cell_base + l);
     const int N = tile_width(cnt, nclusters), ntiles = (cnt + N - 1) / N;
-    const int PPW = N >> 4, half = N >> 1;
+    const int PPW = N >> 4;
     bool waited = false;
     for (int tile = cluster_id; tile < ntiles; tile += nclusters) {
       const int t0 = tile * N;
@@ -1061,11 +901,7 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
       int idx = 0;
       float wt = 0.f;
       if (E0 + (lane & 7) < E1) { idx = __ldg(a.bn_dst + E0 + (lane & 7)); wt = __ldg(a.bn_w + E0 + (lane & 7)); }
-      if (!FLOW && !waited) {
-        if (a.pdl) pdl_wait();                               // per-level launch: the previous level's grid has completed
-        gb.wait();                                           // (ends with a CTA barrier; no-op for a launch's first level)
-        if (a.pdl) __syncthreads();
-      }
+      if (!waited) gb.wait();                                // ends with a CTA barrier
       else __syncthreads();                                  // the previous tile's epilogue still reads the scales
       waited = true;
       c.stamp(PH_CPRE);
@@ -1095,10 +931,6 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
               idx = ok ? __ldg(a.bn_dst + i + (lane & 7)) : 0;
               wt = ok ? __ldg(a.bn_w + i + (lane & 7)) : 0.f;
             }
-            if (FLOW) {
-              if (i + (lane & 7) < E1) wait_flag(a.ready_n + idx);
-              __syncwarp();
-            }
             float4 m[8];
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
@@ -1124,7 +956,6 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
             const int row = __ldg(a.bc_row + i);
             const int64_t co = (int64_t)row * D + lane * 4;
             const float4 hv = ldg4(a.H + (int64_t)__shfl_sync(0xffffffffu, vv, q) * D + lane * 4);
-            if (FLOW) wait_flag(a.ready_c + row);
             float4* dst = reinterpret_cast<float4*>(scratch + (r0 + q) * D + lane * 4);
             *dst = f4add(*dst, cell_edge_grad(hv, ldcg4(a.GA + co), ldg4(a.LSE + co), ldg4(a.A + co)));
           }
@@ -1171,7 +1002,6 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
         }
       };
       mlp_tile(c, N, pre1, epi1, [] {});
-      if (a.pdl) pdl_launch_dependents();
       auto fin = [&](int n, int m, int, float val) {
         if (t0 + n < cnt) a.GA[(int64_t)(crow0 + t0 + n) * D + m] = val;
       };
@@ -1184,166 +1014,79 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
             *reinterpret_cast<float4*>(a.G + (int64_t)__shfl_sync(0xffffffffu, vv, r) * D + lane * 4) =
                 *reinterpret_cast<const float4*>(a.GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4);
       }
-      if (FLOW) {
-        __syncthreads();                                     // every warp's GA stores precede the publication
-        if (tid < half && t0 + (int)c.rank * half + tid < cnt) set_flag(a.ready_c + crow0 + t0 + (int)c.rank * half + tid);
-      }
       c.stamp(PH_CPUB);
     }
-    if (!FLOW) {
-      if (!waited) gb.wait();
-      gb.arrive();
-    }
+    if (!waited) gb.wait();
+    gb.arrive();
   }
   ctx_teardown(c);
-}
-
-// sentinel mode: rows of pins that are not scheduled (or beyond the processed levels) go back to zero
-__global__ void gnn_clear_pending_kernel(int64_t n, const int* __restrict__ level, int le, float* __restrict__ H) {
-  const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (w >= n) return;
-  const int l = level[w];
-  if (l < 0 || l >= le) *reinterpret_cast<float4*>(H + w * D + lane * 4) = make_float4(0.f, 0.f, 0.f, 0.f);
-}
-
-// pins of levels < lb were produced by an earlier call: mark them ready
-__global__ void gnn_mark_ready_kernel(const int* __restrict__ order, int count, unsigned int* __restrict__ ready) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < count) ready[order[i]] = 1u;
 }
 
 // ---------------------------------------------------------------------------------------------
 // host
 // ---------------------------------------------------------------------------------------------
 template <class Args>
-int launch_persist(void (*kern)(const Args), const Args& args, cudaStream_t st, const char* what, int want_clusters = 0, bool pdl = false) {
+int launch_persist(void (*kern)(const Args), const Args& args, cudaStream_t st, const char* what) {
   TM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
-  static const int coop = getenv("TM_GNN_COOP") ? atoi(getenv("TM_GNN_COOP")) : 0;
-  static const int max_ctas = getenv("TM_GNN_CTAS") ? atoi(getenv("TM_GNN_CTAS")) : 0;
   cudaLaunchConfig_t cfg = {};
   cfg.blockDim = dim3(THREADS);
   cfg.dynamicSmemBytes = SMEM_BYTES;
   cfg.stream = st;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeCooperative;
-  attr[1].val.cooperative = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  // every CTA must be resident at once (consumers spin on flags their producers set): size the grid by
-  // what the device can hold, one CTA per SM
+  // every CTA must be resident at once (the grid barrier waits for all of them): size the grid by what the
+  // device can hold, one CTA per SM
   cfg.gridDim = dim3((unsigned)(sm_count() & ~1));
   int ncl = 0;
   TM_CUDA(cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg));
   TM_REQUIRE(ncl >= 1, "%s: no 2-CTA cluster with %u bytes of shared memory fits this device", what, SMEM_BYTES);
-  int nblk = 2 * std::min(ncl, sm_count() / 2);
-  if (max_ctas >= 2) nblk = std::min(nblk, max_ctas & ~1);
-  if (want_clusters > 0) nblk = std::min(nblk, 2 * want_clusters);
-  cfg.gridDim = dim3((unsigned)nblk);
-  cfg.numAttrs = coop ? 2 : 1;
-  if (pdl) {                                   // one launch per level, chained by programmatic dependent launch
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-  }
+  cfg.gridDim = dim3((unsigned)(2 * std::min(ncl, sm_count() / 2)));
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   if (e != cudaSuccess) return fail((int)e, "%s: %s", what, cudaGetErrorString(e));
   return 0;
 }
-int prefetch_on() {
-  static const int v = getenv("TM_GNN_PREFETCH") ? atoi(getenv("TM_GNN_PREFETCH")) : 1;
-  return v;
-}
-std::atomic<int> g_flow{-1};      // 0 = grid barrier per level, 1 = per-pin ready flags, 2 = grid barrier + net-level push fusion
-int sync_mode() {
-  int v = g_flow.load(std::memory_order_relaxed);
-  if (v < 0) {
-    v = (getenv("TM_GNN_SYNC") && getenv("TM_GNN_SYNC")[0] == 'f') ? 1 : ((getenv("TM_GNN_FUSE") && atoi(getenv("TM_GNN_FUSE"))) ? 2 : 0);
-    g_flow.store(v, std::memory_order_relaxed);
-  }
-  return v;
-}
-bool flow_sync() { return sync_mode() == 1 || sync_mode() == 3; }
-bool sentinel_sync() { return sync_mode() == 3; }
+
+// workspace: the packed weight planes of both CTA ranks (256-byte aligned), then the grid-barrier counter on a
+// 256-byte slot of its own
+constexpr size_t WS_PLANES = 2 * 4 * W_PLANE, WS_BAR = 256;
+uint8_t* ws_planes(void* ws) { return reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255); }
+unsigned int* ws_bar(void* ws) { return reinterpret_cast<unsigned int*>(ws_planes(ws) + WS_PLANES); }
 }  // namespace
 
 namespace tmk {
-size_t gnn_persist_ws_bytes() { return 512 + 2 * 4 * W_PLANE; }
+size_t gnn_persist_ws_bytes() { return 256 + WS_PLANES + WS_BAR; }
 static long long* g_prof = nullptr;
 void gnn_persist_set_profile(long long* p) { g_prof = p; }
 int gnn_persist_profile_slots() { return PH_COUNT; }
-int gnn_persist_set_flow(int flow) {
-  const int prev = sync_mode();
-  if (flow >= 0) g_flow.store(flow > 3 ? 0 : flow, std::memory_order_relaxed);
-  return prev;
-}
 
-// pack the fc_cell_neigh planes and clear the synchronisation words: once per pass
-int gnn_persist_begin(const tm_schedule* s, const float* Wa, const float* Wb, void* ws, bool flags_all, size_t nflags, cudaStream_t st) {
-  TM_REQUIRE(s->level_ptr && s->cell_base && s->sync_flags,
-             "tm_gnn: schedule lacks the device level_ptr / cell_base / sync_flags arrays");
-  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-  TM_CUDA(cudaMemsetAsync(s->sync_flags, 0, flags_all ? sizeof(unsigned int) * nflags : 256, st));
-  gnn_pack_planes_kernel<<<2 * 2 * 128 * 128 / 256, 256, 0, st>>>(Wa, Wb, planes);
+// pack the fc_cell_neigh planes and clear the barrier counter: once per pass
+int gnn_persist_begin(const tm_schedule* s, const float* Wa, const float* Wb, void* ws, cudaStream_t st) {
+  TM_REQUIRE(s->level_ptr && s->cell_base, "tm_gnn: schedule lacks the device level_ptr / cell_base arrays");
+  TM_CUDA(cudaMemsetAsync(ws_bar(ws), 0, WS_BAR, st));
+  gnn_pack_planes_kernel<<<2 * 2 * 128 * 128 / 256, 256, 0, st>>>(Wa, Wb, ws_planes(ws));
   return check_launch("gnn_pack_planes");
 }
 
 int gnn_persist_forward(const tm_schedule* s, int lb, int le, float* H, const float* S, const float* W1t, const float* b1,
-                        const float* W2t, const float* b2, float* A, float* LSE, float* HIDb, void* ws, cudaStream_t st,
-                        bool begin, bool per_level) {
-  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-  unsigned int* ready = reinterpret_cast<unsigned int*>(s->sync_flags);
-  if (begin) TM_TRY(gnn_persist_begin(s, W1t, W2t, ws, flow_sync() && !per_level, (size_t)s->n, st));
-  if (!per_level && flow_sync() && lb > 0) {
-    const int count = s->h_level_ptr[lb];
-    if (count > 0) {
-      gnn_mark_ready_kernel<<<(count + 255) / 256, 256, 0, st>>>(s->order, count, ready);
-      TM_TRY(check_launch("gnn_mark_ready"));
-    }
-  }
-  const int fuse_env = sync_mode() == 2;
-  // push fusion needs every net-level pin single-driven from an even level (tm_schedule.single_driver), the whole
-  // pass in one call and the barrier ordering
-  const int fuse = (!per_level && fuse_env && s->single_driver && lb == 0 && le == s->num_levels && !flow_sync() && s->bn_ptr && s->bn_dst) ? 1 : 0;
-  FwdArgs a{s->level_ptr, s->cell_base, s->order, s->f_ptr, s->f_src, S, H, planes, b1, b2, A, LSE, HIDb, ready, g_prof,
-            lb, le, per_level ? 0 : prefetch_on(), s->bn_ptr, s->bn_dst, fuse, per_level ? 1 : 0,
-            (!per_level && sentinel_sync() && lb == 0) ? 1 : 0};
-  if (a.sentinel) {
-    // every row the kernel will read starts as "pending"; rows of pins outside the schedule are zeroed afterwards
-    TM_CUDA(cudaMemsetAsync(H, 0xFF, sizeof(float) * (size_t)s->n * D, st));
-  }
-  if (per_level) {                             // ONE cell level: a cluster per 32-pin tile (more pins per tile past 74 clusters)
-    const int cnt = s->h_level_ptr[lb + 1] - s->h_level_ptr[lb];
-    return launch_persist(gnn_persist_fwd_kernel<false>, a, st, "gnn_cell_level_fwd", (cnt + 31) / 32, true);
-  }
-  TM_TRY(flow_sync() ? launch_persist(gnn_persist_fwd_kernel<true>, a, st, "gnn_persist_fwd<flow>")
-                     : launch_persist(gnn_persist_fwd_kernel<false>, a, st, "gnn_persist_fwd"));
-  if (a.sentinel && (s->h_level_ptr[s->num_levels] < s->n || le < s->num_levels)) {
-    gnn_clear_pending_kernel<<<(unsigned)cdiv((int64_t)s->n * 32, 256), 256, 0, st>>>(s->n, s->level, le, H);
-    TM_TRY(check_launch("gnn_clear_pending"));
-  }
-  return 0;
+                        const float* W2t, const float* b2, float* A, float* LSE, float* HIDb, void* ws, cudaStream_t st) {
+  TM_TRY(gnn_persist_begin(s, W1t, W2t, ws, st));
+  FwdArgs a{s->level_ptr, s->cell_base, s->order, s->f_ptr, s->f_src, S, H, ws_planes(ws), b1, b2, A, LSE, HIDb,
+            ws_bar(ws), g_prof, lb, le};
+  return launch_persist(gnn_persist_fwd_kernel, a, st, "gnn_persist_fwd");
 }
 
 int gnn_persist_backward(const tm_schedule* s, const float* H, float* G, const float* W1, const float* W2, const float* A,
                          const float* LSE, const float* HIDb, float* GA, float* GHID, float* GZC, void* ws, cudaStream_t st,
-                         int lb, int le, bool begin, bool per_level) {
-  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-  unsigned int* ready = reinterpret_cast<unsigned int*>(s->sync_flags);
-  if (begin) TM_TRY(gnn_persist_begin(s, W2, W1, ws, flow_sync() && !per_level, (size_t)s->n + (size_t)s->n_cell_rows, st));
-  BwdArgs a{s->level_ptr, s->cell_base, s->order, s->bn_ptr, s->bn_dst, s->bn_w, s->bc_ptr, s->bc_row, H, G, planes,
-            A, LSE, HIDb, GA, GHID, GZC, ready, ready + s->n, g_prof, s->num_levels, per_level ? 0 : prefetch_on(), lb, le,
-            per_level ? 1 : 0};
-  if (per_level) {
-    const int cnt = s->h_level_ptr[lb + 1] - s->h_level_ptr[lb];
-    return launch_persist(gnn_persist_bwd_kernel<false>, a, st, "gnn_cell_level_bwd", (cnt + 31) / 32, true);
-  }
-  return flow_sync() ? launch_persist(gnn_persist_bwd_kernel<true>, a, st, "gnn_persist_bwd<flow>")
-                     : launch_persist(gnn_persist_bwd_kernel<false>, a, st, "gnn_persist_bwd");
+                         int lb, int le) {
+  TM_TRY(gnn_persist_begin(s, W2, W1, ws, st));
+  BwdArgs a{s->level_ptr, s->cell_base, s->order, s->bn_ptr, s->bn_dst, s->bn_w, s->bc_ptr, s->bc_row, H, G, ws_planes(ws),
+            A, LSE, HIDb, GA, GHID, GZC, ws_bar(ws), g_prof, lb, le};
+  return launch_persist(gnn_persist_bwd_kernel, a, st, "gnn_persist_bwd");
 }
 }  // namespace tmk

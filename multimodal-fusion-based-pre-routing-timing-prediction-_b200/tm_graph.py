@@ -224,18 +224,6 @@ class Schedule:
             net_optr=s.net_optr.data_ptr(), net_odst=s.net_odst.data_ptr(),
             cell_optr=s.cell_optr.data_ptr(), cell_odst=s.cell_odst.data_ptr(),
             level_ptr=s.level_ptr.data_ptr(), cell_base=s.cell_base.data_ptr())
-        s.sync_flags = torch.zeros(n + s.n_cell_rows + 64, dtype=torch.int32, device=dev)
-        s.struct.sync_flags = s.sync_flags.data_ptr()
-        # net-level "push" fusion precondition (one more host read per graph): every odd-level pin has exactly one
-        # net in-edge, coming from an even level
-        lvl = s.level.long()
-        odd = (lvl >= 0) & ((lvl & 1) == 1)
-        ndeg = (s.net_iptr[1:] - s.net_iptr[:-1]).long()
-        src_lv = lvl[s.net_isrc.long()] if int(s.net_isrc.numel()) else lvl[:0]
-        dst_of_edge = torch.repeat_interleave(torch.arange(n, device=dev), ndeg)
-        edge_ok = (~odd[dst_of_edge]) | ((src_lv >= 0) & ((src_lv & 1) == 0))
-        s.single_driver = bool(((ndeg[odd] == 1).all() & edge_ok.all()).item()) if n else False
-        s.struct.single_driver = 1 if s.single_driver else 0
         # level-ordered edge lists: what the propagation kernels actually walk
         e_net, e_cell = int(s.net_isrc.numel()), int(s.cell_isrc.numel())
         ns1 = s.n_sched + 1

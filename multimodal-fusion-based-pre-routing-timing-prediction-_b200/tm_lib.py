@@ -30,8 +30,7 @@ class tm_schedule(ctypes.Structure):
                 ("f_ptr", ctypes.c_void_p), ("f_src", ctypes.c_void_p),
                 ("bn_ptr", ctypes.c_void_p), ("bn_dst", ctypes.c_void_p), ("bn_w", ctypes.c_void_p),
                 ("bc_ptr", ctypes.c_void_p), ("bc_row", ctypes.c_void_p),
-                ("level_ptr", ctypes.c_void_p), ("cell_base", ctypes.c_void_p), ("sync_flags", ctypes.c_void_p),
-                ("single_driver", ctypes.c_int32), ("reserved0", ctypes.c_int32)]
+                ("level_ptr", ctypes.c_void_p), ("cell_base", ctypes.c_void_p)]
 
 
 def parse_header(path=HEADER_PATH):

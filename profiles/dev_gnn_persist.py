@@ -65,8 +65,6 @@ def compare(cfg, seed):
                grads=max(rel(a, b) for a, b in zip(gr1, gr0)))
     H1b, _, Gz1b, _ = run(sched, g, ps, G0, 3)
     out["deterministic"] = bool(torch.equal(H1, H1b) and torch.equal(Gz1, Gz1b))
-    H8, s8, Gz8, gr8 = run(sched, g, ps, G0, 8)      # per-level launches of the tcgen05 cluster tile kernel
-    out["impl8_equals_impl3"] = bool(torch.equal(H8, H1) and torch.equal(Gz8, Gz1) and all(torch.equal(a, b) for a, b in zip(gr8, gr1)))
     H16, s16, Gz16, gr16 = run(sched, g, ps, G0, 16)  # per-level kernels, fp16 two-term split cell MLP
     out["h16"] = dict(H=rel(H16, H0), A=rel(s16["A"], s0["A"]), HID=rel(s16["HID"], s0["HID"]), Gz=rel(Gz16, Gz0),
                       grads=max(rel(a, b) for a, b in zip(gr16, gr0)))
@@ -147,8 +145,6 @@ def time_cfg(name, g, n):
 
 if __name__ == "__main__":
     what = sys.argv[1:] or ["compare"]
-    if os.environ.get("TM_DEV_SYNC"):
-        tm_lib.lib().tm_gnn_set_sync(int(os.environ["TM_DEV_SYNC"]))
     if "compare" in what:
         for cfg, seed in (("tiny", 0), ("tiny", 5), ("c1", 1)):
             compare(cfg, seed)

@@ -42,7 +42,7 @@ def test_schedule_struct_layout_matches_header():
     body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
     names = re.findall(r"(\w+)\s*;", body)
     assert names == [f[0] for f in tm_lib.tm_schedule._fields_]
-    assert ctypes.sizeof(tm_lib.tm_schedule) == 8 + 4 + 4 + 22 * 8 + 8
+    assert ctypes.sizeof(tm_lib.tm_schedule) == 8 + 4 + 4 + 21 * 8
 
 
 def test_cuda_sources_target_sm100a_only():
