@@ -530,6 +530,30 @@ int tm_conv3x3_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t 
                           void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * A7 (bf16 mode)  TMA-fed tcgen05 k x k convolutions (odd k <= 9, stride 1, zero padding k/2)
+ * Replaces nn.Conv2d(32, 64, 7, 1, 3) and nn.Conv2d(64, 32, 9, 1, 4) of LayoutNet (src/model.py:227-243) and
+ * their autograd (data + weight gradients) when the image branch runs with bf16 tensor-core operands.  The kernels
+ * of A6 with k*k taps; operand rows are single pixels and the weights stream through the shared-memory ring.
+ * Activations compact bf16 [B][H][W][C] (tm_to_bf16_rows); H and W powers of two; Cin in {16, 32, 64},
+ * Cout in {16, 32, 64, 128}.
+ * ---------------------------------------------------------------------------------- */
+/* 1 when forward, data gradient and weight gradient all take the shape, else 0 */
+int tm_convkxk_bf16_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k);
+/* nn.Conv2d weight w [Cout][Cin][k][k] fp32 -> bf16 operand q [k*k][Nc][KcP] of tm_convkxk_bf16: dgrad = 0: forward
+ * (Nc = Cout, K = Cin padded to KcP); dgrad = 1: data gradient (Nc = Cin, K = Cout padded to KcP, taps reversed). */
+int tm_convkxk_pack_bf16(int64_t Cout, int64_t Cin, int64_t k, const float* w, void* q, int64_t KcP, int dgrad,
+                         void* stream);
+/* y[pix, 0:N] (fp32, row stride ldy) = act(bias + sum_{tap,c} xb[pix + tap, c] * q[tap][n][c]); bias optional,
+ * flags: TM_EPI_RELU.  The data gradient is the same call on bf16(dy) with the dgrad operand and no bias. */
+int tm_convkxk_bf16(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t k, const void* xb, const void* wq,
+                    const float* bias, float* y, int64_t ldy, int flags, int* err, void* stream);
+/* dw[co][ci][ky][kx] (torch layout) = sum_pix dyb[pix, co] * xb[pix + (ky-k/2, kx-k/2), ci]; deterministic.
+ * The bias gradient is tm_colsum of dy. */
+size_t tm_convkxk_bf16_wgrad_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k);
+int tm_convkxk_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k, const void* xb,
+                          const void* dyb, float* dw, void* ws, size_t ws_bytes, int* err, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * N4  fused Adam (torch.optim.Adam defaults, src/train.py:431-435,555)
  * ---------------------------------------------------------------------------------- */
 int tm_adam_step(int64_t n, float* p, const float* g, float* m, float* v, float lr, float beta1,

@@ -1,4 +1,5 @@
-// TMA-fed tcgen05 3x3 convolutions on bf16 NHWC activations (U-Net bf16 mode, Unet.py:8-22).
+// TMA-fed tcgen05 3x3 convolutions on bf16 NHWC activations (U-Net bf16 mode, Unet.py:8-22), and the same kernels
+// with k x k taps for LayoutNet's 7x7 / 9x9 layers (model.py:227-243; end of the file).
 //
 // The activation is a compact bf16 tensor [B][H][W][C] (C a multiple of 16).  A 4-D tensor map
 // (C, W, H, B) lets ONE cp.async.bulk.tensor per (tile, tap) fetch the 128 input pixels a tile of
@@ -195,8 +196,8 @@ struct ConvArgs {
   Geom g;                            // geometry in PACKED pixels (rows of P pixels)
   int Cin, N, stages;                // channels per packed row: Cin = P * cin, N = P * cout
   int P, cpx;                        // pixels per row, output channels per pixel
-  int ntaps, cscale, convt;          // taps (9 / 4 / 1), coordinate scale of the input map, transposed-conv scatter epilogue
-  signed char tdx[9], tdy[9];        // input offset of every tap
+  int ntaps, cscale, convt;          // taps (k*k / 4 / 1), coordinate scale of the input map, transposed-conv scatter epilogue
+  signed char tdx[81], tdy[81];      // input offset of every tap (up to 9x9)
   uint32_t a_bytes, b_bytes, stage_bytes;
   float* y;
   int64_t ldy;
@@ -554,7 +555,8 @@ conv3x3_tma_rows_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_co
 }
 
 // ------------------------------------------------------------------------------------------------
-// wgrad: grid (pixel splits, 3 kernel rows); CTA (z, r) accumulates taps (r, 0..2) over its pixel blocks
+// wgrad: grid (pixel splits, k kernel rows x tap groups); CTA (z, r, grp) accumulates taps (r, grp*tg ..) over its
+// pixel blocks
 // ------------------------------------------------------------------------------------------------
 struct WgradArgs {
   Geom g;
@@ -564,9 +566,12 @@ struct WgradArgs {
   float* part;                       // [splits][taps][Cout][Cin]
   int* err;
   int cscale;                        // coordinate scale of the tapped map (2: transposed-conv gradient, every other pixel)
-  signed char tdx[4], tdy[4];        // NT == 4: offsets of the four taps (transposed conv); NT == 3 / 1 use (u - 1, r - 1)
+  signed char tdx[4], tdy[4];        // NT == 4: offsets of the four taps (transposed conv); NT == 3 / 1 / 0 use (s - k/2, r - k/2)
+  int k, tg, groups;                 // NT == 0 (k x k): kernel size, taps per group, groups per kernel row
 };
 
+// NT: tapped tiles per stage -- 4: transposed conv; 3: a 3x3 kernel row fused; 1: one tap per stage; 0: k x k, a group
+// of a kernel row's taps fused (runtime k / tg / groups; NT == 3 is this with k = tg = 3 as compile-time constants)
 template <int NT>
 __global__ void __launch_bounds__(CONV_THREADS, 1)
 conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmdy, WgradArgs a) {
@@ -577,10 +582,19 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
   __shared__ int abort_s;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int NS = a.stages, Cin = a.Cin, Cout = a.Cout;
-  constexpr int NTOT = NT == 4 ? 4 : 3;                  // taps accumulated by one CTA
-  const int TT = NT == 4 ? 4 : 9;                         // taps in the whole gradient
+  // NT == 0: a kernel row's taps are split into groups of tg, so that a group's accumulators (tg * Cin columns) fit
+  // one MMA (N <= 256); the CTA (z, r, grp) accumulates taps s0 .. s0 + nt - 1 of kernel row r
+  constexpr bool KXK = NT == 0;
+  constexpr int NTOT = NT == 4 ? 4 : 3;                   // taps accumulated by one CTA (NT != 0)
+  const int r = KXK ? (int)blockIdx.y / a.groups : (int)blockIdx.y;
+  const int s0 = KXK ? ((int)blockIdx.y % a.groups) * a.tg : 0;
+  const int nt = KXK ? (a.k - s0 < a.tg ? a.k - s0 : a.tg) : NTOT;
+  const int kw = KXK ? a.k : NTOT;                        // taps per kernel row
+  const int TT = KXK ? a.k * a.k : NT == 4 ? 4 : 9;       // taps in the whole gradient
+  const int half_k = KXK ? a.k / 2 : 1;
+  const int nload = KXK ? nt : NT;                        // tapped tiles per stage
   uint32_t tmem_cols = 32;
-  while (tmem_cols < (uint32_t)(NTOT * Cin)) tmem_cols <<= 1;
+  while (tmem_cols < (uint32_t)((KXK ? a.tg : NTOT) * Cin)) tmem_cols <<= 1;
 
   if (tid == 0) {
     for (int i = 0; i < NS; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
@@ -598,7 +612,6 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
   volatile int* abortp = &abort_s;
   bool ok = true;
   const int64_t G = gridDim.x;
-  const int r = blockIdx.y;                               // kernel row: taps r*3 .. r*3+2
   constexpr int STEPS = NT == 1 ? 3 : 1;                  // stages per pixel block
 
   if (warp == 0) {
@@ -611,13 +624,13 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
           ok = mbar_wait(&empty_bar[s], ph ^ 1u, abortp);
           if (!ok) break;
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
-          mbar_expect_tx(&full_bar[s], a.dy_bytes + NT * a.x_bytes);
+          mbar_expect_tx(&full_bar[s], a.dy_bytes + nload * a.x_bytes);
           for (int j = 0; j < a.nby; ++j)
             tma_load_4d(base + j * (a.dy_bytes / a.nby), &tmdy, j * a.cby, x0, y0, b0, &full_bar[s]);
 #pragma unroll
-          for (int u = 0; u < NT; ++u) {
-            const int cx = NT == 4 ? x0 * a.cscale + a.tdx[u] : x0 + (NT == 3 ? u : st) - 1;
-            const int cy = NT == 4 ? y0 * a.cscale + a.tdy[u] : y0 + r - 1;
+          for (int u = 0; u < nload; ++u) {
+            const int cx = NT == 4 ? x0 * a.cscale + a.tdx[u] : x0 + s0 + (NT == 1 ? st : u) - half_k;
+            const int cy = NT == 4 ? y0 * a.cscale + a.tdy[u] : y0 + r - half_k;
             for (int j = 0; j < a.nbx; ++j)
               tma_load_4d(base + a.dy_bytes + u * a.x_bytes + j * (a.x_bytes / a.nbx), &tmx, j * a.cbx, cx, cy, b0,
                           &full_bar[s]);
@@ -643,10 +656,10 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
           if (!ok) break;
           tc_fence_after();
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
-          if (NT >= 3) {
-            // the NT tapped tiles are one MN-major operand of NT * Cin columns (tile stride = leading byte
-            // offset), their accumulators neighbours in TMEM: ONE MMA per 16 pixels instead of NT
-            const uint32_t idesc3 = idesc_bf16(NT * Cin, true, true);
+          if (NT != 1) {
+            // the tapped tiles are one MN-major operand of nload * Cin columns (tile stride = leading byte
+            // offset), their accumulators neighbours in TMEM: ONE MMA per 16 pixels instead of nload
+            const uint32_t idesc3 = idesc_bf16(nload * Cin, true, true);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
               const uint64_t da = make_desc_sw(base + j * a_kstep, a_lbo, a_sbo, a_ty);
@@ -665,7 +678,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
           }
           umma_commit(&empty_bar[s]);
           if (++s == (uint32_t)NS) { s = 0; ph ^= 1u; }
-          if (NT >= 3 || st == STEPS - 1) first = false;
+          if (NT != 1 || st == STEPS - 1) first = false;
         }
       }
       if (ok) umma_commit(&acc_full);
@@ -678,8 +691,8 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
     if (ok) {
       tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);
-      for (int tl = 0; tl < NTOT; ++tl) {
-        float* pp = a.part + (((int64_t)blockIdx.x * TT + r * NTOT + tl) * Cout + co) * Cin;
+      for (int tl = 0; tl < nt; ++tl) {
+        float* pp = a.part + (((int64_t)blockIdx.x * TT + r * kw + s0 + tl) * Cout + co) * Cin;
         for (int c = 0; c < Cin; c += 16) {
           float v[16];
           tmem_ld16(trow + (uint32_t)(tl * Cin + c), v);
@@ -703,28 +716,31 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
   }
 }
 
-// part [splits][(r,S)][po*Cout+co][pi*CinP+ci] (packed rows of P pixels) -> dw [Cout][Cin][3][3] (torch layout):
-// tap (r, s) collects every (S, po, pi) with S*P + pi - po + 1 == s.  One warp per output element: lane z owns the
+// part [splits][(r,S)][po*Cout+co][pi*CinP+ci] (packed rows of P pixels) -> dw [Cout][Cin][k][k] (torch layout):
+// tap (r, s) collects every (S, po, pi) with S*P + pi - po + k/2 == s.  One warp per output element: lane z owns the
 // splits z, z+32, ..., the lanes are folded by a fixed shuffle tree (deterministic).
-__global__ void wgrad_reduce_kernel(const float* __restrict__ part, int splits, int P, int Cout, int CinP, int Cin,
+// KC: the kernel size as a compile-time constant (3), or 0: k_rt
+template <int KC>
+__global__ void wgrad_reduce_kernel(const float* __restrict__ part, int splits, int P, int Cout, int CinP, int Cin, int k_rt,
                                     float* __restrict__ dw) {
   const int lane = threadIdx.x & 31;
   const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (i >= (int64_t)9 * Cout * Cin) return;
+  const int k = KC ? KC : k_rt, kk = k * k, h = k / 2;
+  if (i >= (int64_t)kk * Cout * Cin) return;
   // ci fastest: neighbouring warps read neighbouring partials
   const int ci = (int)(i % Cin), co = (int)((i / Cin) % Cout), tap = (int)(i / ((int64_t)Cin * Cout));
-  const int r = tap / 3, sx = tap % 3;
+  const int r = tap / k, sx = tap % k;
   const int64_t ldn = (int64_t)P * CinP, per_tap = (int64_t)P * Cout * ldn;
   float s = 0.f;
   for (int z = lane; z < splits; z += 32)
-    for (int S = -1; S <= 1; ++S)
+    for (int S = -h; S <= h; ++S)
       for (int po = 0; po < P; ++po) {
-        const int pi = sx - 1 + po - S * P;
+        const int pi = sx - h + po - S * P;
         if (pi < 0 || pi >= P) continue;
-        s += part[((int64_t)z * 9 + r * 3 + S + 1) * per_tap + ((int64_t)po * Cout + co) * ldn + (int64_t)pi * CinP + ci];
+        s += part[((int64_t)z * kk + r * k + S + h) * per_tap + ((int64_t)po * Cout + co) * ldn + (int64_t)pi * CinP + ci];
       }
   s = warp_sum(s);
-  if (lane == 0) dw[((int64_t)co * Cin + ci) * 9 + tap] = s;
+  if (lane == 0) dw[((int64_t)co * Cin + ci) * kk + tap] = s;
 }
 
 // fp32 rows (stride ld) -> compact bf16 rows of Cp >= C channels (zero padded); 8 channels per thread
@@ -749,26 +765,26 @@ __global__ void to_bf16_kernel(int64_t npix, int C, const float* __restrict__ x,
   *reinterpret_cast<uint4*>(out + p * Cp + c0) = o;
 }
 
-// w [Cout][Cin][3][3] fp32 -> operand of the convolution over rows of P packed pixels:
-//   q[(r,S)][n = po*Nc + nc][k = pi*KcP + kc],  S in {-1,0,1} = neighbouring packed row, po / pi = pixel inside
-//   the output / input row; the entry is the tap s = S*P + pi - po + 1 of kernel row r when 0 <= s <= 2, else 0.
-//   dgrad == 0: n = output channel co, k = input channel ci            (forward operand)
-//   dgrad == 1: n = ci, k = co, taps reversed (r, s) -> (2-r, 2-s)     (data-gradient operand)
-__global__ void pack_w_bf16_kernel(int Cout, int Cin, const float* __restrict__ w, __nv_bfloat16* __restrict__ q, int P,
-                                   int KcP, int dgrad) {
+// w [Cout][Cin][ks][ks] fp32 -> operand of the convolution over rows of P packed pixels:
+//   q[(r,S)][n = po*Nc + nc][k = pi*KcP + kc],  S in {-ks/2..ks/2} = neighbouring packed row, po / pi = pixel inside
+//   the output / input row; the entry is the tap s = S*P + pi - po + ks/2 of kernel row r when 0 <= s < ks, else 0.
+//   dgrad == 0: n = output channel co, k = input channel ci                    (forward operand)
+//   dgrad == 1: n = ci, k = co, taps reversed (r, s) -> (ks-1-r, ks-1-s)       (data-gradient operand)
+__global__ void pack_w_bf16_kernel(int Cout, int Cin, int ks, const float* __restrict__ w, __nv_bfloat16* __restrict__ q,
+                                   int P, int KcP, int dgrad) {
   const int Nc = dgrad ? Cin : Cout, Kc = dgrad ? Cout : Cin;
   const int64_t ldk = (int64_t)P * KcP, rows = (int64_t)P * Nc;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= 9 * rows * ldk) return;
+  if (i >= (int64_t)ks * ks * rows * ldk) return;
   const int k = (int)(i % ldk), n = (int)((i / ldk) % rows), t = (int)(i / (ldk * rows));
-  const int r = t / 3, S = t % 3 - 1;
+  const int h = ks / 2, r = t / ks, S = t % ks - h;
   const int pi = k / KcP, kc = k % KcP, po = n / Nc, nc = n % Nc;
-  const int sx = S * P + pi - po + 1;
+  const int sx = S * P + pi - po + h;
   float v = 0.f;
-  if (sx >= 0 && sx <= 2 && kc < Kc) {
+  if (sx >= 0 && sx < ks && kc < Kc) {
     const int co = dgrad ? kc : nc, ci = dgrad ? nc : kc;
-    const int tap = dgrad ? (2 - r) * 3 + (2 - sx) : r * 3 + sx;
-    v = w[((int64_t)co * Cin + ci) * 9 + tap];
+    const int tap = dgrad ? (ks - 1 - r) * ks + (ks - 1 - sx) : r * ks + sx;
+    v = w[((int64_t)co * Cin + ci) * ks * ks + tap];
   }
   q[i] = __float2bfloat16(v);
 }
@@ -820,8 +836,8 @@ extern "C" int tm_conv3x3_pack_bf16(int64_t Cout, int64_t Cin, const float* w, v
                                     void* stream) {
   TM_REQUIRE(P >= 1 && KcP >= (dgrad ? Cout : Cin), "tm_conv3x3_pack_bf16: bad packing");
   const int64_t n = 9 * P * (dgrad ? Cin : Cout) * P * KcP;
-  pack_w_bf16_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, w, (__nv_bfloat16*)q, (int)P,
-                                                                             (int)KcP, dgrad);
+  pack_w_bf16_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, 3, w, (__nv_bfloat16*)q,
+                                                                             (int)P, (int)KcP, dgrad);
   return check_launch("pack_w_bf16");
 }
 
@@ -989,8 +1005,9 @@ extern "C" int tm_convt2x2_bf16_dgrad(int64_t B, int64_t H, int64_t W, int64_t C
 }
 
 namespace {
-inline int wgrad_splits(const Geom& g) {
-  const int want = sm_count() / 3 > 0 ? sm_count() / 3 : 1;
+// gy: CTAs per pixel split (kernel rows x tap groups)
+inline int wgrad_splits(const Geom& g, int gy = 3) {
+  const int want = sm_count() / gy > 0 ? sm_count() / gy : 1;
   return (int)(g.ntiles < want ? g.ntiles : want);
 }
 }  // namespace
@@ -1102,6 +1119,107 @@ extern "C" int tm_conv3x3_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Ci
   else conv3x3_wgrad_tma_kernel<1><<<grid, CONV_THREADS, smem, st>>>(tmx, tmdy, a);
   TM_TRY(check_launch("conv3x3_wgrad_tma"));
   const int64_t n = 9 * Cout * Cin_real;
-  wgrad_reduce_kernel<<<(unsigned)cdiv(n * 32, 256), 256, 0, st>>>(a.part, splits, P, (int)Cout, (int)Cin, (int)Cin_real, dw);
+  wgrad_reduce_kernel<3><<<(unsigned)cdiv(n * 32, 256), 256, 0, st>>>(a.part, splits, P, (int)Cout, (int)Cin, (int)Cin_real, 3, dw);
+  return check_launch("wgrad_reduce");
+}
+
+// ------------------------------------------------------------------------------------------------
+// k x k convolutions (odd k <= 9, stride 1, zero padding k/2) on the same kernels: LayoutNet's 7x7 / 9x9 layers
+// (src/model.py:227-243).  Operand rows are single pixels (P = 1); the weights stream through the ring with the
+// activation boxes (a whole 7x7 / 9x9 weight does not fit shared memory next to the ring).
+// ------------------------------------------------------------------------------------------------
+namespace {
+inline bool kxk_ok(int64_t k) { return k >= 3 && k <= 9 && (k & 1); }
+// weight gradient: a kernel row's k taps in groups of tg, so that a group's accumulators fit one MMA (tg * Cin <= 256)
+inline void kxk_groups(int64_t Cin, int64_t k, int& tg, int& groups) {
+  tg = (int)(256 / Cin < k ? 256 / Cin : k);
+  groups = (int)cdiv(k, tg);
+  tg = (int)cdiv(k, groups);
+}
+}  // namespace
+
+extern "C" int tm_convkxk_bf16_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k) {
+  return kxk_ok(k) && conv_shape_ok(B, H, W, Cin, Cout) && conv_shape_ok(B, H, W, Cout, Cin) && pow2(Cin) && Cin <= 64 &&
+                 pow2(Cout) && Cout <= 128
+             ? 1
+             : 0;
+}
+
+// q: bf16 [k*k][Nc][KcP]; dgrad = 0: Nc = Cout, Kc = Cin (padded to KcP); dgrad = 1: Nc = Cin, Kc = Cout, taps reversed
+extern "C" int tm_convkxk_pack_bf16(int64_t Cout, int64_t Cin, int64_t k, const float* w, void* q, int64_t KcP, int dgrad,
+                                    void* stream) {
+  TM_REQUIRE(kxk_ok(k) && KcP >= (dgrad ? Cout : Cin), "tm_convkxk_pack_bf16: bad kernel size or packing");
+  const int64_t n = k * k * (dgrad ? Cin : Cout) * KcP;
+  pack_w_bf16_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, (int)k, w,
+                                                                             (__nv_bfloat16*)q, 1, (int)KcP, dgrad);
+  return check_launch("pack_w_bf16");
+}
+
+// y[pix, 0:N] (fp32, row stride ldy) = act(bias + sum_{tap,c} xb[pix + tap, c] * wq[tap][n][c]); flags: TM_EPI_RELU.
+// The data gradient is the same call on bf16(dy) with the dgrad operand (no bias).
+extern "C" int tm_convkxk_bf16(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t k, const void* xb,
+                               const void* wq, const float* bias, float* y, int64_t ldy, int flags, int* err, void* stream) {
+  TM_REQUIRE(kxk_ok(k) && conv_shape_ok(B, H, W, Cin, N),
+             "tm_convkxk_bf16: unsupported shape (odd k <= 9; H, W powers of two; channels multiples of 16)");
+  TM_REQUIRE(ldy % 4 == 0 && reinterpret_cast<uintptr_t>(y) % 16 == 0, "tm_convkxk_bf16: output rows must be 16-byte aligned");
+  TM_REQUIRE(reinterpret_cast<uintptr_t>(xb) % 16 == 0 && reinterpret_cast<uintptr_t>(wq) % 16 == 0,
+             "tm_convkxk_bf16: operands must be 16-byte aligned");
+  const int CK = Cin >= 64 ? 64 : (int)Cin;
+  ConvArgs a;
+  fill_common(a, B, H, W, Cin, N, CK, y, ldy, bias, err);
+  a.flags = (flags & TM_EPI_RELU) | (bias ? TM_EPI_BIAS : 0);
+  a.cpx = (int)N; a.ntaps = (int)(k * k); a.cscale = 1; a.convt = 0;
+  for (int t = 0; t < a.ntaps; ++t) { a.tdx[t] = (signed char)(t % k - k / 2); a.tdy[t] = (signed char)(t / k - k / 2); }
+  CUtensorMap tmx, tmw;
+  TM_TRY(encode_act(&tmx, xb, Cin, W, H, B, CK, a.g.TW, a.g.TH, a.g.TB));
+  TM_TRY(encode_2d(&tmw, wq, Cin, k * k * N, CK, (int)N));
+  return launch_taps(a, tmx, tmw, CK, (cudaStream_t)stream);
+}
+
+extern "C" size_t tm_convkxk_bf16_wgrad_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k) {
+  if (!kxk_ok(k) || Cin <= 0 || Cin > 256) return 0;
+  int tg, groups;
+  kxk_groups(Cin, k, tg, groups);
+  return (size_t)wgrad_splits(make_geom(B, H, W), (int)k * groups) * k * k * Cout * Cin * sizeof(float) + 256;
+}
+
+// dw[co][ci][ky][kx] (torch layout) = sum_pix dyb[pix, co] * xb[pix + (ky - k/2, kx - k/2), ci]
+// Grid (pixel splits, k kernel rows x tap groups); the partials are folded in a fixed order (deterministic).
+extern "C" int tm_convkxk_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k, const void* xb,
+                                     const void* dyb, float* dw, void* ws, size_t ws_bytes, int* err, void* stream) {
+  TM_REQUIRE(tm_convkxk_bf16_supported(B, H, W, Cin, Cout, k), "tm_convkxk_bf16_wgrad: unsupported shape");
+  TM_REQUIRE(ws && ws_bytes >= tm_convkxk_bf16_wgrad_ws(B, H, W, Cin, Cout, k), "tm_convkxk_bf16_wgrad: workspace too small");
+  WgradArgs a;
+  a.g = make_geom(B, H, W);
+  a.Cin = (int)Cin; a.Cout = (int)Cout;
+  a.cbx = (int)Cin; a.nbx = 1;
+  a.cby = Cout > 64 ? 64 : (int)Cout; a.nby = (int)Cout / a.cby;
+  a.x_bytes = 128u * (uint32_t)Cin * 2u;
+  a.dy_bytes = 128u * (uint32_t)Cout * 2u;
+  a.k = (int)k;
+  kxk_groups(Cin, k, a.tg, a.groups);
+  a.stage_bytes = (uint32_t)align_up(a.dy_bytes + a.tg * a.x_bytes, 1024);
+  const int ns = (int)(CONV_SMEM_BUDGET / a.stage_bytes);
+  a.stages = ns > CONV_MAX_STAGES ? CONV_MAX_STAGES : ns;
+  TM_REQUIRE(a.stages >= 2, "tm_convkxk_bf16_wgrad: tile does not fit shared memory");
+  a.part = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  a.err = err;
+  a.cscale = 1;
+  CUtensorMap tmx, tmdy;
+  TM_TRY(encode_act(&tmx, xb, Cin, W, H, B, a.cbx, a.g.TW, a.g.TH, a.g.TB));
+  TM_TRY(encode_act(&tmdy, dyb, Cout, W, H, B, a.cby, a.g.TW, a.g.TH, a.g.TB));
+  const int gy = (int)k * a.groups;
+  const int splits = wgrad_splits(a.g, gy);
+  const size_t smem = (size_t)a.stages * a.stage_bytes + 1024;
+  cudaStream_t st = (cudaStream_t)stream;
+  static bool optin = false;
+  if (!optin) {
+    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
+    optin = true;
+  }
+  conv3x3_wgrad_tma_kernel<0><<<dim3((unsigned)splits, (unsigned)gy), CONV_THREADS, smem, st>>>(tmx, tmdy, a);
+  TM_TRY(check_launch("convkxk_wgrad_tma"));
+  const int64_t n = k * k * Cout * Cin;
+  wgrad_reduce_kernel<0><<<(unsigned)cdiv(n * 32, 256), 256, 0, st>>>(a.part, splits, 1, (int)Cout, (int)Cin, (int)Cin, (int)k, dw);
   return check_launch("wgrad_reduce");
 }

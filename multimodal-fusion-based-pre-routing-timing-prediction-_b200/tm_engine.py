@@ -1,4 +1,4 @@
-"""Fused design step: U-Net + level-wise GNN + mask fusion + head, forward and backward.
+"""Fused design step: image network (U-Net or LayoutNet) + level-wise GNN + mask fusion + head, forward and backward.
 
 ``DesignStep.run(batch)`` performs what one optimisation step of the reference does to one design
 with all sampled endpoints in a batch (src/train.py:465 CNN forward, :490-511 level loop,
@@ -26,8 +26,10 @@ from tm_lib import call, stream
 from tm_ops import D, RELU, gemm_nn, gemm_tn, transpose
 
 
-def build_models(map_size, pooling="max", seed=0, device="cuda"):
-    """Reference wiring (train.py:56-81 with the head sized as model.py:267,280 produce it)."""
+def build_models(map_size, pooling="max", seed=0, device="cuda", cnn="unet"):
+    """Reference wiring (train.py:56-81 with the head sized as model.py:267,280 produce it).  ``cnn``: "unet" (the
+    reference's ``--unet``) or "layoutnet" (its default, train.py:70); LayoutNet takes a 2-channel image of 4x the
+    map size.  ``TM_UNET_MATH`` sets the math mode of either network."""
     import model as M
     import Unet as U
     torch.manual_seed(seed)
@@ -35,10 +37,15 @@ def build_models(map_size, pooling="max", seed=0, device="cuda"):
     fcn = torch.nn.Linear(map_size * map_size, 128)
     torch.nn.init.xavier_uniform_(fcn.weight, gain=torch.nn.init.calculate_gain("relu"))
     mdl = M.PathModel(gnn, None, fcn, None, None, M.MLP(128 + 128 + 32, 2 * (128 + 128 + 32), 1))
-    cnn = U.UNet(pooling)
+    if cnn == "unet":
+        net = U.UNet(pooling)
+    elif cnn == "layoutnet":
+        net = M.LayoutNet(pooling)
+    else:
+        raise ValueError(f"build_models: cnn must be 'unet' or 'layoutnet', not {cnn!r}")
     if os.environ.get("TM_UNET_MATH"):                 # e.g. "bf16": image branch on the TMA-fed bf16 tensor-core path
-        cnn.math = os.environ["TM_UNET_MATH"]
-    return mdl.to(device).train(), cnn.to(device).train()
+        net.math = os.environ["TM_UNET_MATH"]
+    return mdl.to(device).train(), net.to(device).train()
 
 
 class HostDesign:
@@ -172,6 +179,25 @@ class DesignStep:
         self.gnn_params = [sd[k] for k in tm_ops.GNN_PARAM_NAMES]
         self.cnn_names = [k for k, _ in cnn.named_parameters()]
         self.cnn_params = dict(cnn.named_parameters())
+        import model as M
+        self.layoutnet = isinstance(cnn, M.LayoutNet)    # else the U-Net (LayoutNet has no BatchNorm statistics)
+
+    # ---------------------------------------------------------------- image branch
+    def _image_forward(self, image, need_bwd):
+        if self.layoutnet:
+            return tm_unet.layoutnet_forward(self.cnn, image, need_bwd=need_bwd)
+        return tm_unet.unet_forward(self.cnn, image, need_bwd=need_bwd, update_stats=self.cnn.training)
+
+    def _image_backward(self, st, gout):
+        if self.layoutnet:
+            return tm_unet.layoutnet_backward(self.cnn, st, gout)
+        return tm_unet.unet_backward(self.cnn, st, gout)
+
+    @staticmethod
+    def _check_feature_map(fmap, b):
+        if fmap.numel() != b.mask_csr.width:
+            raise ValueError(f"the image network's feature map has {fmap.numel()} pixels ({tuple(fmap.shape)}) but the "
+                             f"path masks are {b.mask_csr.width} columns wide (map_size**2): wrong image size for this CNN")
 
     # ---------------------------------------------------------------- forward pieces
     def _head_image_side(self, b, feat, X):
@@ -207,7 +233,8 @@ class DesignStep:
 
     def forward(self, b):
         """Inference: predictions for the batch's endpoints (validate(), train.py:137-291)."""
-        fmap, _ = tm_unet.unet_forward(self.cnn, b.image, need_bwd=False, update_stats=self.cnn.training)
+        fmap, _ = self._image_forward(b.image, need_bwd=False)
+        self._check_feature_map(fmap, b)
         sched = b.graph.schedule()
         H, _ = tm_ops.gnn_forward(sched, b.cell_feat, b.net_feat,
                                   [p.detach() for p in self.gnn_params], save=False)
@@ -217,7 +244,7 @@ class DesignStep:
     # ---------------------------------------------------------------- full step
     def run(self, b, grad_scale=1.0):
         """Forward + backward.  Returns (loss (1,) device tensor, pred (T,)); fills ``.grad``."""
-        m, cnn = self.model, self.cnn
+        m = self.model
         dev = b.image.device
         main = torch.cuda.current_stream()
         if getattr(b, "dynamic", False):
@@ -241,8 +268,9 @@ class DesignStep:
         img_cap = int(os.environ.get("TM_IMAGE_SM_CAP", "0")) if side is not main else 0
         with torch.cuda.stream(side):
             old_cap = tm_lib.lib().tm_tc_set_grid_cap(img_cap)
-            fmap, ust = tm_unet.unet_forward(cnn, b.image, need_bwd=True, update_stats=cnn.training)
+            fmap, ust = self._image_forward(b.image, need_bwd=True)
             tm_lib.lib().tm_tc_set_grid_cap(old_cap)
+            self._check_feature_map(fmap, b)
             feat = fmap.reshape(-1)
             # everything of the head that does not read H runs here, off the netlist branch's critical path
             # (the image stream is idle long before the 101 levels finish): mask fusion, level embedding, G = 0
@@ -279,7 +307,7 @@ class DesignStep:
         self._assign(pairs)
         with torch.cuda.stream(side):
             old_cap = tm_lib.lib().tm_tc_set_grid_cap(img_cap)
-            ug = tm_unet.unet_backward(cnn, ust, dF.reshape(fmap.shape))
+            ug = self._image_backward(ust, dF.reshape(fmap.shape))
             tm_lib.lib().tm_tc_set_grid_cap(old_cap)
             upairs = [(self.cnn_params[k], ug[k]) for k in self.cnn_names]
             self._assign(upairs)

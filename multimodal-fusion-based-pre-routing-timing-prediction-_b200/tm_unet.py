@@ -443,6 +443,25 @@ class UNetFn(torch.autograd.Function):
 LAYOUT_SPEC = [(0, 2, 32, 9, True), (3, 32, 64, 7, True), (6, 64, 32, 9, False), (8, 32, 1, 7, False)]
 
 
+def _tma_kxk_ok(B, H, W, cin, cout, k):
+    """bf16 mode and a shape the TMA-fed k x k kernels take.  encode.0 (Cin = 2) and encode.8 (Cout = 1) never do:
+    padded to 16 channels they would waste 8x / 16x of every MMA."""
+    return (USE_TMA and _prec(None) == 0 and cin % 16 == 0 and cout % 16 == 0
+            and tm_lib.ws_bytes("tm_convkxk_bf16_supported", B, H, W, cin, cout, k) == 1)
+
+
+def _pack_kxk_bf16(w, need_dgrad):
+    """-> (forward operand [k*k][Cout][Cin], data-gradient operand [k*k][Cin][Cout] or None), bf16."""
+    cout, cin, k, _ = w.shape
+    wc = w.detach().float().contiguous()
+
+    def one(nc, kc, dgrad):
+        q = torch.empty(k * k, nc, kc, dtype=torch.bfloat16, device=w.device)
+        call("tm_convkxk_pack_bf16", cout, cin, k, wc, q, kc, dgrad, stream())
+        return q
+    return one(cout, cin, 0), (one(cin, cout, 1) if need_dgrad else None)
+
+
 def layoutnet_forward(net, x, need_bwd=True):
     _enter(net)
     squeeze = x.dim() == 3
@@ -460,11 +479,20 @@ def layoutnet_forward(net, x, need_bwd=True):
     h, w = H, W
     for li, (idx, cin, cout, k, pool) in enumerate(LAYOUT_SPEC):
         conv = net.encode[idx]
-        wf, wb = _pack(conv.weight, need_bwd)
         last = li == len(LAYOUT_SPEC) - 1
         y = _empty(B * h * w, cout, dev=dev)
-        _conv(cur, cin, B, h, w, cin, cout, k, wf, conv.bias.detach(), y, cout, 0 if last else RELU)
-        rec = dict(x=cur, y=y, cin=cin, cout=cout, k=k, H=h, W=w, wb=wb, pool=None, name=f"encode.{idx}")
+        rec = dict(x=cur, y=y, cin=cin, cout=cout, k=k, H=h, W=w, pool=None, name=f"encode.{idx}")
+        if _tma_kxk_ok(B, h, w, cin, cout, k):
+            # bf16 mode: TMA-fed tcgen05 k x k convolution; the bf16 copy of x is kept for the weight gradient
+            xb = _to_bf16(cur, cin, B * h * w, cin)
+            wq, wd = _pack_kxk_bf16(conv.weight, need_bwd and li > 0)
+            call("tm_convkxk_bf16", B, h, w, cin, cout, k, xb, wq, conv.bias.detach(), y, cout, 0 if last else RELU,
+                 tm_lib.err_flag(dev), stream())
+            rec.update(tma=True, xb=xb if need_bwd else None, wd=wd)
+        else:
+            wf, wb = _pack(conv.weight, need_bwd)
+            _conv(cur, cin, B, h, w, cin, cout, k, wf, conv.bias.detach(), y, cout, 0 if last else RELU)
+            rec.update(tma=False, wb=wb)
         if last:
             act = _empty(B * h * w, cout, dev=dev)
             call("tm_leaky_relu_forward", B * h * w * cout, y, 0.1, act, stream())
@@ -506,11 +534,25 @@ def layoutnet_backward(net, st, gout):
                 g = dyp
             dy = _empty(npix, cout, dev=dev)
             call("tm_leaky_relu_backward", npix * cout, r["y"], g, 0.0, dy, stream())   # ReLU
-        dw, db = _conv_wgrad(ws, r["x"], cin, dy, cout, B, h, w, cin, cout, k, True)
+        if r["tma"]:
+            # one bf16 copy of dy feeds the weight and the data gradient; the bias gradient sums the fp32 dy
+            dyb = _to_bf16(dy, cout, npix, cout)
+            dw, db = _empty(cout, cin, k, k, dev=dev), _empty(cout, dev=dev)
+            nb = tm_lib.ws_bytes("tm_convkxk_bf16_wgrad_ws", B, h, w, cin, cout, k)
+            call("tm_convkxk_bf16_wgrad", B, h, w, cin, cout, k, r["xb"], dyb, dw, ws.get(nb), nb, tm_lib.err_flag(dev),
+                 stream())
+            nbc = tm_lib.ws_bytes("tm_colsum_ws", npix, cout)
+            call("tm_colsum", npix, cout, dy, cout, None, db, 0, tm_lib.workspace(nbc, dev), nbc, stream())
+        else:
+            dw, db = _conv_wgrad(ws, r["x"], cin, dy, cout, B, h, w, cin, cout, k, True)
         grads[r["name"] + ".weight"], grads[r["name"] + ".bias"] = dw, db
         if li > 0:
             dx = _empty(npix, cin, dev=dev)
-            _conv(dy, cout, B, h, w, cout, cin, k, r["wb"], None, dx, cin)
+            if r["tma"]:
+                call("tm_convkxk_bf16", B, h, w, cout, cin, k, dyb, r["wd"], None, dx, cin, 0, tm_lib.err_flag(dev),
+                     stream())
+            else:
+                _conv(dy, cout, B, h, w, cout, cin, k, r["wb"], None, dx, cin)
             g = dx
     return grads
 
