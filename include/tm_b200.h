@@ -209,6 +209,21 @@ int tm_fuse_forward_runs(int64_t T, int64_t J, int64_t D, const int32_t* run_ptr
 int tm_fuse_backward(int64_t T, int64_t J, int64_t D, const int32_t* csc_ptr, const int32_t* csc_t,
                      const float* g, int64_t ld_g, const float* F, const float* Wt, float* dWt,
                      float* dF, void* stream);
+/* Several designs per step (the reference's per-design loop, src/train.py:461, taken K designs at a time):
+ * design k owns rows ep_off[k]..ep_off[k+1] of out / g (int32 ep_off[K+1] on the device), its feature map F + k*J
+ * and its own selected mask rows, named by design_tab: a device array of K records of five device pointers
+ * {run_ptr, run_lo, run_hi, csc_ptr, csc_t} (the MaskRows buffers of tm_mask_select).
+ * Forward: the K prefix tables are built in one launch (ws: tm_fuse_runs_multi_ws(K, J) bytes); design k's rows are
+ * bit-identical to tm_fuse_forward_runs on design k.
+ * Backward: dF [K][J], dF_k bit-identical to tm_fuse_backward on design k; dWt[j,:] = sum_k F_k[j] * sum_t g[t,:]
+ * over design k's positions t, summed in design order (one [J][D] result, not K). */
+size_t tm_fuse_runs_multi_ws(int64_t K, int64_t J);
+int tm_fuse_forward_runs_multi(int64_t K, int64_t T, int64_t J, int64_t D, const void* design_tab,
+                               const int32_t* ep_off, const float* F, const float* Wt, const float* bias,
+                               float* out, int64_t ld_out, void* ws, size_t ws_bytes, void* stream);
+int tm_fuse_backward_multi(int64_t K, int64_t J, int64_t D, const void* design_tab, const int32_t* ep_off,
+                           const float* g, int64_t ld_g, const float* F, const float* Wt, float* dWt, float* dF,
+                           void* stream);
 
 /* ------------------------------------------------------------------------------------
  * N2  path-mask rasteriser (replaces the host code that builds `path_masks`:
@@ -264,6 +279,11 @@ int tm_colsum_absmax(int64_t R, int64_t C, const float* X, int64_t ld, const int
 /* loss[0] = mean((pred-y)^2); grad[i] = 2*(pred[i]-y[i])/T * grad_scale  (nn.MSELoss) */
 int tm_mse(int64_t T, const float* pred, const float* y, float* loss, float* grad,
            float grad_scale, void* stream);
+/* K designs' losses in one step (src/train.py:513-522 per design, averaged over the K designs): design k owns
+ * positions ep_off[k]..ep_off[k+1] (int32 ep_off[K+1] on the device); loss_k[k] and grad on those positions are what
+ * tm_mse computes for them with grad_scale / K; loss[0] = mean of loss_k in design order.  K = 1 equals tm_mse. */
+int tm_mse_multi(int64_t K, const int32_t* ep_off, const float* pred, const float* y, float* loss_k, float* loss,
+                 float* grad, float grad_scale, void* stream);
 /* N4: the per-batch statistics the reference reads back one .item() at a time (train.py:513-549):
  * out8 = [mse, R2 (torchmetrics R2Score), correct, tp, fn, tn, fp, T] with predicted critical <=>
  * required - pred < 0 (judge_critical, train.py:391-395) against label (int64, 0 = non-critical).
@@ -344,6 +364,22 @@ int tm_bn_relu_backward(int64_t npix, int64_t C, const float* x, int64_t ldx, co
                         int64_t ldy, const float* dy, int64_t lddy, const float* gamma, const float* beta,
                         const float* save_mean, const float* save_invstd, float* dx, int64_t lddx,
                         float* dgamma, float* dbeta, void* dx_bf16, void* ws, size_t ws_bytes, void* stream);
+/* The same pair over nseg images of npix pixels each, with each image's OWN statistics: what the reference's
+ * batch-of-one cnn(cnn_inputs) (src/train.py:465) computes for every design of a multi-design step.  Image k's rows
+ * start at x + k*npix*ldx (likewise y, dy, dx; y_bf16 / dx_bf16 compact [nseg*npix][C]); save_mean / save_invstd are
+ * [nseg][C].  Each image uses the block partition and fold order of a single-image call, so its y, statistics and dx
+ * are bit-identical to tm_bn_relu_forward / tm_bn_relu_backward on that image.  The running statistics are updated
+ * nseg times, image 0 first; dgamma / dbeta [C] are the per-image values summed in image order.
+ * ws: tm_bn_seg_ws(nseg, npix, C) bytes. */
+size_t tm_bn_seg_ws(int64_t nseg, int64_t npix, int64_t C);
+int tm_bn_relu_forward_seg(int64_t nseg, int64_t npix, int64_t C, const float* x, int64_t ldx, const float* gamma,
+                           const float* beta, float* running_mean, float* running_var, float momentum, float eps,
+                           float* y, int64_t ldy, float* save_mean, float* save_invstd, void* y_bf16, void* ws,
+                           size_t ws_bytes, void* stream);
+int tm_bn_relu_backward_seg(int64_t nseg, int64_t npix, int64_t C, const float* x, int64_t ldx, const float* y,
+                            int64_t ldy, const float* dy, int64_t lddy, const float* gamma, const float* beta,
+                            const float* save_mean, const float* save_invstd, float* dx, int64_t lddx, float* dgamma,
+                            float* dbeta, void* dx_bf16, void* ws, size_t ws_bytes, void* stream);
 
 /* OutConv (Unet.py:74-75): nn.Conv2d(C, 1, kernel_size=1) as streaming kernels, exact fp32.
  * forward y[p] = x[p,:] . w + bias; dgrad dx[p,c] = dy[p] * w[c]; wgrad dw[c] = sum_p x[p,c] dy[p], dbias = sum_p dy[p]. */

@@ -73,6 +73,9 @@ __global__ void fold4_kernel(int64_t Cout, const float* __restrict__ cs, float* 
 // pixel range; a thread owns VEC consecutive channels (128-bit loads when the layout allows) of every
 // (256 / groups)-th pixel, accumulates in fp64 and the block folds its pixel lanes in shared memory:
 // part[block][C][2].  The finalize kernels add the <= BN_BLOCKS partials per channel in a fixed order.
+// Segmented form (several images of npix pixels each, one U-Net batch with per-image statistics): blockIdx.y is the
+// image; image k sweeps its own pixels with the block partition a single-image call uses, and every per-channel,
+// per-image array ([nseg][C]) is offset by k, so each image's numbers are bit-identical to a call on that image.
 constexpr int BN_BLOCKS = 592;           // 4 per SM
 constexpr int BN_THREADS = 256;
 
@@ -94,6 +97,11 @@ bn_stats_kernel(int64_t npix, int C, const float* __restrict__ x, int64_t ldx, c
                 const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ beta,
                 double* __restrict__ part) {
   extern __shared__ double sh[];                       // [lanes][C][2]
+  const int64_t seg = blockIdx.y;
+  x += seg * npix * ldx;
+  if (y) y += seg * npix * ldy;
+  if (BWD) { dy += seg * npix * lddy; mean += seg * C; invstd += seg * C; }
+  part += seg * gridDim.x * C * 2;
   const int groups = (C + VEC - 1) / VEC;              // channel groups per pixel
   const int lanes = BN_THREADS / groups;               // pixel lanes (groups <= 256)
   const int g = threadIdx.x % groups, pl = threadIdx.x / groups;
@@ -198,24 +206,30 @@ __device__ __forceinline__ void bn_block_sum2(double& a, double& b) {
 }
 
 __global__ void __launch_bounds__(256)
-bn_finalize_kernel(int64_t npix, int64_t C, int nblk, const double* __restrict__ part,
+bn_finalize_kernel(int64_t npix, int64_t C, int nblk, int nseg, const double* __restrict__ part,
                    float* __restrict__ running_mean, float* __restrict__ running_var,
                    float momentum, float eps, float* __restrict__ save_mean,
                    float* __restrict__ save_invstd) {
   const int c = blockIdx.x;
-  double a = 0.0, b = 0.0;
-  for (int i = threadIdx.x; i < nblk; i += 256) { a += part[((int64_t)i * C + c) * 2]; b += part[((int64_t)i * C + c) * 2 + 1]; }
-  bn_block_sum2(a, b);
-  if (threadIdx.x != 0) return;
-  const double mean = a / (double)npix;
-  double var = b / (double)npix - mean * mean;
-  if (var < 0.0) var = 0.0;
-  save_mean[c] = (float)mean;
-  save_invstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-  if (running_mean) {
-    const double unbiased = npix > 1 ? var * (double)npix / (double)(npix - 1) : var;
-    running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)mean;
-    running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
+  // images in order: the running statistics see image 0's update first, as nseg single-image calls would
+  for (int k = 0; k < nseg; ++k) {
+    const double* pk = part + (int64_t)k * nblk * C * 2;
+    double a = 0.0, b = 0.0;
+    for (int i = threadIdx.x; i < nblk; i += 256) { a += pk[((int64_t)i * C + c) * 2]; b += pk[((int64_t)i * C + c) * 2 + 1]; }
+    bn_block_sum2(a, b);
+    if (threadIdx.x == 0) {
+      const double mean = a / (double)npix;
+      double var = b / (double)npix - mean * mean;
+      if (var < 0.0) var = 0.0;
+      save_mean[k * C + c] = (float)mean;
+      save_invstd[k * C + c] = (float)(1.0 / sqrt(var + (double)eps));
+      if (running_mean) {
+        const double unbiased = npix > 1 ? var * (double)npix / (double)(npix - 1) : var;
+        running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)mean;
+        running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
+      }
+    }
+    __syncthreads();                                   // bn_block_sum2's shared slots are reused by the next image
   }
 }
 
@@ -229,6 +243,12 @@ __global__ void bn_relu_apply_kernel(int64_t npix, int C, const float* __restric
   const int groups = C / VEC;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= npix * groups) return;
+  const int64_t seg = blockIdx.y;                      // image (segmented call): its rows and statistics
+  x += seg * npix * ldx;
+  if (y) y += seg * npix * ldy;
+  if (yb) yb += seg * npix * C;
+  mean += seg * C;
+  invstd += seg * C;
   const int64_t p = i / groups;
   const int c = (int)(i - p * groups) * VEC;
   float v[VEC];
@@ -251,13 +271,24 @@ __global__ void bn_relu_apply_kernel(int64_t npix, int C, const float* __restric
 }
 
 __global__ void __launch_bounds__(256)
-bn_bwd_finalize_kernel(int64_t C, int nblk, const double* __restrict__ part, float* __restrict__ dgamma,
-                       float* __restrict__ dbeta) {
+bn_bwd_finalize_kernel(int64_t C, int nblk, int nseg, const double* __restrict__ part, float* dgamma_seg, float* dbeta_seg,
+                       float* dgamma, float* dbeta) {   // (not restrict: nseg == 1 passes the same arrays twice)
   const int c = blockIdx.x;
-  double a = 0.0, b = 0.0;
-  for (int i = threadIdx.x; i < nblk; i += 256) { a += part[((int64_t)i * C + c) * 2]; b += part[((int64_t)i * C + c) * 2 + 1]; }
-  bn_block_sum2(a, b);
-  if (threadIdx.x == 0) { dbeta[c] = (float)a; dgamma[c] = (float)b; }
+  double ga = 0.0, be = 0.0;                           // fold over the images, in image order
+  for (int k = 0; k < nseg; ++k) {
+    const double* pk = part + (int64_t)k * nblk * C * 2;
+    double a = 0.0, b = 0.0;
+    for (int i = threadIdx.x; i < nblk; i += 256) { a += pk[((int64_t)i * C + c) * 2]; b += pk[((int64_t)i * C + c) * 2 + 1]; }
+    bn_block_sum2(a, b);
+    if (threadIdx.x == 0) {
+      dbeta_seg[k * C + c] = (float)a;                 // image k's own sums: its data gradient needs them
+      dgamma_seg[k * C + c] = (float)b;
+      be += (double)(float)a;
+      ga += (double)(float)b;
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) { dbeta[c] = (float)be; dgamma[c] = (float)ga; }
 }
 
 template <int VEC>
@@ -271,6 +302,13 @@ __global__ void bn_bwd_apply_kernel(int64_t npix, int C, const float* __restrict
   const int groups = C / VEC;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= npix * groups) return;
+  const int64_t seg = blockIdx.y;
+  x += seg * npix * ldx;
+  if (y) y += seg * npix * ldy;
+  dy += seg * npix * lddy;
+  if (dx) dx += seg * npix * lddx;
+  if (dxb) dxb += seg * npix * C;
+  mean += seg * C; invstd += seg * C; dgamma += seg * C; dbeta += seg * C;
   const int64_t p = i / groups;
   const int c = (int)(i - p * groups) * VEC;
   float xv[VEC], yv[VEC], gv[VEC], o[VEC];
@@ -652,6 +690,64 @@ extern "C" size_t tm_bn_ws(int64_t npix, int64_t C) {
   return (size_t)BN_BLOCKS * C * 2 * sizeof(double) + 256;
 }
 
+extern "C" size_t tm_bn_seg_ws(int64_t nseg, int64_t npix, int64_t C) {
+  return (size_t)nseg * (BN_BLOCKS * C * 2 * sizeof(double) + 2 * C * sizeof(float)) + 256;
+}
+
+namespace {
+// nseg images of npix pixels each: image k's rows start at x + k * npix * ldx (likewise y, dy, dx; the bf16 copies
+// are compact), its statistics at save_mean + k * C.  nseg == 1 is the plain batch-norm call.
+int bn_relu_forward_impl(int64_t nseg, int64_t npix, int64_t C, const float* x, int64_t ldx, const float* gamma,
+                         const float* beta, float* running_mean, float* running_var, float momentum, float eps, float* y,
+                         int64_t ldy, float* save_mean, float* save_invstd, void* y_bf16, const void* stats_part,
+                         int64_t nparts, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  double* part = (double*)ws;
+  const bool v4 = bn_vec4(C, {{x, ldx}, {y, ldy}});
+  const int nblk = bn_blocks(npix, C, v4);
+  const int groups = v4 ? (int)C / 4 : (int)C;
+  const size_t sh = (size_t)(BN_THREADS / groups) * C * 2 * sizeof(double);
+  const dim3 sgrid((unsigned)nblk, (unsigned)nseg);
+  int nfin = nblk;
+  if (stats_part) {                      // statistics already taken by the producing convolution's epilogue
+    part = (double*)stats_part;
+    nfin = (int)nparts;
+  } else {
+    if (v4) bn_stats_kernel<4, false><<<sgrid, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, nullptr, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr, part);
+    else bn_stats_kernel<1, false><<<sgrid, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, nullptr, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr, part);
+    TM_TRY(check_launch("bn_stats"));
+  }
+  bn_finalize_kernel<<<(unsigned)C, 256, 0, ST>>>(npix, C, nfin, (int)nseg, part, running_mean, running_var,
+                                                             momentum, eps, save_mean, save_invstd);
+  TM_TRY(check_launch("bn_finalize"));
+  if (v4) bn_relu_apply_kernel<4><<<dim3(blocks_for(npix * (C / 4)), (unsigned)nseg), 256, 0, ST>>>(npix, (int)C, x, ldx, gamma, beta, save_mean, save_invstd, y, ldy, (__nv_bfloat16*)y_bf16);
+  else bn_relu_apply_kernel<1><<<dim3(blocks_for(npix * C), (unsigned)nseg), 256, 0, ST>>>(npix, (int)C, x, ldx, gamma, beta, save_mean, save_invstd, y, ldy, (__nv_bfloat16*)y_bf16);
+  return check_launch("bn_relu_apply");
+}
+
+int bn_relu_backward_impl(int64_t nseg, int64_t npix, int64_t C, const float* x, int64_t ldx, const float* y,
+                          int64_t ldy, const float* dy, int64_t lddy, const float* gamma, const float* beta,
+                          const float* save_mean, const float* save_invstd, float* dx, int64_t lddx, float* dgamma,
+                          float* dbeta, void* dx_bf16, void* ws, cudaStream_t stream) {
+  const bool v4 = bn_vec4(C, {{x, ldx}, {y, ldy}, {dy, lddy}, {dx, lddx}});
+  const int nblk = bn_blocks(npix, C, v4);
+  double* part = (double*)ws;
+  // per-image dgamma / dbeta (what image k's data gradient uses); a single image uses the outputs themselves
+  float* dg_seg = nseg > 1 ? reinterpret_cast<float*>(part + nseg * nblk * C * 2) : dgamma;
+  float* db_seg = nseg > 1 ? dg_seg + nseg * C : dbeta;
+  const int groups = v4 ? (int)C / 4 : (int)C;
+  const size_t sh = (size_t)(BN_THREADS / groups) * C * 2 * sizeof(double);
+  const dim3 sgrid((unsigned)nblk, (unsigned)nseg);
+  if (v4) bn_stats_kernel<4, true><<<sgrid, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, save_mean, save_invstd, gamma, beta, part);
+  else bn_stats_kernel<1, true><<<sgrid, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, save_mean, save_invstd, gamma, beta, part);
+  TM_TRY(check_launch("bn_bwd_stats"));
+  bn_bwd_finalize_kernel<<<(unsigned)C, 256, 0, ST>>>(C, nblk, (int)nseg, part, dg_seg, db_seg, dgamma, dbeta);
+  TM_TRY(check_launch("bn_bwd_finalize"));
+  if (v4) bn_bwd_apply_kernel<4><<<dim3(blocks_for(npix * (C / 4)), (unsigned)nseg), 256, 0, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, gamma, beta, save_mean, save_invstd, dg_seg, db_seg, dx, lddx, (__nv_bfloat16*)dx_bf16);
+  else bn_bwd_apply_kernel<1><<<dim3(blocks_for(npix * C), (unsigned)nseg), 256, 0, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, gamma, beta, save_mean, save_invstd, dg_seg, db_seg, dx, lddx, (__nv_bfloat16*)dx_bf16);
+  return check_launch("bn_bwd_apply");
+}
+}  // namespace
+
 /* y_bf16 (optional): compact bf16 copy [npix][C] of y, written by the same pass */
 extern "C" int tm_bn_relu_forward(int64_t npix, int64_t C, const float* x, int64_t ldx, const float* gamma,
                                   const float* beta, float* running_mean, float* running_var,
@@ -660,27 +756,20 @@ extern "C" int tm_bn_relu_forward(int64_t npix, int64_t C, const float* x, int64
                                   size_t ws_bytes, void* stream) {
   TM_REQUIRE(npix > 0 && C > 0 && C <= 256, "tm_bn_relu_forward: bad sizes (C <= 256)");
   TM_REQUIRE(ws_bytes >= tm_bn_ws(npix, C), "tm_bn_relu_forward: workspace too small");
-  double* part = (double*)ws;
-  const bool v4 = bn_vec4(C, {{x, ldx}, {y, ldy}});
-  const int nblk = bn_blocks(npix, C, v4);
-  const int groups = v4 ? (int)C / 4 : (int)C;
-  const size_t sh = (size_t)(BN_THREADS / groups) * C * 2 * sizeof(double);
   TM_REQUIRE(y || y_bf16, "tm_bn_relu_forward: neither y nor y_bf16 given");
-  int nfin = nblk;
-  if (stats_part) {                      // statistics already taken by the producing convolution's epilogue
-    part = (double*)stats_part;
-    nfin = (int)nparts;
-  } else {
-    if (v4) bn_stats_kernel<4, false><<<nblk, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, nullptr, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr, part);
-    else bn_stats_kernel<1, false><<<nblk, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, nullptr, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr, part);
-    TM_TRY(check_launch("bn_stats"));
-  }
-  bn_finalize_kernel<<<(unsigned)C, 256, 0, ST>>>(npix, C, nfin, part, running_mean, running_var,
-                                                             momentum, eps, save_mean, save_invstd);
-  TM_TRY(check_launch("bn_finalize"));
-  if (v4) bn_relu_apply_kernel<4><<<blocks_for(npix * (C / 4)), 256, 0, ST>>>(npix, (int)C, x, ldx, gamma, beta, save_mean, save_invstd, y, ldy, (__nv_bfloat16*)y_bf16);
-  else bn_relu_apply_kernel<1><<<blocks_for(npix * C), 256, 0, ST>>>(npix, (int)C, x, ldx, gamma, beta, save_mean, save_invstd, y, ldy, (__nv_bfloat16*)y_bf16);
-  return check_launch("bn_relu_apply");
+  return bn_relu_forward_impl(1, npix, C, x, ldx, gamma, beta, running_mean, running_var, momentum, eps, y, ldy,
+                              save_mean, save_invstd, y_bf16, stats_part, nparts, ws, ws_bytes, ST);
+}
+
+extern "C" int tm_bn_relu_forward_seg(int64_t nseg, int64_t npix, int64_t C, const float* x, int64_t ldx,
+                                      const float* gamma, const float* beta, float* running_mean, float* running_var,
+                                      float momentum, float eps, float* y, int64_t ldy, float* save_mean,
+                                      float* save_invstd, void* y_bf16, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(nseg > 0 && nseg <= 65535 && npix > 0 && C > 0 && C <= 256, "tm_bn_relu_forward_seg: bad sizes (C <= 256)");
+  TM_REQUIRE(ws_bytes >= tm_bn_seg_ws(nseg, npix, C), "tm_bn_relu_forward_seg: workspace too small");
+  TM_REQUIRE(y || y_bf16, "tm_bn_relu_forward_seg: neither y nor y_bf16 given");
+  return bn_relu_forward_impl(nseg, npix, C, x, ldx, gamma, beta, running_mean, running_var, momentum, eps, y, ldy,
+                              save_mean, save_invstd, y_bf16, nullptr, 0, ws, ws_bytes, ST);
 }
 
 namespace {
@@ -716,19 +805,21 @@ extern "C" int tm_bn_relu_backward(int64_t npix, int64_t C, const float* x, int6
   TM_REQUIRE(dx || dx_bf16, "tm_bn_relu_backward: neither dx nor dx_bf16 given");
   TM_REQUIRE(y || beta, "tm_bn_relu_backward: without the stored activation y the mask is rebuilt from beta");
   TM_REQUIRE(ws_bytes >= tm_bn_ws(npix, C), "tm_bn_relu_backward: workspace too small");
-  double* part = (double*)ws;
-  const bool v4 = bn_vec4(C, {{x, ldx}, {y, ldy}, {dy, lddy}, {dx, lddx}});
-  const int nblk = bn_blocks(npix, C, v4);
-  const int groups = v4 ? (int)C / 4 : (int)C;
-  const size_t sh = (size_t)(BN_THREADS / groups) * C * 2 * sizeof(double);
-  if (v4) bn_stats_kernel<4, true><<<nblk, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, save_mean, save_invstd, gamma, beta, part);
-  else bn_stats_kernel<1, true><<<nblk, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, save_mean, save_invstd, gamma, beta, part);
-  TM_TRY(check_launch("bn_bwd_stats"));
-  bn_bwd_finalize_kernel<<<(unsigned)C, 256, 0, ST>>>(C, nblk, part, dgamma, dbeta);
-  TM_TRY(check_launch("bn_bwd_finalize"));
-  if (v4) bn_bwd_apply_kernel<4><<<blocks_for(npix * (C / 4)), 256, 0, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, gamma, beta, save_mean, save_invstd, dgamma, dbeta, dx, lddx, (__nv_bfloat16*)dx_bf16);
-  else bn_bwd_apply_kernel<1><<<blocks_for(npix * C), 256, 0, ST>>>(npix, (int)C, x, ldx, y, ldy, dy, lddy, gamma, beta, save_mean, save_invstd, dgamma, dbeta, dx, lddx, (__nv_bfloat16*)dx_bf16);
-  return check_launch("bn_bwd_apply");
+  return bn_relu_backward_impl(1, npix, C, x, ldx, y, ldy, dy, lddy, gamma, beta, save_mean, save_invstd, dx, lddx,
+                               dgamma, dbeta, dx_bf16, ws, ST);
+}
+
+extern "C" int tm_bn_relu_backward_seg(int64_t nseg, int64_t npix, int64_t C, const float* x, int64_t ldx,
+                                       const float* y, int64_t ldy, const float* dy, int64_t lddy, const float* gamma,
+                                       const float* beta, const float* save_mean, const float* save_invstd, float* dx,
+                                       int64_t lddx, float* dgamma, float* dbeta, void* dx_bf16, void* ws,
+                                       size_t ws_bytes, void* stream) {
+  TM_REQUIRE(nseg > 0 && nseg <= 65535 && npix > 0 && C > 0 && C <= 256, "tm_bn_relu_backward_seg: bad sizes (C <= 256)");
+  TM_REQUIRE(dx || dx_bf16, "tm_bn_relu_backward_seg: neither dx nor dx_bf16 given");
+  TM_REQUIRE(y || beta, "tm_bn_relu_backward_seg: without the stored activation y the mask is rebuilt from beta");
+  TM_REQUIRE(ws_bytes >= tm_bn_seg_ws(nseg, npix, C), "tm_bn_relu_backward_seg: workspace too small");
+  return bn_relu_backward_impl(nseg, npix, C, x, ldx, y, ldy, dy, lddy, gamma, beta, save_mean, save_invstd, dx, lddx,
+                               dgamma, dbeta, dx_bf16, ws, ST);
 }
 
 extern "C" int tm_conv1x1_c1_forward(int64_t npix, int64_t C, const float* x, int64_t ldx, const float* w,

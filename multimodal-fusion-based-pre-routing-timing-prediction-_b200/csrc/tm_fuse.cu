@@ -78,6 +78,10 @@ __global__ void __launch_bounds__(D)
 prefix_local_kernel(int64_t J, const float* __restrict__ F, const float* __restrict__ Wt,
                     double* __restrict__ P, double* __restrict__ tot) {
   const int c = threadIdx.x;
+  const int64_t k = blockIdx.y;                      // design (batched form): its feature map, table and block totals
+  F += k * J;
+  P += k * (J + 1) * D;
+  tot += k * gridDim.x * D;
   const int64_t j0 = (int64_t)blockIdx.x * PB;
   double acc = 0.0;
 #pragma unroll 8
@@ -96,6 +100,8 @@ __global__ void __launch_bounds__(D)
 prefix_offset_kernel(int64_t J, double* __restrict__ P, const double* __restrict__ tot) {
   const int c = threadIdx.x, b = blockIdx.x;
   if (b == 0) return;
+  P += (int64_t)blockIdx.y * (J + 1) * D;
+  tot += (int64_t)blockIdx.y * gridDim.x * D;
   double off = 0.0;
   for (int i = 0; i < b; ++i) off += tot[(int64_t)i * D + c];      // fixed order: deterministic
   const int64_t j0 = (int64_t)b * PB;
@@ -152,6 +158,80 @@ fuse_bwd_kernel(int64_t J, const int* __restrict__ cptr, const int* __restrict__
   }
   dot = warp_sum(dot);
   if (lane == 0) dF[j] = dot;
+}
+
+// Several designs in one launch.  Design k owns endpoints [ep_off[k], ep_off[k+1]) of the concatenated batch, the
+// feature map F + k*J and its own mask-row selection (run-length and CSC tables, MaskRows buffers) named by a device
+// pointer table.  Every design's numbers are computed with exactly the arithmetic of the one-design kernels above.
+struct FuseDesign { const int* run_ptr; const int* run_lo; const int* run_hi; const int* csc_ptr; const int* csc_t; };
+
+__device__ __forceinline__ int design_of(int t, const int* __restrict__ ep_off, int K) {
+  int k = 0;
+  while (k + 1 < K && ep_off[k + 1] <= t) ++k;
+  return k;
+}
+
+__global__ void __launch_bounds__(D)
+fuse_fwd_runs_multi_kernel(int K, int64_t J, const FuseDesign* __restrict__ tab, const int* __restrict__ ep_off,
+                           const double* __restrict__ P, const float* __restrict__ bias, float* __restrict__ out,
+                           int64_t ldo) {
+  const int t = blockIdx.x, c = threadIdx.x;
+  const int k = design_of(t, ep_off, K);
+  const FuseDesign d = tab[k];
+  const int tl = t - ep_off[k];
+  P += (int64_t)k * (J + 1) * D;
+  const int s = d.run_ptr[tl], e = d.run_ptr[tl + 1];
+  double acc = 0.0;
+  for (int r = s; r < e; r += 4) {
+    double hi[4], lo[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      hi[u] = 0.0; lo[u] = 0.0;
+      if (r + u < e) { hi[u] = P[(int64_t)d.run_hi[r + u] * D + c]; lo[u] = P[(int64_t)d.run_lo[r + u] * D + c]; }
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) acc += hi[u] - lo[u];
+  }
+  out[(int64_t)t * ldo + c] = (float)acc + bias[c];
+}
+
+// one warp per column j pulls every design's CSC column in design order: dF_k[j] as tm_fuse_backward computes it for
+// design k, and dWt[j] = sum_k F_k[j] * acc_k[j] (the K per-design weight gradients are never materialised)
+__global__ void __launch_bounds__(256)
+fuse_bwd_multi_kernel(int K, int64_t J, const FuseDesign* __restrict__ tab, const int* __restrict__ ep_off,
+                      const float* __restrict__ g, int64_t ldg, const float* __restrict__ F,
+                      const float* __restrict__ Wt, float* __restrict__ dWt, float* __restrict__ dF) {
+  const int lane = threadIdx.x & 31;
+  const int64_t j = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (j >= J) return;
+  float4 dw = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int k = 0; k < K; ++k) {
+    const FuseDesign d = tab[k];
+    const float* gk = g + (int64_t)ep_off[k] * ldg;
+    const int s = d.csc_ptr[j], e = d.csc_ptr[j + 1];
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int i = s; i < e; i += 4) {
+      float4 v[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        v[q] = (i + q < e) ? __ldg(reinterpret_cast<const float4*>(gk + (int64_t)d.csc_t[i + q] * ldg + lane * 4))
+                           : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) { acc.x += v[q].x; acc.y += v[q].y; acc.z += v[q].z; acc.w += v[q].w; }
+    }
+    const float f = F[(int64_t)k * J + j];
+    const float4 p = make_float4(f * acc.x, f * acc.y, f * acc.z, f * acc.w);
+    if (k == 0) dw = p;
+    else { dw.x += p.x; dw.y += p.y; dw.z += p.z; dw.w += p.w; }
+    float dot = 0.f;
+    if (e > s) {
+      const float4 w = __ldg(reinterpret_cast<const float4*>(Wt + j * D + lane * 4));
+      dot = acc.x * w.x + acc.y * w.y + acc.z * w.z + acc.w * w.w;
+    }
+    dot = warp_sum(dot);
+    if (lane == 0) dF[(int64_t)k * J + j] = dot;
+  }
+  st4(dWt + j * D + lane * 4, dw);
 }
 
 __global__ void gather_cols_kernel(int64_t T, int64_t w, const float* __restrict__ src, int64_t lds,
@@ -271,6 +351,36 @@ mse_kernel(int64_t T, const float* __restrict__ pred, const float* __restrict__ 
     v = warp_sum(v);
     if (threadIdx.x == 0 && loss) loss[0] = (float)(v / (double)T);
   }
+}
+
+// one block per design: what mse_kernel computes for design k's T_k endpoints, its gradient scaled by gscale / K
+__global__ void __launch_bounds__(1024)
+mse_multi_kernel(int K, const int* __restrict__ ep_off, const float* __restrict__ pred, const float* __restrict__ y,
+                 float* __restrict__ loss_k, float* __restrict__ grad, float gscale) {
+  __shared__ double part[32];
+  const int k = blockIdx.x;
+  const int64_t o = ep_off[k], T = ep_off[k + 1] - o;
+  const float gs = gscale / (float)K;
+  double s = 0.0;
+  for (int64_t i = threadIdx.x; i < T; i += blockDim.x) {
+    const float d = pred[o + i] - y[o + i];
+    s += (double)d * (double)d;
+    if (grad) grad[o + i] = 2.f * d / (float)T * gs;
+  }
+  s = warp_sum(s);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    double v = part[threadIdx.x];
+    v = warp_sum(v);
+    if (threadIdx.x == 0) loss_k[k] = T > 0 ? (float)(v / (double)T) : __int_as_float(0x7fc00000);
+  }
+}
+
+__global__ void mean_fixed_kernel(int K, const float* __restrict__ v, float* __restrict__ out) {
+  double s = 0.0;
+  for (int k = 0; k < K; ++k) s += (double)v[k];
+  out[0] = (float)(s / (double)K);
 }
 
 // N4: every per-batch number the reference's loop reads back with its own .item() (train.py:513-549,
@@ -397,6 +507,43 @@ extern "C" int tm_fuse_backward(int64_t T, int64_t J, int64_t Dd, const int32_t*
   return check_launch("fuse_bwd");
 }
 
+extern "C" size_t tm_fuse_runs_multi_ws(int64_t K, int64_t J) {
+  return (size_t)K * ((J + 1) * D + cdiv(J, PB) * D) * sizeof(double) + 256;
+}
+
+extern "C" int tm_fuse_forward_runs_multi(int64_t K, int64_t T, int64_t J, int64_t Dd, const void* design_tab,
+                                          const int32_t* ep_off, const float* F, const float* Wt, const float* bias,
+                                          float* out, int64_t ld_out, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(Dd == D, "tm_fuse_forward_runs_multi: D must be 128");
+  TM_REQUIRE(K > 0 && K <= 65535 && design_tab && ep_off, "tm_fuse_forward_runs_multi: bad design table");
+  TM_REQUIRE(ws && ws_bytes >= tm_fuse_runs_multi_ws(K, J), "tm_fuse_forward_runs_multi: workspace too small");
+  if (T <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  double* P = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  double* tot = P + K * (J + 1) * D;
+  const unsigned nb = (unsigned)cdiv(J, PB);
+  if (nb > 0) {
+    prefix_local_kernel<<<dim3(nb, (unsigned)K), D, 0, st>>>(J, F, Wt, P, tot);
+    TM_TRY(check_launch("fuse_prefix_local"));
+    prefix_offset_kernel<<<dim3(nb, (unsigned)K), D, 0, st>>>(J, P, tot);
+    TM_TRY(check_launch("fuse_prefix_offset"));
+  }
+  fuse_fwd_runs_multi_kernel<<<(unsigned)T, D, 0, st>>>((int)K, J, reinterpret_cast<const FuseDesign*>(design_tab), ep_off,
+                                                        P, bias, out, ld_out);
+  return check_launch("fuse_fwd_runs_multi");
+}
+
+extern "C" int tm_fuse_backward_multi(int64_t K, int64_t J, int64_t Dd, const void* design_tab, const int32_t* ep_off,
+                                      const float* g, int64_t ld_g, const float* F, const float* Wt, float* dWt,
+                                      float* dF, void* stream) {
+  TM_REQUIRE(Dd == D, "tm_fuse_backward_multi: D must be 128");
+  TM_REQUIRE(K > 0 && design_tab && ep_off, "tm_fuse_backward_multi: bad design table");
+  if (J <= 0) return 0;
+  fuse_bwd_multi_kernel<<<(unsigned)cdiv(J * 32, 256), 256, 0, (cudaStream_t)stream>>>(
+      (int)K, J, reinterpret_cast<const FuseDesign*>(design_tab), ep_off, g, ld_g, F, Wt, dWt, dF);
+  return check_launch("fuse_bwd_multi");
+}
+
 extern "C" int tm_gather_cols(int64_t T, int64_t w, const float* src, int64_t lds, const int32_t* rows,
                               float* dst, int64_t ldd, int64_t col0, void* stream) {
   if (T * w <= 0) return 0;
@@ -490,6 +637,16 @@ extern "C" int tm_mse(int64_t T, const float* pred, const float* y, float* loss,
   TM_REQUIRE(T > 0, "tm_mse: empty batch");
   mse_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(T, pred, y, loss, grad, grad_scale);
   return check_launch("mse");
+}
+
+extern "C" int tm_mse_multi(int64_t K, const int32_t* ep_off, const float* pred, const float* y, float* loss_k,
+                            float* loss, float* grad, float grad_scale, void* stream) {
+  TM_REQUIRE(K > 0 && ep_off && loss_k && loss, "tm_mse_multi: bad arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  mse_multi_kernel<<<(unsigned)K, 1024, 0, st>>>((int)K, ep_off, pred, y, loss_k, grad, grad_scale);
+  TM_TRY(check_launch("mse_multi"));
+  mean_fixed_kernel<<<1, 1, 0, st>>>((int)K, loss_k, loss);
+  return check_launch("mse_mean");
 }
 
 extern "C" int tm_step_metrics(int64_t T, const float* pred, const float* arrival, const float* required,

@@ -72,10 +72,10 @@ class HostDesign:
 
 
 class DesignBatch:
-    """Device-resident batch of one design."""
+    """Device-resident batch of one design, or of K designs joined by ``DesignBatch.concat``."""
 
     def __init__(self, graph, mask_csr, endpoints, endpoint_level, arrival_time, image, cell_feat=None, net_feat=None,
-                 rows=None, dynamic=False):
+                 rows=None, dynamic=False, mask_rows=None):
         self.graph, self.mask_csr = graph, mask_csr
         # per-batch feature tensors (a prefetched batch must not disturb the one in flight through
         # the shared graph object); default: whatever the graph carries
@@ -84,10 +84,21 @@ class DesignBatch:
         self.endpoints = endpoints                 # int32 (T,)
         self.endpoint_level = endpoint_level       # float32 (T,)
         self.arrival_time = arrival_time           # float32 (T,)
-        self.image = image                         # (C,H,W)
+        self.image = image                         # (C,H,W); (K,C,H,W) for K designs
         # rows: the mask row (path id) of every endpoint -- th.index_select(path_masks, 0, paths), train.py:500;
         # None: endpoint t owns row t (one design's endpoints in one batch, test.py:176)
-        self.mask_rows = mask_csr.select(rows) if rows is not None else mask_csr.select_all()
+        if mask_rows is None:
+            mask_rows = [mask_csr.select(rows) if rows is not None else mask_csr.select_all()]
+        # one MaskRows per design; design k owns endpoints ep_off[k]..ep_off[k+1] of this batch
+        self.mask_rows_list = list(mask_rows)
+        self.mask_rows = self.mask_rows_list[0] if len(self.mask_rows_list) == 1 else None
+        self.K = len(self.mask_rows_list)
+        self.width = self.mask_rows_list[0].csr.width
+        self.ep_off_h = np.concatenate([[0], np.cumsum([r.T for r in self.mask_rows_list])]).astype(np.int64)
+        self.ep_off = None                         # int32 (K+1,) on the device: set by concat (K > 1 only)
+        self.pin_off_h = None                      # first pin of every design in the joined netlist (concat)
+        self.design_losses = None                  # (K,) device tensor, rewritten by every step / replay (K > 1)
+        self._fuse_table = None
         # dynamic: the endpoint batch (endpoints / levels / labels / mask rows) is refreshed IN PLACE between steps, so
         # the step re-runs the on-device row selection every time (captured into its CUDA graph): one capture per
         # design serves every shuffled batch of the reference's DataLoader (train.py:470-486)
@@ -105,13 +116,77 @@ class DesignBatch:
             self._cone = ConeGraph(self.graph, self.endpoints)
         return self._cone
 
-    def set_endpoints(self, endpoints, endpoint_level, arrival_time, rows):
-        """Refresh the endpoint batch in place (same batch size): what changes between two DataLoader batches."""
-        self.endpoints.copy_(endpoints, non_blocking=True)
-        self.endpoint_level.copy_(endpoint_level, non_blocking=True)
-        self.arrival_time.copy_(arrival_time, non_blocking=True)
-        self.mask_rows.rows.copy_(rows, non_blocking=True)
+    def set_endpoints(self, endpoints, endpoint_level, arrival_time, rows, design=0):
+        """Refresh the endpoint batch in place (same batch size): what changes between two DataLoader batches.
+        ``design``: which design of a joined batch (its pin ids as in its own netlist)."""
+        s, e = int(self.ep_off_h[design]), int(self.ep_off_h[design + 1])
+        if self.pin_off_h is not None:
+            endpoints = endpoints + int(self.pin_off_h[design])
+        self.endpoints[s:e].copy_(endpoints, non_blocking=True)
+        self.endpoint_level[s:e].copy_(endpoint_level, non_blocking=True)
+        self.arrival_time[s:e].copy_(arrival_time, non_blocking=True)
+        self.mask_rows_list[design].rows.copy_(rows, non_blocking=True)
         self._cone = None
+
+    def fuse_table(self):
+        """int64 (K, 5) device table of every design's mask-row buffers {run_ptr, run_lo, run_hi, csc_ptr, csc_t}
+        (read by the batched fusion kernels).  The buffers are allocated once and rewritten in place by
+        ``MaskRows.rebuild``, so the table stays valid under CUDA-graph replay."""
+        if self._fuse_table is None:
+            rows = []
+            for r in self.mask_rows_list:
+                run_ptr, run_lo, run_hi = r.runs()
+                csc_ptr, csc_t = r.csc()
+                rows.append([t.data_ptr() for t in (run_ptr, run_lo, run_hi, csc_ptr, csc_t)])
+            self._fuse_table = torch.tensor(rows, dtype=torch.int64).to(self.endpoints.device)
+        return self._fuse_table
+
+    @staticmethod
+    def concat(batches):
+        """One batch of K designs (same image size, same map size), stepped as one by ``DesignStep``: the loss is the
+        mean of the designs' losses and every gradient the mean of their gradients (``DesignStep.run``).
+
+        The netlists are joined into one ``TimingGraph`` (pin ids of design k offset by the pins before it), whose
+        level schedule is every design's own schedule side by side (caller-supplied topological levels survive);
+        features, endpoints (offset), levels and labels are concatenated, the images stacked to (K, C, H, W), and the
+        designs' ``MaskRows`` kept as they are.  A batch is dynamic when one of its designs is."""
+        batches = list(batches)
+        if not batches:
+            raise ValueError("DesignBatch.concat: no designs")
+        b0 = batches[0]
+        for k, b in enumerate(batches[1:], 1):
+            for what, a, c in (("image", b0.image.shape, b.image.shape),
+                               ("mask width", (b0.width,), (b.width,)),
+                               ("cell_feat width", tuple(b0.cell_feat.shape[1:]), tuple(b.cell_feat.shape[1:])),
+                               ("net_feat width", tuple(b0.net_feat.shape[1:]), tuple(b.net_feat.shape[1:]))):
+                if tuple(a) != tuple(c):
+                    raise ValueError(f"DesignBatch.concat: design {k} has {what} {tuple(c)} but design 0 has {tuple(a)}")
+            if b.K != 1:
+                raise ValueError(f"DesignBatch.concat: design {k} is already a batch of {b.K} designs")
+        if b0.K != 1:
+            raise ValueError(f"DesignBatch.concat: design 0 is already a batch of {b0.K} designs")
+        dev = b0.endpoints.device
+        ns = [b.graph.number_of_nodes() for b in batches]
+        pin_off = np.concatenate([[0], np.cumsum(ns)]).astype(np.int64)
+        scheds = [b.graph.schedule() for b in batches]
+        edges = {}
+        for et in ("net", "cell"):
+            edges[et] = tuple(torch.cat([b.graph._edges[et][i].to(dev) + int(o) for b, o in zip(batches, pin_off)])
+                              for i in range(2))
+        g = TimingGraph(int(pin_off[-1]), edges["net"], edges["cell"])
+        g._edges = edges                                                   # already on the device
+        g._levels = (torch.cat([s.level for s in scheds]).contiguous(), max(s.num_levels for s in scheds))
+        cell_feat = torch.cat([b.cell_feat for b in batches])
+        net_feat = torch.cat([b.net_feat for b in batches])
+        g.ndata["cell_feat"], g.ndata["net_feat"] = cell_feat, net_feat
+        endpoints = torch.cat([b.endpoints + int(o) for b, o in zip(batches, pin_off)]).to(torch.int32)
+        out = DesignBatch(g, None, endpoints, torch.cat([b.endpoint_level for b in batches]),
+                          torch.cat([b.arrival_time for b in batches]), torch.stack([b.image for b in batches]),
+                          cell_feat=cell_feat, net_feat=net_feat, dynamic=any(b.dynamic for b in batches),
+                          mask_rows=[b.mask_rows for b in batches])
+        out.pin_off_h = pin_off
+        out.ep_off = torch.from_numpy(out.ep_off_h.astype(np.int32)).to(dev)
+        return out
 
     @staticmethod
     def from_host(h, device, graph=None):
@@ -157,6 +232,36 @@ class PreparedDesign:
         return self.replay()
 
 
+class PreparedDesigns:
+    """``DesignStep.prepare_many``: K resident designs, one captured step over all of them."""
+
+    def __init__(self, step, hosts, device, pool=None):
+        self.parts = [DesignBatch.from_host(h, device) for h in hosts]
+        self.batch = DesignBatch.concat(self.parts)
+        torch.cuda.synchronize()
+        self.replay = step.capture(self.batch, pool=pool)
+
+    def upload(self, hosts, stream=None):
+        """Host -> device copy of every design's per-step values into its slices of the graph's static inputs."""
+        if len(hosts) != len(self.parts):
+            raise ValueError(f"PreparedDesigns.upload: {len(hosts)} designs given, {len(self.parts)} prepared")
+        b = self.batch
+        ctx = torch.cuda.stream(stream) if stream is not None else torch.cuda.stream(torch.cuda.current_stream())
+        with ctx:
+            for k, h in enumerate(hosts):
+                p0, p1 = int(b.pin_off_h[k]), int(b.pin_off_h[k + 1])
+                e0, e1 = int(b.ep_off_h[k]), int(b.ep_off_h[k + 1])
+                b.cell_feat[p0:p1].copy_(h.t["cell_feat"], non_blocking=True)
+                b.net_feat[p0:p1].copy_(h.t["net_feat"], non_blocking=True)
+                b.image[k].copy_(h.t["image"], non_blocking=True)
+                b.arrival_time[e0:e1].copy_(h.t["arrival_time"], non_blocking=True)
+
+    def step(self, hosts=None):
+        if hosts is not None:
+            self.upload(hosts)
+        return self.replay()
+
+
 class DesignStep:
     def __init__(self, model, cnn, process_group=None, world_size=1, prune=None):
         """``prune`` (default: environment ``TM_CONE=1``, else off): run the netlist branch on the sub-netlist that can
@@ -186,7 +291,8 @@ class DesignStep:
     def _image_forward(self, image, need_bwd):
         if self.layoutnet:
             return tm_unet.layoutnet_forward(self.cnn, image, need_bwd=need_bwd)
-        return tm_unet.unet_forward(self.cnn, image, need_bwd=need_bwd, update_stats=self.cnn.training)
+        # several designs: each image is normalised with its own statistics, as the reference's batch of one is
+        return tm_unet.unet_forward(self.cnn, image, need_bwd=need_bwd, update_stats=self.cnn.training, per_image=True)
 
     def _image_backward(self, st, gout):
         if self.layoutnet:
@@ -195,9 +301,10 @@ class DesignStep:
 
     @staticmethod
     def _check_feature_map(fmap, b):
-        if fmap.numel() != b.mask_csr.width:
-            raise ValueError(f"the image network's feature map has {fmap.numel()} pixels ({tuple(fmap.shape)}) but the "
-                             f"path masks are {b.mask_csr.width} columns wide (map_size**2): wrong image size for this CNN")
+        per = fmap.numel() // b.K                        # one feature map per design
+        if per * b.K != fmap.numel() or per != b.width:
+            raise ValueError(f"the image network's feature map has {per} pixels per design ({tuple(fmap.shape)}) but the "
+                             f"path masks are {b.width} columns wide (map_size**2): wrong image size for this CNN")
 
     # ---------------------------------------------------------------- forward pieces
     def _head_image_side(self, b, feat, X):
@@ -206,12 +313,14 @@ class DesignStep:
         m = self.model
         T = int(b.endpoints.numel())
         width = X.shape[1]
-        wt = tm_ops.fusion_forward(b.mask_rows, feat, m.fcn.weight.detach(), m.fcn.bias.detach(), X[:, D:], width)
+        tab = b.fuse_table() if b.K > 1 else None
+        wt = tm_ops.fusion_forward_multi(b.mask_rows_list, tab, b.ep_off, feat, m.fcn.weight.detach(),
+                                         m.fcn.bias.detach(), X[:, D:], width)
         a0, a2 = m.mlp_alpha.layers[0], m.mlp_alpha.layers[2]
         lv = b.endpoint_level.reshape(T, 1)
         ha = tm_ops.mlp2_forward(lv, 1, None, T, a0.weight.detach(), a0.bias.detach(), a2.weight.detach(),
                                  a2.bias.detach(), X[:, 2 * D:], width)
-        return dict(X=X, wt=wt, ha=ha, lv=lv, width=width)
+        return dict(X=X, wt=wt, ha=ha, lv=lv, width=width, tab=tab)
 
     def _head_netlist_side(self, H, b, hs, endpoints=None):
         """Endpoint rows of H into columns 0..D of X, then ``mlp_fuse``."""
@@ -232,7 +341,8 @@ class DesignStep:
         return self._head_netlist_side(H, b, hs), hs
 
     def forward(self, b):
-        """Inference: predictions for the batch's endpoints (validate(), train.py:137-291)."""
+        """Inference: predictions for the batch's endpoints (validate(), train.py:137-291); for a joined batch, every
+        design's predictions one after the other."""
         fmap, _ = self._image_forward(b.image, need_bwd=False)
         self._check_feature_map(fmap, b)
         sched = b.graph.schedule()
@@ -243,12 +353,15 @@ class DesignStep:
 
     # ---------------------------------------------------------------- full step
     def run(self, b, grad_scale=1.0):
-        """Forward + backward.  Returns (loss (1,) device tensor, pred (T,)); fills ``.grad``."""
+        """Forward + backward.  Returns (loss (1,) device tensor, pred (T,)); fills ``.grad``.  A batch of K designs
+        (``DesignBatch.concat``) gives loss = mean of the designs' MSEs (``b.design_losses``, (K,)) and every gradient
+        the mean of their gradients; predictions are per design as the one-design step gives them."""
         m = self.model
         dev = b.image.device
         main = torch.cuda.current_stream()
         if getattr(b, "dynamic", False):
-            b.mask_rows.rebuild()                            # this batch's mask-row selection (7 small kernels, no host sync)
+            for r in b.mask_rows_list:                       # this batch's mask-row selection (7 small kernels, no host sync)
+                r.rebuild()
         side = self.image_stream if (self.overlap and self.image_stream is not None) else main
         side.wait_stream(main)                               # fork: inputs / parameters are ready on `main`
         # the netlist branch runs on the sub-netlist that can reach this batch's endpoints (tm_graph.ConeGraph)
@@ -280,7 +393,12 @@ class DesignStep:
         pred = self._head_netlist_side(H, b, hs, endpoints)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         gpred = torch.empty(T, 1, dtype=torch.float32, device=dev)
-        call("tm_mse", T, pred, b.arrival_time, loss, gpred, float(grad_scale), stream())
+        if b.K == 1:
+            call("tm_mse", T, pred, b.arrival_time, loss, gpred, float(grad_scale), stream())
+        else:                                                # mean over designs: each design's gradient scaled by 1/K
+            b.design_losses = torch.empty(b.K, dtype=torch.float32, device=dev)
+            call("tm_mse_multi", b.K, b.ep_off, pred, b.arrival_time, b.design_losses, loss, gpred, float(grad_scale),
+                 stream())
 
         # ---- head backward: mlp_fuse on the netlist stream (its dX seeds the backward sweep) ...
         width = hs["width"]
@@ -294,7 +412,8 @@ class DesignStep:
         with torch.cuda.stream(side):
             da1, dab1, da2, dab2, _ = tm_ops.mlp2_backward(hs["lv"], 1, None, T, a0.weight.detach(), a2.weight.detach(),
                                                            hs["ha"], dX[:, 2 * D:], width, b1=a0.bias.detach())
-            dF, dfw, dfb = tm_ops.fusion_backward(b.mask_rows, feat, hs["wt"], dX[:, D:], width)
+            dF, dfw, dfb = tm_ops.fusion_backward_multi(b.mask_rows_list, hs["tab"], b.ep_off, feat, hs["wt"],
+                                                        dX[:, D:], width)
             head = [(f0.weight, dw1), (f0.bias, db1), (f2.weight, dw2), (f2.bias, db2), (a0.weight, da1),
                     (a0.bias, dab1), (a2.weight, da2), (a2.bias, dab2), (m.fcn.weight, dfw), (m.fcn.bias, dfb)]
             self._assign(head)
@@ -381,6 +500,12 @@ class DesignStep:
         refreshes the per-step VALUES (features, image, labels) from pinned host memory and replays.
         The structure (edges, endpoints, masks) must be the one given here."""
         return PreparedDesign(self, host, device, graph, pool)
+
+    def prepare_many(self, hosts, device, pool=None):
+        """K designs made resident for repeated steps over all of them (``DesignBatch.concat``), captured as ONE CUDA
+        graph.  Returns a ``PreparedDesigns``; its ``step(hosts)`` refreshes the per-step VALUES of all K from pinned
+        host memory and replays.  The structures must be the ones given here."""
+        return PreparedDesigns(self, hosts, device, pool)
 
     @staticmethod
     def _assign(pairs):

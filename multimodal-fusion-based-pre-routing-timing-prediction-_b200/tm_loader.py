@@ -230,6 +230,27 @@ class LoadedDesign:
             yield self.batch(ids[i:i + batch_size])
 
 
+def prepare_many(designs, step, batch_size=1350):
+    """``LoadedDesign.prepare`` for K designs stepped together (``tm_engine.DesignBatch.concat``): ONE CUDA-graph
+    capture, and ``run(list of K path-id lists) -> (loss, pred)`` refreshes every design's endpoint batch in place and
+    replays the captured step, which re-selects every design's mask rows on the device.  Each list must hold
+    ``batch_size`` path ids."""
+    import tm_engine
+    designs = list(designs)
+    parts = [d.batch([d.paths[i % len(d.paths)] for i in range(batch_size)], dynamic=True) for d in designs]
+    b = tm_engine.DesignBatch.concat(parts)
+    replay = step.capture(b)
+
+    def run(path_id_lists):
+        assert len(path_id_lists) == len(designs), "one path-id list per prepared design"
+        for k, (d, ids) in enumerate(zip(designs, path_id_lists)):
+            assert len(ids) == batch_size, "a prepared design replays fixed-size batches"
+            b.set_endpoints(*d.batch_tensors(ids), design=k)
+        return replay()
+    run.batch = b
+    return run
+
+
 def _prepared(tuple_or_path, usage, os_rate, feat_reduce, norm, num_ctypes):
     if isinstance(tuple_or_path, (str, os.PathLike)):
         data_path, fname = os.path.split(str(tuple_or_path))

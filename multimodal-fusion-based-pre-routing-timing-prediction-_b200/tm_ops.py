@@ -485,6 +485,37 @@ def fusion_backward(mask_rows, feat, wt, g, ldg):
     return dF, transpose(dwt), db
 
 
+def fusion_forward_multi(rows, tab, ep_off, feat, fcn_w, fcn_b, out, ldo):
+    """Mask fusion of K designs in one launch: ``rows`` their ``MaskRows``, ``tab`` the device table of their
+    run / CSC buffers, ``ep_off`` int32 (K+1,) endpoint offsets, ``feat`` (K*J,) their feature maps.  Row t of ``out``
+    is what ``fusion_forward`` gives for its design.  K = 1 is ``fusion_forward``.  Returns fcn_w^T."""
+    K = len(rows)
+    if K == 1:
+        return fusion_forward(rows[0], feat, fcn_w, fcn_b, out, ldo)
+    J = int(feat.numel()) // K
+    if fcn_w.shape != (D, J):
+        raise RuntimeError(f"fcn must be Linear({J}, 128); got weight {tuple(fcn_w.shape)}")
+    wt = transpose(fcn_w)
+    nb = tm_lib.ws_bytes("tm_fuse_runs_multi_ws", K, J)
+    call("tm_fuse_forward_runs_multi", K, sum(r.T for r in rows), J, D, tab, ep_off, feat, wt, _f32c(fcn_b), out, ldo,
+         tm_lib.workspace(nb, feat.device), nb, stream())
+    return wt
+
+
+def fusion_backward_multi(rows, tab, ep_off, feat, wt, g, ldg):
+    """Returns (dfeat (K*J,), dfcn_w (128,J) summed over the designs, dfcn_b (128,)).  K = 1 is ``fusion_backward``."""
+    K = len(rows)
+    if K == 1:
+        return fusion_backward(rows[0], feat, wt, g, ldg)
+    J = int(feat.numel()) // K
+    dev = feat.device
+    dwt = torch.empty(J, D, dtype=torch.float32, device=dev)
+    dF = torch.empty(K * J, dtype=torch.float32, device=dev)
+    call("tm_fuse_backward_multi", K, J, D, tab, ep_off, g, ldg, feat, wt, dwt, dF, stream())
+    db = colsum(g, sum(r.T for r in rows), D, ldg)
+    return dF, transpose(dwt), db
+
+
 class MaskFusionFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mask_rows, feat_flat, fcn_w, fcn_b):

@@ -149,6 +149,7 @@ def _pack(w, need_bwd=True):
 
 
 EVAL = False          # set by unet_forward: nn.Module.eval() -> BatchNorm uses its running statistics
+SEG = 1               # set by unet_forward / unet_backward: > 1 -> BatchNorm statistics per image of the batch
 
 
 def _bn_relu_fwd(ws, x, ldx, npix, C, bn, y, ldy, update_stats, yb=None, stats=None):
@@ -160,14 +161,21 @@ def _bn_relu_fwd(ws, x, ldx, npix, C, bn, y, ldy, update_stats, yb=None, stats=N
         call("tm_bn_relu_eval", npix, C, x, ldx, bn.weight.detach(), bn.bias.detach(), bn.running_mean, bn.running_var,
              float(bn.eps), y, ldy, mean, invstd, yb, stream())
         return mean, invstd
-    nb = tm_lib.ws_bytes("tm_bn_ws", npix, C)
     rm = bn.running_mean if update_stats else None
     rv = bn.running_var if update_stats else None
-    call("tm_bn_relu_forward", npix, C, x, ldx, bn.weight.detach(), bn.bias.detach(), rm, rv,
-         float(bn.momentum), float(bn.eps), y, ldy, mean, invstd, yb, stats[0] if stats else None,
-         stats[1] if stats else 0, ws.get(nb), nb, stream())
+    if SEG > 1:
+        # each image its own statistics; the running statistics take SEG updates, image 0 first
+        mean, invstd = _empty(SEG * C, dev=dev), _empty(SEG * C, dev=dev)
+        nb = tm_lib.ws_bytes("tm_bn_seg_ws", SEG, npix // SEG, C)
+        call("tm_bn_relu_forward_seg", SEG, npix // SEG, C, x, ldx, bn.weight.detach(), bn.bias.detach(), rm, rv,
+             float(bn.momentum), float(bn.eps), y, ldy, mean, invstd, yb, ws.get(nb), nb, stream())
+    else:
+        nb = tm_lib.ws_bytes("tm_bn_ws", npix, C)
+        call("tm_bn_relu_forward", npix, C, x, ldx, bn.weight.detach(), bn.bias.detach(), rm, rv,
+             float(bn.momentum), float(bn.eps), y, ldy, mean, invstd, yb, stats[0] if stats else None,
+             stats[1] if stats else 0, ws.get(nb), nb, stream())
     if update_stats and bn.num_batches_tracked is not None:
-        bn.num_batches_tracked += 1
+        bn.num_batches_tracked += SEG
     return mean, invstd
 
 
@@ -176,6 +184,11 @@ def _bn_relu_bwd(ws, x, ldx, dy, lddy, npix, C, gamma, beta, mean, invstd, dx, l
     is rebuilt from x and the saved statistics (bit-identical to the forward), so the activation is not read."""
     dev = x.device
     dg, db = _empty(C, dev=dev), _empty(C, dev=dev)
+    if SEG > 1:
+        nb = tm_lib.ws_bytes("tm_bn_seg_ws", SEG, npix // SEG, C)
+        call("tm_bn_relu_backward_seg", SEG, npix // SEG, C, x, ldx, None, 0, dy, lddy, gamma, beta, mean, invstd, dx,
+             lddx, dg, db, dxb, ws.get(nb), nb, stream())
+        return dg, db
     nb = tm_lib.ws_bytes("tm_bn_ws", npix, C)
     call("tm_bn_relu_backward", npix, C, x, ldx, None, 0, dy, lddy, gamma, beta, mean, invstd, dx, lddx, dg, db, dxb,
          ws.get(nb), nb, stream())
@@ -197,11 +210,12 @@ def _double_conv_fwd(ws, st, name, mods, x, ldx, B, H, W, cin, cout, out, ldo, u
         xb = _to_bf16(x, ldx, npix, cin)
         wq1, wd1 = _pack_bf16(conv1.weight, W, need_bwd and cin % 16 == 0)
         wq2, wd2 = _pack_bf16(conv2.weight, W, need_bwd)
-        s1 = _conv_tma(xb, B, H, W, _cpad(cin), cmid, wq1, r1, cmid, want_stats=True)
+        # the convolution epilogue's statistics cover the whole batch: per-image statistics (SEG > 1) take their own pass
+        s1 = _conv_tma(xb, B, H, W, _cpad(cin), cmid, wq1, r1, cmid, want_stats=SEG == 1)
         a1b = torch.empty(npix, cmid, dtype=torch.bfloat16, device=dev)
         # the mid activation exists only as the bf16 operand of conv2 (the backward rebuilds its ReLU mask from r1)
         m1, i1 = _bn_relu_fwd(ws, r1, cmid, npix, cmid, bn1, None, 0, update_stats, yb=a1b, stats=s1)
-        s2 = _conv_tma(a1b, B, H, W, cmid, cout, wq2, r2, cout, want_stats=True)
+        s2 = _conv_tma(a1b, B, H, W, cmid, cout, wq2, r2, cout, want_stats=SEG == 1)
         m2, i2 = _bn_relu_fwd(ws, r2, cout, npix, cout, bn2, out, ldo, update_stats, stats=s2)
         st[name] = dict(tma=True, xb=xb if need_bwd else None, a1b=a1b if need_bwd else None, wd1=wd1, wd2=wd2,
                         x=x, ldx=ldx, B=B, H=H, W=W, cin=cin, cmid=cmid, cout=cout, r1=r1, r2=r2, out=out,
@@ -263,11 +277,13 @@ def _dc_mods(dc):
     return seq[0], seq[1], seq[3], seq[4]
 
 
-def unet_forward(net, x, need_bwd=True, update_stats=True):
+def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
     """``net``: the UNet module (parameter container).  x: (B,3,H,W) or (3,H,W) on a CUDA device.
-    Returns (out (B,1,H/2,W/2), state)."""
+    Returns (out (B,1,H/2,W/2), state).  ``per_image``: train-mode BatchNorm normalises every image with its own
+    statistics, as B batch-of-one calls would (the fused step over several designs); default: batch statistics,
+    like ``nn.BatchNorm2d``."""
     _enter(net)
-    global EVAL
+    global EVAL, SEG
     EVAL = not net.training
     if EVAL and need_bwd:
         raise NotImplementedError("UNet in eval mode is inference only here (BatchNorm backward with frozen statistics is not "
@@ -279,10 +295,11 @@ def unet_forward(net, x, need_bwd=True, update_stats=True):
     B, C, H, W = x.shape
     if C != 3 or H % 8 or W % 8:
         raise RuntimeError("UNet expects (B,3,H,W) with H and W multiples of 8")
+    SEG = B if per_image and not EVAL else 1
     dev = x.device
     mode = 0 if net.pooling == "max" else 1
     ws = _Ws(dev)
-    st = {"ws": ws, "mode": mode, "B": B, "H": H, "W": W}
+    st = {"ws": ws, "mode": mode, "B": B, "H": H, "W": W, "seg": SEG}
     x0 = _empty(B * H * W, 3, dev=dev)
     call("tm_nchw_to_nhwc", B, 3, H, W, x, x0, 3, stream())
     chans = [16, 32, 64, 128]
@@ -348,6 +365,8 @@ def unet_forward(net, x, need_bwd=True, update_stats=True):
 def unet_backward(net, st, gout):
     """gout: (B,1,H/2,W/2).  Returns {state_dict-style name: gradient} for every parameter."""
     _enter(net)
+    global SEG
+    SEG = st["seg"]
     B, H, W, mode = st["B"], st["H"], st["W"], st["mode"]
     ws, chans, Hs, Ws_, cat = st["ws"], st["chans"], st["Hs"], st["Ws"], st["cat"]
     dev = gout.device
