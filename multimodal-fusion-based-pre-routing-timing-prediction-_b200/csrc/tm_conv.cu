@@ -73,6 +73,10 @@ __global__ void fold4_kernel(int64_t Cout, const float* __restrict__ cs, float* 
 // pixel range; a thread owns VEC consecutive channels (128-bit loads when the layout allows) of every
 // (256 / groups)-th pixel, accumulates in fp64 and the block folds its pixel lanes in shared memory:
 // part[block][C][2].  The finalize kernels add the <= BN_BLOCKS partials per channel in a fixed order.
+// The forward sums are shifted: every pixel contributes x - K_c and (x - K_c)^2, K_c = the image's first pixel of
+// channel c, so that E[x^2] - mean^2 does not cancel catastrophically on a channel whose mean is large against its
+// spread (a constant background: at mean/std = 3000 the unshifted sums lost 3e-3 of the variance).  K_c is the same
+// for every block of an image, so the segmented and single-image results stay bit-identical.
 // Segmented form (several images of npix pixels each, one U-Net batch with per-image statistics): blockIdx.y is the
 // image; image k sweeps its own pixels with the block partition a single-image call uses, and every per-channel,
 // per-image array ([nseg][C]) is offset by k, so each image's numbers are bit-identical to a call on that image.
@@ -109,10 +113,11 @@ bn_stats_kernel(int64_t npix, int C, const float* __restrict__ x, int64_t ldx, c
   const int64_t per = (npix + gridDim.x - 1) / gridDim.x;
   const int64_t p0 = (int64_t)blockIdx.x * per, p1 = p0 + per < npix ? p0 + per : npix;
   double a[VEC], b[VEC];
-  float mu[VEC], is[VEC], ga[VEC], be[VEC];
+  float mu[VEC], is[VEC], ga[VEC], be[VEC], kk[VEC];
 #pragma unroll
   for (int j = 0; j < VEC; ++j) {
     a[j] = 0.0; b[j] = 0.0;
+    kk[j] = (!BWD && c0 + j < C) ? x[c0 + j] : 0.f;     // the forward's shift K_c
     mu[j] = (BWD && c0 + j < C) ? mean[c0 + j] : 0.f;
     is[j] = (BWD && c0 + j < C) ? invstd[c0 + j] : 0.f;
     ga[j] = (BWD && !y && c0 + j < C) ? gamma[c0 + j] : 0.f;
@@ -136,15 +141,16 @@ bn_stats_kernel(int64_t npix, int C, const float* __restrict__ x, int64_t ldx, c
           sa[j] += gg;
           sb[j] = fmaf(gg, (xv[j] - mu[j]) * is[j], sb[j]);
         } else {
-          sa[j] += xv[j];
-          sb[j] = fmaf(xv[j], xv[j], sb[j]);
+          const float d = xv[j] - kk[j];
+          sa[j] += d;
+          sb[j] = fmaf(d, d, sb[j]);
         }
       }
     };
     if constexpr (VEC == 4) {
       // four pixels per iteration, every load issued before the first use: all loads of an iteration in flight together
       constexpr int U = 2;
-      const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+      const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f), k4 = make_float4(kk[0], kk[1], kk[2], kk[3]);
       int it = 0;
       for (int64_t p = p0 + pl; p < p1; p += (int64_t)U * lanes) {
         float4 tx[U], tg[U], ty[U];
@@ -152,7 +158,7 @@ bn_stats_kernel(int64_t npix, int C, const float* __restrict__ x, int64_t ldx, c
         for (int u = 0; u < U; ++u) {
           const int64_t pu = p + (int64_t)u * lanes;
           const bool on = pu < p1;                       // a skipped pixel contributes exact zeros
-          tx[u] = on ? ld4_stream(x + pu * ldx + c0) : z4;
+          tx[u] = on ? ld4_stream(x + pu * ldx + c0) : k4;
           tg[u] = (BWD && on) ? ld4_stream(dy + pu * lddy + c0) : z4;
           ty[u] = (BWD && y && on) ? ld4_stream(y + pu * ldy + c0) : z4;
         }
@@ -207,9 +213,9 @@ __device__ __forceinline__ void bn_block_sum2(double& a, double& b) {
 
 __global__ void __launch_bounds__(256)
 bn_finalize_kernel(int64_t npix, int64_t C, int nblk, int nseg, const double* __restrict__ part,
-                   float* __restrict__ running_mean, float* __restrict__ running_var,
-                   float momentum, float eps, float* __restrict__ save_mean,
-                   float* __restrict__ save_invstd) {
+                   const float* __restrict__ shift_x, int64_t ldx, float* __restrict__ running_mean,
+                   float* __restrict__ running_var, float momentum, float eps, float* __restrict__ save_mean,
+                   float* __restrict__ save_invstd) {   // shift_x: the images whose first pixel shifted the sums, or NULL
   const int c = blockIdx.x;
   // images in order: the running statistics see image 0's update first, as nseg single-image calls would
   for (int k = 0; k < nseg; ++k) {
@@ -218,8 +224,9 @@ bn_finalize_kernel(int64_t npix, int64_t C, int nblk, int nseg, const double* __
     for (int i = threadIdx.x; i < nblk; i += 256) { a += pk[((int64_t)i * C + c) * 2]; b += pk[((int64_t)i * C + c) * 2 + 1]; }
     bn_block_sum2(a, b);
     if (threadIdx.x == 0) {
-      const double mean = a / (double)npix;
-      double var = b / (double)npix - mean * mean;
+      const double m1 = a / (double)npix;              // mean of x - K_c
+      const double mean = (shift_x ? (double)shift_x[(int64_t)k * npix * ldx + c] : 0.0) + m1;
+      double var = b / (double)npix - m1 * m1;
       if (var < 0.0) var = 0.0;
       save_mean[k * C + c] = (float)mean;
       save_invstd[k * C + c] = (float)(1.0 / sqrt(var + (double)eps));
@@ -716,8 +723,8 @@ int bn_relu_forward_impl(int64_t nseg, int64_t npix, int64_t C, const float* x, 
     else bn_stats_kernel<1, false><<<sgrid, BN_THREADS, sh, ST>>>(npix, (int)C, x, ldx, nullptr, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr, part);
     TM_TRY(check_launch("bn_stats"));
   }
-  bn_finalize_kernel<<<(unsigned)C, 256, 0, ST>>>(npix, C, nfin, (int)nseg, part, running_mean, running_var,
-                                                             momentum, eps, save_mean, save_invstd);
+  bn_finalize_kernel<<<(unsigned)C, 256, 0, ST>>>(npix, C, nfin, (int)nseg, part, stats_part ? nullptr : x, ldx,
+                                                  running_mean, running_var, momentum, eps, save_mean, save_invstd);
   TM_TRY(check_launch("bn_finalize"));
   if (v4) bn_relu_apply_kernel<4><<<dim3(blocks_for(npix * (C / 4)), (unsigned)nseg), 256, 0, ST>>>(npix, (int)C, x, ldx, gamma, beta, save_mean, save_invstd, y, ldy, (__nv_bfloat16*)y_bf16);
   else bn_relu_apply_kernel<1><<<dim3(blocks_for(npix * C), (unsigned)nseg), 256, 0, ST>>>(npix, (int)C, x, ldx, gamma, beta, save_mean, save_invstd, y, ldy, (__nv_bfloat16*)y_bf16);

@@ -2,6 +2,7 @@
 
 precision 3 (3xTF32, the default) and 2 (bf16 x6) must meet the fp32 bar (rtol 1e-3; checked much tighter here);
 precision 1 (split bf16 x3) rtol 1e-3; precision 0 (plain bf16) and 4 (single TF32) the bf16 bar (rtol 2e-2)."""
+import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
@@ -319,3 +320,151 @@ def test_rowdot(lib, M, K, gather, relu):
     got = out[cr.long(), 0] if gather else out[:M, 0]
     assert_close(got, ref, 1e-5, 1e-5, "rowdot")
     assert bool((out[:, 1] == 4.0).all())
+
+
+def _mlp_inputs(M, kx, hid, nout, seed, n_src):
+    """Rows as mlp_alpha and fc_net_self see them: integer level ids in [0, 200] in half of the rows, floats of
+    magnitude 1e-3 .. 50 in the others.  Hidden units 0 .. 7 read only the first input with W1 = 0.5 and
+    b1 = -0.5 x0 for an integer x0: their pre-activation is exactly 0 on every row whose first input is x0."""
+    g = torch.Generator(device=DEV).manual_seed(seed)
+    X = torch.randint(0, 201, (n_src, kx), device=DEV, generator=g).float()
+    fl = torch.rand(n_src, device=DEV, generator=g) < 0.5
+    scale = torch.logspace(-3, float(np.log10(50.0)), n_src, device=DEV)[torch.randperm(n_src, device=DEV, generator=g)]
+    X[fl] = (torch.randn(n_src, kx, device=DEV, generator=g) * scale[:, None])[fl]
+    X[::5, 0] = 0.0                                      # level 0 ...
+    X[1::5, 0] = 17.0                                    # ... and 17 on many rows
+    W1 = torch.randn(hid, kx, device=DEV, generator=g) * 0.5
+    b1 = torch.randn(hid, device=DEV, generator=g) * 0.3
+    W1[:8] = 0.0
+    W1[:8, 0] = 0.5
+    b1[:8] = -0.5 * torch.tensor([0.0, 17.0, 0.0, 17.0, 3.0, 200.0, 17.0, 0.0], device=DEV)
+    W2 = torch.randn(nout, hid, device=DEV, generator=g) * (1.0 / hid ** 0.5)
+    b2 = torch.randn(nout, device=DEV, generator=g) * 0.1
+    return X, W1, b1, W2, b2
+
+
+MLP_SHAPES = [(1, 64, 32), (1, 128, 64), (2, 256, 128)]
+
+
+@pytest.mark.parametrize("precision", [3, 4, 2, 1, 0])
+@pytest.mark.parametrize("kx,hid,nout", MLP_SHAPES)
+@pytest.mark.parametrize("M,gather", [(1, False), (77, True), (128, False), (129, True), (1350, False), (1350, True),
+                                      (40000, True)])
+def test_tc_mlp2_smallk_forward(lib, M, gather, kx, hid, nout, precision):
+    """tm_tc_mlp2_smallk_forward (Linear(kx, hid) -> ReLU -> Linear(hid, nout), hidden layer generated in the operand
+    loader): mlp_alpha's 1 -> 64 -> 32 and fc_net_self's 2 -> 256 -> 128 in every precision, against fp64, written
+    at column 256 of a strided buffer as the head writes it (pixel stride 288 for the 32-wide output); rows and
+    columns outside the output keep their sentinel."""
+    torch.manual_seed(M + hid + precision)
+    n_src, n_dst = M + 37, M + 11
+    X, W1, b1, W2, b2 = _mlp_inputs(M, kx, hid, nout, M + hid + precision, n_src)
+    xr = torch.randperm(n_src, device=DEV)[:M].int().contiguous() if gather else None
+    orow = torch.randperm(n_dst, device=DEV)[:M].int().contiguous() if gather else None
+    xs = X[xr.long()] if gather else X[:M]
+    ref = torch.relu(xs.double() @ W1.double().t() + b1.double()) @ W2.double().t() + b2.double()
+    col0 = 256
+    ldo = 288 if nout == 32 else col0 + nout + 16
+    buf = torch.full((n_dst, ldo), -5.0, device=DEV)
+    out = buf[:, col0:col0 + nout]
+    err = _err()
+    lib.call("tm_tc_mlp2_smallk_forward", M, hid, nout, X, kx, xr, kx, W1, b1, W2, b2, out, ldo, orow, precision, err,
+             lib.stream())
+    assert int(err.item()) == 0
+    rows = orow.long() if gather else torch.arange(M, device=DEV)
+    assert_close(out[rows], ref, *TOL[precision], "smallk forward")
+    touched = torch.zeros_like(buf, dtype=torch.bool)
+    touched[rows, col0:col0 + nout] = True
+    assert bool((buf[~touched] == -5.0).all()), "smallk forward wrote outside its rows / columns"
+
+
+@pytest.mark.parametrize("precision", [3, 4, 2, 1, 0])
+@pytest.mark.parametrize("kx,hid,nout", MLP_SHAPES)
+@pytest.mark.parametrize("R,gather", [(1, False), (77, True), (129, False), (1350, True), (40000, True)])
+def test_tc_mlp2_smallk_wgrad2(lib, R, gather, kx, hid, nout, precision):
+    """tm_tc_mlp2_smallk_wgrad2: dW2 = G[g_rows]^T relu(X[x_rows] W1^T + b1) with the hidden layer generated as the B
+    operand, rows of G scaled from 1e-5 to 1, against fp64; two calls give the same bits."""
+    torch.manual_seed(R + hid + precision)
+    n_src = R + 29
+    X, W1, b1, _, _ = _mlp_inputs(R, kx, hid, nout, R + 3 * hid + precision, n_src)
+    G = torch.randn(n_src, nout, device=DEV) * torch.logspace(-5, 0, n_src, device=DEV)[torch.randperm(n_src, device=DEV)][:, None]
+    xr = torch.randperm(n_src, device=DEV)[:R].int().contiguous() if gather else None
+    gr = torch.randperm(n_src, device=DEV)[:R].int().contiguous() if gather else None
+    xs = X[xr.long()] if gather else X[:R]
+    gs = G[gr.long()] if gather else G[:R]
+    ref = gs.double().t() @ torch.relu(xs.double() @ W1.double().t() + b1.double())
+    nb = lib.ws_bytes("tm_tc_gemm_tn_ws", nout, hid, R)
+    err = _err()
+    outs = []
+    for _ in range(2):
+        dW2 = torch.full((nout, hid), 3.0, device=DEV)
+        lib.call("tm_tc_mlp2_smallk_wgrad2", nout, hid, R, G, nout, gr, X, kx, xr, kx, W1, b1, dW2, precision,
+                 lib.workspace(nb, DEV), nb, err, lib.stream())
+        outs.append(dW2)
+    assert int(err.item()) == 0
+    assert_close(outs[0], ref, *TOL[precision], "smallk dW2")
+    assert torch.equal(outs[0], outs[1]), "smallk wgrad2 is not deterministic"
+
+
+@pytest.mark.parametrize("data", ["exact", "float"])
+@pytest.mark.parametrize("K", [32, 128])
+@pytest.mark.parametrize("N", [64, 256])
+@pytest.mark.parametrize("kx", [1, 2])
+@pytest.mark.parametrize("M,gather", [(129, True), (1350, False), (40000, True)])
+def test_tc_mlp1_bwd_fused(lib, M, gather, kx, N, K, data):
+    """tm_tc_mlp1_bwd_fused: db1 = sum dh, dW1 = dh^T X with dh = (G W2) * (pre > 0), the ReLU mask either rebuilt
+    from W1, b1 (H = NULL, the generated-hidden backward) or read from a stored H (ldh % 4 == 0), against fp64.
+    "exact": integer inputs, W1 and b1 multiples of 1/64, so every pre-activation is exact in fp32 and thousands of
+    them are exactly 0 (ReLU off, as torch.relu's gradient): both masks must equal the fp64 one, and the two calls
+    give the same bits.  "float": inputs of magnitude 1e-3 .. 50 (a gate within an ulp of 0 may go either way).
+    Two calls give the same bits."""
+    torch.manual_seed(M + N + K + kx)
+    n_src = M + 41
+    if data == "exact":
+        g = torch.Generator(device=DEV).manual_seed(M + N + K + kx)
+        X = torch.randint(-20, 201, (n_src, kx), device=DEV, generator=g).float()
+        W1 = torch.randint(-64, 65, (N, kx), device=DEV, generator=g).float() / 64
+        b1 = torch.randint(-640, 641, (N,), device=DEV, generator=g).float() / 64
+        W1[::3] = 0.5
+        b1[::3] = -0.5 * torch.randint(0, 20, (len(range(0, N, 3)),), device=DEV, generator=g).float()
+        X[::2, 0] = torch.randint(0, 20, (len(range(0, n_src, 2)),), device=DEV, generator=g).float()
+        if kx == 2:
+            W1[::3, 1] = 0.0
+    else:
+        X, W1, b1, _, _ = _mlp_inputs(M, kx, N, K, M + N + K, n_src)
+    W2 = torch.randn(K, N, device=DEV) / N ** 0.5
+    G = torch.randn(n_src, K, device=DEV)
+    G[::7] *= 1e-4
+    xr = torch.randperm(n_src, device=DEV)[:M].int().contiguous() if gather else None
+    gr = torch.randperm(n_src, device=DEV)[:M].int().contiguous() if gather else None
+    xs = X[xr.long()] if gather else X[:M]
+    gs = G[gr.long()] if gather else G[:M]
+    pre = xs.double() @ W1.double().t() + b1.double()
+    if data == "exact":
+        assert int((pre == 0).sum()) > M // 10, "the exact data lost its zero pre-activations"
+    dh = (gs.double() @ W2.double()) * (pre > 0)
+    ref_db, ref_dw = dh.sum(0), dh.t() @ xs.double()
+    ldh = N + 8
+    Hbuf = torch.full((M, ldh), float("nan"), device=DEV)
+    Hbuf[:, :N] = torch.relu(pre).float()                # the stored hidden layer: zero wherever pre <= 0
+    W2t = W2.t().contiguous()
+    nb = lib.ws_bytes("tm_tc_mlp1_bwd_ws", N)
+    err = _err()
+    res = {}
+    for mode in ("gen", "gen2", "stored"):
+        H = Hbuf if mode == "stored" else None
+        dW1 = torch.full((N, kx), 9.0, device=DEV)
+        db1 = torch.full((N,), 9.0, device=DEV)
+        lib.call("tm_tc_mlp1_bwd_fused", M, N, K, G, K, gr, W2t, H, ldh, X, kx, xr, kx, W1 if H is None else None,
+                 b1 if H is None else None, dW1, db1, lib.workspace(nb, DEV), nb, err, lib.stream())
+        res[mode] = (dW1, db1)
+    assert int(err.item()) == 0
+    bad = 0 if data == "exact" else 4                    # "float": a gate at |pre| ~ 1 ulp may go either way
+    for mode in ("gen", "stored"):
+        dW1, db1 = res[mode]
+        assert_close(db1, ref_db, 1e-4, 2e-5, f"{mode} db1", max_bad=bad)
+        assert_close(dW1, ref_dw, 1e-4, 2e-5, f"{mode} dW1", max_bad=2 * bad)
+    assert torch.equal(res["gen"][0], res["gen2"][0]) and torch.equal(res["gen"][1], res["gen2"][1]), \
+        "mlp1_bwd_fused is not deterministic"
+    if data == "exact":
+        assert torch.equal(res["gen"][0], res["stored"][0]) and torch.equal(res["gen"][1], res["stored"][1]), \
+            "the regenerated ReLU mask differs from the stored hidden layer's"
