@@ -566,6 +566,47 @@ int tm_conv3x3_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t 
                           void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * A6' (tf32x3 mode)  The A6 kernels with fp32-class operands: 3xTF32 products (hi*hi + hi*lo + lo*hi,
+ * lo = x - trunc_tf32(x)), the arithmetic of precision 3.  The operands are the fp32 activations read in
+ * place by TMA through their pixel stride (16-byte aligned rows; packed rows, P > 1, need compact rows);
+ * the lo planes are formed in shared memory, so no operand copy exists.  Weights packed in fp32.  Layers
+ * whose tiles leave SMs idle split K over taps and channel steps; the fp32 partials (workspace) are folded
+ * in a fixed order, so every call is deterministic.
+ * ---------------------------------------------------------------------------------- */
+/* 1 when forward and weight gradient take the shape (Cin -> Cout; the data gradient is the Cout -> Cin forward) */
+int tm_conv3x3_tf32_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout);
+/* pixels per packed row (rows of 32 fp32 channels); pack weights with it as for tm_conv3x3_bf16_pack */
+int tm_conv3x3_tf32_pack(int64_t W, int64_t Cin, int64_t Cout);
+/* the operand of tm_conv3x3_pack_bf16, fp32: q [9][P*Nc][P*KcP] */
+int tm_conv3x3_pack_f32(int64_t Cout, int64_t Cin, const float* w, float* q, int64_t P, int64_t KcP, int dgrad,
+                        void* stream);
+/* workspace of tm_conv3x3_tf32 (0: the launch is not split; only then may it take stats) */
+size_t tm_conv3x3_tf32_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t P);
+/* y[pix, 0:N] (row stride ldy) = act(bias + sum_{tap,c} x[pix + tap, c] * W[tap][n][c]); x fp32 rows of stride ldx.
+ * stats as for tm_conv3x3_bf16 (unsplit launches only). */
+int tm_conv3x3_tf32(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t P, const float* x, int64_t ldx,
+                    const float* wq, const float* bias, float* y, int64_t ldy, int flags, void* stats, void* ws,
+                    size_t ws_bytes, int* err, void* stream);
+size_t tm_conv3x3_tf32_wgrad_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout);
+/* dw[co][ci][ky][kx] (ci < Cin_real) = sum_pix dy[pix, co] * x[pix + (ky-1,kx-1), ci] */
+int tm_conv3x3_tf32_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cin_real, int64_t Cout,
+                          const float* x, int64_t ldx, const float* dy, int64_t lddy, float* dw, void* ws,
+                          size_t ws_bytes, int* err, void* stream);
+/* nn.ConvTranspose2d(k=2, s=2) as tm_convt2x2_bf16*: forward and data gradient take every convt2x2 shape; the
+ * weight gradient needs Cin, Cout multiples of 32 (Cin <= 128, Cout <= 64).  One workspace size for all three. */
+int tm_convt2x2_tf32_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout);
+int tm_convt2x2_tf32_wgrad_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout);
+int tm_convt2x2_pack_f32(int64_t Cin, int64_t Cout, const float* w, float* wf, float* wd, void* stream);
+size_t tm_convt2x2_tf32_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout);
+int tm_convt2x2_tf32(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const float* x, int64_t ldx,
+                     const float* wf, const float* bias, float* y, int64_t ldy, void* ws, size_t ws_bytes, int* err,
+                     void* stream);
+int tm_convt2x2_tf32_dgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const float* dy, int64_t lddy,
+                           const float* wd, float* dx, int64_t lddx, void* ws, size_t ws_bytes, int* err, void* stream);
+int tm_convt2x2_tf32_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const float* x, int64_t ldx,
+                           const float* dy, int64_t lddy, float* dw, void* ws, size_t ws_bytes, int* err, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * A7 (bf16 mode)  TMA-fed tcgen05 k x k convolutions (odd k <= 9, stride 1, zero padding k/2)
  * Replaces nn.Conv2d(32, 64, 7, 1, 3) and nn.Conv2d(64, 32, 9, 1, 4) of LayoutNet (src/model.py:227-243) and
  * their autograd (data + weight gradients) when the image branch runs with bf16 tensor-core operands.  The kernels

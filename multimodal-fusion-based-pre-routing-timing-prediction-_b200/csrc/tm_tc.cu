@@ -226,6 +226,16 @@ inline int conv_splits(int64_t M, int64_t N, int64_t K, int precision, int64_t* 
 }
 }  // namespace
 
+namespace tmk {
+namespace tc {
+int conv_split_fold(const float* part, int64_t M, int64_t N, int splits, const float* bias, int relu, float* y, int64_t ldy,
+                    cudaStream_t st) {
+  conv_split_reduce_kernel<<<(unsigned)cdiv(M * (N >> 2), 256), 256, 0, st>>>(part, M, N, splits, bias, relu, y, ldy);
+  return check_launch("conv_split_reduce");
+}
+}  // namespace tc
+}  // namespace tmk
+
 extern "C" size_t tm_tc_conv2d_splitk_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k, int precision) {
   int64_t kps;
   const int splits = conv_splits(B * H * W, Cout, k * k * Cin, precision, &kps);
@@ -259,9 +269,7 @@ extern "C" int tm_tc_conv2d_nhwc_splitk(int64_t B, int64_t H, int64_t W, int64_t
     default: TM_CONV_SPLIT_CASE(32); break;
   }
 #undef TM_CONV_SPLIT_CASE
-  conv_split_reduce_kernel<<<(unsigned)cdiv(M * (Cout >> 2), 256), 256, 0, st>>>(part, M, Cout, splits, bias,
-                                                                                  (flags & TM_EPI_RELU) ? 1 : 0, y, ldy);
-  return check_launch("conv_split_reduce");
+  return tc::conv_split_fold(part, M, Cout, splits, bias, (flags & TM_EPI_RELU) ? 1 : 0, y, ldy, st);
 }
 
 extern "C" size_t tm_tc_conv2d_wgrad_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k) {

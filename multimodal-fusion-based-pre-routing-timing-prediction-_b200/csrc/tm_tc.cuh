@@ -1532,5 +1532,10 @@ int launch(const AL& al, const BL& bl, const EP& ep, int64_t M, int64_t N, int64
 #undef TM_TC_CASE
 }
 
+// Y[m][0:N] (row stride ldy) = act(bias + sum_z P[z][m][0:N]): folds the fp32 partials of a K-split convolution in a
+// fixed order (deterministic); N % 4 == 0.
+int conv_split_fold(const float* part, int64_t M, int64_t N, int splits, const float* bias, int relu, float* y, int64_t ldy,
+                    cudaStream_t st);
+
 }  // namespace tc
 }  // namespace tmk

@@ -53,32 +53,37 @@ inline CUtensorMapSwizzle swizzle_for(int inner_bytes) {
                                                                             : CU_TENSOR_MAP_SWIZZLE_32B;
 }
 
-// bf16 [B][H][W][C] with a box of (boxC channels, TW, TH, TB)
+// [B][H][W][C] with a box of (boxC channels, TW, TH, TB); bf16 (esz 2) or fp32 (esz 4) elements, pixel stride ld
+// elements (0: C).  mn32: fp32 boxes of 32 channels read as MN-major operands -- 128-byte swizzle with 32-byte atoms,
+// the layout tcgen05 calls SWIZZLE_128B_BASE32B (descriptor layout type 1)
 int encode_act(CUtensorMap* m, const void* ptr, int64_t C, int64_t W, int64_t H, int64_t B, int boxC, int TW,
-               int TH, int TB, int step = 1) {   // step 2: every other pixel in W and H (transposed-conv gradients)
+               int TH, int TB, int step = 1, int esz = 2, int64_t ld = 0, bool mn32 = false) {   // step 2: every other pixel in W and H (transposed-conv gradients)
   EncodeTiledFn enc = encoder();
   if (!enc) return fail(TM_EINVAL, "cuTensorMapEncodeTiled is not available from the driver");
+  if (ld <= 0) ld = C;
   cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
+  cuuint64_t strides[3] = {(cuuint64_t)(ld * esz), (cuuint64_t)(W * ld * esz), (cuuint64_t)(H * W * ld * esz)};
   cuuint32_t box[4] = {(cuuint32_t)boxC, (cuuint32_t)(TW * step), (cuuint32_t)(TH * step), (cuuint32_t)TB};
   cuuint32_t es[4] = {1, (cuuint32_t)step, (cuuint32_t)step, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(boxC * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+  CUresult r = enc(m, esz == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4,
+                   const_cast<void*>(ptr), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   mn32 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : swizzle_for(boxC * esz), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(TM_EINVAL, "cuTensorMapEncodeTiled(activation) failed: %d", (int)r);
   return 0;
 }
 
-// bf16 [rows][C] with a box of (boxC, boxRows)
-int encode_2d(CUtensorMap* m, const void* ptr, int64_t C, int64_t rows, int boxC, int boxRows) {
+// [rows][C] with a box of (boxC, boxRows); bf16 (esz 2) or fp32 (esz 4)
+int encode_2d(CUtensorMap* m, const void* ptr, int64_t C, int64_t rows, int boxC, int boxRows, int esz = 2) {
   EncodeTiledFn enc = encoder();
   if (!enc) return fail(TM_EINVAL, "cuTensorMapEncodeTiled is not available from the driver");
   cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)C * 2};
+  cuuint64_t strides[1] = {(cuuint64_t)(C * esz)};
   cuuint32_t box[2] = {(cuuint32_t)boxC, (cuuint32_t)boxRows};
   cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(boxC * 2), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+  CUresult r = enc(m, esz == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
+                   const_cast<void*>(ptr), dims, strides, box, es,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(boxC * esz), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(TM_EINVAL, "cuTensorMapEncodeTiled(weights) failed: %d", (int)r);
   return 0;
@@ -170,12 +175,13 @@ struct Geom {
 
 inline bool pow2(int64_t v) { return v > 0 && (v & (v - 1)) == 0; }
 
-inline Geom make_geom(int64_t B, int64_t H, int64_t W) {
+// tiles of `tile` pixels (128: one MMA row block; the tf32x3 weight gradient also takes 64 / 32 per pipeline stage)
+inline Geom make_geom(int64_t B, int64_t H, int64_t W, int tile = 128) {
   Geom g;
   g.B = (int)B; g.H = (int)H; g.W = (int)W;
-  g.TW = (int)(W < 128 ? W : 128);
-  g.TH = (int)(H < 128 / g.TW ? H : 128 / g.TW);
-  g.TB = 128 / (g.TW * g.TH);
+  g.TW = (int)(W < tile ? W : tile);
+  g.TH = (int)(H < tile / g.TW ? H : tile / g.TW);
+  g.TB = tile / (g.TW * g.TH);
   g.tiles_x = (int)(W / g.TW);
   g.tiles_y = (int)(H / g.TH);
   g.ntiles = (int64_t)g.tiles_x * g.tiles_y * cdiv(B, g.TB);
@@ -192,6 +198,31 @@ constexpr int FWD_EPI_WARPS = 8;
 constexpr int FWD_THREADS = (2 + FWD_EPI_WARPS) * 32;
 constexpr uint32_t FWD_SMEM_BUDGET = 184 * 1024;
 
+// Operand formats.  FMT_BF16: one bf16 plane per operand, kind::f16.  FMT_TF32X3: fp32 operands read in place by TMA
+// (tcgen05.mma.kind::tf32 uses the upper 19 bits of each word, so the fp32 word is the "hi" operand); the residual
+// lo = x - trunc_tf32(x), exact in fp32, is formed in shared memory next to it, and every 32-byte K chunk issues
+// hi*hi + hi*lo + lo*hi into one fp32 accumulator -- the 3xTF32 product of tf_gemm_kernel (tm_tc.cuh).
+constexpr int FMT_BF16 = 0, FMT_TF32X3 = 1;
+// tf32x3 forward / data gradient: warps that form the lo planes of a stage once TMA has landed its hi planes
+constexpr int SPLIT_WARPS = 4;
+
+// lo = x - trunc_tf32(x) for the `bytes` of hi operand at st, written at st + lo_off.  Elementwise at the same
+// offset, so the lo plane has the hi plane's swizzled layout whatever the swizzle.
+__device__ __forceinline__ void split_lo(uint8_t* st, uint32_t bytes, uint32_t lo_off, int t, int nthr) {
+  const float4* hi = reinterpret_cast<const float4*>(st);
+  float4* lo = reinterpret_cast<float4*>(st + lo_off);
+#pragma unroll 4
+  for (int i = t; i < (int)(bytes >> 4); i += nthr) {
+    const float4 x = hi[i];
+    float4 l;
+    l.x = x.x - __uint_as_float(__float_as_uint(x.x) & TF32_MASK);
+    l.y = x.y - __uint_as_float(__float_as_uint(x.y) & TF32_MASK);
+    l.z = x.z - __uint_as_float(__float_as_uint(x.z) & TF32_MASK);
+    l.w = x.w - __uint_as_float(__float_as_uint(x.w) & TF32_MASK);
+    lo[i] = l;
+  }
+}
+
 struct ConvArgs {
   Geom g;                            // geometry in PACKED pixels (rows of P pixels)
   int Cin, N, stages;                // channels per packed row: Cin = P * cin, N = P * cout
@@ -199,6 +230,9 @@ struct ConvArgs {
   int ntaps, cscale, convt;          // taps (k*k / 4 / 1), coordinate scale of the input map, transposed-conv scatter epilogue
   signed char tdx[81], tdy[81];      // input offset of every tap (up to 9x9)
   uint32_t a_bytes, b_bytes, stage_bytes;
+  uint32_t hi_bytes;                 // FMT_TF32X3: offset of the lo planes inside a stage
+  int ksplit, kper;                  // FMT_TF32X3: K splits (k-steps kper each); split z writes y + z * zstride
+  int64_t zstride;
   float* y;
   int64_t ldy;
   const float* bias;
@@ -210,12 +244,16 @@ struct ConvArgs {
 // ------------------------------------------------------------------------------------------------
 // fprop / dgrad
 // ------------------------------------------------------------------------------------------------
-template <int CK>
-__global__ void __launch_bounds__(FWD_THREADS, 1)
+// FMT_TF32X3: CK fp32 channels per k-step (128- or 64-byte rows); a stage holds the hi planes of A and B (TMA) and,
+// hi_bytes further, their lo planes (SPLIT_WARPS warps).  ksplit > 1: work unit = (tile, K split), fp32 partials.
+template <int CK, int FMT>
+__global__ void __launch_bounds__(FWD_THREADS + (FMT == FMT_TF32X3 ? SPLIT_WARPS * 32 : 0), 1)
 conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmw, ConvArgs a) {
+  constexpr bool TF = FMT == FMT_TF32X3;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* ring = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   __shared__ __align__(8) uint64_t full_bar[CONV_MAX_STAGES], empty_bar[CONV_MAX_STAGES], acc_full[2], acc_empty[2];
+  __shared__ __align__(8) uint64_t lo_bar[TF ? CONV_MAX_STAGES : 1];   // TF: lo planes of the stage written
   __shared__ float epi_scr[FWD_EPI_WARPS][32 * 17];
   __shared__ double epi_stat[FWD_EPI_WARPS][STAT_MAX_N * 2];       // per epilogue warp: column sums / sums of squares (a.stats)
   __shared__ uint32_t tmem_base_s;
@@ -225,7 +263,10 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
   const uint32_t tmem_cols = 2 * N < 32 ? 32u : (uint32_t)(2 * N);
 
   if (tid == 0) {
-    for (int i = 0; i < NS; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
+    for (int i = 0; i < NS; ++i) {
+      mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1);
+      if (TF) mbar_init(&lo_bar[i], SPLIT_WARPS);
+    }
     mbar_init(&acc_full[0], 1); mbar_init(&acc_full[1], 1);
     mbar_init(&acc_empty[0], FWD_EPI_WARPS); mbar_init(&acc_empty[1], FWD_EPI_WARPS);
     abort_s = 0;
@@ -242,17 +283,31 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
   bool ok = true;
   const int64_t G = gridDim.x;
   const int csteps = a.Cin / CK;
+  const int ksteps = a.ntaps * csteps;
+  const int64_t nunits = TF ? a.g.ntiles * a.ksplit : a.g.ntiles;
+  // work unit u -> tile t, K split z, k-steps [k0, k1)
+  auto unit = [&](int64_t u, int64_t& t, int& z, int& k0, int& k1) {
+    if (TF) {
+      t = u / a.ksplit; z = (int)(u - t * a.ksplit);
+      k0 = z * a.kper; k1 = k0 + a.kper < ksteps ? k0 + a.kper : ksteps;
+    } else {
+      t = u; z = 0; k0 = 0; k1 = ksteps;
+    }
+  };
 
   if (warp == 0) {
     // ======================= TMA producer =======================
     if (lane == 0) {
       uint32_t s = 0, ph = 0;
-      for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G) {
+      for (int64_t u = blockIdx.x; u < nunits && ok; u += G) {
+        int64_t t; int z, k0, k1;
+        unit(u, t, z, k0, k1);
         int x0, y0, b0;
         a.g.origin(t, x0, y0, b0);
         for (int tap = 0; tap < a.ntaps && ok; ++tap) {
           const int dx = a.tdx[tap], dy = a.tdy[tap];
           for (int cs = 0; cs < csteps; ++cs) {
+            if (TF && (tap * csteps + cs < k0 || tap * csteps + cs >= k1)) continue;
             ok = mbar_wait(&empty_bar[s], ph ^ 1u, abortp);
             if (!ok) break;
             const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
@@ -268,27 +323,37 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
   } else if (warp == 1) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      const uint32_t idesc = idesc_bf16(N, false, false);
-      constexpr uint32_t TY = sw_type(CK * 2), SBO = 8u * CK * 2u;
+      const uint32_t idesc = TF ? make_idesc_tf32(N, false, false) : idesc_bf16(N, false, false);
+      constexpr int RB = CK * (TF ? 4 : 2);                 // bytes per operand row; one MMA takes 32 of them
+      constexpr uint32_t TY = sw_type(RB), SBO = 8u * RB;
       uint32_t s = 0, ph = 0;
       int li = 0;
-      for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G, ++li) {
+      for (int64_t u = blockIdx.x; u < nunits && ok; u += G, ++li) {
+        int64_t t; int z, k0, k1;
+        unit(u, t, z, k0, k1);
         const int buf = li & 1;
         ok = mbar_wait(&acc_empty[buf], (((uint32_t)(li >> 1)) & 1u) ^ 1u, abortp);
         if (!ok) break;
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + (uint32_t)(buf * N);
-        const int ksteps = a.ntaps * csteps;
-        for (int ks = 0; ks < ksteps; ++ks) {
-          ok = mbar_wait(&full_bar[s], ph, abortp);
+        for (int ks = k0; ks < k1; ++ks) {
+          ok = mbar_wait(TF ? &lo_bar[s] : &full_bar[s], ph, abortp);
           if (!ok) break;
           tc_fence_after();
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
 #pragma unroll
-          for (int j = 0; j < CK / 16; ++j) {
+          for (int j = 0; j < RB / 32; ++j) {
             const uint64_t da = make_desc_sw(base + j * 32, 16, SBO, TY);
             const uint64_t db = make_desc_sw(base + a.a_bytes + j * 32, 16, SBO, TY);
-            umma(tmem_d, da, db, idesc, (ks > 0 || j > 0) ? 1u : 0u);
+            if (TF) {
+              const uint64_t dal = make_desc_sw(base + a.hi_bytes + j * 32, 16, SBO, TY);
+              const uint64_t dbl = make_desc_sw(base + a.hi_bytes + a.a_bytes + j * 32, 16, SBO, TY);
+              umma_tf32(tmem_d, da, db, idesc, (ks > k0 || j > 0) ? 1u : 0u);
+              umma_tf32(tmem_d, da, dbl, idesc, 1u);
+              umma_tf32(tmem_d, dal, db, idesc, 1u);
+            } else {
+              umma(tmem_d, da, db, idesc, (ks > k0 || j > 0) ? 1u : 0u);
+            }
           }
           umma_commit(&empty_bar[s]);
           if (++s == (uint32_t)NS) { s = 0; ph ^= 1u; }
@@ -298,6 +363,23 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
       }
     }
     __syncwarp();
+  } else if (TF && warp >= 2 + FWD_EPI_WARPS) {
+    // ======================= lo planes (tf32x3) =======================
+    const int rt = tid - (2 + FWD_EPI_WARPS) * 32;
+    uint32_t s = 0, ph = 0;
+    for (int64_t u = blockIdx.x; u < nunits && ok; u += G) {
+      int64_t t; int z, k0, k1;
+      unit(u, t, z, k0, k1);
+      for (int ks = k0; ks < k1; ++ks) {
+        ok = mbar_wait(&full_bar[s], ph, abortp);
+        if (!ok) break;
+        split_lo(ring + (size_t)s * a.stage_bytes, a.a_bytes + a.b_bytes, a.hi_bytes, rt, SPLIT_WARPS * 32);
+        fence_async_smem();                                // generic stores -> async proxy (the MMAs)
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&lo_bar[s]);
+        if (++s == (uint32_t)NS) { s = 0; ph ^= 1u; }
+      }
+    }
   } else {
     // ======================= epilogue =======================
     const int q = warp & 3;                               // TMEM lane quarter this warp may read
@@ -309,7 +391,10 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
       __syncwarp();
     }
     int li = 0;
-    for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G, ++li) {
+    for (int64_t u = blockIdx.x; u < nunits && ok; u += G, ++li) {
+      int64_t t; int z, k0, k1;
+      unit(u, t, z, k0, k1);
+      float* const yz = TF ? a.y + z * a.zstride : a.y;
       const int buf = li & 1;
       ok = mbar_wait(&acc_full[buf], ((uint32_t)(li >> 1)) & 1u, abortp);
       if (!ok) break;
@@ -323,11 +408,11 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
         const int tw = m % a.g.TW, th = (m / a.g.TW) % a.g.TH, tb = m / (a.g.TW * a.g.TH);
         if (a.convt)       // transposed conv k2 s2: the row is the 2x2 output window of input pixel (y0+th, x0+tw)
           rowp[pass] = b0 + tb < a.g.B
-                           ? a.y + (((int64_t)(b0 + tb) * 2 * a.g.H + 2 * (y0 + th)) * 2 * a.g.W + 2 * (x0 + tw)) * a.ldy
+                           ? yz + (((int64_t)(b0 + tb) * 2 * a.g.H + 2 * (y0 + th)) * 2 * a.g.W + 2 * (x0 + tw)) * a.ldy
                            : nullptr;
         else
           rowp[pass] = b0 + tb < a.g.B
-                           ? a.y + (((int64_t)(b0 + tb) * a.g.H + (y0 + th)) * a.g.W + (x0 + tw)) * a.P * a.ldy
+                           ? yz + (((int64_t)(b0 + tb) * a.g.H + (y0 + th)) * a.g.W + (x0 + tw)) * a.P * a.ldy
                            : nullptr;
       }
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * N);
@@ -568,16 +653,22 @@ struct WgradArgs {
   int cscale;                        // coordinate scale of the tapped map (2: transposed-conv gradient, every other pixel)
   signed char tdx[4], tdy[4];        // NT == 4: offsets of the four taps (transposed conv); NT == 3 / 1 / 0 use (s - k/2, r - k/2)
   int k, tg, groups;                 // NT == 0 (k x k): kernel size, taps per group, groups per kernel row
+  uint32_t hi_bytes;                 // FMT_TF32X3: offset of the lo planes inside a stage
+  int tp;                            // FMT_TF32X3: pixels per stage (128 / 64 / 32: the tile of a.g)
 };
 
 // NT: tapped tiles per stage -- 4: transposed conv; 3: a 3x3 kernel row fused; 1: one tap per stage; 0: k x k, a group
 // of a kernel row's taps fused (runtime k / tg / groups; NT == 3 is this with k = tg = 3 as compile-time constants)
-template <int NT>
+// FMT_TF32X3: fp32 boxes of 32 channels, MN-major SWIZZLE_128B_BASE32B; a.tp pixels per stage; the epilogue warps,
+// idle until the last MMA, form each stage's lo planes first.
+template <int NT, int FMT>
 __global__ void __launch_bounds__(CONV_THREADS, 1)
 conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constant__ CUtensorMap tmdy, WgradArgs a) {
+  constexpr bool TF = FMT == FMT_TF32X3;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* ring = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   __shared__ __align__(8) uint64_t full_bar[CONV_MAX_STAGES], empty_bar[CONV_MAX_STAGES], acc_full;
+  __shared__ __align__(8) uint64_t lo_bar[TF ? CONV_MAX_STAGES : 1];
   __shared__ uint32_t tmem_base_s;
   __shared__ int abort_s;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -597,7 +688,10 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
   while (tmem_cols < (uint32_t)((KXK ? a.tg : NTOT) * Cin)) tmem_cols <<= 1;
 
   if (tid == 0) {
-    for (int i = 0; i < NS; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
+    for (int i = 0; i < NS; ++i) {
+      mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1);
+      if (TF) mbar_init(&lo_bar[i], 4);
+    }
     mbar_init(&acc_full, 1);
     abort_s = 0;
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -642,7 +736,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
     __syncwarp();
   } else if (warp == 1) {
     if (lane == 0) {
-      const uint32_t idesc = idesc_bf16(Cin, true, true);
+      const uint32_t idesc = TF ? make_idesc_tf32(Cin, true, true) : idesc_bf16(Cin, true, true);
       // MN-major operand tiles: pixel row k at k * (cb*2) bytes; 8-pixel groups at SBO; the next 64-channel box at LBO
       const uint32_t a_ty = sw_type(a.cby * 2), b_ty = sw_type(a.cbx * 2);
       const uint32_t a_sbo = 8u * a.cby * 2u, b_sbo = 8u * a.cbx * 2u;
@@ -652,11 +746,29 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
       bool first = true;
       for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G) {
         for (int st = 0; st < STEPS && ok; ++st) {
-          ok = mbar_wait(&full_bar[s], ph, abortp);
+          ok = mbar_wait(TF ? &lo_bar[s] : &full_bar[s], ph, abortp);
           if (!ok) break;
           tc_fence_after();
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
-          if (NT != 1) {
+          if (TF) {
+            // 32-channel boxes of tp pixels x 128 bytes: 4-pixel groups at SBO = 512, 8 pixels (one MMA) = 1024 bytes,
+            // the next 32 channels (box) at LBO; the tapped tiles' boxes are uniformly spaced, so NT != 1 is again ONE
+            // MMA of nload * Cin columns.  LBO 0: a single box, re-read for M rows beyond Cout (never stored).
+            const uint32_t box_y = a.dy_bytes / a.nby, box_x = a.x_bytes / a.nbx;
+            const uint32_t lbo_y = a.nby > 1 ? box_y : 0u;
+            const uint32_t idn = NT != 1 ? make_idesc_tf32(nload * Cin, true, true) : idesc;
+            const uint32_t tmem_d = tmem_base + (uint32_t)(NT != 1 ? 0 : st * Cin);
+            const uint32_t xb = base + a.dy_bytes;
+            for (int j = 0; j < a.tp / 8; ++j) {
+              const uint64_t da = make_desc_sw(base + j * 1024, lbo_y, 512, 1);
+              const uint64_t db = make_desc_sw(xb + j * 1024, box_x, 512, 1);
+              const uint64_t dal = make_desc_sw(base + a.hi_bytes + j * 1024, lbo_y, 512, 1);
+              const uint64_t dbl = make_desc_sw(xb + a.hi_bytes + j * 1024, box_x, 512, 1);
+              umma_tf32(tmem_d, da, db, idn, (!first || j > 0) ? 1u : 0u);
+              umma_tf32(tmem_d, da, dbl, idn, 1u);
+              umma_tf32(tmem_d, dal, db, idn, 1u);
+            }
+          } else if (NT != 1) {
             // the tapped tiles are one MN-major operand of nload * Cin columns (tile stride = leading byte
             // offset), their accumulators neighbours in TMEM: ONE MMA per 16 pixels instead of nload
             const uint32_t idesc3 = idesc_bf16(nload * Cin, true, true);
@@ -687,7 +799,22 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
   } else {
     const int q = warp & 3;
     const int co = q * 32 + lane;
-    ok = mbar_wait(&acc_full, 0, abortp);
+    if (TF) {
+      // lo planes of every stage of this CTA, in the producer's order
+      uint32_t s = 0, ph = 0;
+      for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G) {
+        for (int st = 0; st < STEPS && ok; ++st) {
+          ok = mbar_wait(&full_bar[s], ph, abortp);
+          if (!ok) break;
+          split_lo(ring + (size_t)s * a.stage_bytes, a.dy_bytes + nload * a.x_bytes, a.hi_bytes, tid - 64, 128);
+          fence_async_smem();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&lo_bar[s]);
+          if (++s == (uint32_t)NS) { s = 0; ph ^= 1u; }
+        }
+      }
+    }
+    if (ok) ok = mbar_wait(&acc_full, 0, abortp);
     if (ok) {
       tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);
@@ -770,8 +897,11 @@ __global__ void to_bf16_kernel(int64_t npix, int C, const float* __restrict__ x,
 //   the output / input row; the entry is the tap s = S*P + pi - po + ks/2 of kernel row r when 0 <= s < ks, else 0.
 //   dgrad == 0: n = output channel co, k = input channel ci                    (forward operand)
 //   dgrad == 1: n = ci, k = co, taps reversed (r, s) -> (ks-1-r, ks-1-s)       (data-gradient operand)
-__global__ void pack_w_bf16_kernel(int Cout, int Cin, int ks, const float* __restrict__ w, __nv_bfloat16* __restrict__ q,
-                                   int P, int KcP, int dgrad) {
+__device__ __forceinline__ void put(__nv_bfloat16* q, int64_t i, float v) { q[i] = __float2bfloat16(v); }
+__device__ __forceinline__ void put(float* q, int64_t i, float v) { q[i] = v; }
+template <typename T>
+__global__ void pack_w_kernel(int Cout, int Cin, int ks, const float* __restrict__ w, T* __restrict__ q, int P, int KcP,
+                              int dgrad) {
   const int Nc = dgrad ? Cin : Cout, Kc = dgrad ? Cout : Cin;
   const int64_t ldk = (int64_t)P * KcP, rows = (int64_t)P * Nc;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -786,7 +916,7 @@ __global__ void pack_w_bf16_kernel(int Cout, int Cin, int ks, const float* __res
     const int tap = dgrad ? (ks - 1 - r) * ks + (ks - 1 - sx) : r * ks + sx;
     v = w[((int64_t)co * Cin + ci) * ks * ks + tap];
   }
-  q[i] = __float2bfloat16(v);
+  put(q, i, v);
 }
 
 inline bool conv_shape_ok(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N) {
@@ -836,7 +966,7 @@ extern "C" int tm_conv3x3_pack_bf16(int64_t Cout, int64_t Cin, const float* w, v
                                     void* stream) {
   TM_REQUIRE(P >= 1 && KcP >= (dgrad ? Cout : Cin), "tm_conv3x3_pack_bf16: bad packing");
   const int64_t n = 9 * P * (dgrad ? Cin : Cout) * P * KcP;
-  pack_w_bf16_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, 3, w, (__nv_bfloat16*)q,
+  pack_w_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, 3, w, (__nv_bfloat16*)q,
                                                                              (int)P, (int)KcP, dgrad);
   return check_launch("pack_w_bf16");
 }
@@ -914,11 +1044,11 @@ int launch_taps(const ConvArgs& a, const CUtensorMap& tmx, const CUtensorMap& tm
   do {                                                                                                        \
     static bool optin = false;                                                                                \
     if (!optin) {                                                                                             \
-      TM_CUDA(cudaFuncSetAttribute(conv3x3_tma_kernel<CK_>, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
+      TM_CUDA(cudaFuncSetAttribute(conv3x3_tma_kernel<CK_, FMT_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
                                    (int)FWD_SMEM_BUDGET + 1024));                                             \
       optin = true;                                                                                           \
     }                                                                                                         \
-    conv3x3_tma_kernel<CK_><<<grid, FWD_THREADS, smem, st>>>(tmx, tmw, a);                                    \
+    conv3x3_tma_kernel<CK_, FMT_BF16><<<grid, FWD_THREADS, smem, st>>>(tmx, tmw, a);                                    \
   } while (0)
   if (CK == 64) TM_LAUNCH_CONV(64);
   else if (CK == 32) TM_LAUNCH_CONV(32);
@@ -927,20 +1057,20 @@ int launch_taps(const ConvArgs& a, const CUtensorMap& tmx, const CUtensorMap& tm
   return check_launch("conv_tma");
 }
 
-__global__ void pack_convt_bf16_kernel(int Cin, int Cout, const float* __restrict__ w, __nv_bfloat16* __restrict__ wf,
-                                       __nv_bfloat16* __restrict__ wd) {
+template <typename T>
+__global__ void pack_convt_kernel(int Cin, int Cout, const float* __restrict__ w, T* __restrict__ wf, T* __restrict__ wd) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (int64_t)Cin * Cout * 4) return;
   const int q = (int)(i % 4), co = (int)((i / 4) % Cout), ci = (int)(i / (4 * Cout));   // w[ci][co][dy][dx], q = dy*2+dx
-  const __nv_bfloat16 v = __float2bfloat16(w[i]);
-  if (wf) wf[((int64_t)q * Cout + co) * Cin + ci] = v;         // forward operand  [(q,co)][ci]
-  if (wd) wd[((int64_t)q * Cin + ci) * Cout + co] = v;         // data-gradient operand, tap q: [ci][co]
+  const float v = w[i];
+  if (wf) put(wf, ((int64_t)q * Cout + co) * Cin + ci, v);     // forward operand  [(q,co)][ci]
+  if (wd) put(wd, ((int64_t)q * Cin + ci) * Cout + co, v);     // data-gradient operand, tap q: [ci][co]
 }
 }  // namespace
 
 // nn.ConvTranspose2d(k=2, s=2) weight w [Cin][Cout][2][2] fp32 -> wf bf16 [4*Cout][Cin], wd bf16 [4][Cin][Cout]
 extern "C" int tm_convt2x2_pack_bf16(int64_t Cin, int64_t Cout, const float* w, void* wf, void* wd, void* stream) {
-  pack_convt_bf16_kernel<<<(unsigned)cdiv(Cin * Cout * 4, 256), 256, 0, (cudaStream_t)stream>>>((int)Cin, (int)Cout, w,
+  pack_convt_kernel<<<(unsigned)cdiv(Cin * Cout * 4, 256), 256, 0, (cudaStream_t)stream>>>((int)Cin, (int)Cout, w,
                                                                                               (__nv_bfloat16*)wf, (__nv_bfloat16*)wd);
   return check_launch("pack_convt_bf16");
 }
@@ -1068,10 +1198,10 @@ extern "C" int tm_convt2x2_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t C
   cudaStream_t st = (cudaStream_t)stream;
   static bool optin = false;
   if (!optin) {
-    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
+    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<4, FMT_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
     optin = true;
   }
-  conv3x3_wgrad_tma_kernel<4><<<dim3((unsigned)splits, 1), CONV_THREADS, smem, st>>>(tm_tap, tm_m, a);
+  conv3x3_wgrad_tma_kernel<4, FMT_BF16><<<dim3((unsigned)splits, 1), CONV_THREADS, smem, st>>>(tm_tap, tm_m, a);
   TM_TRY(check_launch("convt_wgrad_tma"));
   convt_wgrad_reduce_kernel<<<(unsigned)cdiv(4 * Cin * Cout, 256), 256, 0, st>>>(a.part, splits, (int)Cin, (int)Cout, dw);
   return check_launch("convt_wgrad_reduce");
@@ -1111,16 +1241,339 @@ extern "C" int tm_conv3x3_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Ci
   dim3 grid((unsigned)splits, 3);
   static bool optin = false;
   if (!optin) {
-    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
-    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
+    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<3, FMT_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
+    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<1, FMT_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
     optin = true;
   }
-  if (NT == 3) conv3x3_wgrad_tma_kernel<3><<<grid, CONV_THREADS, smem, st>>>(tmx, tmdy, a);
-  else conv3x3_wgrad_tma_kernel<1><<<grid, CONV_THREADS, smem, st>>>(tmx, tmdy, a);
+  if (NT == 3) conv3x3_wgrad_tma_kernel<3, FMT_BF16><<<grid, CONV_THREADS, smem, st>>>(tmx, tmdy, a);
+  else conv3x3_wgrad_tma_kernel<1, FMT_BF16><<<grid, CONV_THREADS, smem, st>>>(tmx, tmdy, a);
   TM_TRY(check_launch("conv3x3_wgrad_tma"));
   const int64_t n = 9 * Cout * Cin_real;
   wgrad_reduce_kernel<3><<<(unsigned)cdiv(n * 32, 256), 256, 0, st>>>(a.part, splits, P, (int)Cout, (int)Cin, (int)Cin_real, 3, dw);
   return check_launch("wgrad_reduce");
+}
+
+// ------------------------------------------------------------------------------------------------
+// tf32x3 (fp32-class) forms of the 3x3 and transposed convolutions: the kernels above with FMT_TF32X3.  The operands
+// are the fp32 activations themselves, read in place through their pixel stride; the weights are packed in fp32.
+// Rows of 32 fp32 channels are 128 bytes, so narrow layers pack P = 2 pixels per row (16 channels), not 4.
+// ------------------------------------------------------------------------------------------------
+namespace {
+inline int conv_pack_f32(int64_t W, int64_t cin, int64_t cout) {
+  int P = 1;
+  while (P * cin < 32 && 2 * P <= W && 2 * P * cout <= 256) P *= 2;
+  return P;
+}
+inline int wgrad_pack_f32(int64_t W, int64_t cin, int64_t cout) {
+  const int64_t lo = cin < cout ? cin : cout, hi = cin < cout ? cout : cin;
+  int P = 1;
+  while (P * lo < 32 && 2 * P <= W && 2 * P * hi <= 128) P *= 2;
+  return P;
+}
+// MN-major fp32 operands come in boxes of 32 channels (128 bytes; the only MN-major 32-bit layout tcgen05 takes)
+inline bool wgrad_f32_ok(int64_t Cp, int64_t Np) {
+  return Cp % 32 == 0 && Np % 32 == 0 && Cp <= 128 && Np <= 128 && pow2(Cp) && pow2(Np);
+}
+
+// Stage geometry of a forward / data-gradient launch (a.Cin = K, a.N set): CK fp32 channels per k-step, 32 (128-byte
+// rows) unless that leaves fewer than 3 stages -- then 16.  A stage is twice a bf16 stage of the same CK (hi and lo
+// planes), so the 184 KB ring holds 2-4 stages of CK = 32 (N = 128 / 64 / 32); N = 128 and the transposed
+// convolution's N = 256 run at CK = 16 with 5 / 3 stages.  K splits when the tiles leave SMs idle, as
+// tm_tc_conv2d_splitk_ws does: tiles x splits fills the GPU, at least two k-steps per split.  Returns the splits.
+int tf_plan(ConvArgs& a, int& CK) {
+  auto hi = [&](int ck) { return (uint32_t)(128 * ck * 4 + align_up((size_t)a.N * ck * 4, 1024)); };
+  CK = a.Cin >= 32 ? 32 : 16;
+  if (CK == 32 && FWD_SMEM_BUDGET / (2 * hi(32)) < 3) CK = 16;
+  a.a_bytes = 128u * CK * 4u;
+  a.b_bytes = (uint32_t)a.N * CK * 4u;
+  a.hi_bytes = hi(CK);
+  a.stage_bytes = 2 * a.hi_bytes;
+  const int ns = (int)(FWD_SMEM_BUDGET / a.stage_bytes);
+  a.stages = ns > CONV_MAX_STAGES ? CONV_MAX_STAGES : ns;
+  const int ksteps = a.ntaps * (a.Cin / CK);
+  a.ksplit = 1; a.kper = ksteps; a.zstride = 0;
+  int64_t want = (int64_t)sm_count() / a.g.ntiles;
+  if (want > ksteps / 2) want = ksteps / 2;
+  if (want >= 2) {
+    a.kper = (int)cdiv(ksteps, want);
+    a.ksplit = (int)cdiv(ksteps, a.kper);
+  }
+  return a.ksplit;
+}
+inline size_t tf_ws(ConvArgs a, int64_t mout) {
+  int CK;
+  const int splits = tf_plan(a, CK);
+  return splits > 1 ? (size_t)splits * mout * a.cpx * sizeof(float) + 256 : 0;
+}
+
+// a: geometry, channels, taps and stats set.  x: fp32 map (xC channels, xW x xH, pixel stride ldx elements; step 2:
+// every other pixel), wq: fp32 operand of wrows rows.  mout rows of a.cpx outputs; split launches write fp32 partials
+// into ws and fold them (fixed order) into y with the bias and ReLU.
+int run_tf32(ConvArgs a, const float* x, int64_t xC, int64_t xW, int64_t xH, int64_t ldx, int step, const float* wq,
+             int64_t wrows, int64_t mout, const float* bias, int relu, float* y, int64_t ldy, void* ws, size_t ws_bytes,
+             int* err, cudaStream_t st) {
+  TM_REQUIRE(ldx % 4 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(wq) % 16 == 0,
+             "tf32x3 convolution: operand rows must be 16-byte aligned");
+  TM_REQUIRE(ldy % 4 == 0 && reinterpret_cast<uintptr_t>(y) % 16 == 0, "tf32x3 convolution: output rows must be 16-byte aligned");
+  int CK;
+  const int splits = tf_plan(a, CK);
+  a.err = err;
+  float* part = nullptr;
+  if (splits > 1) {
+    TM_REQUIRE(!a.stats, "tf32x3 convolution: fused statistics need an unsplit launch");
+    TM_REQUIRE(ws && ws_bytes >= (size_t)splits * mout * a.cpx * sizeof(float) + 256, "tf32x3 convolution: workspace too small");
+    part = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+    a.y = part; a.ldy = a.cpx; a.zstride = mout * a.cpx;
+    a.bias = nullptr; a.flags = 0;
+  } else {
+    a.y = y; a.ldy = ldy; a.bias = bias;
+    a.flags = (relu ? TM_EPI_RELU : 0) | (bias ? TM_EPI_BIAS : 0);
+  }
+  if (a.stats) TM_CUDA(cudaMemsetAsync(a.stats, 0, tm_conv3x3_bf16_stats_bytes(a.cpx, a.P), st));   // slots of idle CTAs
+  CUtensorMap tmx, tmw;
+  TM_TRY(encode_act(&tmx, x, xC, xW, xH, a.g.B, CK, a.g.TW, a.g.TH, a.g.TB, step, 4, ldx));
+  TM_TRY(encode_2d(&tmw, wq, a.Cin, wrows, CK, a.N, 4));
+  const int64_t units = a.g.ntiles * a.ksplit;
+  const int grid = (int)(units < sm_count() ? units : sm_count());
+  const size_t smem = (size_t)a.stages * a.stage_bytes + 1024;
+  constexpr int threads = FWD_THREADS + SPLIT_WARPS * 32;
+#define TM_LAUNCH_TF(CK_)                                                                                     \
+  do {                                                                                                        \
+    static bool optin = false;                                                                                \
+    if (!optin) {                                                                                             \
+      TM_CUDA(cudaFuncSetAttribute(conv3x3_tma_kernel<CK_, FMT_TF32X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                   (int)FWD_SMEM_BUDGET + 1024));                                             \
+      optin = true;                                                                                           \
+    }                                                                                                         \
+    conv3x3_tma_kernel<CK_, FMT_TF32X3><<<grid, threads, smem, st>>>(tmx, tmw, a);                            \
+  } while (0)
+  if (CK == 32) TM_LAUNCH_TF(32);
+  else TM_LAUNCH_TF(16);
+#undef TM_LAUNCH_TF
+  TM_TRY(check_launch("conv_tma_tf32"));
+  if (splits > 1) return tc::conv_split_fold(part, mout, a.cpx, splits, bias, relu, y, ldy, st);
+  return 0;
+}
+
+ConvArgs conv3x3_args(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t P) {
+  ConvArgs a;
+  a.g = make_geom(B, H, W / P);
+  a.Cin = (int)(P * Cin); a.N = (int)(P * N); a.P = (int)P; a.cpx = (int)N;
+  a.ntaps = 9; a.cscale = 1; a.convt = 0;
+  for (int t = 0; t < 9; ++t) { a.tdx[t] = (signed char)(t % 3 - 1); a.tdy[t] = (signed char)(t / 3 - 1); }
+  a.stats = nullptr;
+  return a;
+}
+ConvArgs convt_args(int64_t B, int64_t H, int64_t W, int64_t K, int64_t N, int64_t cpx, int ntaps) {
+  ConvArgs a;
+  a.g = make_geom(B, H, W);
+  a.Cin = (int)K; a.N = (int)N; a.P = 1; a.cpx = (int)cpx;
+  a.ntaps = ntaps; a.cscale = ntaps == 4 ? 2 : 1; a.convt = ntaps == 1;
+  for (int q = 0; q < 4; ++q) { a.tdx[q] = (signed char)(ntaps == 4 ? q & 1 : 0); a.tdy[q] = (signed char)(ntaps == 4 ? q >> 1 : 0); }
+  a.stats = nullptr;
+  return a;
+}
+
+// weight-gradient stage geometry: tapped tiles per stage (3: a kernel row fused, when 3 * Cin <= 192; else 1) and
+// pixels per stage (128 / 64 / 32), the first that leaves at least 3 stages -- a tf32x3 stage is twice a bf16 stage
+// of the same pixels, and 128 pixels of a 128-channel layer would not fit twice
+void tf_wgrad_plan(WgradArgs& a, int64_t B, int64_t H, int64_t Wp, int nt_max, int& NT) {
+  const int nts[2] = {nt_max, nt_max == 3 ? 1 : nt_max};    // the transposed conv (4) has no one-tap form
+  for (int min_st = 3; min_st >= 2; --min_st)
+    for (int i = 0; i < 2; ++i) {
+      if (i == 1 && nts[1] == nts[0]) break;
+      for (int tp = 128; tp >= 32; tp >>= 1) {
+        const uint32_t hi = (uint32_t)align_up((size_t)tp * a.Cout * 4 + (size_t)nts[i] * tp * a.Cin * 4, 1024);
+        if (CONV_SMEM_BUDGET / (2 * hi) >= (uint32_t)min_st) {
+          NT = nts[i];
+          a.tp = tp;
+          a.g = make_geom(B, H, Wp, tp);
+          a.cbx = 32; a.nbx = a.Cin / 32;
+          a.cby = 32; a.nby = a.Cout / 32;
+          a.x_bytes = (uint32_t)tp * a.Cin * 4;
+          a.dy_bytes = (uint32_t)tp * a.Cout * 4;
+          a.hi_bytes = hi;
+          a.stage_bytes = 2 * hi;
+          const int ns = (int)(CONV_SMEM_BUDGET / a.stage_bytes);
+          a.stages = ns > CONV_MAX_STAGES ? CONV_MAX_STAGES : ns;
+          return;
+        }
+      }
+    }
+  NT = 0;   // no fit (not reached for Cin, Cout <= 128)
+}
+
+template <int NT>
+int launch_wgrad_tf32(const WgradArgs& a, const CUtensorMap& tmx, const CUtensorMap& tmdy, dim3 grid, cudaStream_t st) {
+  static bool optin = false;
+  if (!optin) {
+    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<NT, FMT_TF32X3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)CONV_SMEM_BUDGET + 1024));
+    optin = true;
+  }
+  conv3x3_wgrad_tma_kernel<NT, FMT_TF32X3><<<grid, CONV_THREADS, (size_t)a.stages * a.stage_bytes + 1024, st>>>(tmx, tmdy, a);
+  return check_launch("wgrad_tma_tf32");
+}
+}  // namespace
+
+extern "C" int tm_conv3x3_tf32_pack(int64_t W, int64_t Cin, int64_t Cout) { return conv_pack_f32(W, Cin, Cout); }
+
+extern "C" int tm_conv3x3_tf32_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  if (W <= 0 || Cin <= 0 || Cout <= 0 || Cin % 16 || Cout % 16) return 0;
+  const int P = conv_pack_f32(W, Cin, Cout), Pw = wgrad_pack_f32(W, Cin, Cout);
+  return conv_shape_ok(B, H, W / P, P * Cin, P * Cout) && conv_shape_ok(B, H, W / Pw, Pw * Cin, Pw * Cout) &&
+                 wgrad_f32_ok(Pw * Cin, Pw * Cout)
+             ? 1
+             : 0;
+}
+
+extern "C" int tm_conv3x3_pack_f32(int64_t Cout, int64_t Cin, const float* w, float* q, int64_t P, int64_t KcP, int dgrad,
+                                   void* stream) {
+  TM_REQUIRE(P >= 1 && KcP >= (dgrad ? Cout : Cin), "tm_conv3x3_pack_f32: bad packing");
+  const int64_t n = 9 * P * (dgrad ? Cin : Cout) * P * KcP;
+  pack_w_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, 3, w, q, (int)P, (int)KcP, dgrad);
+  return check_launch("pack_w_f32");
+}
+
+extern "C" size_t tm_conv3x3_tf32_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t P) {
+  if (P < 1 || W % P || !conv_shape_ok(B, H, W / P, P * Cin, P * N)) return 0;
+  return tf_ws(conv3x3_args(B, H, W, Cin, N, P), B * H * W);
+}
+
+extern "C" int tm_conv3x3_tf32(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t N, int64_t P, const float* x, int64_t ldx,
+                               const float* wq, const float* bias, float* y, int64_t ldy, int flags, void* stats, void* ws,
+                               size_t ws_bytes, int* err, void* stream) {
+  TM_REQUIRE(P >= 1 && W % P == 0 && conv_shape_ok(B, H, W / P, P * Cin, P * N),
+             "tm_conv3x3_tf32: unsupported shape (H, W powers of two; channels multiples of 16)");
+  TM_REQUIRE(P == 1 || ldx == Cin, "tm_conv3x3_tf32: packed rows (P > 1) need compact input rows (ldx == Cin)");
+  ConvArgs a = conv3x3_args(B, H, W, Cin, N, P);
+  if (stats) {
+    TM_REQUIRE(!bias && a.N <= STAT_MAX_N, "tm_conv3x3_tf32: fused statistics need no bias and P * N <= 128");
+    a.stats = (double*)stats;
+  }
+  return run_tf32(a, x, P * Cin, W / P, H, P * ldx, 1, wq, 9 * P * N, B * H * W, bias, flags & TM_EPI_RELU, y, ldy, ws,
+                  ws_bytes, err, (cudaStream_t)stream);
+}
+
+extern "C" size_t tm_conv3x3_tf32_wgrad_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  const int P = wgrad_pack_f32(W, Cin, Cout);
+  if (!wgrad_f32_ok(P * Cin, P * Cout)) return 0;
+  WgradArgs a;
+  a.Cin = (int)(P * Cin); a.Cout = (int)(P * Cout);
+  int NT;
+  tf_wgrad_plan(a, B, H, W / P, a.Cin <= 64 ? 3 : 1, NT);
+  return (size_t)wgrad_splits(a.g) * 9 * a.Cout * a.Cin * sizeof(float) + 256;
+}
+
+// dw[co][ci][ky][kx] (ci < Cin_real) = sum_pix dy[pix, co] * x[pix + (ky-1, kx-1), ci]; x, dy fp32 rows of stride ldx / lddy
+extern "C" int tm_conv3x3_tf32_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cin_real, int64_t Cout,
+                                     const float* x, int64_t ldx, const float* dy, int64_t lddy, float* dw, void* ws,
+                                     size_t ws_bytes, int* err, void* stream) {
+  TM_REQUIRE(tm_conv3x3_tf32_supported(B, H, W, Cin, Cout), "tm_conv3x3_tf32_wgrad: unsupported shape");
+  const int P = wgrad_pack_f32(W, Cin, Cout);
+  TM_REQUIRE(P == 1 || (ldx == Cin && lddy == Cout), "tm_conv3x3_tf32_wgrad: packed rows (P > 1) need compact rows");
+  TM_REQUIRE(ldx % 4 == 0 && lddy % 4 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(dy) % 16 == 0,
+             "tm_conv3x3_tf32_wgrad: operand rows must be 16-byte aligned");
+  TM_REQUIRE(ws && ws_bytes >= tm_conv3x3_tf32_wgrad_ws(B, H, W, Cin, Cout), "tm_conv3x3_tf32_wgrad: workspace too small");
+  const int64_t Wp = W / P;
+  WgradArgs a;
+  a.Cin = (int)(P * Cin); a.Cout = (int)(P * Cout);
+  int NT;
+  tf_wgrad_plan(a, B, H, Wp, a.Cin <= 64 ? 3 : 1, NT);
+  TM_REQUIRE(NT > 0, "tm_conv3x3_tf32_wgrad: tile does not fit shared memory");
+  a.part = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  a.err = err;
+  CUtensorMap tmx, tmdy;
+  TM_TRY(encode_act(&tmx, x, a.Cin, Wp, H, B, 32, a.g.TW, a.g.TH, a.g.TB, 1, 4, P * ldx, true));
+  TM_TRY(encode_act(&tmdy, dy, a.Cout, Wp, H, B, 32, a.g.TW, a.g.TH, a.g.TB, 1, 4, P * lddy, true));
+  const int splits = wgrad_splits(a.g);
+  cudaStream_t st = (cudaStream_t)stream;
+  const dim3 grid((unsigned)splits, 3);
+  TM_TRY(NT == 3 ? launch_wgrad_tf32<3>(a, tmx, tmdy, grid, st) : launch_wgrad_tf32<1>(a, tmx, tmdy, grid, st));
+  const int64_t n = 9 * Cout * Cin_real;
+  wgrad_reduce_kernel<3><<<(unsigned)cdiv(n * 32, 256), 256, 0, st>>>(a.part, splits, P, (int)Cout, (int)Cin, (int)Cin_real, 3, dw);
+  return check_launch("wgrad_reduce");
+}
+
+extern "C" int tm_convt2x2_tf32_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  return convt_shape_ok(B, H, W, Cin, Cout) ? 1 : 0;
+}
+extern "C" int tm_convt2x2_tf32_wgrad_supported(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  return convt_shape_ok(B, H, W, Cin, Cout) && Cin % 32 == 0 && Cout % 32 == 0 && Cin <= 128 && Cout <= 64 && pow2(Cin) &&
+                 pow2(Cout)
+             ? 1
+             : 0;
+}
+
+// w [Cin][Cout][2][2] fp32 -> wf fp32 [4*Cout][Cin], wd fp32 [4][Cin][Cout] (either may be NULL)
+extern "C" int tm_convt2x2_pack_f32(int64_t Cin, int64_t Cout, const float* w, float* wf, float* wd, void* stream) {
+  pack_convt_kernel<<<(unsigned)cdiv(Cin * Cout * 4, 256), 256, 0, (cudaStream_t)stream>>>((int)Cin, (int)Cout, w, wf, wd);
+  return check_launch("pack_convt_f32");
+}
+
+namespace {
+void convt_tf_wgrad_plan(WgradArgs& a, int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  // kernel roles: "dy" slot = the untapped M-side operand (x), "x" slot = the four tapped N-side tiles (dy)
+  a.Cin = (int)Cout; a.Cout = (int)Cin;
+  int NT;
+  tf_wgrad_plan(a, B, H, W, 4, NT);
+}
+}  // namespace
+
+// workspace of tm_convt2x2_tf32, _dgrad and _wgrad (the largest of the three)
+extern "C" size_t tm_convt2x2_tf32_ws(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout) {
+  if (!convt_shape_ok(B, H, W, Cin, Cout)) return 0;
+  size_t n = tf_ws(convt_args(B, H, W, Cin, 4 * Cout, Cout, 1), 4 * B * H * W);
+  const size_t d = tf_ws(convt_args(B, H, W, Cout, Cin, Cin, 4), B * H * W);
+  if (d > n) n = d;
+  if (tm_convt2x2_tf32_wgrad_supported(B, H, W, Cin, Cout)) {
+    WgradArgs a;
+    convt_tf_wgrad_plan(a, B, H, W, Cin, Cout);
+    const size_t w = (size_t)convt_wgrad_splits(a.g) * 4 * Cin * Cout * sizeof(float) + 256;
+    if (w > n) n = w;
+  }
+  return n;
+}
+
+// y[b, 2y+dy, 2x+dx, co] (row stride ldy) = bias[co] + sum_ci x[b,y,x,ci] * w[ci][co][dy][dx]; x fp32 rows of stride ldx
+extern "C" int tm_convt2x2_tf32(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const float* x, int64_t ldx,
+                                const float* wf, const float* bias, float* y, int64_t ldy, void* ws, size_t ws_bytes, int* err,
+                                void* stream) {
+  TM_REQUIRE(convt_shape_ok(B, H, W, Cin, Cout), "tm_convt2x2_tf32: unsupported shape");
+  return run_tf32(convt_args(B, H, W, Cin, 4 * Cout, Cout, 1), x, Cin, W, H, ldx, 1, wf, 4 * Cout, 4 * B * H * W, bias, 0,
+                  y, ldy, ws, ws_bytes, err, (cudaStream_t)stream);
+}
+
+// dx[b,y,x,ci] (row stride lddx) = sum_{dy,dx,co} dy[b, 2y+dy, 2x+dx, co] * w[ci][co][dy][dx]; dy fp32 rows of stride lddy
+extern "C" int tm_convt2x2_tf32_dgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const float* dy, int64_t lddy,
+                                      const float* wd, float* dx, int64_t lddx, void* ws, size_t ws_bytes, int* err, void* stream) {
+  TM_REQUIRE(convt_shape_ok(B, H, W, Cin, Cout), "tm_convt2x2_tf32_dgrad: unsupported shape");
+  return run_tf32(convt_args(B, H, W, Cout, Cin, Cin, 4), dy, Cout, 2 * W, 2 * H, lddy, 2, wd, 4 * Cin, B * H * W, nullptr, 0,
+                  dx, lddx, ws, ws_bytes, err, (cudaStream_t)stream);
+}
+
+// dw[ci][co][dy][dx] = sum_{b,y,x} x[b,y,x,ci] * dy[b, 2y+dy, 2x+dx, co]; x, dy fp32 rows of stride ldx / lddy
+extern "C" int tm_convt2x2_tf32_wgrad(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const float* x, int64_t ldx,
+                                      const float* dy, int64_t lddy, float* dw, void* ws, size_t ws_bytes, int* err,
+                                      void* stream) {
+  TM_REQUIRE(tm_convt2x2_tf32_wgrad_supported(B, H, W, Cin, Cout), "tm_convt2x2_tf32_wgrad: unsupported shape");
+  TM_REQUIRE(ldx % 4 == 0 && lddy % 4 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(dy) % 16 == 0,
+             "tm_convt2x2_tf32_wgrad: operand rows must be 16-byte aligned");
+  TM_REQUIRE(ws && ws_bytes >= tm_convt2x2_tf32_ws(B, H, W, Cin, Cout), "tm_convt2x2_tf32_wgrad: workspace too small");
+  WgradArgs a;
+  convt_tf_wgrad_plan(a, B, H, W, Cin, Cout);
+  a.part = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  a.err = err;
+  a.cscale = 2;
+  for (int q = 0; q < 4; ++q) { a.tdx[q] = (signed char)(q & 1); a.tdy[q] = (signed char)(q >> 1); }
+  CUtensorMap tm_tap, tm_m;
+  TM_TRY(encode_act(&tm_tap, dy, Cout, 2 * W, 2 * H, B, 32, a.g.TW, a.g.TH, a.g.TB, 2, 4, lddy, true));
+  TM_TRY(encode_act(&tm_m, x, Cin, W, H, B, 32, a.g.TW, a.g.TH, a.g.TB, 1, 4, ldx, true));
+  const int splits = convt_wgrad_splits(a.g);
+  cudaStream_t st = (cudaStream_t)stream;
+  TM_TRY(launch_wgrad_tf32<4>(a, tm_tap, tm_m, dim3((unsigned)splits, 1), st));
+  convt_wgrad_reduce_kernel<<<(unsigned)cdiv(4 * Cin * Cout, 256), 256, 0, st>>>(a.part, splits, (int)Cin, (int)Cout, dw);
+  return check_launch("convt_wgrad_reduce");
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1150,7 +1603,7 @@ extern "C" int tm_convkxk_pack_bf16(int64_t Cout, int64_t Cin, int64_t k, const 
                                     void* stream) {
   TM_REQUIRE(kxk_ok(k) && KcP >= (dgrad ? Cout : Cin), "tm_convkxk_pack_bf16: bad kernel size or packing");
   const int64_t n = k * k * (dgrad ? Cin : Cout) * KcP;
-  pack_w_bf16_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, (int)k, w,
+  pack_w_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((int)Cout, (int)Cin, (int)k, w,
                                                                              (__nv_bfloat16*)q, 1, (int)KcP, dgrad);
   return check_launch("pack_w_bf16");
 }
@@ -1214,10 +1667,10 @@ extern "C" int tm_convkxk_bf16_wgrad(int64_t B, int64_t H, int64_t W, int64_t Ci
   cudaStream_t st = (cudaStream_t)stream;
   static bool optin = false;
   if (!optin) {
-    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
+    TM_CUDA(cudaFuncSetAttribute(conv3x3_wgrad_tma_kernel<0, FMT_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONV_SMEM_BUDGET + 1024));
     optin = true;
   }
-  conv3x3_wgrad_tma_kernel<0><<<dim3((unsigned)splits, (unsigned)gy), CONV_THREADS, smem, st>>>(tmx, tmdy, a);
+  conv3x3_wgrad_tma_kernel<0, FMT_BF16><<<dim3((unsigned)splits, (unsigned)gy), CONV_THREADS, smem, st>>>(tmx, tmdy, a);
   TM_TRY(check_launch("convkxk_wgrad_tma"));
   const int64_t n = k * k * Cout * Cin;
   wgrad_reduce_kernel<0><<<(unsigned)cdiv(n * 32, 256), 256, 0, st>>>(a.part, splits, 1, (int)Cout, (int)Cin, (int)Cin, (int)k, dw);

@@ -49,18 +49,30 @@ def _enter(net):
     _CUR = getattr(net, "math", None)
 
 
-USE_TMA = os.environ.get("TM_CONV_TMA", "1") != "0"   # bf16 mode: TMA-fed 3x3 convolutions on bf16 activations
+USE_TMA = os.environ.get("TM_CONV_TMA", "1") != "0"   # bf16 / tf32x3 mode: TMA-fed 3x3 and transposed convolutions
 
 
 def _cpad(c):
     return max(16, (c + 15) // 16 * 16)
 
 
+def _tma_fmt():
+    """Operand format of the TMA-fed kernels for the current arithmetic: "bf16" (bf16 mode), "tf32" (tf32x3: fp32
+    operands read in place, 3xTF32 products) or None (tc6, tc3, tf32, fp32 keep the cp.async / CUDA-core kernels)."""
+    return {0: "bf16", 3: "tf32"}.get(_prec(None)) if USE_TMA else None
+
+
 def _tma_ok(B, H, W, cin, cout):
-    """bf16 mode and a shape the TMA kernels take (H, W powers of two; channels multiples of 16)."""
-    return (USE_TMA and _prec(None) == 0 and cout <= 128 and _cpad(cin) <= 128
-            and tm_lib.ws_bytes("tm_conv3x3_bf16_supported", B, H, W, _cpad(cin), cout) == 1
-            and (cin % 16 != 0 or tm_lib.ws_bytes("tm_conv3x3_bf16_supported", B, H, W, cout, cin) == 1))
+    """-> the TMA operand format when it serves the current arithmetic and the kernels take the shape (H, W powers
+    of two; channels multiples of 16), else None."""
+    fmt = _tma_fmt()
+    if fmt is None or cout > 128 or _cpad(cin) > 128:
+        return None
+    fn = f"tm_conv3x3_{fmt}_supported"
+    if (tm_lib.ws_bytes(fn, B, H, W, _cpad(cin), cout) == 1
+            and (cin % 16 != 0 or tm_lib.ws_bytes(fn, B, H, W, cout, cin) == 1)):
+        return fmt
+    return None
 
 
 def _to_bf16(x, ldx, npix, C):
@@ -70,17 +82,18 @@ def _to_bf16(x, ldx, npix, C):
     return out
 
 
-def _pack_bf16(w, W, need_dgrad):
-    """-> ((forward operand, P), (data-gradient operand, P) or None) for images W wide."""
+def _pack_tma(w, W, need_dgrad, fmt="bf16"):
+    """-> ((forward operand, P), (data-gradient operand, P) or None) for images W wide; bf16 or fp32 ("tf32")."""
     cout, cin = w.shape[0], w.shape[1]
     dev = w.device
     wc = w.detach().float().contiguous()
+    dtype, pack = (torch.bfloat16, "tm_conv3x3_pack_bf16") if fmt == "bf16" else (torch.float32, "tm_conv3x3_pack_f32")
 
     def one(nc, kc, dgrad):
         kp = _cpad(kc)
-        P = tm_lib.ws_bytes("tm_conv3x3_bf16_pack", W, kp, nc)
-        q = torch.empty(9, P * nc, P * kp, dtype=torch.bfloat16, device=dev)
-        call("tm_conv3x3_pack_bf16", cout, cin, wc, q, P, kp, dgrad, stream())
+        P = tm_lib.ws_bytes(f"tm_conv3x3_{fmt}_pack", W, kp, nc)
+        q = torch.empty(9, P * nc, P * kp, dtype=dtype, device=dev)
+        call(pack, cout, cin, wc, q, P, kp, dgrad, stream())
         return q, P
     return one(cout, cin, 0), (one(cin, cout, 1) if need_dgrad else None)
 
@@ -98,6 +111,33 @@ def _conv_tma(xb, B, H, W, cinp, cout, wq, y, ldy, want_stats=False):
     call("tm_conv3x3_bf16", B, H, W, cinp, cout, P, xb, q, None, y, ldy, 0, stats[0] if stats else None,
          tm_lib.err_flag(y.device), stream())
     return stats
+
+
+def _conv_tf(ws, x, ldx, B, H, W, cinp, cout, wq, y, ldy, want_stats=False):
+    """tf32x3 on the TMA kernels, x read in place.  Deep layers split K (workspace); only unsplit launches take the
+    batch-norm statistics in their epilogue.  -> (stats buffer, number of partials) or None."""
+    q, P = wq
+    nb = tm_lib.ws_bytes("tm_conv3x3_tf32_ws", B, H, W, cinp, cout, P)
+    stats = None
+    if want_stats and FUSE_BN_STATS and nb == 0 and P * cout <= 128:
+        ns = tm_lib.ws_bytes("tm_conv3x3_bf16_stats_bytes", cout, P)
+        stats = (torch.empty(ns, dtype=torch.uint8, device=y.device), ns // (16 * cout))
+    call("tm_conv3x3_tf32", B, H, W, cinp, cout, P, x, ldx, q, None, y, ldy, 0, stats[0] if stats else None,
+         ws.get(nb) if nb else None, nb, tm_lib.err_flag(y.device), stream())
+    return stats
+
+
+def _wgrad_tf(ws, x, ldx, dy, lddy, B, H, W, cinp, cin, cout):
+    if min(cin, cout) >= 64:
+        # measured slower on the TMA kernel (profiles/bench_unet_tf32_layers.py: 128 -> 128 at 32x32 70 us against
+        # 31 us): few pixels, 32-pixel stages and one-tap stages; these stay on the cp.async tf_gemm route
+        return _conv_wgrad(ws, x, ldx, dy, lddy, B, H, W, cin, cout, 3, False)[0]
+    dev = dy.device
+    dw = _empty(cout, cin, 3, 3, dev=dev)
+    nb = tm_lib.ws_bytes("tm_conv3x3_tf32_wgrad_ws", B, H, W, cinp, cout)
+    call("tm_conv3x3_tf32_wgrad", B, H, W, cinp, cin, cout, x, ldx, dy, lddy, dw, ws.get(nb), nb, tm_lib.err_flag(dev),
+         stream())
+    return dw
 
 
 def _wgrad_tma(ws, xb, dyb, B, H, W, cin, cout):
@@ -205,11 +245,26 @@ def _double_conv_fwd(ws, st, name, mods, x, ldx, B, H, W, cin, cout, out, ldo, u
     npix = B * H * W
     cmid = conv1.weight.shape[0]
     r1, r2 = _empty(npix, cmid, dev=dev), _empty(npix, cout, dev=dev)
-    if _tma_ok(B, H, W, cin, cmid) and _tma_ok(B, H, W, cmid, cout):
+    route = _tma_ok(B, H, W, cin, cmid) if _tma_ok(B, H, W, cmid, cout) else None
+    if route == "tf32":
+        # tf32x3 mode: the TMA-fed kernels read the fp32 activations in place (x: compact rows, or 16 zero-padded
+        # channels for the 3-channel input)
+        wq1, wd1 = _pack_tma(conv1.weight, W, need_bwd and cin % 16 == 0, "tf32")
+        wq2, wd2 = _pack_tma(conv2.weight, W, need_bwd, "tf32")
+        a1 = _empty(npix, cmid, dev=dev)
+        s1 = _conv_tf(ws, x, ldx, B, H, W, _cpad(cin), cmid, wq1, r1, cmid, want_stats=SEG == 1)
+        m1, i1 = _bn_relu_fwd(ws, r1, cmid, npix, cmid, bn1, a1, cmid, update_stats, stats=s1)
+        s2 = _conv_tf(ws, a1, cmid, B, H, W, cmid, cout, wq2, r2, cout, want_stats=SEG == 1)
+        m2, i2 = _bn_relu_fwd(ws, r2, cout, npix, cout, bn2, out, ldo, update_stats, stats=s2)
+        st[name] = dict(tf=True, x=x, ldx=ldx, a1=a1, wd1=wd1, wd2=wd2, B=B, H=H, W=W, cin=cin, cmid=cmid, cout=cout,
+                        r1=r1, r2=r2, out=out, ldo=ldo, m1=m1, i1=i1, m2=m2, i2=i2, g1=bn1.weight.detach(),
+                        g2=bn2.weight.detach(), be1=bn1.bias.detach(), be2=bn2.bias.detach())
+        return
+    if route == "bf16":
         # bf16 mode: TMA-fed tcgen05 convolutions on compact bf16 copies of the activations (kept for wgrad)
         xb = _to_bf16(x, ldx, npix, cin)
-        wq1, wd1 = _pack_bf16(conv1.weight, W, need_bwd and cin % 16 == 0)
-        wq2, wd2 = _pack_bf16(conv2.weight, W, need_bwd)
+        wq1, wd1 = _pack_tma(conv1.weight, W, need_bwd and cin % 16 == 0)
+        wq2, wd2 = _pack_tma(conv2.weight, W, need_bwd)
         # the convolution epilogue's statistics cover the whole batch: per-image statistics (SEG > 1) take their own pass
         s1 = _conv_tma(xb, B, H, W, _cpad(cin), cmid, wq1, r1, cmid, want_stats=SEG == 1)
         a1b = torch.empty(npix, cmid, dtype=torch.bfloat16, device=dev)
@@ -240,7 +295,19 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx):
     npix = B * H * W
     dev = dout.device
     da1 = _empty(npix, cmid, dev=dev)
-    if s.get("tma"):
+    if s.get("tf"):
+        dr2 = _empty(npix, cout, dev=dev)
+        dg2, db2 = _bn_relu_bwd(ws, s["r2"], cout, dout, lddo, npix, cout, s["g2"], s["be2"], s["m2"], s["i2"],
+                                dr2, cout)
+        dw2 = _wgrad_tf(ws, s["a1"], cmid, dr2, cout, B, H, W, cmid, cmid, cout)
+        _conv_tf(ws, dr2, cout, B, H, W, cout, cmid, s["wd2"], da1, cmid)
+        dr1 = _empty(npix, cmid, dev=dev)
+        dg1, db1 = _bn_relu_bwd(ws, s["r1"], cmid, da1, cmid, npix, cmid, s["g1"], s["be1"], s["m1"], s["i1"],
+                                dr1, cmid)
+        dw1 = _wgrad_tf(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, _cpad(cin), cin, cmid)
+        if dx is not None:
+            _conv_tf(ws, dr1, cmid, B, H, W, cmid, cin, s["wd1"], dx, lddx)
+    elif s.get("tma"):
         # the batch-norm backward emits its result directly as the bf16 operand shared by the weight and the
         # data gradient; the fp32 copy is never needed
         dr2b = torch.empty(npix, cout, dtype=torch.bfloat16, device=dev)
@@ -300,15 +367,17 @@ def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
     mode = 0 if net.pooling == "max" else 1
     ws = _Ws(dev)
     st = {"ws": ws, "mode": mode, "B": B, "H": H, "W": W, "seg": SEG}
-    x0 = _empty(B * H * W, 3, dev=dev)
-    call("tm_nchw_to_nhwc", B, 3, H, W, x, x0, 3, stream())
+    # tf32x3 mode reads the input in place: 16 channels, zero padded (a 12-byte pixel stride is no TMA stride)
+    c0 = 16 if _tma_fmt() == "tf32" else 3
+    x0 = (torch.zeros if c0 > 3 else torch.empty)(B * H * W, c0, dtype=torch.float32, device=dev)
+    call("tm_nchw_to_nhwc", B, 3, H, W, x, x0, c0, stream())
     chans = [16, 32, 64, 128]
     Hs = [H, H // 2, H // 4, H // 8]
     Ws_ = [W, W // 2, W // 4, W // 8]
     cat = [_empty(B * Hs[i] * Ws_[i], 2 * chans[i], dev=dev) for i in range(3)]     # [skip | up]
     x4 = _empty(B * Hs[3] * Ws_[3], 128, dev=dev)
     enc = [net.inc, net.down1.maxpool_conv[1], net.down2.maxpool_conv[1], net.down3.maxpool_conv[1]]
-    cur, ld, cin = x0, 3, 3
+    cur, ld, cin = x0, c0, 3
     st["pool"] = []
     for i in range(4):
         if i > 0:                                      # Down = pool -> DoubleConv (Unet.py:33-36)
@@ -330,8 +399,19 @@ def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
         cout_t = cy // 2
         half = cat[i][:, chans[i]:]                    # second half of the concat buffer
         wup = up.up.weight.detach().float().contiguous()
-        if (USE_TMA and _prec(None) == 0
-                and tm_lib.ws_bytes("tm_convt2x2_bf16_supported", B, Hs[i + 1], Ws_[i + 1], cy, cout_t) == 1):
+        fmt = _tma_fmt()
+        if fmt and tm_lib.ws_bytes(f"tm_convt2x2_{fmt}_supported", B, Hs[i + 1], Ws_[i + 1], cy, cout_t) != 1:
+            fmt = None
+        if fmt == "tf32":
+            # tf32x3 mode: the same one-tap TMA convolution on the fp32 activation, read in place
+            wfq = _empty(4 * cout_t, cy, dev=dev)
+            wdq = _empty(4, cy, cout_t, dev=dev) if need_bwd else None
+            call("tm_convt2x2_pack_f32", cy, cout_t, wup, wfq, wdq, stream())
+            nb = tm_lib.ws_bytes("tm_convt2x2_tf32_ws", B, Hs[i + 1], Ws_[i + 1], cy, cout_t)
+            call("tm_convt2x2_tf32", B, Hs[i + 1], Ws_[i + 1], cy, cout_t, y, ldy, wfq, up.up.bias.detach(), half,
+                 2 * chans[i], ws.get(nb) if nb else None, nb, tm_lib.err_flag(dev), stream())
+            st[f"up{j}"] = dict(x=y, ldx=ldy, cin=cy, cout=cout_t, wdf=wdq, i=i)
+        elif fmt == "bf16":
             # bf16 mode: one-tap TMA convolution whose epilogue scatters the 2x2 output windows
             yb = _to_bf16(y, ldy, B * Hs[i + 1] * Ws_[i + 1], cy)
             wfq = torch.empty(4 * cout_t, cy, dtype=torch.bfloat16, device=dev)
@@ -404,14 +484,32 @@ def unet_backward(net, st, gout):
             call("tm_convt2x2_bf16_dgrad", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"], halfb, u["wdq"], dy, u["cin"],
                  tm_lib.err_flag(dev), stream())
         else:
-            nb = tm_lib.ws_bytes("tm_convt2x2_wgrad_ws", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"])
-            dwt, dbt = _empty(u["cin"], 4 * u["cout"], dev=dev), _empty(u["cout"], dev=dev)
-            call("tm_convt2x2_wgrad_nhwc", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"], u["x"], u["ldx"], half,
-                 2 * chans[i], Hs[i], Ws_[i], 0, 0, dwt, dbt, ws.get(nb), nb, stream())
-            dwu = _empty(u["cin"], u["cout"], 2, 2, dev=dev)
-            call("tm_convt_unpack_wgrad", u["cin"], u["cout"], dwt, dwu, stream())
-            call("tm_convt2x2_dgrad_nhwc", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"], half, 2 * chans[i], Hs[i],
-                 Ws_[i], 0, 0, u["wtT"], dy, u["cin"], stream())
+            tf = u.get("wdf") is not None
+            shape = (B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"])
+            if tf and tm_lib.ws_bytes("tm_convt2x2_tf32_wgrad_supported", *shape) == 1:
+                # tf32x3 mode: weight gradient on the TMA path (its N side needs 32-channel boxes: Cout >= 32)
+                nb = tm_lib.ws_bytes("tm_convt2x2_tf32_ws", *shape)
+                dwu, dbt = _empty(u["cin"], u["cout"], 2, 2, dev=dev), _empty(u["cout"], dev=dev)
+                call("tm_convt2x2_tf32_wgrad", *shape, u["x"], u["ldx"], half, 2 * chans[i], dwu, ws.get(nb), nb,
+                     tm_lib.err_flag(dev), stream())
+                npo = B * Hs[i] * Ws_[i]
+                nbc = tm_lib.ws_bytes("tm_colsum_ws", npo, u["cout"])
+                call("tm_colsum", npo, u["cout"], half, 2 * chans[i], None, dbt, 0, tm_lib.workspace(nbc, dev), nbc,
+                     stream())
+            else:
+                nb = tm_lib.ws_bytes("tm_convt2x2_wgrad_ws", *shape)
+                dwt, dbt = _empty(u["cin"], 4 * u["cout"], dev=dev), _empty(u["cout"], dev=dev)
+                call("tm_convt2x2_wgrad_nhwc", *shape, u["x"], u["ldx"], half,
+                     2 * chans[i], Hs[i], Ws_[i], 0, 0, dwt, dbt, ws.get(nb), nb, stream())
+                dwu = _empty(u["cin"], u["cout"], 2, 2, dev=dev)
+                call("tm_convt_unpack_wgrad", u["cin"], u["cout"], dwt, dwu, stream())
+            if tf:
+                nb = tm_lib.ws_bytes("tm_convt2x2_tf32_ws", *shape)
+                call("tm_convt2x2_tf32_dgrad", *shape, half, 2 * chans[i], u["wdf"], dy, u["cin"],
+                     ws.get(nb) if nb else None, nb, tm_lib.err_flag(dev), stream())
+            else:
+                call("tm_convt2x2_dgrad_nhwc", *shape, half, 2 * chans[i], Hs[i],
+                     Ws_[i], 0, 0, u["wtT"], dy, u["cin"], stream())
         grads[f"{names[j]}.up.weight"], grads[f"{names[j]}.up.bias"] = dwu, dbt
         lddy = u["cin"]
     # encoder, deepest first; dy is the gradient of x4
