@@ -391,6 +391,15 @@ size_t tm_conv1x1_c1_wgrad_ws(int64_t C);
 int tm_conv1x1_c1_wgrad(int64_t npix, int64_t C, const float* x, int64_t ldx, const float* dy, int64_t lddy, float* dw,
                         float* dbias, void* ws, size_t ws_bytes, void* stream);
 
+/* Gradient w.r.t. the input image of the first convolution of each image network (U-Net inc.double_conv.0: k = 3,
+ * 16 -> 3; LayoutNet encode.0: k = 9, 32 -> 2): dx = conv_transpose2d(dy, w) for nn.Conv2d(Cin, Cout, k, stride 1,
+ * padding k/2).  dy: NHWC [B][H][W], pixel stride lddy, Cout channels, fp32 (dy_bf16 = 0) or bf16 (dy_bf16 = 1);
+ * w: the nn.Conv2d weight [Cout][Cin][k][k] fp32; dx: NCHW fp32 [B][Cin][H][W], every element written.
+ * k in {3, 9}, 1 <= Cin <= 4, Cout % 8 == 0, lddy % 8 == 0, dy 16-byte aligned.  Direct convolution on the CUDA
+ * cores (fp32 products and accumulation in a fixed order: deterministic, fp32-class for fp32 dy). */
+int tm_conv_dgrad_narrow(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k, const void* dy,
+                         int64_t lddy, int dy_bf16, const float* w, float* dx, void* stream);
+
 /* 2x2 stride-2 pooling (Unet.py:89-91, model.py:222-224). mode 0 = max (idx: uint8 argmax
  * saved for backward, first maximum in row-major window order), 1 = avg (idx unused).
  * flags: TM_EPI_RELU applies ReLU after pooling (OutConv, Unet.py:76-77). */

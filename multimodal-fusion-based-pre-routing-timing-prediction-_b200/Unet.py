@@ -89,5 +89,5 @@ class UNet(nn.Module):
 
     def forward(self, x):
         params = list(self.parameters())
-        need = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+        need = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
         return tm_unet.UNetFn.apply(self, x, need, *params)

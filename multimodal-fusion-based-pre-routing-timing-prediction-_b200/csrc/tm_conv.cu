@@ -426,6 +426,108 @@ __global__ void conv1x1_c1_wgrad_final_kernel(int C, int nblk, const double* __r
   else if (dbias) dbias[0] = (float)a;
 }
 
+// ------------------------------------------------------------------------------ narrow data gradient (input image)
+// dx = conv_transpose2d(dy, w) of the first convolution of each image network (U-Net inc: k = 3, 16 -> 3; LayoutNet
+// encode.0: k = 9, 32 -> 2).  With 2-4 output channels an implicit GEMM padded to 16 would waste 4-8x of every MMA, so
+// this is a direct correlation with the flipped taps on CUDA cores: a CTA owns a 32 x 32 tile of dx for every input
+// channel; dy (tile + halo, NDG_CC channels at a time) and the weights live in shared memory; a thread owns a column of
+// NDG_RPT pixels, loads the NDG_RPT + K - 1 dy values a tap column needs once and reuses them over the K taps of that
+// column.  fp32 accumulate in a fixed order (deterministic); dx is written straight to NCHW.
+constexpr int NDG_THREADS = 128, NDG_RPT = 8, NDG_TW = 32, NDG_TH = NDG_RPT * NDG_THREADS / 32, NDG_CC = 8;
+
+__host__ __device__ constexpr int ndg_cinp(int cin) { return cin == 3 ? 4 : cin; }
+
+__device__ __forceinline__ void ndg_load8(const float* p, float* v) {
+  const float4 a = ld4(p), b = ld4(p + 4);
+  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void ndg_load8(const __nv_bfloat16* p, float* v) {
+  const uint4 a = *reinterpret_cast<const uint4*>(p);
+  const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&a);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 f = __bfloat1622float2(h[j]);
+    v[2 * j] = f.x;
+    v[2 * j + 1] = f.y;
+  }
+}
+
+template <int K, int CIN, typename T>
+__global__ void __launch_bounds__(NDG_THREADS)
+conv_dgrad_narrow_kernel(int H, int W, int Cout, const T* __restrict__ dy, int64_t lddy, const float* __restrict__ w,
+                         float* __restrict__ dx) {
+  constexpr int P = K / 2, SW = NDG_TW + K - 1, SH = NDG_TH + K - 1, CP = ndg_cinp(CIN);
+  extern __shared__ float4 ndg_sh[];
+  float* sw = reinterpret_cast<float*>(ndg_sh);       // [Cout][K][K][CP], taps flipped
+  float* sd = sw + Cout * K * K * CP;                  // [NDG_CC][SH][SW]
+  const int b = blockIdx.z, x0 = blockIdx.x * NDG_TW, y0 = blockIdx.y * NDG_TH;
+  for (int i = threadIdx.x; i < Cout * K * K * CP; i += NDG_THREADS) {
+    const int ci = i % CP, tap = (i / CP) % (K * K), co = i / (CP * K * K);
+    sw[i] = ci < CIN ? __ldg(w + ((int64_t)co * CIN + ci) * K * K + (K * K - 1 - tap)) : 0.f;
+  }
+  const int lane = threadIdx.x & 31, r0 = (threadIdx.x >> 5) * NDG_RPT;
+  float acc[NDG_RPT][CIN];
+#pragma unroll
+  for (int i = 0; i < NDG_RPT; ++i)
+#pragma unroll
+    for (int ci = 0; ci < CIN; ++ci) acc[i][ci] = 0.f;
+  const T* dyb = dy + (int64_t)b * H * W * lddy;
+  for (int c0 = 0; c0 < Cout; c0 += NDG_CC) {
+    __syncthreads();
+    for (int p = threadIdx.x; p < SH * SW; p += NDG_THREADS) {
+      const int ly = p / SW, lx = p - ly * SW, gy = y0 - P + ly, gx = x0 - P + lx;
+      float v[NDG_CC];
+      if (gy >= 0 && gy < H && gx >= 0 && gx < W) {
+        ndg_load8(dyb + ((int64_t)gy * W + gx) * lddy + c0, v);
+      } else {
+#pragma unroll
+        for (int c = 0; c < NDG_CC; ++c) v[c] = 0.f;
+      }
+#pragma unroll
+      for (int c = 0; c < NDG_CC; ++c) sd[(c * SH + ly) * SW + lx] = v[c];
+    }
+    __syncthreads();
+    for (int c = 0; c < NDG_CC; ++c) {
+      const float* s = sd + (c * SH + r0) * SW + lane;
+      const float* wc = sw + (c0 + c) * K * K * CP;
+#pragma unroll
+      for (int v = 0; v < K; ++v) {
+        float col[NDG_RPT + K - 1];
+#pragma unroll
+        for (int i = 0; i < NDG_RPT + K - 1; ++i) col[i] = s[i * SW + v];
+#pragma unroll
+        for (int u = 0; u < K; ++u) {
+          float wv[CP];
+          const float* wp = wc + (u * K + v) * CP;
+          if constexpr (CP == 4) {
+            const float4 t = *reinterpret_cast<const float4*>(wp);
+            wv[0] = t.x; wv[1] = t.y; wv[2] = t.z; wv[3] = t.w;
+          } else if constexpr (CP == 2) {
+            const float2 t = *reinterpret_cast<const float2*>(wp);
+            wv[0] = t.x; wv[1] = t.y;
+          } else {
+            wv[0] = wp[0];
+          }
+#pragma unroll
+          for (int i = 0; i < NDG_RPT; ++i)
+#pragma unroll
+            for (int ci = 0; ci < CIN; ++ci) acc[i][ci] = fmaf(col[i + u], wv[ci], acc[i][ci]);
+        }
+      }
+    }
+  }
+  const int gx = x0 + lane;
+  if (gx >= W) return;
+#pragma unroll
+  for (int i = 0; i < NDG_RPT; ++i) {
+    const int gy = y0 + r0 + i;
+    if (gy < H) {
+#pragma unroll
+      for (int ci = 0; ci < CIN; ++ci) dx[(((int64_t)b * CIN + ci) * H + gy) * W + gx] = acc[i][ci];
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------ pooling etc.
 __global__ void pool_fwd_kernel(int64_t B, int64_t H, int64_t W, int64_t C, int mode,
                                 const float* __restrict__ x, int64_t ldx, float* __restrict__ y, int64_t ldy,
@@ -857,6 +959,53 @@ extern "C" int tm_conv1x1_c1_wgrad(int64_t npix, int64_t C, const float* x, int6
   TM_TRY(check_launch("conv1x1_c1_wgrad"));
   conv1x1_c1_wgrad_final_kernel<<<(unsigned)cdiv((C + 1) * 32, 128), 128, 0, ST>>>((int)C, nblk, (const double*)ws, dw, dbias);
   return check_launch("conv1x1_c1_wgrad_final");
+}
+
+namespace {
+template <int K, int CIN, typename T>
+int conv_dgrad_narrow_launch(int64_t B, int64_t H, int64_t W, int64_t Cout, const void* dy, int64_t lddy, const float* w,
+                             float* dx, cudaStream_t st) {
+  auto kern = conv_dgrad_narrow_kernel<K, CIN, T>;
+  const size_t sh = sizeof(float) * ((size_t)Cout * K * K * ndg_cinp(CIN) + (size_t)NDG_CC * (NDG_TH + K - 1) *
+                                     (NDG_TW + K - 1));
+  TM_REQUIRE(sh <= 227 * 1024, "tm_conv_dgrad_narrow: Cout = %lld needs %zu bytes of shared memory", (long long)Cout, sh);
+  TM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sh));
+  const dim3 grid((unsigned)cdiv(W, NDG_TW), (unsigned)cdiv(H, NDG_TH), (unsigned)B);
+  kern<<<grid, NDG_THREADS, sh, st>>>((int)H, (int)W, (int)Cout, (const T*)dy, lddy, w, dx);
+  return check_launch("conv_dgrad_narrow");
+}
+template <int K, typename T>
+int conv_dgrad_narrow_cin(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, const void* dy, int64_t lddy,
+                          const float* w, float* dx, cudaStream_t st) {
+  switch (Cin) {
+    case 1: return conv_dgrad_narrow_launch<K, 1, T>(B, H, W, Cout, dy, lddy, w, dx, st);
+    case 2: return conv_dgrad_narrow_launch<K, 2, T>(B, H, W, Cout, dy, lddy, w, dx, st);
+    case 3: return conv_dgrad_narrow_launch<K, 3, T>(B, H, W, Cout, dy, lddy, w, dx, st);
+    default: return conv_dgrad_narrow_launch<K, 4, T>(B, H, W, Cout, dy, lddy, w, dx, st);
+  }
+}
+template <typename T>
+int conv_dgrad_narrow_k(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k, const void* dy,
+                        int64_t lddy, const float* w, float* dx, cudaStream_t st) {
+  switch (k) {
+    case 3: return conv_dgrad_narrow_cin<3, T>(B, H, W, Cin, Cout, dy, lddy, w, dx, st);
+    default: return conv_dgrad_narrow_cin<9, T>(B, H, W, Cin, Cout, dy, lddy, w, dx, st);
+  }
+}
+}  // namespace
+
+extern "C" int tm_conv_dgrad_narrow(int64_t B, int64_t H, int64_t W, int64_t Cin, int64_t Cout, int64_t k,
+                                    const void* dy, int64_t lddy, int dy_bf16, const float* w, float* dx,
+                                    void* stream) {
+  TM_REQUIRE(B > 0 && H > 0 && W > 0 && B <= 65535 && H * W <= INT32_MAX, "tm_conv_dgrad_narrow: bad sizes");
+  TM_REQUIRE(Cin >= 1 && Cin <= 4, "tm_conv_dgrad_narrow: Cin must be 1..4 (got %lld)", (long long)Cin);
+  TM_REQUIRE(k == 3 || k == 9, "tm_conv_dgrad_narrow: k must be 3 or 9 (got %lld)", (long long)k);
+  TM_REQUIRE(Cout > 0 && Cout % NDG_CC == 0 && lddy >= Cout && lddy % 8 == 0 && ((uintptr_t)dy & 15) == 0,
+             "tm_conv_dgrad_narrow: dy needs Cout %% 8 == 0, a pixel stride lddy >= Cout with lddy %% 8 == 0 and 16-byte "
+             "alignment (Cout %lld, lddy %lld)", (long long)Cout, (long long)lddy);
+  if (dy_bf16)
+    return conv_dgrad_narrow_k<__nv_bfloat16>(B, H, W, Cin, Cout, k, dy, lddy, w, dx, ST);
+  return conv_dgrad_narrow_k<float>(B, H, W, Cin, Cout, k, dy, lddy, w, dx, ST);
 }
 
 extern "C" int tm_pool2x2_forward(int64_t B, int64_t H, int64_t W, int64_t C, int mode, const float* x,

@@ -156,7 +156,7 @@ class LayoutNet(nn.Module):
 
     def forward(self, x):
         params = list(self.parameters())
-        need = th.is_grad_enabled() and any(p.requires_grad for p in params)
+        need = th.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
         return tm_unet.LayoutNetFn.apply(self, x, need, *params)
 
 

@@ -435,6 +435,10 @@ class GnnPropagateFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gH):
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            raise NotImplementedError("PathConv: gradients w.r.t. cell_feat / net_feat are not implemented; the "
+                                      "propagation differentiates its parameters only (set requires_grad=False on "
+                                      "the features)")
         G = gH.contiguous().clone()                      # consumed in place by the sweep
         grads = gnn_backward(ctx.sched, ctx.saved, ctx.params, G)
         return (None, None, None, None) + tuple(grads)

@@ -289,8 +289,16 @@ def _double_conv_fwd(ws, st, name, mods, x, ldx, B, H, W, cin, cout, out, ldo, u
                     g2=bn2.weight.detach(), be1=bn1.bias.detach(), be2=bn2.bias.detach())
 
 
-def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx):
-    """dout: gradient w.r.t. the block output (strided).  Writes dx (if not None)."""
+def _dgrad_image(dr, lddr, bf16, s, w, dimg):
+    """Gradient w.r.t. the network's input image from the gradient of its first convolution's output: the narrow
+    direct kernel (2-4 image channels), written straight to NCHW."""
+    call("tm_conv_dgrad_narrow", s["B"], s["H"], s["W"], s["cin"], w.shape[0], w.shape[2], dr, lddr, int(bf16), w, dimg,
+         stream())
+
+
+def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx, dimg=None, w1=None):
+    """dout: gradient w.r.t. the block output (strided).  Writes dx (if not None); dimg (NCHW, optional): the gradient
+    w.r.t. the block input when it is the input image, through the first convolution's weight w1."""
     B, H, W, cin, cmid, cout = s["B"], s["H"], s["W"], s["cin"], s["cmid"], s["cout"]
     npix = B * H * W
     dev = dout.device
@@ -307,6 +315,8 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx):
         dw1 = _wgrad_tf(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, _cpad(cin), cin, cmid)
         if dx is not None:
             _conv_tf(ws, dr1, cmid, B, H, W, cmid, cin, s["wd1"], dx, lddx)
+        if dimg is not None:
+            _dgrad_image(dr1, cmid, False, s, w1, dimg)
     elif s.get("tma"):
         # the batch-norm backward emits its result directly as the bf16 operand shared by the weight and the
         # data gradient; the fp32 copy is never needed
@@ -321,6 +331,8 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx):
         dw1 = _wgrad_tma(ws, s["xb"], dr1b, B, H, W, cin, cmid)
         if dx is not None:
             _conv_tma(dr1b, B, H, W, cmid, cin, s["wd1"], dx, lddx)
+        if dimg is not None:
+            _dgrad_image(dr1b, cmid, True, s, w1, dimg)
     else:
         dr2 = _empty(npix, cout, dev=dev)
         dg2, db2 = _bn_relu_bwd(ws, s["r2"], cout, dout, lddo, npix, cout, s["g2"], s["be2"], s["m2"], s["i2"],
@@ -333,6 +345,8 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx):
         dw1, _ = _conv_wgrad(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, cin, cmid, 3, False)
         if dx is not None:
             _conv(dr1, cmid, B, H, W, cmid, cin, 3, s["wb1"], None, dx, lddx)
+        if dimg is not None:
+            _dgrad_image(dr1, cmid, False, s, w1, dimg)
     grads[prefix + ".0.weight"] = dw1
     grads[prefix + ".1.weight"], grads[prefix + ".1.bias"] = dg1, db1
     grads[prefix + ".3.weight"] = dw2
@@ -355,7 +369,8 @@ def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
     if EVAL and need_bwd:
         raise NotImplementedError("UNet in eval mode is inference only here (BatchNorm backward with frozen statistics is not "
                                   "built): call it under torch.no_grad(), or keep the module in train mode like the reference")
-    if x.dim() == 3:                                   # train.py:465 passes (C,H,W)
+    squeeze = x.dim() == 3
+    if squeeze:                                        # train.py:465 passes (C,H,W)
         x = x.unsqueeze(0)
     x = x.detach().float().contiguous()
     tm_lib.require_cuda(x, "UNet input")
@@ -366,7 +381,8 @@ def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
     dev = x.device
     mode = 0 if net.pooling == "max" else 1
     ws = _Ws(dev)
-    st = {"ws": ws, "mode": mode, "B": B, "H": H, "W": W, "seg": SEG}
+    st = {"ws": ws, "mode": mode, "B": B, "H": H, "W": W, "seg": SEG, "squeeze": squeeze,
+          "w_in": net.inc.double_conv[0].weight.detach().float().contiguous()}
     # tf32x3 mode reads the input in place: 16 channels, zero padded (a 12-byte pixel stride is no TMA stride)
     c0 = 16 if _tma_fmt() == "tf32" else 3
     x0 = (torch.zeros if c0 > 3 else torch.empty)(B * H * W, c0, dtype=torch.float32, device=dev)
@@ -442,8 +458,9 @@ def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
     return out, st
 
 
-def unet_backward(net, st, gout):
-    """gout: (B,1,H/2,W/2).  Returns {state_dict-style name: gradient} for every parameter."""
+def unet_backward(net, st, gout, need_dx=False):
+    """gout: (B,1,H/2,W/2).  Returns {state_dict-style name: gradient} for every parameter; with ``need_dx``
+    (grads, dx), dx the gradient w.r.t. the input image in its layout: (B,3,H,W), or (3,H,W) for a 3-D input."""
     _enter(net)
     global SEG
     SEG = st["seg"]
@@ -527,8 +544,11 @@ def unet_backward(net, st, gout):
                  p["idx"], dprev, chans[i - 1], 0, dskip[i - 1], 2 * chans[i - 1], stream())
             dy, lddy = dprev, chans[i - 1]
         else:
-            _double_conv_bwd(ws, s, dy, lddy, grads, enc_names[0], None, 0)
-    return grads
+            dx = _empty(B, 3, H, W, dev=dev) if need_dx else None
+            _double_conv_bwd(ws, s, dy, lddy, grads, enc_names[0], None, 0, dimg=dx, w1=st["w_in"])
+    if not need_dx:
+        return grads
+    return grads, (dx[0] if st["squeeze"] else dx)
 
 
 UNET_PARAM_ORDER = None
@@ -543,14 +563,17 @@ class UNetFn(torch.autograd.Function):
     def forward(ctx, net, x, need, *params):
         # `need` is decided by the caller: grad mode is always off inside Function.forward
         out, st = unet_forward(net, x, need_bwd=need, update_stats=net.training)
-        ctx.net, ctx.st = net, st
+        ctx.net, ctx.st, ctx.x_dtype = net, st, x.dtype
         ctx.names = unet_param_names(net)
         return out
 
     @staticmethod
     def backward(ctx, gout):
-        grads = unet_backward(ctx.net, ctx.st, gout)
-        return (None, None, None) + tuple(grads[k] for k in ctx.names)
+        if not ctx.needs_input_grad[1]:
+            grads = unet_backward(ctx.net, ctx.st, gout)
+            return (None, None, None) + tuple(grads[k] for k in ctx.names)
+        grads, dx = unet_backward(ctx.net, ctx.st, gout, need_dx=True)
+        return (None, dx.to(ctx.x_dtype), None) + tuple(grads[k] for k in ctx.names)
 
 
 # --------------------------------------------------------------------------------------------
@@ -599,6 +622,8 @@ def layoutnet_forward(net, x, need_bwd=True):
         last = li == len(LAYOUT_SPEC) - 1
         y = _empty(B * h * w, cout, dev=dev)
         rec = dict(x=cur, y=y, cin=cin, cout=cout, k=k, H=h, W=w, pool=None, name=f"encode.{idx}")
+        if li == 0:                                       # for the gradient w.r.t. the input image
+            rec["w"] = conv.weight.detach().float().contiguous()
         if _tma_kxk_ok(B, h, w, cin, cout, k):
             # bf16 mode: TMA-fed tcgen05 k x k convolution; the bf16 copy of x is kept for the weight gradient
             xb = _to_bf16(cur, cin, B * h * w, cin)
@@ -629,7 +654,9 @@ def layoutnet_forward(net, x, need_bwd=True):
     return (out[0] if squeeze else out), st
 
 
-def layoutnet_backward(net, st, gout):
+def layoutnet_backward(net, st, gout, need_dx=False):
+    """gout: the output's gradient.  Returns {state_dict-style name: gradient}; with ``need_dx`` (grads, dx), dx the
+    gradient w.r.t. the input image in its layout: (B,2,H,W), or (2,H,W) for a 3-D input."""
     _enter(net)
     B, mode, ws = st["B"], st["mode"], st["ws"]
     dev = gout.device
@@ -671,18 +698,27 @@ def layoutnet_backward(net, st, gout):
             else:
                 _conv(dy, cout, B, h, w, cout, cin, k, r["wb"], None, dx, cin)
             g = dx
-    return grads
+        elif need_dx:
+            # encode.0 (Cin = 2) never takes the TMA route (_tma_kxk_ok): its dy is fp32
+            dimg = _empty(B, cin, h, w, dev=dev)
+            call("tm_conv_dgrad_narrow", B, h, w, cin, cout, k, dy, cout, 0, r["w"], dimg, stream())
+    if not need_dx:
+        return grads
+    return grads, (dimg[0] if st["squeeze"] else dimg)
 
 
 class LayoutNetFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, net, x, need, *params):
         out, st = layoutnet_forward(net, x, need_bwd=need)
-        ctx.net, ctx.st = net, st
+        ctx.net, ctx.st, ctx.x_dtype = net, st, x.dtype
         ctx.names = [k for k, _ in net.named_parameters()]
         return out
 
     @staticmethod
     def backward(ctx, gout):
-        grads = layoutnet_backward(ctx.net, ctx.st, gout)
-        return (None, None, None) + tuple(grads[k] for k in ctx.names)
+        if not ctx.needs_input_grad[1]:
+            grads = layoutnet_backward(ctx.net, ctx.st, gout)
+            return (None, None, None) + tuple(grads[k] for k in ctx.names)
+        grads, dx = layoutnet_backward(ctx.net, ctx.st, gout, need_dx=True)
+        return (None, dx.to(ctx.x_dtype), None) + tuple(grads[k] for k in ctx.names)
