@@ -80,6 +80,9 @@ struct Carver {
 #ifdef __CUDACC__
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ float4 f4add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+__device__ __forceinline__ float4 f4scale(float4 a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
+__device__ __forceinline__ float4 f4relu(float4 a) { return make_float4(fmaxf(a.x, 0.f), fmaxf(a.y, 0.f), fmaxf(a.z, 0.f), fmaxf(a.w, 0.f)); }
 // streaming 128-bit load that does not allocate in L1 (rows read once per kernel)
 __device__ __forceinline__ float4 ld4_stream(const float* p) {
   float4 r;

@@ -21,8 +21,11 @@
 #include <stdlib.h>
 
 #include "tm_common.cuh"
+#include "tm_sm100.cuh"
+#include "tm_split.cuh"
 
 using namespace tmk;
+using namespace tmk::sm100;
 
 namespace {
 constexpr int D = 128;     // out_feat_dim (model.py:43, options.py:10)
@@ -36,10 +39,6 @@ constexpr int CT = 256;    // threads per CTA on a cell level (8 warps: two per 
 // the previous grid has completed and its writes are visible.
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-__device__ __forceinline__ float4 f4add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
-__device__ __forceinline__ float4 f4scale(float4 a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
-__device__ __forceinline__ float4 f4relu(float4 a) { return make_float4(fmaxf(a.x, 0.f), fmaxf(a.y, 0.f), fmaxf(a.z, 0.f), fmaxf(a.w, 0.f)); }
 
 // ---------------------------------------------------------------------------------------------
 // forward, level 0 and odd (net) levels: one warp per pin
@@ -162,27 +161,24 @@ __global__ void gnn_pack_kernel(const float* __restrict__ src, int R, int C, flo
   dst[i] = (c < C) ? src[(size_t)r * C + c] : 0.f;
 }
 
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
 // one elected thread: chunk c of the packed weights -> ring slot c % NSTAGE, completion on wfull
 __device__ __forceinline__ void issue_chunk(const Tiles& T, const float* __restrict__ Wa,
                                             const float* __restrict__ Wb, int c) {
   if (c >= NCHUNK) return;
   const float* src = (c < 8) ? Wa + (size_t)c * CHUNK_A : Wb + (size_t)(c - 8) * CHUNK_B;
   const uint32_t bytes = (uint32_t)((c < 8 ? CHUNK_A : CHUNK_B) * sizeof(float));
-  const uint32_t bar = smem_addr(&T.wfull[c % NSTAGE]), dst = smem_addr(T.wbuf + (c % NSTAGE) * SLOT);
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+  mbar_expect_tx(&T.wfull[c % NSTAGE], bytes);
+  bulk_copy_g2s(smem_u32(T.wbuf + (c % NSTAGE) * SLOT), src, bytes, &T.wfull[c % NSTAGE]);
 }
+// A lost bulk copy traps after 2^24 probes.  Unlike mbar_wait_trap, the bound is tested before the exit: with
+// mbar_wait_trap's order the compiler reschedules the cell kernels, and the config-2 design step measured 1% slower
+// (one B200 at 1000 W).
 __device__ __forceinline__ void wait_chunk(const Tiles& T, int c) {
-  const uint32_t bar = smem_addr(&T.wfull[c % NSTAGE]), parity = (uint32_t)(c / NSTAGE) & 1u;
-  uint32_t done = 0;
+  const uint32_t bar = smem_u32(&T.wfull[c % NSTAGE]), parity = (uint32_t)(c / NSTAGE) & 1u;
+  bool done = false;
   for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (spin > (1u << 24)) __trap();      // a lost bulk copy must fail the launch, not hang the GPU
+    done = mbar_try_wait(bar, parity);
+    if (spin > (1u << 24)) __trap();
   }
 }
 
@@ -190,10 +186,9 @@ __device__ __forceinline__ void wait_chunk(const Tiles& T, int c) {
 __device__ __forceinline__ void mlp_prologue(const Tiles& T, const float* Wa, const float* Wb, int tid) {
   if (tid == 0) {
 #pragma unroll
-    for (int i = 0; i < NSTAGE; ++i)
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&T.wfull[i])));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    for (int i = 0; i < NSTAGE; ++i) mbar_init(&T.wfull[i], 1);
+    fence_mbarrier_init();
+    fence_async_smem();
 #pragma unroll
     for (int c = 0; c < NSTAGE - 1; ++c) issue_chunk(T, Wa, Wb, c);
   }
@@ -284,37 +279,16 @@ __device__ __forceinline__ void mlp_tile(const Tiles& T, const float* Wa, const 
 }
 
 // =============================================================================================
-// fp16 two-term split variant of the tile MLP (TM_GNN_CELL_MATH=h16, round 2; see tm_gnn_persist.cu):
-//   x s = hi + lo,  hi = fp16(x s),  lo' = fp16((x s - hi) 2^11),  s = per-pin power of two (row maximum -> [1, 2))
-//   acc_main += hi hi;  acc_corr += hi lo' + lo' hi;  result = (acc_main + 2^-11 acc_corr) / s
+// fp16 two-term split variant of the tile MLP (TM_GNN_CELL_MATH=h16, round 2): the split of tm_split.cuh, per-pin scale,
 // on mma.sync.m16n8k16 (f16 operands, fp32 accumulate): 3 tensor instructions per k16 step and n-tile instead of the 6 of
 // 3xTF32 (m16n8k8), and the operand fragments are single 32-bit shared-memory words (half2 k-pairs), no on-the-fly split.
 // The weights are packed ONCE per call into the same chunk geometry as the fp32 path (so the cp.async.bulk ring is
 // unchanged): chunk c < 8 = k16 step c of Wa as [plane hi | lo'][8 k-pairs][264 words], chunk 8 + c = two k16 steps of
 // Wb as [plane][16 k-pairs][136 words].
 // =============================================================================================
-constexpr float LO_SCALE = 2048.f, LO_INV = 1.f / 2048.f;
-__device__ __forceinline__ void split_h(float x, __half& hi, __half& lo) {
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * LO_SCALE);
-}
-__device__ __forceinline__ uint32_t pack_h2(__half a, __half b) {
-  return (uint32_t)__half_as_ushort(a) | ((uint32_t)__half_as_ushort(b) << 16);
-}
-__device__ __forceinline__ void row_scale(float rowmax, int emin, float& sc, float& inv) {
-  int e = (int)((__float_as_uint(rowmax) >> 23) & 0xffu) - 127;
-  e = max(emin, min(e, 100));
-  sc = __uint_as_float((uint32_t)(127 - e) << 23);
-  inv = __uint_as_float((uint32_t)(127 + e) << 23);
-}
-__device__ __forceinline__ float warp_max_f(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 // one tile row (this lane: channels 4 lane .. 4 lane + 3) -> scale, split, half2 planes
 __device__ __forceinline__ void store_row_h(const Tiles& T, int row, int lane, float4 x, int emin) {
-  const float rm = warp_max_f(fmaxf(fmaxf(fabsf(x.x), fabsf(x.y)), fmaxf(fabsf(x.z), fabsf(x.w))));
+  const float rm = warp_max(fmaxf(fmaxf(fabsf(x.x), fabsf(x.y)), fmaxf(fabsf(x.z), fabsf(x.w))));
   float sc, inv;
   row_scale(rm, emin, sc, inv);
   __half h0, h1, h2, h3, l0, l1, l2, l3;

@@ -17,11 +17,9 @@
 // still spreads over every SM.  The two partial out^T tiles are exchanged through distributed shared
 // memory (each CTA finalises half of the tile's pins).
 //
-// Arithmetic: fp16 two-term split, the exact analogue of 3xTF32 at half the bytes.  x*s = hi + lo
-// with hi = fp16(x*s), lo' = fp16((x*s - hi) * 2^11); s is a per-pin power of two that brings the
-// row's largest magnitude into [1, 2) (exact, undone in the epilogue), so gradients of any size keep
-// 22 significant bits.  acc_main += hi*hi; acc_corr += hi*lo' + lo'*hi (both fp32 in TMEM);
-// result = acc_main + acc_corr * 2^-11: ~22-bit products, fp32 accumulation.
+// Arithmetic: the fp16 two-term split (tm_split.cuh), the exact analogue of 3xTF32 at half the bytes,
+// with a per-pin scale, so gradients of any size keep 22 significant bits; acc_main and acc_corr are
+// both fp32 in TMEM.
 //
 // Net levels / level 0 (mean over net in-edges) are processed by sub-warp groups (8 / 16 / 32 lanes
 // per pin, chosen per level so that every pin gets its own group when the level fits).
@@ -29,8 +27,11 @@
 #include <cuda_fp16.h>
 
 #include "tm_common.cuh"
+#include "tm_sm100.cuh"
+#include "tm_split.cuh"
 
 using namespace tmk;
+using namespace tmk::sm100;
 
 namespace {
 constexpr int D = 128;
@@ -55,16 +56,12 @@ static_assert(2 * B_PLANE >= NMAX * D * 4, "backward scratch must fit the operan
 static_assert(SMEM_BYTES <= 232448, "shared memory budget");
 
 constexpr uint32_t TM_MAIN1 = 0, TM_CORR1 = 128, TM_MAIN2 = 256, TM_CORR2 = 384, TM_COLS = 512;
-constexpr float LO_SCALE = 2048.f, LO_INV = 1.f / 2048.f;
+constexpr uint32_t MBAR_SPINS = 1u << 22;         // mbarrier waits trap after this many probes
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ float4 ldcg4(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ float4 f4zero() { return make_float4(0.f, 0.f, 0.f, 0.f); }
-__device__ __forceinline__ float4 f4add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
 __device__ __forceinline__ float4 f4fma(float4 a, float s, float4 c) { return make_float4(fmaf(a.x, s, c.x), fmaf(a.y, s, c.y), fmaf(a.z, s, c.z), fmaf(a.w, s, c.w)); }
-__device__ __forceinline__ float4 f4scale(float4 a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
-__device__ __forceinline__ float4 f4relu(float4 a) { return make_float4(fmaxf(a.x, 0.f), fmaxf(a.y, 0.f), fmaxf(a.z, 0.f), fmaxf(a.w, 0.f)); }
 __device__ __forceinline__ float4 relu_mask(float4 hv, float4 g) {
   return make_float4(hv.x > 0.f ? g.x : 0.f, hv.y > 0.f ? g.y : 0.f, hv.z > 0.f ? g.z : 0.f, hv.w > 0.f ? g.w : 0.f);
 }
@@ -120,70 +117,14 @@ __device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) {
   asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
 }
 
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-    if (done) return;
-    if (spin > (1u << 22)) __trap();       // a tensor-core fault must fail the launch, not hang the GPU
-  }
-}
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// ---------------------------------------------------------------------------------------------
-// tcgen05
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {   // one full warp
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols));
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {     // same warp
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols));
-}
-// shared-memory matrix descriptor, SWIZZLE_NONE, K-major (see tm_tc.cuh: make_desc)
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46);
-}
-// kind::f16 instruction descriptor: D = f32, A = B = fp16 (format 0), both K-major, M = 128, N = n
-__device__ __forceinline__ uint32_t make_idesc_f16(int n) {
-  return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-
 // one product  acc = W (128 x 128, resident planes) . tile^T (N x 128, pin planes):  8 k-steps of
 // 16, three MMAs each (hi*hi -> main; hi*lo' + lo'*hi -> corr), then one commit.  One thread.
 __device__ __forceinline__ void issue_gemm(uint32_t w_hi, uint32_t w_lo, uint32_t b_hi, uint32_t b_lo, uint32_t t_main,
                                            uint32_t t_corr, uint32_t idesc, uint64_t* bar) {
 #pragma unroll
   for (int ks = 0; ks < 8; ++ks) {
-    const uint64_t ah = make_desc(w_hi + ks * 2 * W_LBO, W_LBO, W_SBO), al = make_desc(w_lo + ks * 2 * W_LBO, W_LBO, W_SBO);
-    const uint64_t bh = make_desc(b_hi + ks * 2 * B_LBO, B_LBO, B_SBO), bl = make_desc(b_lo + ks * 2 * B_LBO, B_LBO, B_SBO);
+    const uint64_t ah = smem_desc(w_hi + ks * 2 * W_LBO, W_LBO, W_SBO), al = smem_desc(w_lo + ks * 2 * W_LBO, W_LBO, W_SBO);
+    const uint64_t bh = smem_desc(b_hi + ks * 2 * B_LBO, B_LBO, B_SBO), bl = smem_desc(b_lo + ks * 2 * B_LBO, B_LBO, B_SBO);
     umma_f16(t_main, ah, bh, idesc, ks > 0);
     umma_f16(t_corr, ah, bl, idesc, ks > 0);
     umma_f16(t_corr, al, bh, idesc, 1u);
@@ -191,35 +132,6 @@ __device__ __forceinline__ void issue_gemm(uint32_t w_hi, uint32_t w_lo, uint32_
   umma_commit(bar);
 }
 
-// ---------------------------------------------------------------------------------------------
-// fp16 two-term split
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void split_h(float x, __half& hi, __half& lo) {
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * LO_SCALE);
-}
-__device__ __forceinline__ uint32_t pack_h2(__half a, __half b) {
-  return (uint32_t)__half_as_ushort(a) | ((uint32_t)__half_as_ushort(b) << 16);
-}
-__device__ __forceinline__ void split_h4(float4 x, uint2& hi, uint2& lo) {
-  __half h0, h1, h2, h3, l0, l1, l2, l3;
-  split_h(x.x, h0, l0); split_h(x.y, h1, l1); split_h(x.z, h2, l2); split_h(x.w, h3, l3);
-  hi = make_uint2(pack_h2(h0, h1), pack_h2(h2, h3));
-  lo = make_uint2(pack_h2(l0, l1), pack_h2(l2, l3));
-}
-// power-of-two scale of a row whose largest magnitude is rowmax: s = 2^-e, inv = 2^e, e = floor(log2(rowmax))
-// clamped to [emin, 100]
-__device__ __forceinline__ void row_scale(float rowmax, int emin, float& s, float& inv) {
-  int e = (int)((__float_as_uint(rowmax) >> 23) & 0xffu) - 127;
-  e = max(emin, min(e, 100));
-  s = __uint_as_float((uint32_t)(127 - e) << 23);
-  inv = __uint_as_float((uint32_t)(127 + e) << 23);
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
 __device__ __forceinline__ uint32_t pin_off(int row, int k) {       // byte offset inside a pin plane
   return (uint32_t)(row >> 3) * B_SBO + (uint32_t)(k >> 3) * B_LBO + (uint32_t)(row & 7) * 16 + (uint32_t)(k & 7) * 2;
 }
@@ -295,7 +207,7 @@ template <class Pre1, class Epi1, class Pre2>
 __device__ __forceinline__ void mlp_tile(Ctx& c, int N, Pre1 pre1, Epi1 epi1, Pre2 pre2) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t sW = smem_u32(c.smem + OFF_W), sB = smem_u32(c.smem + OFF_B);
-  const uint32_t idesc = make_idesc_f16(N);
+  const uint32_t idesc = make_idesc(Fmt::F16, N);
   const int qd = warp & 3, cg = warp >> 2, m = qd * 32 + lane, nper = N >> 2;
   const uint32_t tl = c.tmem + ((uint32_t)(qd * 32) << 16);
   fence_async_smem();                    // the pin planes were written through the generic proxy
@@ -307,7 +219,7 @@ __device__ __forceinline__ void mlp_tile(Ctx& c, int N, Pre1 pre1, Epi1 epi1, Pr
     issue_gemm(sW, sW + W_PLANE, sB, sB + B_PLANE, c.tmem + TM_MAIN1, c.tmem + TM_CORR1, idesc, c.mbar);
   }
   pre1();
-  mbar_wait(c.mbar, c.mphase);
+  mbar_wait_trap<MBAR_SPINS>(c.mbar, c.mphase);
   c.mphase ^= 1u;
   tc_fence_after();
   c.stamp(PH_MMA1);
@@ -340,7 +252,7 @@ __device__ __forceinline__ void mlp_tile(Ctx& c, int N, Pre1 pre1, Epi1 epi1, Pr
     issue_gemm(sW + 2 * W_PLANE, sW + 3 * W_PLANE, sB, sB + B_PLANE, c.tmem + TM_MAIN2, c.tmem + TM_CORR2, idesc, c.mbar);
   }
   pre2();
-  mbar_wait(c.mbar, c.mphase);
+  mbar_wait_trap<MBAR_SPINS>(c.mbar, c.mphase);
   c.mphase ^= 1u;
   tc_fence_after();
   c.stamp(PH_MMA2);
@@ -411,18 +323,17 @@ __device__ __forceinline__ void ctx_setup(Ctx& c, uint8_t* smem, const uint8_t* 
   if (warp == 0) tmem_alloc(slot, TM_COLS);
   if (tid == 32) {
     mbar_init(c.mbar, 1);
+    fence_mbarrier_init();
     mbar_init(wbar, 1);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    const uint32_t bar = smem_u32(wbar);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(4u * W_PLANE) : "memory");
+    fence_mbarrier_init();
+    fence_async_smem();
+    mbar_expect_tx(wbar, 4u * W_PLANE);
 #pragma unroll
     for (int i = 0; i < 4; ++i)
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(smem_u32(smem + OFF_W + i * W_PLANE)), "l"(planes + (size_t)c.rank * 4 * W_PLANE + (size_t)i * W_PLANE),
-                     "r"(W_PLANE), "r"(bar) : "memory");
+      bulk_copy_g2s(smem_u32(smem + OFF_W + i * W_PLANE), planes + (size_t)c.rank * 4 * W_PLANE + (size_t)i * W_PLANE, W_PLANE, wbar);
   }
   __syncthreads();                       // the barriers are initialised
-  mbar_wait(wbar, 0);                    // the weights have landed (async proxy: what the MMAs read through)
+  mbar_wait_trap<MBAR_SPINS>(wbar, 0);   // the weights have landed (async proxy: what the MMAs read through)
   fence_async_smem();
   tc_fence_before();
   __syncthreads();

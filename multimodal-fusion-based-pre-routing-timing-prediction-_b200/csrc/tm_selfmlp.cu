@@ -6,9 +6,8 @@
 //
 // Why a kernel of its own: the generic streaming GEMM (tm_tc.cuh) is bound by the shared-memory traffic of fp32-sized
 // operands -- 2 100 cycles per 32-wide k-block, 266 us for this product.  Here
-//   * operands are the fp16 two-term split of tm_gnn_persist.cu (x s = hi + lo, lo' = fp16((x s - hi) 2^11), per-row
-//     power-of-two scale s; hi hi -> acc_main, hi lo' + lo' hi -> acc_corr, result = (main + 2^-11 corr) / s: ~22-bit
-//     products at the fp16 MMA rate and half the operand bytes);
+//   * operands are the fp16 two-term split (tm_split.cuh) with a per-row scale: ~22-bit products at the fp16 MMA rate
+//     and half the operand bytes;
 //   * W2 is split ONCE (tm_selfmlp_pack) and stays resident in shared memory (2 x 64 KB planes), so a k-step reads
 //     8 KB instead of 24 KB and nothing is re-staged per tile;
 //   * the per-row scale comes from a bound (|x0| max|w0| + |x1| max|w1| + max|b1| >= every hidden unit of the row), so
@@ -21,8 +20,11 @@
 #include <stdlib.h>
 
 #include "tm_common.cuh"
+#include "tm_sm100.cuh"
+#include "tm_split.cuh"
 
 using namespace tmk;
+using namespace tmk::sm100;
 
 namespace tmk {   // tm_gemm.cu: C[m][n] (+)= sum_k P[k][m*N + n], fixed order
 __global__ void split_reduce_kernel(const float* __restrict__ P, int64_t count, int splits, float* __restrict__ C, int64_t N,
@@ -53,90 +55,7 @@ constexpr uint32_t OFF_BAR = OFF_P + (3 * HIDF + NOUT + 4) * 4;
 constexpr uint32_t SMEM_BYTES = OFF_BAR + 16 * 8 + 16;
 static_assert(SMEM_BYTES <= 232448, "shared memory budget");
 constexpr uint32_t TM_COLS = 512;                          // [acc buffer 2][main 128 | corr 128]
-constexpr float LO_SCALE = 2048.f, LO_INV = 1.f / 2048.f;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  for (uint32_t spin = 0;; ++spin) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-    if (done) return;
-    if (spin > (1u << 22)) __trap();       // a lost arrival must fail the launch, not hang the GPU
-  }
-}
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {   // one full warp
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols));
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {     // same warp
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols));
-}
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46);
-}
-// kind::f16 instruction descriptor: D = f32, A = B = fp16 (format 0), both K-major, M = 128, N = n
-__device__ __forceinline__ uint32_t make_idesc_f16(int n) {
-  return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,"
-      "%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-        "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-        "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void split_h(float x, __half& hi, __half& lo) {
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * LO_SCALE);
-}
-// Two values in [0, 2) -> packed (hi, hi) and (lo', lo') words.  hi is taken by Veltkamp's splitting (x rounded to 11
-// significant bits in fp32: exactly an fp16 number when x >= 2^-14) so that only TWO packed conversions are issued
-// per pair instead of six scalar ones -- the conversions, not the FMAs, bounded the generator; below 2^-14 the
-// conversion of hi rounds once more, by at most 2^-25 of the row's scale.
-__device__ __forceinline__ void split_pair(float y0, float y1, uint32_t& hi, uint32_t& lo) {
-  const float C = 8193.f;                                     // 2^13 + 1
-  const float t0 = __fmul_rn(y0, C), t1 = __fmul_rn(y1, C);
-  const float h0 = __fsub_rn(t0, __fsub_rn(t0, y0)), h1 = __fsub_rn(t1, __fsub_rn(t1, y1));
-  const __half2 hh = __floats2half2_rn(h0, h1);
-  const __half2 ll = __floats2half2_rn(__fmul_rn(__fsub_rn(y0, h0), LO_SCALE), __fmul_rn(__fsub_rn(y1, h1), LO_SCALE));
-  hi = *reinterpret_cast<const uint32_t*>(&hh);
-  lo = *reinterpret_cast<const uint32_t*>(&ll);
-}
-// s = 2^-e, inv = 2^e with 2^e <= bound < 2^(e+1): every |value| <= bound lands in [0, 2) after scaling
-__device__ __forceinline__ void bound_scale(float bound, float& s, float& inv) {
-  int e = (int)((__float_as_uint(bound) >> 23) & 0xffu) - 127;
-  e = max(-100, min(e, 100));
-  s = __uint_as_float((uint32_t)(127 - e) << 23);
-  inv = __uint_as_float((uint32_t)(127 + e) << 23);
-}
+constexpr uint32_t MBAR_SPINS = 1u << 22;                  // mbarrier waits trap after this many probes
 
 // W2 [NOUT][HIDF] fp32 (nn.Linear layout: K-major as it is) -> the shared-memory image of the (hi, lo') planes
 __global__ void selfmlp_pack_kernel(const float* __restrict__ W2, uint8_t* __restrict__ out) {
@@ -192,15 +111,12 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_fwd_kernel(Args a) {
       mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], EPI_W);
     }
     mbar_init(wbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     fence_async_smem();
     // resident weight planes: 128 KB in four bulk copies
-    const uint32_t bar = smem_u32(wbar);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(2 * W_PLANE) : "memory");
+    mbar_expect_tx(wbar, 2 * W_PLANE);
     for (int i = 0; i < 4; ++i)
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(smem_u32(smem + OFF_W + i * (W_PLANE / 2))), "l"(a.wplanes + (size_t)i * (W_PLANE / 2)), "r"(W_PLANE / 2), "r"(bar)
-                   : "memory");
+      bulk_copy_g2s(smem_u32(smem + OFF_W + i * (W_PLANE / 2)), a.wplanes + (size_t)i * (W_PLANE / 2), W_PLANE / 2, wbar);
   }
   for (int j = tid; j < HIDF; j += THREADS) {
     w0_s[j] = LOADED ? 0.f : a.W1[(size_t)j * a.kx];
@@ -255,7 +171,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_fwd_kernel(Args a) {
           const int64_t r = a.h_rows ? (int64_t)a.h_rows[m] : m;
           hp[i] = a.H + r * a.ldh + kq * 4;
           float inv;
-          bound_scale(a.rowmax[r], sc[i], inv);
+          row_scale(a.rowmax[r], -100, sc[i], inv);
         }
       }
       float4 cur[8], nxt[8];
@@ -271,7 +187,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_fwd_kernel(Args a) {
       for (int c = 0; c < NCH; ++c, ++g) {
         if (c + 1 < NCH) fetch(c + 1, nxt);
         const uint32_t buf = g & 1u;
-        mbar_wait(&h_empty[buf], ((g >> 1) & 1u) ^ 1u);
+        mbar_wait_trap<MBAR_SPINS>(&h_empty[buf], ((g >> 1) & 1u) ^ 1u);
         uint8_t* hi_p = smem + OFF_H + buf * 2 * H_PLANE + (uint32_t)(kq >> 1) * H_LBO + (uint32_t)(kq & 1) * 8;
         uint8_t* lo_p = hi_p + H_PLANE;
 #pragma unroll
@@ -314,12 +230,12 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_fwd_kernel(Args a) {
       for (int rb = 0; rb < 4; ++rb) {
         row_x(t * TM + rb * 32 + lane, x0[rb], x1[rb]);
         float inv;
-        bound_scale(fmaf(fabsf(x0[rb]), wm0, fmaf(fabsf(x1[rb]), wm1, bm)), sc[rb], inv);
+        row_scale(fmaf(fabsf(x0[rb]), wm0, fmaf(fabsf(x1[rb]), wm1, bm)), -100, sc[rb], inv);
       }
 #pragma unroll
       for (int c = 0; c < NCH; ++c, ++g) {
         const uint32_t buf = g & 1u;
-        mbar_wait(&h_empty[buf], ((g >> 1) & 1u) ^ 1u);       // the MMAs that read this buffer two chunks ago are done
+        mbar_wait_trap<MBAR_SPINS>(&h_empty[buf], ((g >> 1) & 1u) ^ 1u);       // the MMAs that read this buffer two chunks ago are done
         uint8_t* hi_p = smem + OFF_H + buf * 2 * H_PLANE + (uint32_t)gw * H_LBO;
         uint8_t* lo_p = hi_p + H_PLANE;
 #pragma unroll
@@ -344,26 +260,26 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_fwd_kernel(Args a) {
   } else if (warp == MMA_WARP) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      mbar_wait(wbar, 0);
-      const uint32_t idesc = make_idesc_f16(NOUT);
+      mbar_wait_trap<MBAR_SPINS>(wbar, 0);
+      const uint32_t idesc = make_idesc(Fmt::F16, NOUT);
       const uint32_t w_hi = smem_u32(smem + OFF_W), w_lo = w_hi + W_PLANE;
       uint32_t g = 0;
       int li = 0;
       for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++li) {
         const uint32_t ab = (uint32_t)li & 1u;
-        mbar_wait(&acc_empty[ab], (((uint32_t)li >> 1) & 1u) ^ 1u);   // the epilogue drained this accumulator pair
+        mbar_wait_trap<MBAR_SPINS>(&acc_empty[ab], (((uint32_t)li >> 1) & 1u) ^ 1u);   // the epilogue drained this accumulator pair
         tc_fence_after();
         const uint32_t t_main = tmem_base + ab * 256u, t_corr = t_main + 128u;
         for (int c = 0; c < NCH; ++c, ++g) {
           const uint32_t buf = g & 1u;
-          mbar_wait(&h_full[buf], (g >> 1) & 1u);
+          mbar_wait_trap<MBAR_SPINS>(&h_full[buf], (g >> 1) & 1u);
           tc_fence_after();
           const uint32_t h_hi = smem_u32(smem + OFF_H + buf * 2 * H_PLANE), h_lo = h_hi + H_PLANE;
 #pragma unroll
           for (int ks = 0; ks < KC / 16; ++ks) {
             const uint32_t wk = (uint32_t)(c * (KC / 8) + ks * 2) * W_LBO;
-            const uint64_t ah = make_desc(h_hi + ks * 2 * H_LBO, H_LBO, H_SBO), al = make_desc(h_lo + ks * 2 * H_LBO, H_LBO, H_SBO);
-            const uint64_t bh = make_desc(w_hi + wk, W_LBO, W_SBO), bl = make_desc(w_lo + wk, W_LBO, W_SBO);
+            const uint64_t ah = smem_desc(h_hi + ks * 2 * H_LBO, H_LBO, H_SBO), al = smem_desc(h_lo + ks * 2 * H_LBO, H_LBO, H_SBO);
+            const uint64_t bh = smem_desc(w_hi + wk, W_LBO, W_SBO), bl = smem_desc(w_lo + wk, W_LBO, W_SBO);
             const uint32_t acc = (c > 0 || ks > 0) ? 1u : 0u;
             umma_f16(t_main, ah, bh, idesc, acc);
             umma_f16(t_corr, ah, bl, idesc, acc);
@@ -384,15 +300,15 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_fwd_kernel(Args a) {
       float s, inv;
       if constexpr (LOADED) {
         s = 1.f; inv = 1.f;
-        if (m < a.M) bound_scale(a.rowmax[a.h_rows ? (int64_t)a.h_rows[m] : m], s, inv);
+        if (m < a.M) row_scale(a.rowmax[a.h_rows ? (int64_t)a.h_rows[m] : m], -100, s, inv);
       } else {
         float x0, x1;
         row_x(m, x0, x1);
-        bound_scale(fmaf(fabsf(x0), wm0, fmaf(fabsf(x1), wm1, bm)), s, inv);
+        row_scale(fmaf(fabsf(x0), wm0, fmaf(fabsf(x1), wm1, bm)), -100, s, inv);
       }
       float* op = nullptr;
       if (m < a.M) op = a.out + (a.out_rows ? (int64_t)a.out_rows[m] : m) * a.ldo;
-      mbar_wait(&acc_full[ab], ((uint32_t)li >> 1) & 1u);
+      mbar_wait_trap<MBAR_SPINS>(&acc_full[ab], ((uint32_t)li >> 1) & 1u);
       tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16) + ab * 256u;
 #pragma unroll 1
@@ -448,10 +364,6 @@ constexpr uint32_t WG_OFF_BAR = WG_OFF_X + 2 * 2 * WG_KS * 4;
 constexpr uint32_t WG_SMEM = WG_OFF_BAR + 8 * 8 + 16;
 static_assert(WG_SMEM <= 232448, "shared memory budget");
 
-__device__ __forceinline__ uint32_t make_idesc_f16_n(int n) {
-  return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
-
 // max |x0|, max |x1| over the rows (non-negative floats order like their bit patterns)
 __global__ void selfmlp_xmax_kernel(int64_t M, const float* __restrict__ X, int64_t ldx, const int* __restrict__ x_rows, int kx,
                                     unsigned int* __restrict__ out2) {
@@ -501,7 +413,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) selfmlp_gen_wgrad2_kernel(WgArg
   if (tid == 0) {
     for (int i = 0; i < 2; ++i) { mbar_init(&full[i], GEN_W + WG_TR_W); mbar_init(&empty[i], 1); }
     mbar_init(done, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == 0) tmem_alloc(tmem_slot, TM_COLS);
   if (warp == 1) {                                            // bounds of the first layer
@@ -524,25 +436,25 @@ __global__ void __launch_bounds__(WG_THREADS, 1) selfmlp_gen_wgrad2_kernel(WgArg
   const uint32_t tmem_base = *tmem_slot;
   // global operand scales (powers of two)
   float sg, ig, sh, ih;
-  bound_scale(fmaxf(a.gmax[0], 1e-37f), sg, ig);
-  bound_scale(fmaf(a.xmax[0], wmax_s[0], fmaf(a.xmax[1], wmax_s[1], wmax_s[2])), sh, ih);
+  row_scale(fmaxf(a.gmax[0], 1e-37f), -100, sg, ig);
+  row_scale(fmaf(a.xmax[0], wmax_s[0], fmaf(a.xmax[1], wmax_s[1], wmax_s[2])), -100, sh, ih);
 
   if (warp == 0) {
     // ======================= MMA issuer =======================
     if (lane == 0 && s1 > s0) {
-      const uint32_t idesc = make_idesc_f16_n(HIDF);
+      const uint32_t idesc = make_idesc(Fmt::F16, HIDF);
       const uint32_t t_main = tmem_base, t_corr = tmem_base + 256u;
       uint32_t g = 0;
       for (int64_t st = s0; st < s1; ++st, ++g) {
         const uint32_t buf = g & 1u;
-        mbar_wait(&full[buf], (g >> 1) & 1u);
+        mbar_wait_trap<MBAR_SPINS>(&full[buf], (g >> 1) & 1u);
         tc_fence_after();
         const uint32_t a_hi = smem_u32(smem + buf * WG_BUF), a_lo = a_hi + WG_A_PLANE;
         const uint32_t b_hi = a_hi + 2 * WG_A_PLANE, b_lo = b_hi + WG_B_PLANE;
 #pragma unroll
         for (int ks = 0; ks < WG_KS / 16; ++ks) {
-          const uint64_t ah = make_desc(a_hi + ks * 2 * WG_LBO, WG_LBO, WG_A_SBO), al = make_desc(a_lo + ks * 2 * WG_LBO, WG_LBO, WG_A_SBO);
-          const uint64_t bh = make_desc(b_hi + ks * 2 * WG_LBO, WG_LBO, WG_SBO), bl = make_desc(b_lo + ks * 2 * WG_LBO, WG_LBO, WG_SBO);
+          const uint64_t ah = smem_desc(a_hi + ks * 2 * WG_LBO, WG_LBO, WG_A_SBO), al = smem_desc(a_lo + ks * 2 * WG_LBO, WG_LBO, WG_A_SBO);
+          const uint64_t bh = smem_desc(b_hi + ks * 2 * WG_LBO, WG_LBO, WG_SBO), bl = smem_desc(b_lo + ks * 2 * WG_LBO, WG_LBO, WG_SBO);
           const uint32_t acc = (g > 0 || ks > 0) ? 1u : 0u;
           umma_f16(t_main, ah, bh, idesc, acc);
           umma_f16(t_corr, ah, bl, idesc, acc);
@@ -561,7 +473,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) selfmlp_gen_wgrad2_kernel(WgArg
     uint32_t g = 0;
     for (int64_t st = s0; st < s1; ++st, ++g) {
       const uint32_t buf = g & 1u;
-      mbar_wait(&empty[buf], ((g >> 1) & 1u) ^ 1u);
+      mbar_wait_trap<MBAR_SPINS>(&empty[buf], ((g >> 1) & 1u) ^ 1u);
       float* xs = reinterpret_cast<float*>(smem + WG_OFF_X) + buf * 2 * WG_KS;
       if (j < WG_KS) {                                        // the step's inputs (rows past M: 0, and G is 0 there too)
         const int64_t r = st * WG_KS + j;
@@ -623,7 +535,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) selfmlp_gen_wgrad2_kernel(WgArg
     uint32_t g = 0;
     for (int64_t st = s0; st < s1; ++st, ++g) {
       const uint32_t buf = g & 1u;
-      mbar_wait(&empty[buf], ((g >> 1) & 1u) ^ 1u);
+      mbar_wait_trap<MBAR_SPINS>(&empty[buf], ((g >> 1) & 1u) ^ 1u);
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const int rg = tw + 4 * h;
@@ -652,7 +564,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) selfmlp_gen_wgrad2_kernel(WgArg
     const int q = warp & 3;
     float* prow = a.part + ((size_t)blockIdx.x * NOUT + (q * 32 + lane)) * HIDF;
     if (s1 > s0) {
-      mbar_wait(done, 0);
+      mbar_wait_trap<MBAR_SPINS>(done, 0);
       tc_fence_after();
       const float unscale = ig * ih;
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);
@@ -773,14 +685,11 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
     mbar_init(a_full, GEN_W); mbar_init(a_empty, 1);
     for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], EPI_W); }
     mbar_init(wbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     fence_async_smem();
-    const uint32_t bar = smem_u32(wbar);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(2 * B1_W_PLANE) : "memory");
+    mbar_expect_tx(wbar, 2 * B1_W_PLANE);
     for (int i = 0; i < 4; ++i)
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(smem_u32(smem + B1_OFF_W + i * (B1_W_PLANE / 2))), "l"(a.wplanes + (size_t)i * (B1_W_PLANE / 2)),
-                     "r"(B1_W_PLANE / 2), "r"(bar) : "memory");
+      bulk_copy_g2s(smem_u32(smem + B1_OFF_W + i * (B1_W_PLANE / 2)), a.wplanes + (size_t)i * (B1_W_PLANE / 2), B1_W_PLANE / 2, wbar);
   }
   if constexpr (!STORE) {
     for (int j = tid; j < HIDF; j += THREADS) {
@@ -813,7 +722,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
     if ((int64_t)blockIdx.x < ntiles) fetch(blockIdx.x);
     uint32_t li = 0;
     for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++li) {
-      mbar_wait(a_empty, (li & 1u) ^ 1u);                      // the MMAs of the previous tile are done with the planes
+      mbar_wait_trap<MBAR_SPINS>(a_empty, (li & 1u) ^ 1u);                      // the MMAs of the previous tile are done with the planes
       uint8_t* hi_p = smem + B1_OFF_A + (uint32_t)(lane >> 1) * B1_A_LBO + (uint32_t)(lane & 1) * 8;
 #pragma unroll
       for (int e = 0; e < 16; ++e) {
@@ -823,7 +732,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) rm = fmaxf(rm, __shfl_xor_sync(0xffffffffu, rm, o));
         float sc, inv;
-        bound_scale(rm, sc, inv);
+        row_scale(rm, -100, sc, inv);
         uint32_t h0, l0, h1, l1;
         split_pair(x.x * sc, x.y * sc, h0, l0);
         split_pair(x.z * sc, x.w * sc, h1, l1);
@@ -840,23 +749,23 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
   } else if (warp == MMA_WARP) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      mbar_wait(wbar, 0);
-      const uint32_t idesc = make_idesc_f16(NOUT);             // N = 128 columns per half
+      mbar_wait_trap<MBAR_SPINS>(wbar, 0);
+      const uint32_t idesc = make_idesc(Fmt::F16, NOUT);             // N = 128 columns per half
       const uint32_t a_hi = smem_u32(smem + B1_OFF_A), a_lo = a_hi + B1_A_PLANE;
       const uint32_t w_hi = smem_u32(smem + B1_OFF_W), w_lo = w_hi + B1_W_PLANE;
       uint32_t li = 0;
       for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++li) {
-        mbar_wait(a_full, li & 1u);
+        mbar_wait_trap<MBAR_SPINS>(a_full, li & 1u);
         tc_fence_after();
         for (uint32_t half = 0; half < 2; ++half) {
-          mbar_wait(&acc_empty[half], (li & 1u) ^ 1u);         // the epilogue drained this half's accumulators
+          mbar_wait_trap<MBAR_SPINS>(&acc_empty[half], (li & 1u) ^ 1u);         // the epilogue drained this half's accumulators
           tc_fence_after();
           const uint32_t t_main = tmem_base + half * 256u, t_corr = t_main + 128u;
           const uint32_t wh = w_hi + half * 16u * B1_W_SBO, wl = w_lo + half * 16u * B1_W_SBO;
 #pragma unroll
           for (int ks = 0; ks < NOUT / 16; ++ks) {
-            const uint64_t ah = make_desc(a_hi + ks * 2 * B1_A_LBO, B1_A_LBO, B1_A_SBO), al = make_desc(a_lo + ks * 2 * B1_A_LBO, B1_A_LBO, B1_A_SBO);
-            const uint64_t bh = make_desc(wh + ks * 2 * 128u, 128u, B1_W_SBO), bl = make_desc(wl + ks * 2 * 128u, 128u, B1_W_SBO);
+            const uint64_t ah = smem_desc(a_hi + ks * 2 * B1_A_LBO, B1_A_LBO, B1_A_SBO), al = smem_desc(a_lo + ks * 2 * B1_A_LBO, B1_A_LBO, B1_A_SBO);
+            const uint64_t bh = smem_desc(wh + ks * 2 * 128u, 128u, B1_W_SBO), bl = smem_desc(wl + ks * 2 * 128u, 128u, B1_W_SBO);
             const uint32_t acc = ks > 0 ? 1u : 0u;
             umma_f16(t_main, ah, bh, idesc, acc);
             umma_f16(t_corr, ah, bl, idesc, acc);
@@ -882,7 +791,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
       }
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
-        mbar_wait(&acc_full[half], li & 1u);
+        mbar_wait_trap<MBAR_SPINS>(&acc_full[half], li & 1u);
         tc_fence_after();
         const float inv = inv_s[(li & 1u) * TM + warp * 32 + lane];
         const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)half * 256u;
@@ -936,7 +845,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
       __syncwarp();
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
-        mbar_wait(&acc_full[half], li & 1u);
+        mbar_wait_trap<MBAR_SPINS>(&acc_full[half], li & 1u);
         tc_fence_after();
         const float inv = inv_s[(li & 1u) * TM + warp * 32 + lane];   // (written before a_full of this tile was signalled)
         const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)half * 256u;
@@ -1035,14 +944,11 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_lin1_kernel(L1Args a) {
     mbar_init(a_full, L1_LOAD_W); mbar_init(a_empty, 1);
     for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], EPI_W); }
     mbar_init(wbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     fence_async_smem();
-    const uint32_t bar = smem_u32(wbar);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(2 * L1_W_PLANE) : "memory");
+    mbar_expect_tx(wbar, 2 * L1_W_PLANE);
     for (int i = 0; i < 2; ++i)
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(smem_u32(smem + L1_OFF_W + i * L1_W_PLANE)), "l"(a.wplanes + (size_t)i * L1_W_PLANE), "r"(L1_W_PLANE), "r"(bar)
-                   : "memory");
+      bulk_copy_g2s(smem_u32(smem + L1_OFF_W + i * L1_W_PLANE), a.wplanes + (size_t)i * L1_W_PLANE, L1_W_PLANE, wbar);
   }
   for (int j = tid; j < HIDF; j += THREADS) b1_s[j] = a.b1[j];
   if (warp == MMA_WARP) tmem_alloc(tmem_slot, TM_COLS);
@@ -1070,12 +976,12 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_lin1_kernel(L1Args a) {
     if ((int64_t)blockIdx.x < ntiles) fetch(blockIdx.x);
     uint32_t li = 0;
     for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++li) {
-      mbar_wait(a_empty, (li & 1u) ^ 1u);
+      mbar_wait_trap<MBAR_SPINS>(a_empty, (li & 1u) ^ 1u);
       float rm = 0.f;
 #pragma unroll
       for (int q = 0; q < L1_K / 4; ++q) rm = fmaxf(rm, fmaxf(fmaxf(fabsf(v[q].x), fabsf(v[q].y)), fmaxf(fabsf(v[q].z), fabsf(v[q].w))));
       float sc, inv;
-      bound_scale(rm, sc, inv);
+      row_scale(rm, -100, sc, inv);
       uint8_t* hi_p = smem + L1_OFF_A + (uint32_t)(row >> 3) * L1_SBO + (uint32_t)(row & 7) * 16;
 #pragma unroll
       for (int kg = 0; kg < L1_K / 8; ++kg) {
@@ -1095,23 +1001,23 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_lin1_kernel(L1Args a) {
     }
   } else if (warp == MMA_WARP) {
     if (lane == 0) {
-      mbar_wait(wbar, 0);
-      const uint32_t idesc = make_idesc_f16(NOUT);
+      mbar_wait_trap<MBAR_SPINS>(wbar, 0);
+      const uint32_t idesc = make_idesc(Fmt::F16, NOUT);
       const uint32_t a_hi = smem_u32(smem + L1_OFF_A), a_lo = a_hi + L1_A_PLANE;
       const uint32_t w_hi = smem_u32(smem + L1_OFF_W), w_lo = w_hi + L1_W_PLANE;
       uint32_t li = 0;
       for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++li) {
-        mbar_wait(a_full, li & 1u);
+        mbar_wait_trap<MBAR_SPINS>(a_full, li & 1u);
         tc_fence_after();
         for (uint32_t half = 0; half < 2; ++half) {
-          mbar_wait(&acc_empty[half], (li & 1u) ^ 1u);
+          mbar_wait_trap<MBAR_SPINS>(&acc_empty[half], (li & 1u) ^ 1u);
           tc_fence_after();
           const uint32_t t_main = tmem_base + half * 256u, t_corr = t_main + 128u;
           const uint32_t wh = w_hi + half * 16u * L1_SBO, wl = w_lo + half * 16u * L1_SBO;
 #pragma unroll
           for (int ks = 0; ks < L1_K / 16; ++ks) {
-            const uint64_t ah = make_desc(a_hi + ks * 256u, 128u, L1_SBO), al = make_desc(a_lo + ks * 256u, 128u, L1_SBO);
-            const uint64_t bh = make_desc(wh + ks * 256u, 128u, L1_SBO), bl = make_desc(wl + ks * 256u, 128u, L1_SBO);
+            const uint64_t ah = smem_desc(a_hi + ks * 256u, 128u, L1_SBO), al = smem_desc(a_lo + ks * 256u, 128u, L1_SBO);
+            const uint64_t bh = smem_desc(wh + ks * 256u, 128u, L1_SBO), bl = smem_desc(wl + ks * 256u, 128u, L1_SBO);
             const uint32_t acc = ks > 0 ? 1u : 0u;
             umma_f16(t_main, ah, bh, idesc, acc);
             umma_f16(t_corr, ah, bl, idesc, acc);
@@ -1132,7 +1038,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_lin1_kernel(L1Args a) {
       float rmax = 0.f;
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
-        mbar_wait(&acc_full[half], li & 1u);
+        mbar_wait_trap<MBAR_SPINS>(&acc_full[half], li & 1u);
         tc_fence_after();
         const float inv = inv_s[(li & 1u) * TM + warp * 32 + lane];
         const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)half * 256u;

@@ -28,6 +28,8 @@
 #include <stdlib.h>
 
 #include "tm_gemm.cuh"
+#include "tm_sm100.cuh"
+#include "tm_split.cuh"
 
 // Bottleneck-bisection switches (TM_TC_DEBUG bits) and the clock64 timeline (TM_TC_TRACE) are compiled
 // in only with -DTM_TC_INSTRUMENT=1 (make INSTRUMENT=1); production kernels carry none of it.
@@ -40,6 +42,8 @@
 namespace tmk {
 namespace tc {
 
+using namespace sm100;
+
 constexpr int BM = 128;
 constexpr int BK = 32;
 constexpr int EPI_WARPS = 4;        // warps 0..3: TMEM lane group = warp index
@@ -48,78 +52,6 @@ constexpr int PROD_WARP0 = 5;
 constexpr int PROD_WARPS = 8;
 constexpr int PROD_THREADS = PROD_WARPS * 32;
 constexpr int THREADS = (EPI_WARPS + 1 + PROD_WARPS) * 32;   // 416
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// Bounded wait: a tensor-core fault must not turn into a hung GPU.  Returns false on timeout or
-// when another role of the CTA already gave up (*abort != 0).
-__device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, volatile int* abort) {
-  const uint32_t addr = smem_u32(bar);
-  for (uint32_t spin = 0; spin < (1u << 24); ++spin) {
-    if ((spin & 1023u) == 1023u && *abort) return false;
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (done) return true;
-  }
-  return false;
-}
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {   // one full warp
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols));
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {     // same warp
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols));
-}
-
-// K-major, SWIZZLE_NONE shared-memory matrix descriptor (cute::UMMA::SmemDescriptor layout):
-//   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 (between the two 8-element k
-//   groups of one MMA) | [32,46) stride byte offset >> 4 (between 8-row groups) | [46,48) version 1
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) |
-         (1ull << 46);
-}
-// kind::f16 instruction descriptor: D = f32, A = B = bf16, both K-major, M = 128
-__host__ __device__ constexpr uint32_t make_idesc(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-}
-__device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
 
 // cp.async (LDGSTS): global -> shared without a register round trip; bytes past `nbytes` are
 // zero-filled, so out-of-matrix elements need no branch in the consumer
@@ -642,21 +574,6 @@ struct Cfg {
   static constexpr int B_CH = (BN * BK / 4 + PROD_THREADS - 1) / PROD_THREADS;   // 1..8
 };
 
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
 // tile index -> (m tile, n tile, k split): splits fastest, then n, so that concurrently running
 // CTAs share A rows through L2
 struct TileMap {
@@ -700,7 +617,7 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
     mbar_init(&acc_full[0], 1); mbar_init(&acc_full[1], 1);
     mbar_init(&acc_empty[0], EPI_WARPS); mbar_init(&acc_empty[1], EPI_WARPS);
     abort_s = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == MMA_WARP) tmem_alloc(&tmem_base_s, C::TMEM_COLS);
   tc_fence_before();
@@ -829,7 +746,7 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
     for (uint32_t g = 0; g < total; ++g) {
       if (tr_on && tr_n < 64) TM_TRACEPTR[tr_n * 4 + 0] = clock64();
       cp_async_wait<ND - 1>();                                         // my copies of k-block g have landed
-      if (!mbar_wait(&empty_bar[s], ph ^ 1u, abortp)) abort_s = 1;    // MMAs that read this stage are done
+      if (!mbar_wait_abort(&empty_bar[s], ph ^ 1u, abortp)) abort_s = 1;    // MMAs that read this stage are done
       if (COOP) asm volatile("bar.sync 1, %0;" ::"n"(PROD_THREADS) : "memory");   // everybody's copies landed
       else __syncwarp();
       if (*abortp) { ok = false; break; }                              // (uniform across the barrier)
@@ -869,13 +786,13 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
   } else if (warp == MMA_WARP) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(BN);
+      constexpr uint32_t idesc = make_idesc(Fmt::BF16, BN);
       uint32_t s = 0, ph = 0;
       int li = 0;
       for (int64_t t = blockIdx.x; t < tm.total && ok; t += G, ++li) {
         const int buf = li & 1;
         const uint32_t aph = (uint32_t)(li >> 1) & 1u;
-        ok = mbar_wait(&acc_empty[buf], aph ^ 1u, abortp);               // epilogue drained this accumulator
+        ok = mbar_wait_abort(&acc_empty[buf], aph ^ 1u, abortp);               // epilogue drained this accumulator
         if (!ok) break;
         tc_fence_after();
         int64_t m0, nq, kb0; int zi, nkb;
@@ -884,7 +801,7 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
         for (int kb = 0; kb < nkb; ++kb) {
           const bool tr_on = TM_TRACEPTR && blockIdx.x == 0 && li == 0 + (kb >> 6) && kb < 64;
           if (tr_on) TM_TRACEPTR[256 + kb * 4 + 0] = clock64();
-          ok = mbar_wait(&full_bar[s], ph, abortp);
+          ok = mbar_wait_abort(&full_bar[s], ph, abortp);
           if (!ok) break;
           tc_fence_after();
           if (tr_on) TM_TRACEPTR[256 + kb * 4 + 1] = clock64();
@@ -896,16 +813,16 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
             uint64_t da[PARTS], db[PARTS];
 #pragma unroll
             for (int p = 0; p < PARTS; ++p) {
-              da[p] = make_desc(sa + p * A_BYTES + koff, 128, 512);
-              db[p] = make_desc(sb + p * B_BYTES + koff, 128, 512);
+              da[p] = smem_desc(sa + p * A_BYTES + koff, 128, 512);
+              db[p] = smem_desc(sb + p * B_BYTES + koff, 128, 512);
             }
             // products in decreasing magnitude; parts: 0 = hi, 1 = mid, 2 = lo
-            umma(tmem_d, da[0], db[0], idesc, (kb > 0 || ks > 0) ? 1u : 0u);
-            if (PARTS >= 2) { umma(tmem_d, da[0], db[1], idesc, 1u); umma(tmem_d, da[1], db[0], idesc, 1u); }
+            umma_f16(tmem_d, da[0], db[0], idesc, (kb > 0 || ks > 0) ? 1u : 0u);
+            if (PARTS >= 2) { umma_f16(tmem_d, da[0], db[1], idesc, 1u); umma_f16(tmem_d, da[1], db[0], idesc, 1u); }
             if (PARTS >= 3) {
-              umma(tmem_d, da[1], db[1], idesc, 1u);
-              umma(tmem_d, da[0], db[2], idesc, 1u);
-              umma(tmem_d, da[2], db[0], idesc, 1u);
+              umma_f16(tmem_d, da[1], db[1], idesc, 1u);
+              umma_f16(tmem_d, da[0], db[2], idesc, 1u);
+              umma_f16(tmem_d, da[2], db[0], idesc, 1u);
             }
           }
           umma_commit(&empty_bar[s]);                                    // stage reusable once these MMAs retire
@@ -926,7 +843,7 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
       const uint32_t aph = (uint32_t)(li >> 1) & 1u;
       const bool tr_on = TM_TRACEPTR && blockIdx.x == 0 && warp == 0 && lane == 0 && li < 16;
       if (tr_on) TM_TRACEPTR[512 + li * 4 + 0] = clock64();
-      ok = mbar_wait(&acc_full[buf], aph, abortp);
+      ok = mbar_wait_abort(&acc_full[buf], aph, abortp);
       if (!ok) break;
       tc_fence_after();
       if (tr_on) TM_TRACEPTR[512 + li * 4 + 1] = clock64();
@@ -1007,35 +924,17 @@ tc_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
 // Both are written directly by 16-byte cp.async's (whole 128-byte lines per quarter warp in HBM
 // and in shared memory), so weight gradients (both operands transposed) need no transposition.
 // =============================================================================================
-constexpr uint32_t TF32_MASK = 0xFFFFE000u;
 // 16 producer warps: the copy phase is bound by cp.async issue and the lo pass by ALU latency, both of
 // which scale with the number of warps in flight (the kernel needs < 64 registers per thread)
 constexpr int TF_PROD_WARPS = 16;
 constexpr int TF_PROD_THREADS = TF_PROD_WARPS * 32;
 constexpr int TF_THREADS = (EPI_WARPS + 1 + TF_PROD_WARPS) * 32;   // 672
 
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int n, bool a_mn, bool b_mn) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
-         ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-}
-// swizzled descriptor, version 1; layout type (bits [61,64)): 2 = SWIZZLE_128B, 1 = SWIZZLE_128B_BASE32B
-__device__ __forceinline__ uint64_t make_desc_sw128(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t type = 2) {
-  return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) |
-         (1ull << 46) | ((uint64_t)type << 61);
-}
 // byte offset of the 16-byte chunk (k, rc) of an MN-major plane
 __device__ __forceinline__ uint32_t mn_chunk_off(int k, int rc) {
   const uint32_t j = (uint32_t)(rc & 7), k4 = (uint32_t)(k & 3);
   return (uint32_t)(rc >> 3) * 4096u + (uint32_t)(k >> 2) * 512u + k4 * 128u + (((((j >> 1) ^ k4) << 1) | (j & 1u)) << 4);
 }
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-
 template <int BN, int PLANES>
 struct TfCfg {
   static constexpr uint32_t PLANE_A = BM * BK * 4, PLANE_B = BN * BK * 4;
@@ -1071,7 +970,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
     mbar_init(&acc_full[0], 1); mbar_init(&acc_full[1], 1);
     mbar_init(&acc_empty[0], EPI_WARPS); mbar_init(&acc_empty[1], EPI_WARPS);
     abort_s = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
   }
   if (warp == MMA_WARP) tmem_alloc(&tmem_base_s, C::TMEM_COLS);
   tc_fence_before();
@@ -1144,7 +1043,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
     uint32_t ls = 0, lph = 0;                                        // slot / phase of the next k-block to load
     auto issue = [&]() -> bool {                                     // always commits exactly one group
       if (lvalid) {
-        if (!mbar_wait(&empty_bar[ls], lph ^ 1u, abortp)) return false;   // MMAs that read this slot are done
+        if (!mbar_wait_abort(&empty_bar[ls], lph ^ 1u, abortp)) return false;   // MMAs that read this slot are done
         if (!(TM_DBGBITS & 2)) {
           const uint32_t base = smem_u32(ring + (size_t)ls * SLOT);
 #pragma unroll
@@ -1183,13 +1082,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
       if (PLANES == 2 && !(TM_DBGBITS & 4)) {
         uint8_t* base = ring + (size_t)s * SLOT;
         auto residual = [&](uint32_t hi_off, uint32_t lo_off) {
-          const float4 x = *reinterpret_cast<const float4*>(base + hi_off);
-          float4 l;
-          l.x = x.x - __uint_as_float(__float_as_uint(x.x) & TF32_MASK);
-          l.y = x.y - __uint_as_float(__float_as_uint(x.y) & TF32_MASK);
-          l.z = x.z - __uint_as_float(__float_as_uint(x.z) & TF32_MASK);
-          l.w = x.w - __uint_as_float(__float_as_uint(x.w) & TF32_MASK);
-          *reinterpret_cast<float4*>(base + lo_off) = l;
+          *reinterpret_cast<float4*>(base + lo_off) = tf32_lo(*reinterpret_cast<const float4*>(base + hi_off));
         };
 #pragma unroll
         for (int j = 0; j < A_CH; ++j) residual(OFF_AHI + a_o[j], OFF_ALO + a_o[j]);
@@ -1210,7 +1103,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
   } else if (warp == MMA_WARP) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc_tf32(BN, AL::kTransposed, BL::kTransposed);
+      constexpr uint32_t idesc = make_idesc(Fmt::TF32, BN, AL::kTransposed, BL::kTransposed);
       // per MMA (K = 8): K-major advances 32 bytes inside the swizzle atom, MN-major two 512-byte k groups
       constexpr uint32_t A_KSTEP = AL::kTransposed ? 1024u : 32u, B_KSTEP = BL::kTransposed ? 1024u : 32u;
       constexpr uint32_t A_LBO = AL::kTransposed ? 4096u : 16u, B_LBO = BL::kTransposed ? 4096u : 16u;
@@ -1221,7 +1114,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
       for (int64_t t = blockIdx.x; t < tm.total && ok; t += G, ++li) {
         const int buf = li & 1;
         const uint32_t aph = (uint32_t)(li >> 1) & 1u;
-        ok = mbar_wait(&acc_empty[buf], aph ^ 1u, abortp);               // epilogue drained this accumulator
+        ok = mbar_wait_abort(&acc_empty[buf], aph ^ 1u, abortp);               // epilogue drained this accumulator
         if (!ok) break;
         tc_fence_after();
         int64_t m0, nq, kb0; int zi, nkb;
@@ -1230,7 +1123,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
         for (int kb = 0; kb < nkb; ++kb) {
           const bool tr_on = TM_TRACEPTR && blockIdx.x == 0 && li == 0 && kb < 64;
           if (tr_on) TM_TRACEPTR[256 + kb * 4 + 0] = clock64();
-          ok = mbar_wait(&full_bar[s], ph, abortp);
+          ok = mbar_wait_abort(&full_bar[s], ph, abortp);
           if (!ok) break;
           tc_fence_after();
           if (tr_on) TM_TRACEPTR[256 + kb * 4 + 1] = clock64();
@@ -1238,12 +1131,12 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
           if (!(TM_DBGBITS & 8))
 #pragma unroll
           for (int ks = 0; ks < BK / 8; ++ks) {
-            const uint64_t ah = make_desc_sw128(base + OFF_AHI + ks * A_KSTEP, A_LBO, A_SBO, A_TY);
-            const uint64_t bh = make_desc_sw128(base + OFF_BHI + ks * B_KSTEP, B_LBO, B_SBO, B_TY);
+            const uint64_t ah = smem_desc(base + OFF_AHI + ks * A_KSTEP, A_LBO, A_SBO, A_TY);
+            const uint64_t bh = smem_desc(base + OFF_BHI + ks * B_KSTEP, B_LBO, B_SBO, B_TY);
             umma_tf32(tmem_d, ah, bh, idesc, (kb > 0 || ks > 0) ? 1u : 0u);
             if (PLANES == 2) {
-              const uint64_t alo = make_desc_sw128(base + OFF_ALO + ks * A_KSTEP, A_LBO, A_SBO, A_TY);
-              const uint64_t blo = make_desc_sw128(base + OFF_BLO + ks * B_KSTEP, B_LBO, B_SBO, B_TY);
+              const uint64_t alo = smem_desc(base + OFF_ALO + ks * A_KSTEP, A_LBO, A_SBO, A_TY);
+              const uint64_t blo = smem_desc(base + OFF_BLO + ks * B_KSTEP, B_LBO, B_SBO, B_TY);
               umma_tf32(tmem_d, ah, blo, idesc, 1u);
               umma_tf32(tmem_d, alo, bh, idesc, 1u);
             }
@@ -1268,7 +1161,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
       for (int64_t t = blockIdx.x; t < tm.total && ok; t += G, ++li) {
         const int buf = li & 1;
         const uint32_t aph = (uint32_t)(li >> 1) & 1u;
-        ok = mbar_wait(&acc_full[buf], aph, abortp);
+        ok = mbar_wait_abort(&acc_full[buf], aph, abortp);
         if (!ok) break;
         tc_fence_after();
         int64_t m0, nq, kb0; int zi, nkb;
@@ -1367,7 +1260,7 @@ tf_gemm_kernel(AL al, BL bl, EP ep, int64_t M, int64_t N, TileMap tm, int* __res
     for (int64_t t = blockIdx.x; t < tm.total && ok; t += G, ++li) {
       const int buf = li & 1;
       const uint32_t aph = (uint32_t)(li >> 1) & 1u;
-      ok = mbar_wait(&acc_full[buf], aph, abortp);
+      ok = mbar_wait_abort(&acc_full[buf], aph, abortp);
       if (!ok) break;
       tc_fence_after();
       int64_t m0, nq, kb0; int zi, nkb;

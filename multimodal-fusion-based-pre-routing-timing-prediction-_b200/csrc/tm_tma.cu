@@ -92,9 +92,6 @@ int encode_2d(CUtensorMap* m, const void* ptr, int64_t C, int64_t rows, int boxC
 // ------------------------------------------------------------------------------------------------
 // device helpers
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3,
                                             uint64_t* bar) {
   asm volatile(
@@ -111,17 +108,8 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
 __device__ __forceinline__ void prefetch_map(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
-// shared-memory matrix descriptor, version 1.  type: 2 = SWIZZLE_128B, 4 = SWIZZLE_64B, 6 = SWIZZLE_32B
-__device__ __forceinline__ uint64_t make_desc_sw(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t type) {
-  return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) |
-         (1ull << 46) | ((uint64_t)type << 61);
-}
+// shared-memory descriptor layout of a swizzled row of inner_bytes: 2 = SWIZZLE_128B, 4 = SWIZZLE_64B, 6 = SWIZZLE_32B
 __host__ __device__ constexpr uint32_t sw_type(int inner_bytes) { return inner_bytes >= 128 ? 2u : inner_bytes == 64 ? 4u : 6u; }
-// kind::f16, D = f32, A = B = bf16, M = 128; a_mn / b_mn: operand is MN-major
-__host__ __device__ constexpr uint32_t idesc_bf16(int n, bool a_mn, bool b_mn) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
-         ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
 
 // Store one 16-column chunk of a 32-row accumulator slab.  After tcgen05.ld lane = row; writing from that layout
 // would touch 32 different lines with 16 bytes each per instruction.  The chunk is transposed through a padded
@@ -200,7 +188,7 @@ constexpr uint32_t FWD_SMEM_BUDGET = 184 * 1024;
 
 // Operand formats.  FMT_BF16: one bf16 plane per operand, kind::f16.  FMT_TF32X3: fp32 operands read in place by TMA
 // (tcgen05.mma.kind::tf32 uses the upper 19 bits of each word, so the fp32 word is the "hi" operand); the residual
-// lo = x - trunc_tf32(x), exact in fp32, is formed in shared memory next to it, and every 32-byte K chunk issues
+// lo = x - trunc_tf32(x) (tm_split.cuh) is formed in shared memory next to it, and every 32-byte K chunk issues
 // hi*hi + hi*lo + lo*hi into one fp32 accumulator -- the 3xTF32 product of tf_gemm_kernel (tm_tc.cuh).
 constexpr int FMT_BF16 = 0, FMT_TF32X3 = 1;
 // tf32x3 forward / data gradient: warps that form the lo planes of a stage once TMA has landed its hi planes
@@ -212,15 +200,7 @@ __device__ __forceinline__ void split_lo(uint8_t* st, uint32_t bytes, uint32_t l
   const float4* hi = reinterpret_cast<const float4*>(st);
   float4* lo = reinterpret_cast<float4*>(st + lo_off);
 #pragma unroll 4
-  for (int i = t; i < (int)(bytes >> 4); i += nthr) {
-    const float4 x = hi[i];
-    float4 l;
-    l.x = x.x - __uint_as_float(__float_as_uint(x.x) & TF32_MASK);
-    l.y = x.y - __uint_as_float(__float_as_uint(x.y) & TF32_MASK);
-    l.z = x.z - __uint_as_float(__float_as_uint(x.z) & TF32_MASK);
-    l.w = x.w - __uint_as_float(__float_as_uint(x.w) & TF32_MASK);
-    lo[i] = l;
-  }
+  for (int i = t; i < (int)(bytes >> 4); i += nthr) lo[i] = tf32_lo(hi[i]);
 }
 
 struct ConvArgs {
@@ -270,7 +250,7 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
     mbar_init(&acc_full[0], 1); mbar_init(&acc_full[1], 1);
     mbar_init(&acc_empty[0], FWD_EPI_WARPS); mbar_init(&acc_empty[1], FWD_EPI_WARPS);
     abort_s = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     prefetch_map(&tmx);
     prefetch_map(&tmw);
   }
@@ -308,7 +288,7 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
           const int dx = a.tdx[tap], dy = a.tdy[tap];
           for (int cs = 0; cs < csteps; ++cs) {
             if (TF && (tap * csteps + cs < k0 || tap * csteps + cs >= k1)) continue;
-            ok = mbar_wait(&empty_bar[s], ph ^ 1u, abortp);
+            ok = mbar_wait_abort(&empty_bar[s], ph ^ 1u, abortp);
             if (!ok) break;
             const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
             mbar_expect_tx(&full_bar[s], a.a_bytes + a.b_bytes);
@@ -323,7 +303,7 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
   } else if (warp == 1) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      const uint32_t idesc = TF ? make_idesc_tf32(N, false, false) : idesc_bf16(N, false, false);
+      const uint32_t idesc = TF ? make_idesc(Fmt::TF32, N) : make_idesc(Fmt::BF16, N);
       constexpr int RB = CK * (TF ? 4 : 2);                 // bytes per operand row; one MMA takes 32 of them
       constexpr uint32_t TY = sw_type(RB), SBO = 8u * RB;
       uint32_t s = 0, ph = 0;
@@ -332,27 +312,27 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
         int64_t t; int z, k0, k1;
         unit(u, t, z, k0, k1);
         const int buf = li & 1;
-        ok = mbar_wait(&acc_empty[buf], (((uint32_t)(li >> 1)) & 1u) ^ 1u, abortp);
+        ok = mbar_wait_abort(&acc_empty[buf], (((uint32_t)(li >> 1)) & 1u) ^ 1u, abortp);
         if (!ok) break;
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + (uint32_t)(buf * N);
         for (int ks = k0; ks < k1; ++ks) {
-          ok = mbar_wait(TF ? &lo_bar[s] : &full_bar[s], ph, abortp);
+          ok = mbar_wait_abort(TF ? &lo_bar[s] : &full_bar[s], ph, abortp);
           if (!ok) break;
           tc_fence_after();
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
 #pragma unroll
           for (int j = 0; j < RB / 32; ++j) {
-            const uint64_t da = make_desc_sw(base + j * 32, 16, SBO, TY);
-            const uint64_t db = make_desc_sw(base + a.a_bytes + j * 32, 16, SBO, TY);
+            const uint64_t da = smem_desc(base + j * 32, 16, SBO, TY);
+            const uint64_t db = smem_desc(base + a.a_bytes + j * 32, 16, SBO, TY);
             if (TF) {
-              const uint64_t dal = make_desc_sw(base + a.hi_bytes + j * 32, 16, SBO, TY);
-              const uint64_t dbl = make_desc_sw(base + a.hi_bytes + a.a_bytes + j * 32, 16, SBO, TY);
+              const uint64_t dal = smem_desc(base + a.hi_bytes + j * 32, 16, SBO, TY);
+              const uint64_t dbl = smem_desc(base + a.hi_bytes + a.a_bytes + j * 32, 16, SBO, TY);
               umma_tf32(tmem_d, da, db, idesc, (ks > k0 || j > 0) ? 1u : 0u);
               umma_tf32(tmem_d, da, dbl, idesc, 1u);
               umma_tf32(tmem_d, dal, db, idesc, 1u);
             } else {
-              umma(tmem_d, da, db, idesc, (ks > k0 || j > 0) ? 1u : 0u);
+              umma_f16(tmem_d, da, db, idesc, (ks > k0 || j > 0) ? 1u : 0u);
             }
           }
           umma_commit(&empty_bar[s]);
@@ -371,7 +351,7 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
       int64_t t; int z, k0, k1;
       unit(u, t, z, k0, k1);
       for (int ks = k0; ks < k1; ++ks) {
-        ok = mbar_wait(&full_bar[s], ph, abortp);
+        ok = mbar_wait_abort(&full_bar[s], ph, abortp);
         if (!ok) break;
         split_lo(ring + (size_t)s * a.stage_bytes, a.a_bytes + a.b_bytes, a.hi_bytes, rt, SPLIT_WARPS * 32);
         fence_async_smem();                                // generic stores -> async proxy (the MMAs)
@@ -396,7 +376,7 @@ conv3x3_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_constan
       unit(u, t, z, k0, k1);
       float* const yz = TF ? a.y + z * a.zstride : a.y;
       const int buf = li & 1;
-      ok = mbar_wait(&acc_full[buf], ((uint32_t)(li >> 1)) & 1u, abortp);
+      ok = mbar_wait_abort(&acc_full[buf], ((uint32_t)(li >> 1)) & 1u, abortp);
       if (!ok) break;
       tc_fence_after();
       int x0, y0, b0;
@@ -486,7 +466,7 @@ conv3x3_tma_rows_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_co
     mbar_init(&acc_empty[0], FWD_EPI_WARPS); mbar_init(&acc_empty[1], FWD_EPI_WARPS);
     mbar_init(&w_full, 1);
     abort_s = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     prefetch_map(&tmx);
     prefetch_map(&tmw);
   }
@@ -515,7 +495,7 @@ conv3x3_tma_rows_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_co
         const int b = (int)(t / ((int64_t)tiles_x * tiles_y));
         for (int iy = -1; iy <= ROWS && ok; ++iy) {
           for (int S = 0; S < 3; ++S) {
-            ok = mbar_wait(&empty_bar[s], ph ^ 1u, abortp);
+            ok = mbar_wait_abort(&empty_bar[s], ph ^ 1u, abortp);
             if (!ok) break;
             if (a.flags & 0x400) { mbar_arrive(&full_bar[s]); }
             else {
@@ -530,19 +510,19 @@ conv3x3_tma_rows_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_co
     __syncwarp();
   } else if (warp == 1) {
     if (lane == 0) {
-      const uint32_t idesc = idesc_bf16(N, false, false);
-      ok = mbar_wait(&w_full, 0, abortp);
+      const uint32_t idesc = make_idesc(Fmt::BF16, N);
+      ok = mbar_wait_abort(&w_full, 0, abortp);
       uint32_t s = 0, ph = 0;
       int li = 0;
       for (int64_t t = blockIdx.x; t < ntiles && ok; t += G, ++li) {
         const int buf = li & 1;
-        ok = mbar_wait(&acc_empty[buf], (((uint32_t)(li >> 1)) & 1u) ^ 1u, abortp);
+        ok = mbar_wait_abort(&acc_empty[buf], (((uint32_t)(li >> 1)) & 1u) ^ 1u, abortp);
         if (!ok) break;
         tc_fence_after();
         const uint32_t acc0 = tmem_base + (uint32_t)(buf * ROWS * N);
         for (int iy = -1; iy <= ROWS && ok; ++iy) {
           for (int S = 0; S < 3; ++S) {
-            ok = mbar_wait(&full_bar[s], ph, abortp);
+            ok = mbar_wait_abort(&full_bar[s], ph, abortp);
             if (!ok) break;
             tc_fence_after();
             const uint32_t abase = smem_u32(ring + (size_t)s * a.a_bytes);
@@ -553,21 +533,21 @@ conv3x3_tma_rows_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_co
               const uint32_t wS = smem_u32(wsm + (size_t)(S * 3) * w_tap);       // stacked [r=2; r=1; r=0] for this shift
 #pragma unroll
               for (int k = 0; k < 4; ++k) {
-                const uint64_t da = make_desc_sw(abase + k * 32, 16, 1024, 2);
+                const uint64_t da = smem_desc(abase + k * 32, 16, 1024, 2);
                 int hi = r_hi;
                 if (S == 0 && k == 0 && r_lo == 0) {
                   // first touch of accumulator j = iy + 1 (kernel row 0): overwrite instead of accumulate
-                  umma(acc0 + (uint32_t)((iy + 1) * N), da, make_desc_sw(wS + 2 * w_tap + k * 32, 16, 1024, 2), idesc, 0u);
+                  umma_f16(acc0 + (uint32_t)((iy + 1) * N), da, smem_desc(wS + 2 * w_tap + k * 32, 16, 1024, 2), idesc, 0u);
                   if (r_hi == 0) continue;
                   // the remaining rows r = 1 .. r_hi accumulate: handled below with r_lo' = 1
                   const int nr = r_hi;                                             // rows 1 .. r_hi
-                  umma(acc0 + (uint32_t)((iy + 1 - r_hi) * N), da, make_desc_sw(wS + (uint32_t)(2 - r_hi) * w_tap + k * 32, 16, 1024, 2),
-                       idesc_bf16(nr * N, false, false), 1u);
+                  umma_f16(acc0 + (uint32_t)((iy + 1 - r_hi) * N), da, smem_desc(wS + (uint32_t)(2 - r_hi) * w_tap + k * 32, 16, 1024, 2),
+                       make_idesc(Fmt::BF16, nr * N), 1u);
                   continue;
                 }
                 const int nr = hi - r_lo + 1;
-                umma(acc0 + (uint32_t)((iy + 1 - hi) * N), da, make_desc_sw(wS + (uint32_t)(2 - hi) * w_tap + k * 32, 16, 1024, 2),
-                     idesc_bf16(nr * N, false, false), 1u);
+                umma_f16(acc0 + (uint32_t)((iy + 1 - hi) * N), da, smem_desc(wS + (uint32_t)(2 - hi) * w_tap + k * 32, 16, 1024, 2),
+                     make_idesc(Fmt::BF16, nr * N), 1u);
               }
             }
             umma_commit(&empty_bar[s]);
@@ -591,7 +571,7 @@ conv3x3_tma_rows_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_co
     int li = 0;
     for (int64_t t = blockIdx.x; t < ntiles && ok; t += G, ++li) {
       const int buf = li & 1;
-      ok = mbar_wait(&acc_full[buf], ((uint32_t)(li >> 1)) & 1u, abortp);
+      ok = mbar_wait_abort(&acc_full[buf], ((uint32_t)(li >> 1)) & 1u, abortp);
       if (!ok) break;
       tc_fence_after();
       const int x0 = (int)(t % tiles_x) * 128, y0 = (int)((t / tiles_x) % tiles_y) * ROWS;
@@ -694,7 +674,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
     }
     mbar_init(&acc_full, 1);
     abort_s = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbarrier_init();
     prefetch_map(&tmx);
     prefetch_map(&tmdy);
   }
@@ -715,7 +695,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
         int x0, y0, b0;
         a.g.origin(t, x0, y0, b0);
         for (int st = 0; st < STEPS && ok; ++st) {
-          ok = mbar_wait(&empty_bar[s], ph ^ 1u, abortp);
+          ok = mbar_wait_abort(&empty_bar[s], ph ^ 1u, abortp);
           if (!ok) break;
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
           mbar_expect_tx(&full_bar[s], a.dy_bytes + nload * a.x_bytes);
@@ -736,7 +716,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
     __syncwarp();
   } else if (warp == 1) {
     if (lane == 0) {
-      const uint32_t idesc = TF ? make_idesc_tf32(Cin, true, true) : idesc_bf16(Cin, true, true);
+      const uint32_t idesc = TF ? make_idesc(Fmt::TF32, Cin, true, true) : make_idesc(Fmt::BF16, Cin, true, true);
       // MN-major operand tiles: pixel row k at k * (cb*2) bytes; 8-pixel groups at SBO; the next 64-channel box at LBO
       const uint32_t a_ty = sw_type(a.cby * 2), b_ty = sw_type(a.cbx * 2);
       const uint32_t a_sbo = 8u * a.cby * 2u, b_sbo = 8u * a.cbx * 2u;
@@ -746,7 +726,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
       bool first = true;
       for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G) {
         for (int st = 0; st < STEPS && ok; ++st) {
-          ok = mbar_wait(TF ? &lo_bar[s] : &full_bar[s], ph, abortp);
+          ok = mbar_wait_abort(TF ? &lo_bar[s] : &full_bar[s], ph, abortp);
           if (!ok) break;
           tc_fence_after();
           const uint32_t base = smem_u32(ring + (size_t)s * a.stage_bytes);
@@ -756,14 +736,14 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
             // MMA of nload * Cin columns.  LBO 0: a single box, re-read for M rows beyond Cout (never stored).
             const uint32_t box_y = a.dy_bytes / a.nby, box_x = a.x_bytes / a.nbx;
             const uint32_t lbo_y = a.nby > 1 ? box_y : 0u;
-            const uint32_t idn = NT != 1 ? make_idesc_tf32(nload * Cin, true, true) : idesc;
+            const uint32_t idn = NT != 1 ? make_idesc(Fmt::TF32, nload * Cin, true, true) : idesc;
             const uint32_t tmem_d = tmem_base + (uint32_t)(NT != 1 ? 0 : st * Cin);
             const uint32_t xb = base + a.dy_bytes;
             for (int j = 0; j < a.tp / 8; ++j) {
-              const uint64_t da = make_desc_sw(base + j * 1024, lbo_y, 512, 1);
-              const uint64_t db = make_desc_sw(xb + j * 1024, box_x, 512, 1);
-              const uint64_t dal = make_desc_sw(base + a.hi_bytes + j * 1024, lbo_y, 512, 1);
-              const uint64_t dbl = make_desc_sw(xb + a.hi_bytes + j * 1024, box_x, 512, 1);
+              const uint64_t da = smem_desc(base + j * 1024, lbo_y, 512, 1);
+              const uint64_t db = smem_desc(xb + j * 1024, box_x, 512, 1);
+              const uint64_t dal = smem_desc(base + a.hi_bytes + j * 1024, lbo_y, 512, 1);
+              const uint64_t dbl = smem_desc(xb + a.hi_bytes + j * 1024, box_x, 512, 1);
               umma_tf32(tmem_d, da, db, idn, (!first || j > 0) ? 1u : 0u);
               umma_tf32(tmem_d, da, dbl, idn, 1u);
               umma_tf32(tmem_d, dal, db, idn, 1u);
@@ -771,21 +751,21 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
           } else if (NT != 1) {
             // the tapped tiles are one MN-major operand of nload * Cin columns (tile stride = leading byte
             // offset), their accumulators neighbours in TMEM: ONE MMA per 16 pixels instead of nload
-            const uint32_t idesc3 = idesc_bf16(nload * Cin, true, true);
+            const uint32_t idesc3 = make_idesc(Fmt::BF16, nload * Cin, true, true);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
-              const uint64_t da = make_desc_sw(base + j * a_kstep, a_lbo, a_sbo, a_ty);
-              const uint64_t db = make_desc_sw(base + a.dy_bytes + j * b_kstep, a.x_bytes, b_sbo, b_ty);
-              umma(tmem_base, da, db, idesc3, (!first || j > 0) ? 1u : 0u);
+              const uint64_t da = smem_desc(base + j * a_kstep, a_lbo, a_sbo, a_ty);
+              const uint64_t db = smem_desc(base + a.dy_bytes + j * b_kstep, a.x_bytes, b_sbo, b_ty);
+              umma_f16(tmem_base, da, db, idesc3, (!first || j > 0) ? 1u : 0u);
             }
           } else {
             const uint32_t tmem_d = tmem_base + (uint32_t)(st * Cin);       // tap inside the kernel row
             const uint32_t xb = base + a.dy_bytes;
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
-              const uint64_t da = make_desc_sw(base + j * a_kstep, a_lbo, a_sbo, a_ty);
-              const uint64_t db = make_desc_sw(xb + j * b_kstep, b_lbo, b_sbo, b_ty);
-              umma(tmem_d, da, db, idesc, (!first || j > 0) ? 1u : 0u);
+              const uint64_t da = smem_desc(base + j * a_kstep, a_lbo, a_sbo, a_ty);
+              const uint64_t db = smem_desc(xb + j * b_kstep, b_lbo, b_sbo, b_ty);
+              umma_f16(tmem_d, da, db, idesc, (!first || j > 0) ? 1u : 0u);
             }
           }
           umma_commit(&empty_bar[s]);
@@ -804,7 +784,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
       uint32_t s = 0, ph = 0;
       for (int64_t t = blockIdx.x; t < a.g.ntiles && ok; t += G) {
         for (int st = 0; st < STEPS && ok; ++st) {
-          ok = mbar_wait(&full_bar[s], ph, abortp);
+          ok = mbar_wait_abort(&full_bar[s], ph, abortp);
           if (!ok) break;
           split_lo(ring + (size_t)s * a.stage_bytes, a.dy_bytes + nload * a.x_bytes, a.hi_bytes, tid - 64, 128);
           fence_async_smem();
@@ -814,7 +794,7 @@ conv3x3_wgrad_tma_kernel(const __grid_constant__ CUtensorMap tmx, const __grid_c
         }
       }
     }
-    if (ok) ok = mbar_wait(&acc_full, 0, abortp);
+    if (ok) ok = mbar_wait_abort(&acc_full, 0, abortp);
     if (ok) {
       tc_fence_after();
       const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);

@@ -54,6 +54,53 @@ def test_cuda_sources_target_sm100a_only():
             assert "triton" not in src.lower()
 
 
+def _strip_c_comments(src):
+    """Source text with // and /* */ comments blanked out; string and character literals are kept."""
+    return re.sub(r'//[^\n]*|/\*.*?\*/|("(?:\\.|[^"\\])*"|\'(?:\\.|[^\'\\])*\')',
+                  lambda m: m.group(1) or " ", src, flags=re.S)
+
+
+def _asm_statements(src):
+    """The concatenated string literals of every asm statement in comment-free source."""
+    out = []
+    for m in re.finditer(r"\basm\b(\s+volatile\b)?\s*\(", src):
+        depth, i = 1, m.end()
+        while depth:
+            c = src[i]
+            if c == '"':
+                i = re.compile(r'"(?:\\.|[^"\\])*"').match(src, i).end()
+                continue
+            depth += (c == "(") - (c == ")")
+            i += 1
+        out.append("".join(re.findall(r'"((?:\\.|[^"\\])*)"', src[m.end():i])))
+    return out
+
+
+def test_sm100_primitives_are_defined_once():
+    """mbarrier / tcgen05 / async-proxy PTX and the fp16 split live in tm_sm100.cuh and tm_split.cuh only."""
+    csrc = os.path.join(PKG, "csrc")
+    srcs = {f: _strip_c_comments(open(os.path.join(csrc, f)).read())
+            for f in sorted(os.listdir(csrc)) if f.endswith((".cu", ".cuh"))}
+    assert "tm_sm100.cuh" in srcs and "tm_split.cuh" in srcs
+    forbidden = ("mbarrier.", "tcgen05.", "fence.proxy.async", "fence.mbarrier_init",
+                 "cp.async.bulk.shared::cluster.global")
+    n_asm = 0
+    for f, src in srcs.items():
+        for stmt in _asm_statements(src):
+            n_asm += 1
+            if f != "tm_sm100.cuh":
+                assert not any(k in stmt for k in forbidden), f"{f}: {stmt}"
+    assert n_asm > 20
+    defs = {
+        "LO_SCALE": r"\bLO_SCALE\s*=",
+        "split_h": r"\bsplit_h\s*\([^;{}]*\)\s*\{",
+        "__cvta_generic_to_shared": r"\b__cvta_generic_to_shared\b",
+    }
+    for name, pat in defs.items():
+        where = [f for f, src in srcs.items() if re.search(pat, src)]
+        assert len(where) == 1, f"{name} is defined in {where}"
+
+
 def test_product_never_imports_oracle():
     for f in os.listdir(PKG):
         if f.endswith(".py"):
