@@ -468,6 +468,13 @@ size_t tm_selfmlp_bwd1_ws_bytes(void);
 int tm_selfmlp_gen_bwd1(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
                         const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* W2,
                         float* dW1, float* db1, void* ws, size_t ws_bytes, void* stream);
+/* The same kernel with the input's data gradient as well: dX[r, 0:kx] = dh W1 for row m, r = x_rows ? x_rows[m] : m
+ * (the row the forward read), summed over the 256 hidden units in a fixed order: deterministic.  dW1 / db1 are bitwise
+ * those of tm_selfmlp_gen_bwd1.  The rows r must be distinct (each row of dX is written by one thread, never
+ * accumulated); rows of dX that no m maps to are left untouched.  ws: tm_selfmlp_bwd1_ws_bytes(). */
+int tm_selfmlp_gen_bwd1_dx(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
+                           const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* W2,
+                           float* dW1, float* db1, float* dX, int64_t lddx, void* ws, size_t ws_bytes, void* stream);
 /* The same product for an MLP whose hidden activations H were STORED (fc_cell_self, 36 inputs): the hidden-layer
  * gradient DH[r] = (G[g_rows[m]] @ W2) * (H[r] > 0), r = h_rows ? h_rows[m] : m, written out (it feeds the first-layer
  * weight gradient).  Replaces the masked data-gradient GEMM of the general MLP backward. */

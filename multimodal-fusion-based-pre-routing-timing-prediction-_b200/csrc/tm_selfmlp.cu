@@ -664,11 +664,15 @@ struct B1Args {
   const int* h_rows;      // row of H (and of DH) that belongs to row m (NULL: m)
   float* DH;
   int64_t lddh;
+  // DX form (tm_selfmlp_gen_bwd1_dx): the input's data gradient dh W1, written to the row of X the forward read
+  float* dX;
+  int64_t lddx;
 };
 
-// STORE == false: first-layer gradients of the generated MLP (above).  STORE == true: the same product with the epilogue
+// STORE == false: first-layer gradients of the generated MLP (above); DX adds the data gradient dX = dh W1, two FMAs per
+// hidden unit in the lane that owns the row, in hidden-unit order.  STORE == true: the same product with the epilogue
 // of the general MLP backward -- dh = (G W2) * (H > 0) written to DH (fc_cell_self: 36 inputs, the hidden layer is stored).
-template <bool STORE>
+template <bool STORE, bool DX>
 __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   float* w0_s = reinterpret_cast<float*>(smem + B1_OFF_P);
@@ -843,6 +847,7 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
       __syncwarp();
       xs0[lane] = x0; xs1[lane] = x1;
       __syncwarp();
+      float dx0 = 0.f, dx1 = 0.f;                                      // (DX) this row's data gradient
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         mbar_wait_trap<MBAR_SPINS>(&acc_full[half], li & 1u);
@@ -859,7 +864,12 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
           for (int i = 0; i < 32; ++i) {
             const float pre = fmaf(w0_s[j0 + i], x0, fmaf(w1_s[j0 + i], x1, b1_s[j0 + i]));
             const float dh = fmaf(vc[i], LO_INV, vm[i]) * inv;
-            scr[lane * 33 + i] = pre > 0.f ? dh : 0.f;
+            const float d = pre > 0.f ? dh : 0.f;
+            scr[lane * 33 + i] = d;
+            if constexpr (DX) {
+              dx0 = fmaf(d, w0_s[j0 + i], dx0);
+              dx1 = fmaf(d, w1_s[j0 + i], dx1);
+            }
           }
           __syncwarp();
           float s = 0.f, s0 = 0.f, s1 = 0.f;
@@ -877,6 +887,13 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_empty[half]);
+      }
+      if constexpr (DX) {
+        if (m < a.M) {
+          float* dp = a.dX + (a.x_rows ? (int64_t)a.x_rows[m] : m) * a.lddx;
+          dp[0] = dx0;
+          if (a.kx > 1) dp[1] = dx1;
+        }
       }
     }
     float* pp = a.part + ((size_t)blockIdx.x * EPI_W + warp) * 3 * HIDF;
@@ -1130,12 +1147,14 @@ extern "C" int tm_selfmlp_gen_wgrad2(int64_t M, const float* G, int64_t ldg, con
 
 extern "C" size_t tm_selfmlp_bwd1_ws_bytes() { return 2 * (size_t)B1_W_PLANE + (size_t)sm_count() * EPI_W * 3 * HIDF * sizeof(float) + 1024; }
 
-extern "C" int tm_selfmlp_gen_bwd1(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
-                                   const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* W2,
-                                   float* dW1, float* db1, void* ws, size_t ws_bytes, void* stream) {
-  TM_REQUIRE(kx == 1 || kx == 2, "tm_selfmlp_gen_bwd1: the first layer must have 1 or 2 inputs");
-  TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_bwd1_ws_bytes(), "tm_selfmlp_gen_bwd1: workspace too small (tm_selfmlp_bwd1_ws_bytes)");
-  TM_REQUIRE((ldg & 3) == 0 && (reinterpret_cast<uintptr_t>(G) & 15) == 0, "tm_selfmlp_gen_bwd1: G rows must be 16-byte aligned");
+namespace {
+// tm_selfmlp_gen_bwd1 (dX == nullptr) and tm_selfmlp_gen_bwd1_dx
+int gen_bwd1(const char* name, int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
+             const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* W2, float* dW1, float* db1,
+             float* dX, int64_t lddx, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(kx == 1 || kx == 2, "%s: the first layer must have 1 or 2 inputs", name);
+  TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_bwd1_ws_bytes(), "%s: workspace too small (tm_selfmlp_bwd1_ws_bytes)", name);
+  TM_REQUIRE((ldg & 3) == 0 && (reinterpret_cast<uintptr_t>(G) & 15) == 0, "%s: G rows must be 16-byte aligned", name);
   cudaStream_t st = (cudaStream_t)stream;
   if (M <= 0) {
     TM_CUDA(cudaMemsetAsync(dW1, 0, (size_t)HIDF * kx * sizeof(float), st));
@@ -1146,14 +1165,38 @@ extern "C" int tm_selfmlp_gen_bwd1(int64_t M, const float* G, int64_t ldg, const
   float* part = reinterpret_cast<float*>(planes + 2 * B1_W_PLANE);
   selfmlp_pack_t_kernel<<<(NOUT * HIDF + 255) / 256, 256, 0, st>>>(W2, planes);
   TM_TRY(check_launch("selfmlp_pack_t"));
-  TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
   const int64_t ntiles = (M + TM - 1) / TM;
   const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
-  B1Args a{M, G, ldg, g_rows, X, ldx, x_rows, (int)kx, W1, b1, planes, part, nullptr, 0, nullptr, nullptr, 0};
-  selfmlp_gen_bwd1_kernel<false><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
-  TM_TRY(check_launch("selfmlp_gen_bwd1"));
+  B1Args a{M, G, ldg, g_rows, X, ldx, x_rows, (int)kx, W1, b1, planes, part, nullptr, 0, nullptr, nullptr, 0, dX, lddx};
+  if (dX) {
+    TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+    selfmlp_gen_bwd1_kernel<false, true><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+    TM_TRY(check_launch("selfmlp_gen_bwd1_dx"));
+  } else {
+    TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+    selfmlp_gen_bwd1_kernel<false, false><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+    TM_TRY(check_launch("selfmlp_gen_bwd1"));
+  }
   selfmlp_bwd1_reduce_kernel<<<HIDF / 32, 256, 0, st>>>(part, grid * EPI_W, (int)kx, dW1, db1);
   return check_launch("selfmlp_bwd1_reduce");
+}
+}  // namespace
+
+extern "C" int tm_selfmlp_gen_bwd1(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
+                                   const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* W2,
+                                   float* dW1, float* db1, void* ws, size_t ws_bytes, void* stream) {
+  return gen_bwd1("tm_selfmlp_gen_bwd1", M, G, ldg, g_rows, X, ldx, x_rows, kx, W1, b1, W2, dW1, db1, nullptr, 0, ws,
+                  ws_bytes, stream);
+}
+
+/* ... and the input's data gradient dX[x_rows ? x_rows[m] : m, 0:kx] = dh W1 (declared in tm_b200.h). */
+extern "C" int tm_selfmlp_gen_bwd1_dx(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X,
+                                      int64_t ldx, const int32_t* x_rows, int64_t kx, const float* W1, const float* b1,
+                                      const float* W2, float* dW1, float* db1, float* dX, int64_t lddx, void* ws,
+                                      size_t ws_bytes, void* stream) {
+  TM_REQUIRE(dX && lddx >= kx, "tm_selfmlp_gen_bwd1_dx: dX missing or its row stride lddx < kx");
+  return gen_bwd1("tm_selfmlp_gen_bwd1_dx", M, G, ldg, g_rows, X, ldx, x_rows, kx, W1, b1, W2, dW1, db1, dX, lddx, ws,
+                  ws_bytes, stream);
 }
 
 extern "C" size_t tm_selfmlp_rows_dh_ws_bytes() { return 2 * (size_t)B1_W_PLANE + 256; }
@@ -1172,11 +1215,11 @@ extern "C" int tm_selfmlp_rows_dh(int64_t M, const float* G, int64_t ldg, const 
   uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
   selfmlp_pack_t_kernel<<<(NOUT * HIDF + 255) / 256, 256, 0, st>>>(W2, planes);
   TM_TRY(check_launch("selfmlp_pack_t"));
-  TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+  TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
   const int64_t ntiles = (M + TM - 1) / TM;
   const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
   B1Args a{M, G, ldg, g_rows, nullptr, 0, nullptr, 0, nullptr, nullptr, planes, nullptr, H, ldh, h_rows, DH, lddh};
-  selfmlp_gen_bwd1_kernel<true><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+  selfmlp_gen_bwd1_kernel<true, false><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
   return check_launch("selfmlp_rows_dh");
 }
 

@@ -98,6 +98,7 @@ class DesignBatch:
         self.ep_off = None                         # int32 (K+1,) on the device: set by concat (K > 1 only)
         self.pin_off_h = None                      # first pin of every design in the joined netlist (concat)
         self.design_losses = None                  # (K,) device tensor, rewritten by every step / replay (K > 1)
+        self.input_grads = None                    # {"cell_feat", "net_feat", "image"}: DesignStep.run(input_grads=True)
         self._fuse_table = None
         # dynamic: the endpoint batch (endpoints / levels / labels / mask rows) is refreshed IN PLACE between steps, so
         # the step re-runs the on-device row selection every time (captured into its CUDA graph): one capture per
@@ -209,12 +210,12 @@ class DesignBatch:
 class PreparedDesign:
     VALUE_FIELDS = ("cell_feat", "net_feat", "image", "arrival_time")
 
-    def __init__(self, step, host, device, graph=None, pool=None):
+    def __init__(self, step, host, device, graph=None, pool=None, input_grads=False):
         self.batch = DesignBatch.from_host(host, device, graph=graph)
         self.static = {"cell_feat": self.batch.cell_feat, "net_feat": self.batch.net_feat,
                        "image": self.batch.image, "arrival_time": self.batch.arrival_time}
         torch.cuda.synchronize()
-        self.replay = step.capture(self.batch, pool=pool)
+        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads)
 
     def upload(self, host, stream=None):
         """Host -> device copy of the per-step values into the graph's static inputs."""
@@ -235,11 +236,11 @@ class PreparedDesign:
 class PreparedDesigns:
     """``DesignStep.prepare_many``: K resident designs, one captured step over all of them."""
 
-    def __init__(self, step, hosts, device, pool=None):
+    def __init__(self, step, hosts, device, pool=None, input_grads=False):
         self.parts = [DesignBatch.from_host(h, device) for h in hosts]
         self.batch = DesignBatch.concat(self.parts)
         torch.cuda.synchronize()
-        self.replay = step.capture(self.batch, pool=pool)
+        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads)
 
     def upload(self, hosts, stream=None):
         """Host -> device copy of every design's per-step values into its slices of the graph's static inputs."""
@@ -294,10 +295,10 @@ class DesignStep:
         # several designs: each image is normalised with its own statistics, as the reference's batch of one is
         return tm_unet.unet_forward(self.cnn, image, need_bwd=need_bwd, update_stats=self.cnn.training, per_image=True)
 
-    def _image_backward(self, st, gout):
+    def _image_backward(self, st, gout, need_dx=False):
         if self.layoutnet:
-            return tm_unet.layoutnet_backward(self.cnn, st, gout)
-        return tm_unet.unet_backward(self.cnn, st, gout)
+            return tm_unet.layoutnet_backward(self.cnn, st, gout, need_dx=need_dx)
+        return tm_unet.unet_backward(self.cnn, st, gout, need_dx=need_dx)
 
     @staticmethod
     def _check_feature_map(fmap, b):
@@ -352,10 +353,29 @@ class DesignStep:
         return pred.squeeze(-1)
 
     # ---------------------------------------------------------------- full step
-    def run(self, b, grad_scale=1.0):
+    def run(self, b, grad_scale=1.0, input_grads=False, pred_grad=None):
         """Forward + backward.  Returns (loss (1,) device tensor, pred (T,)); fills ``.grad``.  A batch of K designs
         (``DesignBatch.concat``) gives loss = mean of the designs' MSEs (``b.design_losses``, (K,)) and every gradient
-        the mean of their gradients; predictions are per design as the one-design step gives them."""
+        the mean of their gradients; predictions are per design as the one-design step gives them.
+
+        ``input_grads``: also fill ``b.input_grads`` = {"cell_feat", "net_feat", "image"}, the gradients of what the step
+        differentiates with respect to the batch's inputs, shaped like ``b.cell_feat`` / ``b.net_feat`` / ``b.image``
+        and rewritten by every run or replay.  Feature rows the propagation never reads (net-class pins in
+        "cell_feat", cell-class pins in "net_feat", pins outside the schedule or, with ``prune``, outside the cone) are
+        exactly zero.  In a joined batch design k owns the rows ``b.pin_off_h[k]:b.pin_off_h[k + 1]`` and ``image[k]``.
+        With several ranks these gradients belong to the rank's own designs and are not all-reduced.
+        ``pred_grad``: (T,) float32 device tensor, dObjective/dpred, that seeds the backward instead of the MSE's
+        gradient, taken as given (no 1/T or 1/K factor; ``grad_scale`` must stay 1): every ``.grad`` and input gradient
+        is then the vector-Jacobian product ``pred.backward(pred_grad)`` gives.  The loss is still computed.  Neither
+        option changes the parameter gradients' arithmetic: with ``pred_grad`` unset they are the same bits."""
+        if pred_grad is not None:
+            T = int(b.endpoints.numel())
+            if grad_scale != 1.0:
+                raise ValueError("DesignStep.run: pred_grad is taken as given; scale the seed instead of grad_scale")
+            if (pred_grad.shape != (T,) or pred_grad.dtype != torch.float32 or not pred_grad.is_contiguous()
+                    or pred_grad.device != b.endpoints.device):
+                raise ValueError(f"DesignStep.run: pred_grad must be a contiguous float32 ({T},) tensor on "
+                                 f"{b.endpoints.device}, got {pred_grad.dtype} {tuple(pred_grad.shape)} on {pred_grad.device}")
         m = self.model
         dev = b.image.device
         main = torch.cuda.current_stream()
@@ -399,6 +419,8 @@ class DesignStep:
             b.design_losses = torch.empty(b.K, dtype=torch.float32, device=dev)
             call("tm_mse_multi", b.K, b.ep_off, pred, b.arrival_time, b.design_losses, loss, gpred, float(grad_scale),
                  stream())
+        if pred_grad is not None:
+            gpred = pred_grad.reshape(T, 1)
 
         # ---- head backward: mlp_fuse on the netlist stream (its dX seeds the backward sweep) ...
         width = hs["width"]
@@ -421,13 +443,19 @@ class DesignStep:
 
         # ---- GNN backward (main stream) next to the U-Net backward (image stream)
         call("tm_scatter_add_cols", T, D, dX, width, 0, endpoints, G, D, stream())
-        ggrads = tm_ops.gnn_backward(sched, saved, gp, G)
+        if input_grads:
+            ggrads, dcf, dnf = tm_ops.gnn_backward(sched, saved, gp, G, need_dx=True)
+        else:
+            ggrads = tm_ops.gnn_backward(sched, saved, gp, G)
         pairs = list(zip(self.gnn_params, ggrads))
         self._assign(pairs)
         with torch.cuda.stream(side):
             old_cap = tm_lib.lib().tm_tc_set_grid_cap(img_cap)
-            ug = self._image_backward(ust, dF.reshape(fmap.shape))
+            ug = self._image_backward(ust, dF.reshape(fmap.shape), need_dx=input_grads)
             tm_lib.lib().tm_tc_set_grid_cap(old_cap)
+            if input_grads:
+                ug, dimg = ug
+                b.input_grads = {"cell_feat": dcf, "net_feat": dnf, "image": dimg}
             upairs = [(self.cnn_params[k], ug[k]) for k in self.cnn_names]
             self._assign(upairs)
         main.wait_stream(side)                               # join: every gradient exists on `main`
@@ -442,22 +470,23 @@ class DesignStep:
         return loss, pred.squeeze(-1)
 
     # ---------------------------------------------------------------- CUDA graph
-    def capture(self, b, warmup=2, pool=None):
-        """Capture ``run(b)`` (about 500 launches on two streams) into one CUDA graph.  The batch's
-        tensors become the graph's static inputs: refresh them in place (``tensor.copy_``) and call
-        the returned function, which replays the graph and returns the same (loss, pred) tensors;
-        ``param.grad`` tensors are rewritten in place by every replay.  On the data-parallel path the
+    def capture(self, b, warmup=2, pool=None, input_grads=False, pred_grad=None):
+        """Capture ``run(b, input_grads=input_grads, pred_grad=pred_grad)`` (about 500 launches on two streams) into
+        one CUDA graph.  The batch's tensors -- and ``pred_grad`` -- become the graph's static inputs: refresh them in
+        place (``tensor.copy_``) and call the returned function, which replays the graph and returns the same (loss,
+        pred) tensors; ``param.grad`` tensors and ``b.input_grads`` are rewritten in place by every replay.  On the data-parallel path the
         bucketed NCCL all-reduces (head + fusion early, GNN + U-Net after the join) are captured INSIDE the graph (persistent flat buffers,
         ``tm_dp.FlatBucket``), where they overlap the backward as in the eager schedule; with
         ``TM_DP_GRAPH=0`` the graph holds the rank's compute only and one exchange is posted after each
         replay.  ``pool``: a ``torch.cuda.graph_pool_handle()`` shared by graphs that are replayed one
         after the other (several prepared designs of one rank share their activation memory).
         Call ``close()`` before ``torch.distributed.destroy_process_group()``."""
+        opts = dict(input_grads=input_grads, pred_grad=pred_grad)
         if self.world <= 1 or os.environ.get("TM_DP_GRAPH", "1") != "0":
-            return self._capture_local(b, warmup, pool)
+            return self._capture_local(b, warmup, pool, opts)
         world, self.world = self.world, 1                  # no collectives inside the captured region
         try:
-            replay_local = self._capture_local(b, warmup, pool)
+            replay_local = self._capture_local(b, warmup, pool, opts)
         finally:
             self.world = world
         params = [p for p in list(self.model.parameters()) + list(self.cnn.parameters())]
@@ -470,42 +499,47 @@ class DesignStep:
         replay.graph = replay_local.graph
         return replay
 
-    def _capture_local(self, b, warmup=2, pool=None):
+    def _capture_local(self, b, warmup=2, pool=None, opts=None):
+        opts = opts or {}
         cur = torch.cuda.current_stream()
         s = torch.cuda.Stream(priority=int(os.environ.get("TM_MAIN_PRIORITY", "0")))   # (a higher priority for the netlist branch was measured: no effect)
         s.wait_stream(cur)
         with torch.cuda.stream(s):
             for _ in range(warmup):
-                self.run(b)
+                self.run(b, **opts)
         cur.wait_stream(s)
         torch.cuda.synchronize()
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, pool=pool):
-            loss, pred = self.run(b)
+            loss, pred = self.run(b, **opts)
         self._graphs.append(g)
         grads = [(p, p.grad) for p in list(self.model.parameters()) + list(self.cnn.parameters()) if p.grad is not None]
+        igrads = b.input_grads if opts.get("input_grads") else None
 
         def replay():
             g.replay()
             for p, gr in grads:                      # several captured steps may coexist: re-point .grad
                 p.grad = gr
+            if igrads is not None:
+                b.input_grads = igrads
             return loss, pred
         replay.graph = g
         return replay
 
-    def prepare(self, host, device, graph=None, pool=None):
+    def prepare(self, host, device, graph=None, pool=None, input_grads=False):
         """A design made resident for repeated steps: uploads everything once, builds the structure
         that depends only on the netlist and the endpoint batch (level schedule, CSRs, mask runs / CSC)
         and captures the step as a CUDA graph.  Returns a ``PreparedDesign``; its ``step(host)``
         refreshes the per-step VALUES (features, image, labels) from pinned host memory and replays.
-        The structure (edges, endpoints, masks) must be the one given here."""
-        return PreparedDesign(self, host, device, graph, pool)
+        The structure (edges, endpoints, masks) must be the one given here.  ``input_grads``: every replay also
+        rewrites ``batch.input_grads`` (see ``run``)."""
+        return PreparedDesign(self, host, device, graph, pool, input_grads)
 
-    def prepare_many(self, hosts, device, pool=None):
+    def prepare_many(self, hosts, device, pool=None, input_grads=False):
         """K designs made resident for repeated steps over all of them (``DesignBatch.concat``), captured as ONE CUDA
         graph.  Returns a ``PreparedDesigns``; its ``step(hosts)`` refreshes the per-step VALUES of all K from pinned
-        host memory and replays.  The structures must be the ones given here."""
-        return PreparedDesigns(self, hosts, device, pool)
+        host memory and replays.  The structures must be the ones given here.  ``input_grads``: as in ``prepare``."""
+        return PreparedDesigns(self, hosts, device, pool, input_grads)
 
     @staticmethod
     def _assign(pairs):

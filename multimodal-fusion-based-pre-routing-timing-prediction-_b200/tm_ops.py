@@ -228,14 +228,17 @@ def _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, h_rows, dh):
 
 
 def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=False, b1=None, wgrad_stream=None,
-                  h_rows=None):
+                  h_rows=None, dx_out=None):
     """Gradients of a two-layer MLP.  ``g``: dLoss/d(out) rows (optionally gathered by ``g_rows``).
     ``h``: the hidden activations mlp2_forward returned, or None when they were generated on the fly
     (then ``b1`` is required).  Returns (dw1, db1, dw2, db2, dx or None).
     ``wgrad_stream`` (with ``need_dx``): the data gradient is computed first on the current stream and the four
     parameter gradients on ``wgrad_stream`` (which waits for it); the caller joins that stream before reading them.
     ``h_rows``: row of ``h`` that belongs to MLP row i (default i) -- set when ``rows`` / ``g_rows`` are a subset of
-    the rows the forward pass ran on (``tm_graph.BackwardCone``)."""
+    the rows the forward pass ran on (``tm_graph.BackwardCone``).
+    ``dx_out`` (with ``need_dx``; required when ``rows`` gathers): the data gradient of MLP row i is written to row
+    ``rows[i]`` of ``dx_out`` -- the row of ``x`` it read, so ``rows`` must be distinct -- and ``dx_out`` is returned as dx;
+    its other rows are left as they are.  The parameter gradients are the same bits as without ``need_dx``."""
     hid, kin = w1.shape
     nout = w2.shape[0]
     dev = g.device
@@ -243,13 +246,17 @@ def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=
     db2 = torch.empty(nout, dtype=torch.float32, device=dev)
     dw1 = torch.empty(hid, kin, dtype=torch.float32, device=dev)
     db1 = torch.empty(hid, dtype=torch.float32, device=dev)
+    if need_dx and dx_out is None and rows is not None:
+        raise RuntimeError("mlp2_backward: a data gradient of gathered rows needs dx_out")
     if n_rows == 0:
         for t in (dw1, db1, dw2, db2):
             t.zero_()
-        return dw1, db1, dw2, db2, None
+        return dw1, db1, dw2, db2, dx_out if need_dx else None
+    if need_dx and dx_out is None:
+        dx_out = torch.empty(n_rows, kin, dtype=torch.float32, device=dev)
     if h is None:                                            # generated hidden layer (kin <= 2)
-        if b1 is None or need_dx:
-            raise RuntimeError("mlp2_backward: generated hidden activations need b1 (and have no dx path)")
+        if b1 is None:
+            raise RuntimeError("mlp2_backward: generated hidden activations need b1")
         prec = _precision()
         prec = 3 if prec is None else prec
         fused = FUSED_SELF_MLP and hid == 256 and nout == 128 and prec == 3 and ldg % 4 == 0 and g.data_ptr() % 16 == 0
@@ -269,19 +276,31 @@ def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=
                  prec, tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
         if fused:
             nb = tm_lib.ws_bytes("tm_selfmlp_bwd1_ws_bytes")
-            call("tm_selfmlp_gen_bwd1", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2), dw1, db1,
-                 tm_lib.workspace(nb, dev), nb, stream())
+            if need_dx:                                      # the same kernel with dX = dh W1 in its epilogue
+                call("tm_selfmlp_gen_bwd1_dx", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2),
+                     dw1, db1, dx_out, dx_out.stride(0), tm_lib.workspace(nb, dev), nb, stream())
+            else:
+                call("tm_selfmlp_gen_bwd1", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2),
+                     dw1, db1, tm_lib.workspace(nb, dev), nb, stream())
         else:
             nb = tm_lib.ws_bytes("tm_tc_mlp1_bwd_ws", hid)
             call("tm_tc_mlp1_bwd_fused", n_rows, hid, nout, g, ldg, g_rows, transpose(_f32c(w2)), None, 0, x, ldx, rows, kin,
                  _f32c(w1), _f32c(b1), dw1, db1, tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
+            if need_dx:
+                # no fused data-gradient kernel in this precision: the hidden layer is materialised for the data
+                # gradient alone (the parameter gradients above are untouched)
+                hm = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
+                gemm_nn(n_rows, hid, kin, x, ldx, _f32c(w1), kin, hm, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True)
+                dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
+                _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, hm, None, dh)
+                gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx_out, dx_out.stride(0), c_rows=rows)
         aux_join()
-        return dw1, db1, dw2, db2, None
+        return dw1, db1, dw2, db2, dx_out if need_dx else None
     if need_dx and wgrad_stream is not None:
         dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
         gemm_nn(n_rows, hid, nout, g, ldg, _f32c(w2), hid, dh, hid, a_rows=g_rows, mask=h, ldmask=hid)
-        dx = torch.empty(n_rows, kin, dtype=torch.float32, device=dev)
-        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx, kin)
+        dx = dx_out
+        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx, dx.stride(0), c_rows=rows)
         wgrad_stream.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(wgrad_stream):
             gemm_tn(nout, hid, n_rows, g, ldg, h, hid, dw2, hid, a_rows=g_rows, colsum_a=db2)
@@ -309,12 +328,10 @@ def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=
     dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
     _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, None, dh)
     gemm_tn(hid, kin, n_rows, dh, hid, x, ldx, dw1, kin, b_rows=rows, colsum_a=db1)
-    dx = None
     if need_dx:
-        dx = torch.empty(n_rows, kin, dtype=torch.float32, device=dev)
-        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx, kin)
+        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx_out, dx_out.stride(0), c_rows=rows)
     aux_join()
-    return dw1, db1, dw2, db2, dx
+    return dw1, db1, dw2, db2, dx_out if need_dx else None
 
 
 # --------------------------------------------------------------------------------------------
@@ -377,11 +394,18 @@ def gnn_forward(sched, cell_feat, net_feat, params, save=True, impl=None, x_rows
     return H, saved
 
 
-def gnn_backward(sched, saved, params, G, cone=None):
+def gnn_backward(sched, saved, params, G, cone=None, need_dx=False):
     """``G`` (N,128): dLoss/dH, consumed (overwritten with dLoss/d pre-activation).
     Returns the 12 parameter gradients in GNN_PARAM_NAMES order.
     ``cone`` (``tm_graph.BackwardCone`` of the endpoints that seeded G): the weight-gradient contractions run over
-    the cone's rows only -- every other row of dLoss/dz is exactly zero."""
+    the cone's rows only -- every other row of dLoss/dz is exactly zero.
+    ``need_dx``: returns ``(grads, dcell_feat, dnet_feat)``, the gradients with respect to the features, shaped like
+    the ``cell_feat`` / ``net_feat`` the forward read.  The self-term S enters each pin's pre-activation linearly, so
+    after the sweep G is dLoss/dS and the feature gradient is the self MLPs' data gradient of it.  Rows the
+    propagation never reads are exactly zero: net-class pins in ``dcell_feat``, cell-class pins in ``dnet_feat``,
+    unscheduled pins in both.  The parameter gradients are the same bits as without ``need_dx``."""
+    if need_dx and cone is not None:
+        raise RuntimeError("gnn_backward: a BackwardCone has no feature-gradient path")
     (cs1w, cs1b, cs2w, cs2b, ns1w, ns1b, ns2w, ns2b, cn1w, cn1b, cn2w, cn2b) = [_f32c(p) for p in params]
     dev = G.device
     ncr = sched.n_cell_rows
@@ -415,12 +439,17 @@ def gnn_backward(sched, saved, params, G, cone=None):
         xc, xn = cpins, npins
         cpos = cone.cell_pos if saved["hc"] is not None else None
     nc, nn_ = int(cpins.numel()), int(npins.numel())
+    dcf = torch.zeros(cf.shape, dtype=torch.float32, device=dev) if need_dx else None
+    dnf = torch.zeros(nf.shape, dtype=torch.float32, device=dev) if need_dx else None
     dcs1w, dcs1b, dcs2w, dcs2b, _ = mlp2_backward(cf, cf.stride(0), xc, nc, cs1w, cs2w,
-                                                  saved["hc"], G, D, g_rows=cpins, b1=cs1b, h_rows=cpos)
+                                                  saved["hc"], G, D, g_rows=cpins, b1=cs1b, h_rows=cpos,
+                                                  need_dx=need_dx, dx_out=dcf)
     dns1w, dns1b, dns2w, dns2b, _ = mlp2_backward(nf, nf.stride(0), xn, nn_, ns1w, ns2w,
                                                   saved["hn"], G, D, g_rows=npins, b1=ns1b,
-                                                  h_rows=(cone.net_pos if cone is not None and saved["hn"] is not None else None))
-    return (dcs1w, dcs1b, dcs2w, dcs2b, dns1w, dns1b, dns2w, dns2b, dcn1w, dcn1b, dcn2w, dcn2b)
+                                                  h_rows=(cone.net_pos if cone is not None and saved["hn"] is not None else None),
+                                                  need_dx=need_dx, dx_out=dnf)
+    grads = (dcs1w, dcs1b, dcs2w, dcs2b, dns1w, dns1b, dns2w, dns2b, dcn1w, dcn1b, dcn2w, dcn2b)
+    return (grads, dcf, dnf) if need_dx else grads
 
 
 class GnnPropagateFn(torch.autograd.Function):
