@@ -180,7 +180,8 @@ int tm_gnn_forward(const tm_schedule* s, int32_t level_begin, int32_t level_end,
  *              out: dLoss/d(pre-activation) of every scheduled pin == dLoss/dS;
  *   W1[256,128], W2[128,256]: fc_cell_neigh weights as stored by nn.Linear;
  *   GA[n_cell_rows,128] scratch; GHID[n_cell_rows,256], GZC[n_cell_rows,128] out: operands of
- *   the hoisted weight-gradient GEMMs (dW1 = GHID^T A, dW2 = GZC^T HID). */
+ *   the hoisted weight-gradient GEMMs (dW1 = GHID^T A, dW2 = GZC^T HID).  GHID = GZC = NULL (both or neither): the
+ *   data gradient alone, a compile-time variant of either back end that stores neither; G is the same bits. */
 int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, const float* W1,
                     const float* W2, const float* A, const float* LSE, const float* HID,
                     float* GA, float* GHID, float* GZC, void* ws, size_t ws_bytes, void* stream);
@@ -205,7 +206,8 @@ int tm_fuse_forward_runs(int64_t T, int64_t J, int64_t D, const int32_t* run_ptr
                          float* out, int64_t ld_out, void* ws, size_t ws_bytes, void* stream);
 /* Column-major pull (deterministic, no atomics): csc_ptr[J+1], csc_t[nnz] list the positions t
  * (0..T-1) whose mask contains column j.
- *   dWt[j,:] = F[j] * sum_t g[t,:];   dF[j] = sum_t sum_c g[t,c] * Wt[j,c]. */
+ *   dWt[j,:] = F[j] * sum_t g[t,:];   dF[j] = sum_t sum_c g[t,c] * Wt[j,c].
+ * dWt = NULL (here and in tm_fuse_backward_multi): dF alone, the same bits. */
 int tm_fuse_backward(int64_t T, int64_t J, int64_t D, const int32_t* csc_ptr, const int32_t* csc_t,
                      const float* g, int64_t ld_g, const float* F, const float* Wt, float* dWt,
                      float* dF, void* stream);
@@ -471,7 +473,8 @@ int tm_selfmlp_gen_bwd1(int64_t M, const float* G, int64_t ldg, const int32_t* g
 /* The same kernel with the input's data gradient as well: dX[r, 0:kx] = dh W1 for row m, r = x_rows ? x_rows[m] : m
  * (the row the forward read), summed over the 256 hidden units in a fixed order: deterministic.  dW1 / db1 are bitwise
  * those of tm_selfmlp_gen_bwd1.  The rows r must be distinct (each row of dX is written by one thread, never
- * accumulated); rows of dX that no m maps to are left untouched.  ws: tm_selfmlp_bwd1_ws_bytes(). */
+ * accumulated); rows of dX that no m maps to are left untouched.  dW1 = db1 = NULL: dX alone (the column accumulators and
+ * their reduction are compiled out), the same bits.  ws: tm_selfmlp_bwd1_ws_bytes(). */
 int tm_selfmlp_gen_bwd1_dx(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
                            const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* W2,
                            float* dW1, float* db1, float* dX, int64_t lddx, void* ws, size_t ws_bytes, void* stream);
@@ -492,6 +495,13 @@ size_t tm_selfmlp_rows_dh_ws_bytes(void);
 int tm_selfmlp_rows_dh(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* W2, const float* H,
                        int64_t ldh, const int32_t* h_rows, float* DH, int64_t lddh, void* ws, size_t ws_bytes,
                        void* stream);
+/* The data gradient of that MLP in one pass: dX[r, 0:kin] = ((G[g_rows[m]] @ W2) * (H[h_rows[m]] > 0)) @ W1,
+ * r = x_rows ? x_rows[m] : m (distinct), W1 [256][kin] as stored, kin % 4 == 0, kin <= 48.  The first product runs as in
+ * tm_selfmlp_rows_dh (the same ReLU gates); the hidden gradient is never written: the lane that owns a row multiplies it
+ * into W1 in hidden-unit order, so the result is deterministic.  ws: tm_selfmlp_rows_dh_ws_bytes(). */
+int tm_selfmlp_rows_dx(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* W2, const float* H,
+                       int64_t ldh, const int32_t* h_rows, const float* W1, int64_t kin, float* dX, int64_t lddx,
+                       const int32_t* x_rows, void* ws, size_t ws_bytes, void* stream);
 size_t tm_selfmlp_wgrad2_ws_bytes(void);
 int tm_selfmlp_gen_wgrad2(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
                           const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* gmax,

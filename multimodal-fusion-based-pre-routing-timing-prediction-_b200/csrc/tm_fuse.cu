@@ -131,6 +131,8 @@ fuse_fwd_runs_kernel(const int* __restrict__ run_ptr, const int* __restrict__ ru
   out[(int64_t)t * ldo + c] = (float)acc + bias[c];
 }
 
+// WG == false: dF only, the weight gradient dWt is neither computed nor written (dF is the same bits)
+template <bool WG>
 __global__ void __launch_bounds__(256)
 fuse_bwd_kernel(int64_t J, const int* __restrict__ cptr, const int* __restrict__ ct,
                 const float* __restrict__ g, int64_t ldg, const float* __restrict__ F,
@@ -149,8 +151,10 @@ fuse_bwd_kernel(int64_t J, const int* __restrict__ cptr, const int* __restrict__
 #pragma unroll
     for (int q = 0; q < 4; ++q) { acc.x += v[q].x; acc.y += v[q].y; acc.z += v[q].z; acc.w += v[q].w; }
   }
-  const float f = F[j];
-  st4(dWt + j * D + lane * 4, make_float4(f * acc.x, f * acc.y, f * acc.z, f * acc.w));
+  if constexpr (WG) {
+    const float f = F[j];
+    st4(dWt + j * D + lane * 4, make_float4(f * acc.x, f * acc.y, f * acc.z, f * acc.w));
+  }
   float dot = 0.f;
   if (e > s) {
     const float4 w = __ldg(reinterpret_cast<const float4*>(Wt + j * D + lane * 4));
@@ -197,6 +201,7 @@ fuse_fwd_runs_multi_kernel(int K, int64_t J, const FuseDesign* __restrict__ tab,
 
 // one warp per column j pulls every design's CSC column in design order: dF_k[j] as tm_fuse_backward computes it for
 // design k, and dWt[j] = sum_k F_k[j] * acc_k[j] (the K per-design weight gradients are never materialised)
+template <bool WG>
 __global__ void __launch_bounds__(256)
 fuse_bwd_multi_kernel(int K, int64_t J, const FuseDesign* __restrict__ tab, const int* __restrict__ ep_off,
                       const float* __restrict__ g, int64_t ldg, const float* __restrict__ F,
@@ -219,10 +224,12 @@ fuse_bwd_multi_kernel(int K, int64_t J, const FuseDesign* __restrict__ tab, cons
 #pragma unroll
       for (int q = 0; q < 4; ++q) { acc.x += v[q].x; acc.y += v[q].y; acc.z += v[q].z; acc.w += v[q].w; }
     }
-    const float f = F[(int64_t)k * J + j];
-    const float4 p = make_float4(f * acc.x, f * acc.y, f * acc.z, f * acc.w);
-    if (k == 0) dw = p;
-    else { dw.x += p.x; dw.y += p.y; dw.z += p.z; dw.w += p.w; }
+    if constexpr (WG) {
+      const float f = F[(int64_t)k * J + j];
+      const float4 p = make_float4(f * acc.x, f * acc.y, f * acc.z, f * acc.w);
+      if (k == 0) dw = p;
+      else { dw.x += p.x; dw.y += p.y; dw.z += p.z; dw.w += p.w; }
+    }
     float dot = 0.f;
     if (e > s) {
       const float4 w = __ldg(reinterpret_cast<const float4*>(Wt + j * D + lane * 4));
@@ -231,7 +238,7 @@ fuse_bwd_multi_kernel(int K, int64_t J, const FuseDesign* __restrict__ tab, cons
     dot = warp_sum(dot);
     if (lane == 0) dF[(int64_t)k * J + j] = dot;
   }
-  st4(dWt + j * D + lane * 4, dw);
+  if constexpr (WG) st4(dWt + j * D + lane * 4, dw);
 }
 
 __global__ void gather_cols_kernel(int64_t T, int64_t w, const float* __restrict__ src, int64_t lds,
@@ -501,9 +508,12 @@ extern "C" int tm_fuse_backward(int64_t T, int64_t J, int64_t Dd, const int32_t*
                                 const int32_t* csc_t, const float* g, int64_t ld_g, const float* F,
                                 const float* Wt, float* dWt, float* dF, void* stream) {
   TM_REQUIRE(Dd == D, "tm_fuse_backward: D must be 128");
+  TM_REQUIRE(dF, "tm_fuse_backward: dF missing");
   (void)T;
   if (J <= 0) return 0;
-  fuse_bwd_kernel<<<(unsigned)cdiv(J * 32, 256), 256, 0, (cudaStream_t)stream>>>(J, csc_ptr, csc_t, g, ld_g, F, Wt, dWt, dF);
+  const unsigned grid = (unsigned)cdiv(J * 32, 256);
+  if (dWt) fuse_bwd_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(J, csc_ptr, csc_t, g, ld_g, F, Wt, dWt, dF);
+  else fuse_bwd_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(J, csc_ptr, csc_t, g, ld_g, F, Wt, dWt, dF);
   return check_launch("fuse_bwd");
 }
 
@@ -538,9 +548,12 @@ extern "C" int tm_fuse_backward_multi(int64_t K, int64_t J, int64_t Dd, const vo
                                       float* dF, void* stream) {
   TM_REQUIRE(Dd == D, "tm_fuse_backward_multi: D must be 128");
   TM_REQUIRE(K > 0 && design_tab && ep_off, "tm_fuse_backward_multi: bad design table");
+  TM_REQUIRE(dF, "tm_fuse_backward_multi: dF missing");
   if (J <= 0) return 0;
-  fuse_bwd_multi_kernel<<<(unsigned)cdiv(J * 32, 256), 256, 0, (cudaStream_t)stream>>>(
-      (int)K, J, reinterpret_cast<const FuseDesign*>(design_tab), ep_off, g, ld_g, F, Wt, dWt, dF);
+  const unsigned grid = (unsigned)cdiv(J * 32, 256);
+  const FuseDesign* tab = reinterpret_cast<const FuseDesign*>(design_tab);
+  if (dWt) fuse_bwd_multi_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>((int)K, J, tab, ep_off, g, ld_g, F, Wt, dWt, dF);
+  else fuse_bwd_multi_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>((int)K, J, tab, ep_off, g, ld_g, F, Wt, dWt, dF);
   return check_launch("fuse_bwd_multi");
 }
 

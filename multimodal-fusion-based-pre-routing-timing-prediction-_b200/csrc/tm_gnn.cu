@@ -612,7 +612,8 @@ gnn_net_bwd_kernel(SchedDev s, int p0, int cnt, const float* __restrict__ H, flo
   st4(G + off, relu_mask(hv, g));
 }
 
-template <bool H16>
+// WG == false: G and GA only -- the operands of the hoisted weight-gradient GEMMs (GZC, GHID) are not stored
+template <bool H16, bool WG>
 __global__ void __launch_bounds__(CT)
 gnn_cell_bwd_kernel(SchedDev s, int p0, int cnt, int crow0, const float* __restrict__ H, float* G,
                     const float* __restrict__ W1, const float* __restrict__ W2, float* GA,
@@ -710,7 +711,7 @@ gnn_cell_bwd_kernel(SchedDev s, int p0, int cnt, int crow0, const float* __restr
           *reinterpret_cast<float4*>(&T.in_lo[(r0 + r) * IN_LD + lane * 4]) = gzl;
         }
         st4(G + (int64_t)__shfl_sync(0xffffffffu, vv, r) * D + lane * 4, gz);
-        st4(GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4, gz);
+        if constexpr (WG) st4(GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4, gz);
       } else if constexpr (H16) {
         store_row_h(T, r0 + r, lane, make_float4(0.f, 0.f, 0.f, 0.f), -100);
       } else {
@@ -735,7 +736,7 @@ gnn_cell_bwd_kernel(SchedDev s, int p0, int cnt, int crow0, const float* __restr
 #pragma unroll
   for (int i = 0; i < TILE * HID / 4 / CT; ++i) {
     const int q = tid + i * CT, row = q >> 6, c4 = (q & 63) * 4;
-    if (t0 + row < cnt) {
+    if (WG && t0 + row < cnt) {
       if constexpr (H16)
         st4(GHID + (int64_t)(crow0 + t0 + row) * HID + c4, *reinterpret_cast<const float4*>(&T.hid_f[row * MID_LD + c4]));
       else
@@ -772,9 +773,11 @@ int launch_pdl(void (*kern)(KArgs...), unsigned grid, unsigned block, size_t sme
 int cell_smem_optin() {
   // the attribute is per function AND per device: set it on every call (cheap), so a second device works
   TM_CUDA(cudaFuncSetAttribute(gnn_cell_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
-  TM_CUDA(cudaFuncSetAttribute(gnn_cell_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
+  TM_CUDA(cudaFuncSetAttribute(gnn_cell_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
+  TM_CUDA(cudaFuncSetAttribute(gnn_cell_bwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
   TM_CUDA(cudaFuncSetAttribute(gnn_cell_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
-  TM_CUDA(cudaFuncSetAttribute(gnn_cell_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
+  TM_CUDA(cudaFuncSetAttribute(gnn_cell_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
+  TM_CUDA(cudaFuncSetAttribute(gnn_cell_bwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CELL_SMEM));
   return 0;
 }
 
@@ -898,6 +901,8 @@ extern "C" int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, c
                                const float* W2_in, const float* A, const float* LSE, const float* HIDb,
                                float* GA, float* GHID, float* GZC, void* ws, size_t ws_bytes, void* stream) {
   TM_REQUIRE(s && s->h_level_ptr && s->bn_ptr && s->bc_ptr, "tm_gnn_backward: bad schedule");
+  TM_REQUIRE((GHID == nullptr) == (GZC == nullptr), "tm_gnn_backward: GHID and GZC must be both set or both NULL");
+  const bool wg = GHID != nullptr;
   cudaStream_t st = (cudaStream_t)stream;
   const bool wide = s->num_levels > 0 && s->h_level_ptr[s->num_levels] / s->num_levels >= 6000;
   if ((gnn_impl() & 2) || ((gnn_impl() & 4) && wide)) {
@@ -921,7 +926,9 @@ extern "C" int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, c
     if (!cell) {
       TM_TRY(launch_pdl(gnn_net_bwd_kernel, (unsigned)cdiv(cnt, 8), 256, 0, st, "gnn_net_bwd", d, p0, cnt, H, G, (const float*)GA, A, LSE));
     } else {
-      TM_TRY(launch_pdl(h16 ? gnn_cell_bwd_kernel<true> : gnn_cell_bwd_kernel<false>, (unsigned)cdiv(cnt, TILE), CT, CELL_SMEM, st, "gnn_cell_bwd", d, p0, cnt, crow_end, H,
+      auto kern = h16 ? (wg ? gnn_cell_bwd_kernel<true, true> : gnn_cell_bwd_kernel<true, false>)
+                      : (wg ? gnn_cell_bwd_kernel<false, true> : gnn_cell_bwd_kernel<false, false>);
+      TM_TRY(launch_pdl(kern, (unsigned)cdiv(cnt, TILE), CT, CELL_SMEM, st, "gnn_cell_bwd", d, p0, cnt, crow_end, H,
                         G, W1, W2, GA, A, LSE, HIDb, GHID, GZC));
     }
   }

@@ -768,6 +768,9 @@ __device__ __forceinline__ void bwd_net_level(const BwdArgs& a, int p0, int cnt,
   c.stamp(PH_NBODY);
 }
 
+// WG == false: G and GA only.  GHID / GZC (the operands of the hoisted weight-gradient GEMMs) are not stored; g_z stays
+// in registers until the pair's exchange barrier instead of being staged in GZC.
+template <bool WG>
 __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -881,7 +884,7 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
         if (r < PPW && r < npin) {
           const float4 hv = ldg4(a.H + (int64_t)__shfl_sync(0xffffffffu, vv, r) * D + lane * 4);
           gz[r] = relu_mask(hv, *reinterpret_cast<const float4*>(scratch + (r0 + r) * D + lane * 4));
-          if (owner) *reinterpret_cast<float4*>(a.GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4) = gz[r];
+          if (WG && owner) *reinterpret_cast<float4*>(a.GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4) = gz[r];
         }
       }
       __syncthreads();                                       // every warp is done with the scratch rows
@@ -907,7 +910,7 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
           float gh = 0.f;
           if (t0 + n0 + j < cnt) {
             gh = hsel(hraw, n0 - cg * nper + j) > 0.f ? fmaf(vc[j], LO_INV, vm[j]) : 0.f;
-            a.GHID[(int64_t)(crow0 + t0 + n0 + j) * HID + c.rank * 128 + m] = gh * c.inv_s[n0 + j];
+            if constexpr (WG) a.GHID[(int64_t)(crow0 + t0 + n0 + j) * HID + c.rank * 128 + m] = gh * c.inv_s[n0 + j];
           }
           vm[j] = gh;
         }
@@ -923,7 +926,7 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
         for (int r = 0; r < NMAX / 16; ++r)
           if (r < PPW && r < npin)
             *reinterpret_cast<float4*>(a.G + (int64_t)__shfl_sync(0xffffffffu, vv, r) * D + lane * 4) =
-                *reinterpret_cast<const float4*>(a.GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4);
+                WG ? *reinterpret_cast<const float4*>(a.GZC + (int64_t)(crow0 + t0 + r0 + r) * D + lane * 4) : gz[r];
       }
       c.stamp(PH_CPUB);
     }
@@ -998,6 +1001,7 @@ int gnn_persist_backward(const tm_schedule* s, const float* H, float* G, const f
   TM_TRY(gnn_persist_begin(s, W2, W1, ws, st));
   BwdArgs a{s->level_ptr, s->cell_base, s->order, s->bn_ptr, s->bn_dst, s->bn_w, s->bc_ptr, s->bc_row, H, G, ws_planes(ws),
             A, LSE, HIDb, GA, GHID, GZC, ws_bar(ws), g_prof, lb, le};
-  return launch_persist(gnn_persist_bwd_kernel, a, st, "gnn_persist_bwd");
+  if (GHID) return launch_persist(gnn_persist_bwd_kernel<true>, a, st, "gnn_persist_bwd");
+  return launch_persist(gnn_persist_bwd_kernel<false>, a, st, "gnn_persist_bwd");
 }
 }  // namespace tmk

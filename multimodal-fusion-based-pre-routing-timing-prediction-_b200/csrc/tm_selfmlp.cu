@@ -664,15 +664,18 @@ struct B1Args {
   const int* h_rows;      // row of H (and of DH) that belongs to row m (NULL: m)
   float* DH;
   int64_t lddh;
-  // DX form (tm_selfmlp_gen_bwd1_dx): the input's data gradient dh W1, written to the row of X the forward read
+  // DX form (tm_selfmlp_gen_bwd1_dx, tm_selfmlp_rows_dx): the input's data gradient dh W1, written to the row of X the
+  // forward read (x_rows)
   float* dX;
   int64_t lddx;
 };
 
 // STORE == false: first-layer gradients of the generated MLP (above); DX adds the data gradient dX = dh W1, two FMAs per
-// hidden unit in the lane that owns the row, in hidden-unit order.  STORE == true: the same product with the epilogue
-// of the general MLP backward -- dh = (G W2) * (H > 0) written to DH (fc_cell_self: 36 inputs, the hidden layer is stored).
-template <bool STORE, bool DX>
+// hidden unit in the lane that owns the row, in hidden-unit order; WG == false (with DX) drops the first-layer weight
+// gradients and leaves dX the same bits.  STORE == true: the same product with the epilogue of the general MLP
+// backward -- dh = (G W2) * (H > 0) written to DH (fc_cell_self: 36 inputs, the hidden layer is stored); with DX, dh is
+// not written but multiplied into dX = dh W1 (kx <= 48 inputs) in the lane that owns the row, in hidden-unit order.
+template <bool STORE, bool DX, bool WG = true>
 __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   float* w0_s = reinterpret_cast<float*>(smem + B1_OFF_P);
@@ -781,6 +784,68 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
       }
     }
     __syncwarp();
+  } else if constexpr (STORE && DX) {
+    // ======================= epilogue (rows_dx): a lane owns one row: mask from H, dX = dh W1 in registers ==========
+    // W1 [256][kx] rows are read as warp-uniform 16-byte loads (one transaction per warp, L1-resident)
+    const int nk4 = a.kx >> 2;
+    float* dsc = reinterpret_cast<float*>(smem + B1_OFF_SCR + warp * B1_SCR_W) + lane * 9;   // this row's 8 gated dh values
+    uint32_t li = 0;
+    for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x, ++li) {
+      const int64_t m = t * TM + warp * 32 + lane;
+      const float* hp = nullptr;
+      if (m < a.M) hp = a.H + (a.h_rows ? (int64_t)a.h_rows[m] : m) * a.ldh;
+      float dx[48];
+#pragma unroll
+      for (int k = 0; k < 48; ++k) dx[k] = 0.f;
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {
+        mbar_wait_trap<MBAR_SPINS>(&acc_full[half], li & 1u);
+        tc_fence_after();
+        const float inv = inv_s[(li & 1u) * TM + warp * 32 + lane];
+        const uint32_t trow = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)half * 256u;
+#pragma unroll 1
+        for (int c = 0; c < 16; ++c) {
+          const int j0 = half * 128 + c * 8;
+          float4 mk[2];
+#pragma unroll
+          for (int e = 0; e < 2; ++e) mk[e] = hp ? ld4(hp + j0 + 4 * e) : make_float4(0.f, 0.f, 0.f, 0.f);
+          float vm[8], vc[8];
+          tmem_ld8(trow + (uint32_t)(c * 8), vm);
+          tmem_ld8(trow + 128u + (uint32_t)(c * 8), vc);
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            dsc[4 * e] = mk[e].x > 0.f ? fmaf(vc[4 * e], LO_INV, vm[4 * e]) * inv : 0.f;
+            dsc[4 * e + 1] = mk[e].y > 0.f ? fmaf(vc[4 * e + 1], LO_INV, vm[4 * e + 1]) * inv : 0.f;
+            dsc[4 * e + 2] = mk[e].z > 0.f ? fmaf(vc[4 * e + 2], LO_INV, vm[4 * e + 2]) * inv : 0.f;
+            dsc[4 * e + 3] = mk[e].w > 0.f ? fmaf(vc[4 * e + 3], LO_INV, vm[4 * e + 3]) * inv : 0.f;
+          }
+#pragma unroll 1
+          for (int i = 0; i < 8; ++i) {                      // (the loop stays rolled: 48 accumulators fill the budget)
+            const float d = dsc[i];
+            const float4* wr = reinterpret_cast<const float4*>(a.W1 + (size_t)(j0 + i) * a.kx);
+#pragma unroll
+            for (int k4 = 0; k4 < 12; ++k4) {
+              if (k4 < nk4) {
+                const float4 w = __ldg(wr + k4);
+                dx[4 * k4] = fmaf(d, w.x, dx[4 * k4]);
+                dx[4 * k4 + 1] = fmaf(d, w.y, dx[4 * k4 + 1]);
+                dx[4 * k4 + 2] = fmaf(d, w.z, dx[4 * k4 + 2]);
+                dx[4 * k4 + 3] = fmaf(d, w.w, dx[4 * k4 + 3]);
+              }
+            }
+          }
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&acc_empty[half]);
+      }
+      if (m < a.M) {
+        float* dp = a.dX + (a.x_rows ? (int64_t)a.x_rows[m] : m) * a.lddx;
+#pragma unroll
+        for (int k4 = 0; k4 < 12; ++k4)
+          if (k4 < nk4) st4(dp + 4 * k4, make_float4(dx[4 * k4], dx[4 * k4 + 1], dx[4 * k4 + 2], dx[4 * k4 + 3]));
+      }
+    }
   } else if constexpr (STORE) {
     // ======================= epilogue (STORE): a lane owns one row: mask from H, 128-bit stores to DH ===============
     uint32_t li = 0;
@@ -865,24 +930,26 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
             const float pre = fmaf(w0_s[j0 + i], x0, fmaf(w1_s[j0 + i], x1, b1_s[j0 + i]));
             const float dh = fmaf(vc[i], LO_INV, vm[i]) * inv;
             const float d = pre > 0.f ? dh : 0.f;
-            scr[lane * 33 + i] = d;
+            if constexpr (WG) scr[lane * 33 + i] = d;
             if constexpr (DX) {
               dx0 = fmaf(d, w0_s[j0 + i], dx0);
               dx1 = fmaf(d, w1_s[j0 + i], dx1);
             }
           }
-          __syncwarp();
-          float s = 0.f, s0 = 0.f, s1 = 0.f;
+          if constexpr (WG) {
+            __syncwarp();
+            float s = 0.f, s0 = 0.f, s1 = 0.f;
 #pragma unroll
-          for (int r = 0; r < 32; r += 4) {                    // (the rows' inputs: broadcast 16-byte reads)
-            const float4 p = *reinterpret_cast<const float4*>(xs0 + r), q = *reinterpret_cast<const float4*>(xs1 + r);
-            const float d0 = scr[r * 33 + lane], d1 = scr[(r + 1) * 33 + lane], d2 = scr[(r + 2) * 33 + lane], d3 = scr[(r + 3) * 33 + lane];
-            s += (d0 + d1) + (d2 + d3);
-            s0 = fmaf(d0, p.x, fmaf(d1, p.y, fmaf(d2, p.z, fmaf(d3, p.w, s0))));
-            s1 = fmaf(d0, q.x, fmaf(d1, q.y, fmaf(d2, q.z, fmaf(d3, q.w, s1))));
+            for (int r = 0; r < 32; r += 4) {                    // (the rows' inputs: broadcast 16-byte reads)
+              const float4 p = *reinterpret_cast<const float4*>(xs0 + r), q = *reinterpret_cast<const float4*>(xs1 + r);
+              const float d0 = scr[r * 33 + lane], d1 = scr[(r + 1) * 33 + lane], d2 = scr[(r + 2) * 33 + lane], d3 = scr[(r + 3) * 33 + lane];
+              s += (d0 + d1) + (d2 + d3);
+              s0 = fmaf(d0, p.x, fmaf(d1, p.y, fmaf(d2, p.z, fmaf(d3, p.w, s0))));
+              s1 = fmaf(d0, q.x, fmaf(d1, q.y, fmaf(d2, q.z, fmaf(d3, q.w, s1))));
+            }
+            acc[half * 4 + c][0] += s; acc[half * 4 + c][1] += s0; acc[half * 4 + c][2] += s1;
+            __syncwarp();
           }
-          acc[half * 4 + c][0] += s; acc[half * 4 + c][1] += s0; acc[half * 4 + c][2] += s1;
-          __syncwarp();
         }
         tc_fence_before();
         __syncwarp();
@@ -896,11 +963,13 @@ __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) 
         }
       }
     }
-    float* pp = a.part + ((size_t)blockIdx.x * EPI_W + warp) * 3 * HIDF;
+    if constexpr (WG) {
+      float* pp = a.part + ((size_t)blockIdx.x * EPI_W + warp) * 3 * HIDF;
 #pragma unroll
-    for (int i = 0; i < 8; ++i)
+      for (int i = 0; i < 8; ++i)
 #pragma unroll
-      for (int k = 0; k < 3; ++k) pp[(size_t)k * HIDF + i * 32 + lane] = acc[i][k];
+        for (int k = 0; k < 3; ++k) pp[(size_t)k * HIDF + i * 32 + lane] = acc[i][k];
+    }
   }
   tc_fence_before();
   __syncthreads();
@@ -1155,7 +1224,10 @@ int gen_bwd1(const char* name, int64_t M, const float* G, int64_t ldg, const int
   TM_REQUIRE(kx == 1 || kx == 2, "%s: the first layer must have 1 or 2 inputs", name);
   TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_bwd1_ws_bytes(), "%s: workspace too small (tm_selfmlp_bwd1_ws_bytes)", name);
   TM_REQUIRE((ldg & 3) == 0 && (reinterpret_cast<uintptr_t>(G) & 15) == 0, "%s: G rows must be 16-byte aligned", name);
+  TM_REQUIRE((dW1 == nullptr) == (db1 == nullptr), "%s: dW1 and db1 must be both set or both NULL", name);
+  TM_REQUIRE(dW1 || dX, "%s: dW1 / db1 NULL is served with dX only (tm_selfmlp_gen_bwd1_dx)", name);
   cudaStream_t st = (cudaStream_t)stream;
+  if (M <= 0 && !dW1) return 0;
   if (M <= 0) {
     TM_CUDA(cudaMemsetAsync(dW1, 0, (size_t)HIDF * kx * sizeof(float), st));
     TM_CUDA(cudaMemsetAsync(db1, 0, (size_t)HIDF * sizeof(float), st));
@@ -1168,6 +1240,11 @@ int gen_bwd1(const char* name, int64_t M, const float* G, int64_t ldg, const int
   const int64_t ntiles = (M + TM - 1) / TM;
   const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
   B1Args a{M, G, ldg, g_rows, X, ldx, x_rows, (int)kx, W1, b1, planes, part, nullptr, 0, nullptr, nullptr, 0, dX, lddx};
+  if (!dW1) {                 // data gradient only: no column accumulators, no partials, no reduction
+    TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+    selfmlp_gen_bwd1_kernel<false, true, false><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+    return check_launch("selfmlp_gen_bwd1_dx(no wgrad)");
+  }
   if (dX) {
     TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
     selfmlp_gen_bwd1_kernel<false, true><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
@@ -1221,6 +1298,31 @@ extern "C" int tm_selfmlp_rows_dh(int64_t M, const float* G, int64_t ldg, const 
   B1Args a{M, G, ldg, g_rows, nullptr, 0, nullptr, 0, nullptr, nullptr, planes, nullptr, H, ldh, h_rows, DH, lddh};
   selfmlp_gen_bwd1_kernel<true, false><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
   return check_launch("selfmlp_rows_dh");
+}
+
+/* dX[x_rows[m], 0:kin] = ((G[g_rows[m]] @ W2) * (H[h_rows[m]] > 0)) @ W1 for m < M: the data gradient of
+ * Linear(kin, 256) -> ReLU -> Linear(256, 128) whose hidden activations H were stored (fc_cell_self), in one pass; the
+ * hidden gradient never leaves the SM.  W1 [256][kin] as stored, kin % 4 == 0, kin <= 48.  ws: tm_selfmlp_rows_dh_ws_bytes(). */
+extern "C" int tm_selfmlp_rows_dx(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* W2, const float* H,
+                                  int64_t ldh, const int32_t* h_rows, const float* W1, int64_t kin, float* dX, int64_t lddx,
+                                  const int32_t* x_rows, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(kin > 0 && kin <= 48 && (kin & 3) == 0, "tm_selfmlp_rows_dx: kin must be a multiple of 4, <= 48");
+  TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_rows_dh_ws_bytes(), "tm_selfmlp_rows_dx: workspace too small (tm_selfmlp_rows_dh_ws_bytes)");
+  TM_REQUIRE(G && W2 && H && W1 && dX, "tm_selfmlp_rows_dx: G, W2, H, W1 and dX are required");
+  TM_REQUIRE((ldg & 3) == 0 && (reinterpret_cast<uintptr_t>(G) & 15) == 0 && (ldh & 3) == 0 && (reinterpret_cast<uintptr_t>(H) & 15) == 0 &&
+                 (lddx & 3) == 0 && lddx >= kin && (reinterpret_cast<uintptr_t>(dX) & 15) == 0 && (reinterpret_cast<uintptr_t>(W1) & 15) == 0,
+             "tm_selfmlp_rows_dx: G, H, W1 and dX rows must be 16-byte aligned (lddx >= kin)");
+  if (M <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  selfmlp_pack_t_kernel<<<(NOUT * HIDF + 255) / 256, 256, 0, st>>>(W2, planes);
+  TM_TRY(check_launch("selfmlp_pack_t"));
+  TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+  const int64_t ntiles = (M + TM - 1) / TM;
+  const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
+  B1Args a{M, G, ldg, g_rows, nullptr, 0, x_rows, (int)kin, W1, nullptr, planes, nullptr, H, ldh, h_rows, nullptr, 0, dX, lddx};
+  selfmlp_gen_bwd1_kernel<true, true, false><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+  return check_launch("selfmlp_rows_dx");
 }
 
 extern "C" size_t tm_selfmlp_lin1_ws_bytes() { return 2 * (size_t)L1_W_PLANE + 256; }

@@ -210,12 +210,12 @@ class DesignBatch:
 class PreparedDesign:
     VALUE_FIELDS = ("cell_feat", "net_feat", "image", "arrival_time")
 
-    def __init__(self, step, host, device, graph=None, pool=None, input_grads=False):
+    def __init__(self, step, host, device, graph=None, pool=None, input_grads=False, param_grads=True):
         self.batch = DesignBatch.from_host(host, device, graph=graph)
         self.static = {"cell_feat": self.batch.cell_feat, "net_feat": self.batch.net_feat,
                        "image": self.batch.image, "arrival_time": self.batch.arrival_time}
         torch.cuda.synchronize()
-        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads)
+        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads, param_grads=param_grads)
 
     def upload(self, host, stream=None):
         """Host -> device copy of the per-step values into the graph's static inputs."""
@@ -236,11 +236,11 @@ class PreparedDesign:
 class PreparedDesigns:
     """``DesignStep.prepare_many``: K resident designs, one captured step over all of them."""
 
-    def __init__(self, step, hosts, device, pool=None, input_grads=False):
+    def __init__(self, step, hosts, device, pool=None, input_grads=False, param_grads=True):
         self.parts = [DesignBatch.from_host(h, device) for h in hosts]
         self.batch = DesignBatch.concat(self.parts)
         torch.cuda.synchronize()
-        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads)
+        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads, param_grads=param_grads)
 
     def upload(self, hosts, stream=None):
         """Host -> device copy of every design's per-step values into its slices of the graph's static inputs."""
@@ -289,16 +289,17 @@ class DesignStep:
         self.layoutnet = isinstance(cnn, M.LayoutNet)    # else the U-Net (LayoutNet has no BatchNorm statistics)
 
     # ---------------------------------------------------------------- image branch
-    def _image_forward(self, image, need_bwd):
+    def _image_forward(self, image, need_bwd, update_stats=True):
         if self.layoutnet:
             return tm_unet.layoutnet_forward(self.cnn, image, need_bwd=need_bwd)
         # several designs: each image is normalised with its own statistics, as the reference's batch of one is
-        return tm_unet.unet_forward(self.cnn, image, need_bwd=need_bwd, update_stats=self.cnn.training, per_image=True)
+        return tm_unet.unet_forward(self.cnn, image, need_bwd=need_bwd, update_stats=update_stats and self.cnn.training,
+                                    per_image=True)
 
-    def _image_backward(self, st, gout, need_dx=False):
+    def _image_backward(self, st, gout, need_dx=False, need_wgrad=True):
         if self.layoutnet:
-            return tm_unet.layoutnet_backward(self.cnn, st, gout, need_dx=need_dx)
-        return tm_unet.unet_backward(self.cnn, st, gout, need_dx=need_dx)
+            return tm_unet.layoutnet_backward(self.cnn, st, gout, need_dx=need_dx, need_wgrad=need_wgrad)
+        return tm_unet.unet_backward(self.cnn, st, gout, need_dx=need_dx, need_wgrad=need_wgrad)
 
     @staticmethod
     def _check_feature_map(fmap, b):
@@ -353,7 +354,7 @@ class DesignStep:
         return pred.squeeze(-1)
 
     # ---------------------------------------------------------------- full step
-    def run(self, b, grad_scale=1.0, input_grads=False, pred_grad=None):
+    def run(self, b, grad_scale=1.0, input_grads=False, pred_grad=None, param_grads=True):
         """Forward + backward.  Returns (loss (1,) device tensor, pred (T,)); fills ``.grad``.  A batch of K designs
         (``DesignBatch.concat``) gives loss = mean of the designs' MSEs (``b.design_losses``, (K,)) and every gradient
         the mean of their gradients; predictions are per design as the one-design step gives them.
@@ -367,7 +368,15 @@ class DesignStep:
         ``pred_grad``: (T,) float32 device tensor, dObjective/dpred, that seeds the backward instead of the MSE's
         gradient, taken as given (no 1/T or 1/K factor; ``grad_scale`` must stay 1): every ``.grad`` and input gradient
         is then the vector-Jacobian product ``pred.backward(pred_grad)`` gives.  The loss is still computed.  Neither
-        option changes the parameter gradients' arithmetic: with ``pred_grad`` unset they are the same bits."""
+        option changes the parameter gradients' arithmetic: with ``pred_grad`` unset they are the same bits.
+        ``param_grads=False`` (needs ``input_grads``): a step against a frozen predictor, for layout optimisation or
+        saliency.  The model is left exactly as it was: no ``.grad`` is touched, no parameter changes, U-Net batch norm
+        normalises with the batch's statistics as the training step does but does not update its running statistics
+        or ``num_batches_tracked``, and no gradient all-reduce is posted.  No parameter-gradient kernel runs.  Loss,
+        predictions and the "net_feat" / "image" input gradients are the same bits as with ``param_grads=True``;
+        "cell_feat" comes from a fused data-gradient kernel that sums in another order (fp32-class)."""
+        if not param_grads and not input_grads:
+            raise ValueError("DesignStep.run: param_grads=False computes input gradients only; pass input_grads=True")
         if pred_grad is not None:
             T = int(b.endpoints.numel())
             if grad_scale != 1.0:
@@ -401,7 +410,7 @@ class DesignStep:
         img_cap = int(os.environ.get("TM_IMAGE_SM_CAP", "0")) if side is not main else 0
         with torch.cuda.stream(side):
             old_cap = tm_lib.lib().tm_tc_set_grid_cap(img_cap)
-            fmap, ust = self._image_forward(b.image, need_bwd=True)
+            fmap, ust = self._image_forward(b.image, need_bwd=True, update_stats=param_grads)
             tm_lib.lib().tm_tc_set_grid_cap(old_cap)
             self._check_feature_map(fmap, b)
             feat = fmap.reshape(-1)
@@ -427,50 +436,56 @@ class DesignStep:
         f0, f2 = m.mlp_fuse.layers[0], m.mlp_fuse.layers[2]
         dw1, db1, dw2, db2, dX = tm_ops.mlp2_backward(X, width, None, T, f0.weight.detach(), f2.weight.detach(),
                                                       hs["hf"], gpred, 1, need_dx=True,
-                                                      wgrad_stream=side if side is not main else None)
+                                                      wgrad_stream=side if side is not main else None,
+                                                      need_wgrad=param_grads)
         side.wait_stream(main)                               # dX is ready
         # ... the level embedding and the mask fusion (whose dF starts the U-Net backward) on the image stream
         a0, a2 = m.mlp_alpha.layers[0], m.mlp_alpha.layers[2]
         with torch.cuda.stream(side):
-            da1, dab1, da2, dab2, _ = tm_ops.mlp2_backward(hs["lv"], 1, None, T, a0.weight.detach(), a2.weight.detach(),
-                                                           hs["ha"], dX[:, 2 * D:], width, b1=a0.bias.detach())
+            # (a frozen step: the level embedding's input has no gradient, so mlp_alpha has no backward at all)
+            if param_grads:
+                da1, dab1, da2, dab2, _ = tm_ops.mlp2_backward(hs["lv"], 1, None, T, a0.weight.detach(),
+                                                               a2.weight.detach(), hs["ha"], dX[:, 2 * D:], width,
+                                                               b1=a0.bias.detach())
             dF, dfw, dfb = tm_ops.fusion_backward_multi(b.mask_rows_list, hs["tab"], b.ep_off, feat, hs["wt"],
-                                                        dX[:, D:], width)
-            head = [(f0.weight, dw1), (f0.bias, db1), (f2.weight, dw2), (f2.bias, db2), (a0.weight, da1),
-                    (a0.bias, dab1), (a2.weight, da2), (a2.bias, dab2), (m.fcn.weight, dfw), (m.fcn.bias, dfb)]
-            self._assign(head)
-            self._post_allreduce("head", [p for p, _ in head])
+                                                        dX[:, D:], width, need_wgrad=param_grads)
+            if param_grads:
+                head = [(f0.weight, dw1), (f0.bias, db1), (f2.weight, dw2), (f2.bias, db2), (a0.weight, da1),
+                        (a0.bias, dab1), (a2.weight, da2), (a2.bias, dab2), (m.fcn.weight, dfw), (m.fcn.bias, dfb)]
+                self._assign(head)
+                self._post_allreduce("head", [p for p, _ in head])
 
         # ---- GNN backward (main stream) next to the U-Net backward (image stream)
         call("tm_scatter_add_cols", T, D, dX, width, 0, endpoints, G, D, stream())
         if input_grads:
-            ggrads, dcf, dnf = tm_ops.gnn_backward(sched, saved, gp, G, need_dx=True)
+            ggrads, dcf, dnf = tm_ops.gnn_backward(sched, saved, gp, G, need_dx=True, need_wgrad=param_grads)
         else:
             ggrads = tm_ops.gnn_backward(sched, saved, gp, G)
-        pairs = list(zip(self.gnn_params, ggrads))
+        pairs = list(zip(self.gnn_params, ggrads)) if param_grads else []
         self._assign(pairs)
         with torch.cuda.stream(side):
             old_cap = tm_lib.lib().tm_tc_set_grid_cap(img_cap)
-            ug = self._image_backward(ust, dF.reshape(fmap.shape), need_dx=input_grads)
+            ug = self._image_backward(ust, dF.reshape(fmap.shape), need_dx=input_grads, need_wgrad=param_grads)
             tm_lib.lib().tm_tc_set_grid_cap(old_cap)
             if input_grads:
                 ug, dimg = ug
                 b.input_grads = {"cell_feat": dcf, "net_feat": dnf, "image": dimg}
-            upairs = [(self.cnn_params[k], ug[k]) for k in self.cnn_names]
+            upairs = [(self.cnn_params[k], ug[k]) for k in self.cnn_names] if param_grads else []
             self._assign(upairs)
         main.wait_stream(side)                               # join: every gradient exists on `main`
-        # The GNN and U-Net gradients go out as ONE exchange after the join (2.5 MB): posted separately they were two
-        # latency-bound all-reduces queued behind each other on the communication stream at the very end of the step
-        # (the U-Net's could not start before the GNN's, which waits for the last weight-gradient kernel)
-        self._post_allreduce("tail", [p for p, _ in pairs] + [p for p, _ in upairs])
-        self._wait_allreduce()
+        if param_grads:
+            # The GNN and U-Net gradients go out as ONE exchange after the join (2.5 MB): posted separately they were
+            # two latency-bound all-reduces queued behind each other on the communication stream at the very end of
+            # the step (the U-Net's could not start before the GNN's, which waits for the last weight-gradient kernel)
+            self._post_allreduce("tail", [p for p, _ in pairs] + [p for p, _ in upairs])
+            self._wait_allreduce()
         # a tensor-core kernel whose barrier timed out leaves garbage: the step's loss becomes NaN (loud in any
         # training loop, also under graph replay); tm_lib.check_err_flags() names the cause on the host
         call("tm_poison_on_error", loss, tm_lib.err_flag(dev), stream())
         return loss, pred.squeeze(-1)
 
     # ---------------------------------------------------------------- CUDA graph
-    def capture(self, b, warmup=2, pool=None, input_grads=False, pred_grad=None):
+    def capture(self, b, warmup=2, pool=None, input_grads=False, pred_grad=None, param_grads=True):
         """Capture ``run(b, input_grads=input_grads, pred_grad=pred_grad)`` (about 500 launches on two streams) into
         one CUDA graph.  The batch's tensors -- and ``pred_grad`` -- become the graph's static inputs: refresh them in
         place (``tensor.copy_``) and call the returned function, which replays the graph and returns the same (loss,
@@ -480,9 +495,12 @@ class DesignStep:
         ``TM_DP_GRAPH=0`` the graph holds the rank's compute only and one exchange is posted after each
         replay.  ``pool``: a ``torch.cuda.graph_pool_handle()`` shared by graphs that are replayed one
         after the other (several prepared designs of one rank share their activation memory).
+        ``param_grads=False``: a frozen step (see ``run``); the replay leaves every ``.grad`` alone and posts nothing.
         Call ``close()`` before ``torch.distributed.destroy_process_group()``."""
-        opts = dict(input_grads=input_grads, pred_grad=pred_grad)
-        if self.world <= 1 or os.environ.get("TM_DP_GRAPH", "1") != "0":
+        if not param_grads and not input_grads:
+            raise ValueError("DesignStep.capture: param_grads=False computes input gradients only; pass input_grads=True")
+        opts = dict(input_grads=input_grads, pred_grad=pred_grad, param_grads=param_grads)
+        if self.world <= 1 or not param_grads or os.environ.get("TM_DP_GRAPH", "1") != "0":
             return self._capture_local(b, warmup, pool, opts)
         world, self.world = self.world, 1                  # no collectives inside the captured region
         try:
@@ -513,7 +531,8 @@ class DesignStep:
         with torch.cuda.graph(g, pool=pool):
             loss, pred = self.run(b, **opts)
         self._graphs.append(g)
-        grads = [(p, p.grad) for p in list(self.model.parameters()) + list(self.cnn.parameters()) if p.grad is not None]
+        grads = [(p, p.grad) for p in list(self.model.parameters()) + list(self.cnn.parameters())
+                 if p.grad is not None] if opts.get("param_grads", True) else []
         igrads = b.input_grads if opts.get("input_grads") else None
 
         def replay():
@@ -526,20 +545,21 @@ class DesignStep:
         replay.graph = g
         return replay
 
-    def prepare(self, host, device, graph=None, pool=None, input_grads=False):
+    def prepare(self, host, device, graph=None, pool=None, input_grads=False, param_grads=True):
         """A design made resident for repeated steps: uploads everything once, builds the structure
         that depends only on the netlist and the endpoint batch (level schedule, CSRs, mask runs / CSC)
         and captures the step as a CUDA graph.  Returns a ``PreparedDesign``; its ``step(host)``
         refreshes the per-step VALUES (features, image, labels) from pinned host memory and replays.
         The structure (edges, endpoints, masks) must be the one given here.  ``input_grads``: every replay also
-        rewrites ``batch.input_grads`` (see ``run``)."""
-        return PreparedDesign(self, host, device, graph, pool, input_grads)
+        rewrites ``batch.input_grads`` (see ``run``); ``param_grads=False``: a frozen step (see ``run``)."""
+        return PreparedDesign(self, host, device, graph, pool, input_grads, param_grads)
 
-    def prepare_many(self, hosts, device, pool=None, input_grads=False):
+    def prepare_many(self, hosts, device, pool=None, input_grads=False, param_grads=True):
         """K designs made resident for repeated steps over all of them (``DesignBatch.concat``), captured as ONE CUDA
         graph.  Returns a ``PreparedDesigns``; its ``step(hosts)`` refreshes the per-step VALUES of all K from pinned
-        host memory and replays.  The structures must be the ones given here.  ``input_grads``: as in ``prepare``."""
-        return PreparedDesigns(self, hosts, device, pool, input_grads)
+        host memory and replays.  The structures must be the ones given here.  ``input_grads``, ``param_grads``: as in
+        ``prepare``."""
+        return PreparedDesigns(self, hosts, device, pool, input_grads, param_grads)
 
     @staticmethod
     def _assign(pairs):

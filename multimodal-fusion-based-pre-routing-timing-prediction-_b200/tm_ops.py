@@ -227,8 +227,27 @@ def _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, h_rows, dh):
     gemm_nn(n_rows, hid, nout, g, ldg, _f32c(w2), hid, dh, hid, a_rows=g_rows, c_rows=h_rows, mask=h, ldmask=hid)
 
 
+def _rows_dx(n_rows, g, ldg, g_rows, w1, w2, h, dx_out, rows):
+    """Data gradient alone of an MLP whose hidden activations were stored: dx_out[rows[m]] = ((g[g_rows[m]] @ w2) *
+    (h[m] > 0)) @ w1.  The reference's sizes (256 hidden, 128 outputs, <= 48 inputs) run as one fused kernel
+    (``tm_selfmlp_rows_dx``: the hidden gradient never leaves the SM); others take the two GEMMs."""
+    hid, kin = w1.shape
+    nout = w2.shape[0]
+    w1c = _f32c(w1)
+    if (FUSED_SELF_MLP and hid == 256 and nout == 128 and _precision() == 3 and kin % 4 == 0 and kin <= 48
+            and ldg % 4 == 0 and g.data_ptr() % 16 == 0 and h.stride(0) % 4 == 0 and h.data_ptr() % 16 == 0
+            and dx_out.stride(0) % 4 == 0 and dx_out.data_ptr() % 16 == 0):
+        nb = tm_lib.ws_bytes("tm_selfmlp_rows_dh_ws_bytes")
+        call("tm_selfmlp_rows_dx", n_rows, g, ldg, g_rows, _f32c(w2), h, h.stride(0), None, w1c, kin, dx_out,
+             dx_out.stride(0), rows, tm_lib.workspace(nb, dx_out.device), nb, stream())
+        return
+    dh = torch.empty(n_rows, hid, dtype=torch.float32, device=g.device)
+    _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, None, dh)
+    gemm_nn(n_rows, kin, hid, dh, hid, w1c, kin, dx_out, dx_out.stride(0), c_rows=rows)
+
+
 def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=False, b1=None, wgrad_stream=None,
-                  h_rows=None, dx_out=None):
+                  h_rows=None, dx_out=None, need_wgrad=True):
     """Gradients of a two-layer MLP.  ``g``: dLoss/d(out) rows (optionally gathered by ``g_rows``).
     ``h``: the hidden activations mlp2_forward returned, or None when they were generated on the fly
     (then ``b1`` is required).  Returns (dw1, db1, dw2, db2, dx or None).
@@ -238,10 +257,23 @@ def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=
     the rows the forward pass ran on (``tm_graph.BackwardCone``).
     ``dx_out`` (with ``need_dx``; required when ``rows`` gathers): the data gradient of MLP row i is written to row
     ``rows[i]`` of ``dx_out`` -- the row of ``x`` it read, so ``rows`` must be distinct -- and ``dx_out`` is returned as dx;
-    its other rows are left as they are.  The parameter gradients are the same bits as without ``need_dx``."""
+    its other rows are left as they are.  The parameter gradients are the same bits as without ``need_dx``.
+    ``need_wgrad=False`` (with ``need_dx``): the data gradient alone, no parameter-gradient work; returns
+    (None, None, None, None, dx).  dx is the same bits as with the parameter gradients, except for a stored hidden layer
+    of the reference's sizes (``fc_cell_self``), whose fused kernel sums the second product in another order."""
     hid, kin = w1.shape
     nout = w2.shape[0]
     dev = g.device
+    if not need_wgrad:
+        if not need_dx or h_rows is not None:
+            raise RuntimeError("mlp2_backward: need_wgrad=False needs need_dx and no h_rows")
+        if dx_out is None:
+            if rows is not None:
+                raise RuntimeError("mlp2_backward: a data gradient of gathered rows needs dx_out")
+            dx_out = torch.empty(n_rows, kin, dtype=torch.float32, device=dev)
+        if n_rows > 0:
+            _mlp2_dx(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows, b1, dx_out, wgrad_stream is not None)
+        return None, None, None, None, dx_out
     dw2 = torch.empty(nout, hid, dtype=torch.float32, device=dev)
     db2 = torch.empty(nout, dtype=torch.float32, device=dev)
     dw1 = torch.empty(hid, kin, dtype=torch.float32, device=dev)
@@ -334,6 +366,33 @@ def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=
     return dw1, db1, dw2, db2, dx_out if need_dx else None
 
 
+def _mlp2_dx(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows, b1, dx_out, head):
+    """``mlp2_backward(need_wgrad=False)``: the data-gradient launches of each route, without the weight-gradient ones."""
+    hid, kin = w1.shape
+    nout = w2.shape[0]
+    dev = g.device
+    if h is None:                                            # generated hidden layer (kin <= 2)
+        if b1 is None:
+            raise RuntimeError("mlp2_backward: generated hidden activations need b1")
+        prec = _precision()
+        prec = 3 if prec is None else prec
+        if FUSED_SELF_MLP and hid == 256 and nout == 128 and prec == 3 and ldg % 4 == 0 and g.data_ptr() % 16 == 0:
+            nb = tm_lib.ws_bytes("tm_selfmlp_bwd1_ws_bytes")
+            call("tm_selfmlp_gen_bwd1_dx", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2),
+                 None, None, dx_out, dx_out.stride(0), tm_lib.workspace(nb, dev), nb, stream())
+            return
+        hm = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
+        gemm_nn(n_rows, hid, kin, x, ldx, _f32c(w1), kin, hm, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True)
+        _rows_dx(n_rows, g, ldg, g_rows, w1, w2, hm, dx_out, rows)       # (kin <= 2: the two GEMMs)
+        return
+    if head:                                                 # the head's route (mlp2_backward with wgrad_stream)
+        dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
+        gemm_nn(n_rows, hid, nout, g, ldg, _f32c(w2), hid, dh, hid, a_rows=g_rows, mask=h, ldmask=hid)
+        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx_out, dx_out.stride(0), c_rows=rows)
+        return
+    _rows_dx(n_rows, g, ldg, g_rows, w1, w2, h, dx_out, rows)
+
+
 # --------------------------------------------------------------------------------------------
 # GNN propagation
 # --------------------------------------------------------------------------------------------
@@ -394,7 +453,7 @@ def gnn_forward(sched, cell_feat, net_feat, params, save=True, impl=None, x_rows
     return H, saved
 
 
-def gnn_backward(sched, saved, params, G, cone=None, need_dx=False):
+def gnn_backward(sched, saved, params, G, cone=None, need_dx=False, need_wgrad=True):
     """``G`` (N,128): dLoss/dH, consumed (overwritten with dLoss/d pre-activation).
     Returns the 12 parameter gradients in GNN_PARAM_NAMES order.
     ``cone`` (``tm_graph.BackwardCone`` of the endpoints that seeded G): the weight-gradient contractions run over
@@ -403,13 +462,32 @@ def gnn_backward(sched, saved, params, G, cone=None, need_dx=False):
     the ``cell_feat`` / ``net_feat`` the forward read.  The self-term S enters each pin's pre-activation linearly, so
     after the sweep G is dLoss/dS and the feature gradient is the self MLPs' data gradient of it.  Rows the
     propagation never reads are exactly zero: net-class pins in ``dcell_feat``, cell-class pins in ``dnet_feat``,
-    unscheduled pins in both.  The parameter gradients are the same bits as without ``need_dx``."""
+    unscheduled pins in both.  The parameter gradients are the same bits as without ``need_dx``.
+    ``need_wgrad=False`` (with ``need_dx``): the feature gradients alone, ``(None, dcell_feat, dnet_feat)``; the sweep
+    stores no weight-gradient operands and no parameter gradient is computed.  G and dnet_feat are the same bits;
+    dcell_feat comes from the fused ``fc_cell_self`` data-gradient kernel (``tm_selfmlp_rows_dx``)."""
     if need_dx and cone is not None:
         raise RuntimeError("gnn_backward: a BackwardCone has no feature-gradient path")
+    if not need_wgrad and not need_dx:
+        raise RuntimeError("gnn_backward: need_wgrad=False needs need_dx")
     (cs1w, cs1b, cs2w, cs2b, ns1w, ns1b, ns2w, ns2b, cn1w, cn1b, cn2w, cn2b) = [_f32c(p) for p in params]
     dev = G.device
     ncr = sched.n_cell_rows
     GA = torch.empty(max(ncr, 1), D, dtype=torch.float32, device=dev)
+    if not need_wgrad:
+        nb = tm_lib.ws_bytes("tm_gnn_ws_bytes")
+        call("tm_gnn_backward", sched.struct, saved["H"], G, cn1w, cn2w, saved["A"], saved["LSE"], saved["HID"],
+             GA, None, None, tm_lib.workspace(nb, dev), nb, stream())
+        cf, nf = saved["cell_feat"], saved["net_feat"]
+        cpins, npins = sched.cell_class, sched.net_class
+        xc, xn = saved.get("x_rows") or (cpins, npins)
+        dcf = torch.zeros(cf.shape, dtype=torch.float32, device=dev)
+        dnf = torch.zeros(nf.shape, dtype=torch.float32, device=dev)
+        mlp2_backward(cf, cf.stride(0), xc, int(cpins.numel()), cs1w, cs2w, saved["hc"], G, D, g_rows=cpins, b1=cs1b,
+                      need_dx=True, dx_out=dcf, need_wgrad=False)
+        mlp2_backward(nf, nf.stride(0), xn, int(npins.numel()), ns1w, ns2w, saved["hn"], G, D, g_rows=npins, b1=ns1b,
+                      need_dx=True, dx_out=dnf, need_wgrad=False)
+        return None, dcf, dnf
     GHID = torch.empty(max(ncr, 1), 256, dtype=torch.float32, device=dev)
     GZC = torch.empty(max(ncr, 1), D, dtype=torch.float32, device=dev)
     nb = tm_lib.ws_bytes("tm_gnn_ws_bytes")
@@ -506,14 +584,17 @@ def fusion_forward(mask_rows, feat, fcn_w, fcn_b, out, ldo):
     return wt
 
 
-def fusion_backward(mask_rows, feat, wt, g, ldg):
-    """Returns (dfeat (J,), dfcn_w (128,J), dfcn_b (128,))."""
+def fusion_backward(mask_rows, feat, wt, g, ldg, need_wgrad=True):
+    """Returns (dfeat (J,), dfcn_w (128,J), dfcn_b (128,)); ``need_wgrad=False``: (dfeat, None, None), dfeat the same
+    bits."""
     J = int(feat.numel())
     dev = feat.device
     cptr, ct = mask_rows.csc()
-    dwt = torch.empty(J, D, dtype=torch.float32, device=dev)
+    dwt = torch.empty(J, D, dtype=torch.float32, device=dev) if need_wgrad else None
     dF = torch.empty(J, dtype=torch.float32, device=dev)
     call("tm_fuse_backward", mask_rows.T, J, D, cptr, ct, g, ldg, feat, wt, dwt, dF, stream())
+    if not need_wgrad:
+        return dF, None, None
     db = colsum(g, mask_rows.T, D, ldg)
     return dF, transpose(dwt), db
 
@@ -535,16 +616,19 @@ def fusion_forward_multi(rows, tab, ep_off, feat, fcn_w, fcn_b, out, ldo):
     return wt
 
 
-def fusion_backward_multi(rows, tab, ep_off, feat, wt, g, ldg):
-    """Returns (dfeat (K*J,), dfcn_w (128,J) summed over the designs, dfcn_b (128,)).  K = 1 is ``fusion_backward``."""
+def fusion_backward_multi(rows, tab, ep_off, feat, wt, g, ldg, need_wgrad=True):
+    """Returns (dfeat (K*J,), dfcn_w (128,J) summed over the designs, dfcn_b (128,)).  K = 1 is ``fusion_backward``.
+    ``need_wgrad=False``: (dfeat, None, None)."""
     K = len(rows)
     if K == 1:
-        return fusion_backward(rows[0], feat, wt, g, ldg)
+        return fusion_backward(rows[0], feat, wt, g, ldg, need_wgrad)
     J = int(feat.numel()) // K
     dev = feat.device
-    dwt = torch.empty(J, D, dtype=torch.float32, device=dev)
+    dwt = torch.empty(J, D, dtype=torch.float32, device=dev) if need_wgrad else None
     dF = torch.empty(K * J, dtype=torch.float32, device=dev)
     call("tm_fuse_backward_multi", K, J, D, tab, ep_off, g, ldg, feat, wt, dwt, dF, stream())
+    if not need_wgrad:
+        return dF, None, None
     db = colsum(g, sum(r.T for r in rows), D, ldg)
     return dF, transpose(dwt), db
 

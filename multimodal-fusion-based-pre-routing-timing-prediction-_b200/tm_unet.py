@@ -296,9 +296,10 @@ def _dgrad_image(dr, lddr, bf16, s, w, dimg):
          stream())
 
 
-def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx, dimg=None, w1=None):
+def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx, dimg=None, w1=None, wg=True):
     """dout: gradient w.r.t. the block output (strided).  Writes dx (if not None); dimg (NCHW, optional): the gradient
-    w.r.t. the block input when it is the input image, through the first convolution's weight w1."""
+    w.r.t. the block input when it is the input image, through the first convolution's weight w1.  ``wg=False``: no
+    weight gradient is computed and nothing is added to ``grads`` (the batch-norm backward still reduces: dx needs it)."""
     B, H, W, cin, cmid, cout = s["B"], s["H"], s["W"], s["cin"], s["cmid"], s["cout"]
     npix = B * H * W
     dev = dout.device
@@ -307,12 +308,12 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx, dimg=None, w1=N
         dr2 = _empty(npix, cout, dev=dev)
         dg2, db2 = _bn_relu_bwd(ws, s["r2"], cout, dout, lddo, npix, cout, s["g2"], s["be2"], s["m2"], s["i2"],
                                 dr2, cout)
-        dw2 = _wgrad_tf(ws, s["a1"], cmid, dr2, cout, B, H, W, cmid, cmid, cout)
+        dw2 = _wgrad_tf(ws, s["a1"], cmid, dr2, cout, B, H, W, cmid, cmid, cout) if wg else None
         _conv_tf(ws, dr2, cout, B, H, W, cout, cmid, s["wd2"], da1, cmid)
         dr1 = _empty(npix, cmid, dev=dev)
         dg1, db1 = _bn_relu_bwd(ws, s["r1"], cmid, da1, cmid, npix, cmid, s["g1"], s["be1"], s["m1"], s["i1"],
                                 dr1, cmid)
-        dw1 = _wgrad_tf(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, _cpad(cin), cin, cmid)
+        dw1 = _wgrad_tf(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, _cpad(cin), cin, cmid) if wg else None
         if dx is not None:
             _conv_tf(ws, dr1, cmid, B, H, W, cmid, cin, s["wd1"], dx, lddx)
         if dimg is not None:
@@ -323,12 +324,12 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx, dimg=None, w1=N
         dr2b = torch.empty(npix, cout, dtype=torch.bfloat16, device=dev)
         dg2, db2 = _bn_relu_bwd(ws, s["r2"], cout, dout, lddo, npix, cout, s["g2"], s["be2"], s["m2"], s["i2"],
                                 None, 0, dxb=dr2b)
-        dw2 = _wgrad_tma(ws, s["a1b"], dr2b, B, H, W, cmid, cout)
+        dw2 = _wgrad_tma(ws, s["a1b"], dr2b, B, H, W, cmid, cout) if wg else None
         _conv_tma(dr2b, B, H, W, cout, cmid, s["wd2"], da1, cmid)
         dr1b = torch.empty(npix, cmid, dtype=torch.bfloat16, device=dev)
         dg1, db1 = _bn_relu_bwd(ws, s["r1"], cmid, da1, cmid, npix, cmid, s["g1"], s["be1"], s["m1"], s["i1"],
                                 None, 0, dxb=dr1b)
-        dw1 = _wgrad_tma(ws, s["xb"], dr1b, B, H, W, cin, cmid)
+        dw1 = _wgrad_tma(ws, s["xb"], dr1b, B, H, W, cin, cmid) if wg else None
         if dx is not None:
             _conv_tma(dr1b, B, H, W, cmid, cin, s["wd1"], dx, lddx)
         if dimg is not None:
@@ -338,15 +339,17 @@ def _double_conv_bwd(ws, s, dout, lddo, grads, prefix, dx, lddx, dimg=None, w1=N
         dg2, db2 = _bn_relu_bwd(ws, s["r2"], cout, dout, lddo, npix, cout, s["g2"], s["be2"], s["m2"], s["i2"],
                                 dr2, cout)
         dr1 = _empty(npix, cmid, dev=dev)
-        dw2, _ = _conv_wgrad(ws, s["a1"], cmid, dr2, cout, B, H, W, cmid, cout, 3, False)
+        dw2 = _conv_wgrad(ws, s["a1"], cmid, dr2, cout, B, H, W, cmid, cout, 3, False)[0] if wg else None
         _conv(dr2, cout, B, H, W, cout, cmid, 3, s["wb2"], None, da1, cmid)
         dg1, db1 = _bn_relu_bwd(ws, s["r1"], cmid, da1, cmid, npix, cmid, s["g1"], s["be1"], s["m1"], s["i1"],
                                 dr1, cmid)
-        dw1, _ = _conv_wgrad(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, cin, cmid, 3, False)
+        dw1 = _conv_wgrad(ws, s["x"], s["ldx"], dr1, cmid, B, H, W, cin, cmid, 3, False)[0] if wg else None
         if dx is not None:
             _conv(dr1, cmid, B, H, W, cmid, cin, 3, s["wb1"], None, dx, lddx)
         if dimg is not None:
             _dgrad_image(dr1, cmid, False, s, w1, dimg)
+    if not wg:
+        return
     grads[prefix + ".0.weight"] = dw1
     grads[prefix + ".1.weight"], grads[prefix + ".1.bias"] = dg1, db1
     grads[prefix + ".3.weight"] = dw2
@@ -458,9 +461,11 @@ def unet_forward(net, x, need_bwd=True, update_stats=True, per_image=False):
     return out, st
 
 
-def unet_backward(net, st, gout, need_dx=False):
+def unet_backward(net, st, gout, need_dx=False, need_wgrad=True):
     """gout: (B,1,H/2,W/2).  Returns {state_dict-style name: gradient} for every parameter; with ``need_dx``
-    (grads, dx), dx the gradient w.r.t. the input image in its layout: (B,3,H,W), or (3,H,W) for a 3-D input."""
+    (grads, dx), dx the gradient w.r.t. the input image in its layout: (B,3,H,W), or (3,H,W) for a 3-D input.
+    ``need_wgrad=False`` (a frozen network): no weight-gradient kernel runs on any route and ``grads`` is empty; dx is
+    the same bits."""
     _enter(net)
     global SEG
     SEG = st["seg"]
@@ -471,10 +476,11 @@ def unet_backward(net, st, gout, need_dx=False):
     grads = {}
     d_oraw = _empty(B * H * W, 1, dev=dev)
     call("tm_pool2x2_backward", B, H, W, 1, mode, gout, 1, st["out"], 1, st["oidx"], d_oraw, 1, RELU, None, 0, stream())
-    dw, db = _empty(1, 16, 1, 1, dev=dev), _empty(1, dev=dev)
-    nb = tm_lib.ws_bytes("tm_conv1x1_c1_wgrad_ws", 16)
-    call("tm_conv1x1_c1_wgrad", B * H * W, 16, st["y3"], st["ld3"], d_oraw, 1, dw, db, ws.get(nb), nb, stream())
-    grads["outc.conv.0.weight"], grads["outc.conv.0.bias"] = dw, db
+    if need_wgrad:
+        dw, db = _empty(1, 16, 1, 1, dev=dev), _empty(1, dev=dev)
+        nb = tm_lib.ws_bytes("tm_conv1x1_c1_wgrad_ws", 16)
+        call("tm_conv1x1_c1_wgrad", B * H * W, 16, st["y3"], st["ld3"], d_oraw, 1, dw, db, ws.get(nb), nb, stream())
+        grads["outc.conv.0.weight"], grads["outc.conv.0.bias"] = dw, db
     dy = _empty(B * H * W, 16, dev=dev)
     call("tm_conv1x1_c1_dgrad", B * H * W, 16, d_oraw, 1, st["wo"], dy, 16, stream())
     lddy = 16
@@ -483,7 +489,8 @@ def unet_backward(net, st, gout, need_dx=False):
     for j in (2, 1, 0):
         i = 2 - j
         dcat = _empty(B * Hs[i] * Ws_[i], 2 * chans[i], dev=dev)
-        _double_conv_bwd(ws, st[f"dec{j}"], dy, lddy, grads, f"{names[j]}.conv.double_conv", dcat, 2 * chans[i])
+        _double_conv_bwd(ws, st[f"dec{j}"], dy, lddy, grads, f"{names[j]}.conv.double_conv", dcat, 2 * chans[i],
+                         wg=need_wgrad)
         dskip[i] = dcat                                  # first half = gradient of the skip tensor
         u = st[f"up{j}"]
         half = dcat[:, chans[i]:]
@@ -492,18 +499,19 @@ def unet_backward(net, st, gout, need_dx=False):
             # bf16 mode: weight and data gradient on the TMA path, both from one bf16 copy of the gradient half
             npo = B * Hs[i] * Ws_[i]
             halfb = _to_bf16(half, 2 * chans[i], npo, u["cout"])
-            dwu, dbt = _empty(u["cin"], u["cout"], 2, 2, dev=dev), _empty(u["cout"], dev=dev)
-            nb = tm_lib.ws_bytes("tm_convt2x2_bf16_wgrad_ws", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"])
-            call("tm_convt2x2_bf16_wgrad", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"], u["xb"], halfb, dwu, ws.get(nb), nb,
-                 tm_lib.err_flag(dev), stream())
-            nbc = tm_lib.ws_bytes("tm_colsum_ws", npo, u["cout"])
-            call("tm_colsum", npo, u["cout"], half, 2 * chans[i], None, dbt, 0, tm_lib.workspace(nbc, dev), nbc, stream())
+            if need_wgrad:
+                dwu, dbt = _empty(u["cin"], u["cout"], 2, 2, dev=dev), _empty(u["cout"], dev=dev)
+                nb = tm_lib.ws_bytes("tm_convt2x2_bf16_wgrad_ws", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"])
+                call("tm_convt2x2_bf16_wgrad", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"], u["xb"], halfb, dwu, ws.get(nb),
+                     nb, tm_lib.err_flag(dev), stream())
+                nbc = tm_lib.ws_bytes("tm_colsum_ws", npo, u["cout"])
+                call("tm_colsum", npo, u["cout"], half, 2 * chans[i], None, dbt, 0, tm_lib.workspace(nbc, dev), nbc, stream())
             call("tm_convt2x2_bf16_dgrad", B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"], halfb, u["wdq"], dy, u["cin"],
                  tm_lib.err_flag(dev), stream())
         else:
             tf = u.get("wdf") is not None
             shape = (B, Hs[i + 1], Ws_[i + 1], u["cin"], u["cout"])
-            if tf and tm_lib.ws_bytes("tm_convt2x2_tf32_wgrad_supported", *shape) == 1:
+            if need_wgrad and tf and tm_lib.ws_bytes("tm_convt2x2_tf32_wgrad_supported", *shape) == 1:
                 # tf32x3 mode: weight gradient on the TMA path (its N side needs 32-channel boxes: Cout >= 32)
                 nb = tm_lib.ws_bytes("tm_convt2x2_tf32_ws", *shape)
                 dwu, dbt = _empty(u["cin"], u["cout"], 2, 2, dev=dev), _empty(u["cout"], dev=dev)
@@ -513,7 +521,7 @@ def unet_backward(net, st, gout, need_dx=False):
                 nbc = tm_lib.ws_bytes("tm_colsum_ws", npo, u["cout"])
                 call("tm_colsum", npo, u["cout"], half, 2 * chans[i], None, dbt, 0, tm_lib.workspace(nbc, dev), nbc,
                      stream())
-            else:
+            elif need_wgrad:
                 nb = tm_lib.ws_bytes("tm_convt2x2_wgrad_ws", *shape)
                 dwt, dbt = _empty(u["cin"], 4 * u["cout"], dev=dev), _empty(u["cout"], dev=dev)
                 call("tm_convt2x2_wgrad_nhwc", *shape, u["x"], u["ldx"], half,
@@ -527,7 +535,8 @@ def unet_backward(net, st, gout, need_dx=False):
             else:
                 call("tm_convt2x2_dgrad_nhwc", *shape, half, 2 * chans[i], Hs[i],
                      Ws_[i], 0, 0, u["wtT"], dy, u["cin"], stream())
-        grads[f"{names[j]}.up.weight"], grads[f"{names[j]}.up.bias"] = dwu, dbt
+        if need_wgrad:
+            grads[f"{names[j]}.up.weight"], grads[f"{names[j]}.up.bias"] = dwu, dbt
         lddy = u["cin"]
     # encoder, deepest first; dy is the gradient of x4
     enc_names = ["inc.double_conv", "down1.maxpool_conv.1.double_conv", "down2.maxpool_conv.1.double_conv",
@@ -536,7 +545,7 @@ def unet_backward(net, st, gout, need_dx=False):
         s = st[f"enc{i}"]
         if i > 0:
             dpool = _empty(B * Hs[i] * Ws_[i], chans[i - 1], dev=dev)
-            _double_conv_bwd(ws, s, dy, lddy, grads, enc_names[i], dpool, chans[i - 1])
+            _double_conv_bwd(ws, s, dy, lddy, grads, enc_names[i], dpool, chans[i - 1], wg=need_wgrad)
             p = st["pool"][i - 1]
             dprev = _empty(B * Hs[i - 1] * Ws_[i - 1], chans[i - 1], dev=dev)
             # pooling backward and the gradient arriving through the skip connection (first half of dcat) in one pass
@@ -545,7 +554,7 @@ def unet_backward(net, st, gout, need_dx=False):
             dy, lddy = dprev, chans[i - 1]
         else:
             dx = _empty(B, 3, H, W, dev=dev) if need_dx else None
-            _double_conv_bwd(ws, s, dy, lddy, grads, enc_names[0], None, 0, dimg=dx, w1=st["w_in"])
+            _double_conv_bwd(ws, s, dy, lddy, grads, enc_names[0], None, 0, dimg=dx, w1=st["w_in"], wg=need_wgrad)
     if not need_dx:
         return grads
     return grads, (dx[0] if st["squeeze"] else dx)
@@ -572,8 +581,10 @@ class UNetFn(torch.autograd.Function):
         if not ctx.needs_input_grad[1]:
             grads = unet_backward(ctx.net, ctx.st, gout)
             return (None, None, None) + tuple(grads[k] for k in ctx.names)
-        grads, dx = unet_backward(ctx.net, ctx.st, gout, need_dx=True)
-        return (None, dx.to(ctx.x_dtype), None) + tuple(grads[k] for k in ctx.names)
+        # frozen parameters (requires_grad=False): the image gradient alone, no weight-gradient kernel
+        wg = any(ctx.needs_input_grad[3:])
+        grads, dx = unet_backward(ctx.net, ctx.st, gout, need_dx=True, need_wgrad=wg)
+        return (None, dx.to(ctx.x_dtype), None) + tuple(grads.get(k) for k in ctx.names)
 
 
 # --------------------------------------------------------------------------------------------
@@ -654,9 +665,10 @@ def layoutnet_forward(net, x, need_bwd=True):
     return (out[0] if squeeze else out), st
 
 
-def layoutnet_backward(net, st, gout, need_dx=False):
+def layoutnet_backward(net, st, gout, need_dx=False, need_wgrad=True):
     """gout: the output's gradient.  Returns {state_dict-style name: gradient}; with ``need_dx`` (grads, dx), dx the
-    gradient w.r.t. the input image in its layout: (B,2,H,W), or (2,H,W) for a 3-D input."""
+    gradient w.r.t. the input image in its layout: (B,2,H,W), or (2,H,W) for a 3-D input.  ``need_wgrad=False``: no
+    weight- or bias-gradient kernel runs and ``grads`` is empty; dx is the same bits."""
     _enter(net)
     B, mode, ws = st["B"], st["mode"], st["ws"]
     dev = gout.device
@@ -681,15 +693,17 @@ def layoutnet_backward(net, st, gout, need_dx=False):
         if r["tma"]:
             # one bf16 copy of dy feeds the weight and the data gradient; the bias gradient sums the fp32 dy
             dyb = _to_bf16(dy, cout, npix, cout)
+        if need_wgrad and r["tma"]:
             dw, db = _empty(cout, cin, k, k, dev=dev), _empty(cout, dev=dev)
             nb = tm_lib.ws_bytes("tm_convkxk_bf16_wgrad_ws", B, h, w, cin, cout, k)
             call("tm_convkxk_bf16_wgrad", B, h, w, cin, cout, k, r["xb"], dyb, dw, ws.get(nb), nb, tm_lib.err_flag(dev),
                  stream())
             nbc = tm_lib.ws_bytes("tm_colsum_ws", npix, cout)
             call("tm_colsum", npix, cout, dy, cout, None, db, 0, tm_lib.workspace(nbc, dev), nbc, stream())
-        else:
+        elif need_wgrad:
             dw, db = _conv_wgrad(ws, r["x"], cin, dy, cout, B, h, w, cin, cout, k, True)
-        grads[r["name"] + ".weight"], grads[r["name"] + ".bias"] = dw, db
+        if need_wgrad:
+            grads[r["name"] + ".weight"], grads[r["name"] + ".bias"] = dw, db
         if li > 0:
             dx = _empty(npix, cin, dev=dev)
             if r["tma"]:
@@ -720,5 +734,6 @@ class LayoutNetFn(torch.autograd.Function):
         if not ctx.needs_input_grad[1]:
             grads = layoutnet_backward(ctx.net, ctx.st, gout)
             return (None, None, None) + tuple(grads[k] for k in ctx.names)
-        grads, dx = layoutnet_backward(ctx.net, ctx.st, gout, need_dx=True)
-        return (None, dx.to(ctx.x_dtype), None) + tuple(grads[k] for k in ctx.names)
+        wg = any(ctx.needs_input_grad[3:])                 # frozen parameters: the image gradient alone
+        grads, dx = layoutnet_backward(ctx.net, ctx.st, gout, need_dx=True, need_wgrad=wg)
+        return (None, dx.to(ctx.x_dtype), None) + tuple(grads.get(k) for k in ctx.names)
