@@ -292,6 +292,15 @@ int tm_mse_multi(int64_t K, const int32_t* ep_off, const float* pred, const floa
  * required / label may be NULL (regression statistics only). */
 int tm_step_metrics(int64_t T, const float* pred, const float* arrival, const float* required,
                     const int64_t* label, float* out8, void* stream);
+/* The same statistics per segment, for validate() (train.py:137-291) and test.py's per-design / per-level report:
+ * segment s is the endpoint list seg_idx[seg_ptr[s] .. seg_ptr[s+1]) (int32 on the device; segments may overlap or be
+ * empty).  out (n_seg, 9) float32, row s = [mse, r2, correct, tp, fn, tn, fp, count, mape]: the first eight as out8 of
+ * tm_step_metrics, mape = mean(|pred - y| / max(|y|, 1.17e-6)) (torchmetrics MeanAbsolutePercentageError).  r2 is NaN
+ * for count < 2 or a zero total sum of squares; an empty segment gives count 0, NaN mse / r2 / mape and zero counts.
+ * One CTA per segment, fp64 sums in a fixed order: the same bits on every launch.  No synchronisation (capturable).
+ * required / label may be NULL. */
+int tm_eval_metrics(int32_t n_seg, const int32_t* seg_ptr, const int32_t* seg_idx, const float* pred,
+                    const float* arrival, const float* required, const int64_t* label, float* out, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * G4  U-Net / LayoutNet image branch, fp32 NHWC (replaces the cuDNN/ATen calls behind

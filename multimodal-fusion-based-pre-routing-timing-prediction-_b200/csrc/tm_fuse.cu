@@ -427,6 +427,59 @@ metrics_kernel(int64_t T, const float* __restrict__ pred, const float* __restric
   }
 }
 
+// The same statistics over segments of the batch (validate(), train.py:137-291, and test.py's per-level report): one
+// CTA per segment s = endpoints seg_idx[seg_ptr[s] .. seg_ptr[s+1]), fp64 sums in a fixed order (thread-strided, then
+// the warp / block tree of metrics_kernel), so every launch gives the same bits.  The sums of squares are taken about
+// the segment's first label: the total sum of squares of a constant segment is then exactly 0 (r2 = NaN).
+//   out[s*9 + 0] mse  1 r2  2 correct  3 tp  4 fn  5 tn  6 fp  7 count  8 mape (torchmetrics MeanAbsolutePercentageError)
+constexpr int EVAL_THREADS = 256;
+__global__ void __launch_bounds__(EVAL_THREADS)
+eval_metrics_kernel(const int32_t* __restrict__ seg_ptr, const int32_t* __restrict__ seg_idx,
+                    const float* __restrict__ pred, const float* __restrict__ arrival, const float* __restrict__ required,
+                    const int64_t* __restrict__ label, float* __restrict__ out) {
+  constexpr int NV = 9;
+  __shared__ double part[EVAL_THREADS / 32][NV];
+  const int s0 = seg_ptr[blockIdx.x], s1 = seg_ptr[blockIdx.x + 1];
+  float* o = out + (int64_t)blockIdx.x * 9;
+  if (s1 <= s0) {                                          // empty segment (uniform across the CTA)
+    if (threadIdx.x < 9) o[threadIdx.x] = (threadIdx.x == 0 || threadIdx.x == 1 || threadIdx.x == 8) ? nanf("") : 0.f;
+    return;
+  }
+  const double y0 = arrival[seg_idx[s0]];
+  // sse, sum (y - y0), sum (y - y0)^2, sum ape, correct, tp, fn, tn, fp
+  double v[NV] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  for (int j = s0 + threadIdx.x; j < s1; j += EVAL_THREADS) {
+    const int i = seg_idx[j];
+    const float p = pred[i], yf = arrival[i];
+    const double y = yf, d = (double)p - y, c = y - y0;
+    v[0] += d * d; v[1] += c; v[2] += c * c;
+    v[3] += fabs(d) / (double)fmaxf(fabsf(yf), 1.17e-6f);
+    if (required && label) {
+      const bool crit = (required[i] - p) < 0.f, lab = label[i] != 0;
+      v[4] += (crit == lab) && (label[i] == 0 || label[i] == 1);
+      v[5] += crit && lab; v[6] += !crit && lab; v[7] += !crit && !lab; v[8] += crit && !lab;
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < NV; ++k) v[k] = warp_sum(v[k]);
+  if ((threadIdx.x & 31) == 0)
+#pragma unroll
+    for (int k = 0; k < NV; ++k) part[threadIdx.x >> 5][k] = v[k];
+  __syncthreads();
+  if (threadIdx.x < 32) {
+#pragma unroll
+    for (int k = 0; k < NV; ++k) v[k] = warp_sum(threadIdx.x < EVAL_THREADS / 32 ? part[threadIdx.x][k] : 0.0);
+    if (threadIdx.x == 0) {
+      const double n = (double)(s1 - s0), sst = v[2] - v[1] * v[1] / n;
+      o[0] = (float)(v[0] / n);
+      o[1] = (n >= 2.0 && sst > 0.0) ? (float)(1.0 - v[0] / sst) : nanf("");
+      o[2] = (float)v[4]; o[3] = (float)v[5]; o[4] = (float)v[6]; o[5] = (float)v[7]; o[6] = (float)v[8];
+      o[7] = (float)n;
+      o[8] = (float)(v[3] / n);
+    }
+  }
+}
+
 __global__ void adam_kernel(int64_t n, float* __restrict__ p, const float* __restrict__ g,
                             float* __restrict__ m, float* __restrict__ v, float lr, float b1, float b2,
                             float eps, float wd, float bc1, float bc2, float gscale) {
@@ -667,6 +720,16 @@ extern "C" int tm_step_metrics(int64_t T, const float* pred, const float* arriva
   TM_REQUIRE(T > 0, "tm_step_metrics: empty batch");
   metrics_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(T, pred, arrival, required, label, out8);
   return check_launch("step_metrics");
+}
+
+extern "C" int tm_eval_metrics(int32_t n_seg, const int32_t* seg_ptr, const int32_t* seg_idx, const float* pred,
+                               const float* arrival, const float* required, const int64_t* label, float* out,
+                               void* stream) {
+  if (n_seg <= 0) return 0;
+  TM_REQUIRE(seg_ptr && seg_idx && pred && arrival && out, "tm_eval_metrics: seg_ptr, seg_idx, pred, arrival, out required");
+  eval_metrics_kernel<<<(unsigned)n_seg, EVAL_THREADS, 0, (cudaStream_t)stream>>>(seg_ptr, seg_idx, pred, arrival,
+                                                                                 required, label, out);
+  return check_launch("eval_metrics");
 }
 
 extern "C" int tm_adam_step(int64_t n, float* p, const float* g, float* m, float* v, float lr,

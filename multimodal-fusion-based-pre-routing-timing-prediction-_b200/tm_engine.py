@@ -99,7 +99,12 @@ class DesignBatch:
         self.pin_off_h = None                      # first pin of every design in the joined netlist (concat)
         self.design_losses = None                  # (K,) device tensor, rewritten by every step / replay (K > 1)
         self.input_grads = None                    # {"cell_feat", "net_feat", "image"}: DesignStep.run(input_grads=True)
+        # per-endpoint required time (float32) and critical label (int64, 0 = non-critical), both (T,) on the device:
+        # when set, DesignStep.evaluate counts judge_critical's confusion matrix (train.py:391-395)
+        self.required = None
+        self.label = None
         self._fuse_table = None
+        self._segments = None
         # dynamic: the endpoint batch (endpoints / levels / labels / mask rows) is refreshed IN PLACE between steps, so
         # the step re-runs the on-device row selection every time (captured into its CUDA graph): one capture per
         # design serves every shuffled batch of the reference's DataLoader (train.py:470-486)
@@ -128,6 +133,7 @@ class DesignBatch:
         self.arrival_time[s:e].copy_(arrival_time, non_blocking=True)
         self.mask_rows_list[design].rows.copy_(rows, non_blocking=True)
         self._cone = None
+        self._segments = None
 
     def fuse_table(self):
         """int64 (K, 5) device table of every design's mask-row buffers {run_ptr, run_lo, run_hi, csc_ptr, csc_t}
@@ -141,6 +147,33 @@ class DesignBatch:
                 rows.append([t.data_ptr() for t in (run_ptr, run_lo, run_hi, csc_ptr, csc_t)])
             self._fuse_table = torch.tensor(rows, dtype=torch.int64).to(self.endpoints.device)
         return self._fuse_table
+
+    def eval_segments(self):
+        """(seg_ptr, seg_idx, L): the int32 device CSR of ``DesignStep.evaluate``'s metric rows (cached).  Row 0 is the
+        whole batch, rows 1..K the designs (``ep_off_h``), then K x L rows: design k's endpoints on endpoint level l at
+        row 1 + K + k * L + l, L = the largest endpoint level + 1.  Inside a row the endpoints keep the batch's order.
+        Built on the host from ``endpoint_level`` (one device-to-host read), so build it before a capture; a captured
+        evaluation keeps the levels it was built with."""
+        if self._segments is None:
+            lv = self.endpoint_level.detach().cpu().numpy()
+            if lv.size and (lv.min() < 0 or not np.all(lv == np.round(lv))):
+                raise ValueError("DesignBatch.eval_segments: endpoint levels must be non-negative integers")
+            lv = lv.astype(np.int64)
+            T, K = int(lv.size), self.K
+            L = int(lv.max()) + 1 if T else 1
+            sizes, idx = [T], [np.arange(T)]
+            for k in range(K):
+                s, e = int(self.ep_off_h[k]), int(self.ep_off_h[k + 1])
+                sizes.append(e - s)
+                idx.append(np.arange(s, e))
+            for k in range(K):
+                s, e = int(self.ep_off_h[k]), int(self.ep_off_h[k + 1])
+                sizes.extend(np.bincount(lv[s:e], minlength=L).tolist())
+                idx.append(s + np.argsort(lv[s:e], kind="stable"))
+            ptr = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int32)
+            dev = self.endpoints.device
+            self._segments = (torch.from_numpy(ptr).to(dev), torch.from_numpy(np.concatenate(idx).astype(np.int32)).to(dev), L)
+        return self._segments
 
     @staticmethod
     def concat(batches):
@@ -187,6 +220,10 @@ class DesignBatch:
                           mask_rows=[b.mask_rows for b in batches])
         out.pin_off_h = pin_off
         out.ep_off = torch.from_numpy(out.ep_off_h.astype(np.int32)).to(dev)
+        if all(b.required is not None for b in batches):
+            out.required = torch.cat([b.required for b in batches])
+        if all(b.label is not None for b in batches):
+            out.label = torch.cat([b.label for b in batches])
         return out
 
     @staticmethod
@@ -207,15 +244,35 @@ class DesignBatch:
         return DesignBatch.from_host(HostDesign(d, pin=False), device)
 
 
+class EvalMetrics:
+    """``DesignStep.evaluate``'s metrics: ONE (1 + K + K * L, 9) float32 tensor, columns ``tm_ops.EVAL_COLUMNS``
+    ([mse, r2, correct, tp, fn, tn, fp, count, mape]), and views into it.  Under CUDA-graph replay the tensor is
+    rewritten in place, and so are the views."""
+
+    def __init__(self, table, K, L):
+        self.table, self.K, self.L = table, K, L
+        self.batch = table[0]                                    # (9,) the whole batch
+        self.design = table[1:1 + K]                             # (K, 9) every design of a joined batch
+        self.level = table[1 + K:].view(K, L, table.shape[1])    # (K, L, 9) design k's endpoints on endpoint level l
+
+    def to_host(self):
+        """The same views over one device-to-host copy of the table."""
+        return EvalMetrics(self.table.cpu(), self.K, self.L)
+
+
 class PreparedDesign:
     VALUE_FIELDS = ("cell_feat", "net_feat", "image", "arrival_time")
 
-    def __init__(self, step, host, device, graph=None, pool=None, input_grads=False, param_grads=True):
+    def __init__(self, step, host, device, graph=None, pool=None, input_grads=False, param_grads=True, evaluate=False):
+        _check_evaluate_options(evaluate, input_grads, param_grads)
         self.batch = DesignBatch.from_host(host, device, graph=graph)
         self.static = {"cell_feat": self.batch.cell_feat, "net_feat": self.batch.net_feat,
                        "image": self.batch.image, "arrival_time": self.batch.arrival_time}
         torch.cuda.synchronize()
-        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads, param_grads=param_grads)
+        if evaluate:
+            self.replay = step.capture_evaluate(self.batch, pool=pool)
+        else:
+            self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads, param_grads=param_grads)
 
     def upload(self, host, stream=None):
         """Host -> device copy of the per-step values into the graph's static inputs."""
@@ -236,11 +293,15 @@ class PreparedDesign:
 class PreparedDesigns:
     """``DesignStep.prepare_many``: K resident designs, one captured step over all of them."""
 
-    def __init__(self, step, hosts, device, pool=None, input_grads=False, param_grads=True):
+    def __init__(self, step, hosts, device, pool=None, input_grads=False, param_grads=True, evaluate=False):
+        _check_evaluate_options(evaluate, input_grads, param_grads)
         self.parts = [DesignBatch.from_host(h, device) for h in hosts]
         self.batch = DesignBatch.concat(self.parts)
         torch.cuda.synchronize()
-        self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads, param_grads=param_grads)
+        if evaluate:
+            self.replay = step.capture_evaluate(self.batch, pool=pool)
+        else:
+            self.replay = step.capture(self.batch, pool=pool, input_grads=input_grads, param_grads=param_grads)
 
     def upload(self, hosts, stream=None):
         """Host -> device copy of every design's per-step values into its slices of the graph's static inputs."""
@@ -261,6 +322,12 @@ class PreparedDesigns:
         if hosts is not None:
             self.upload(hosts)
         return self.replay()
+
+
+def _check_evaluate_options(evaluate, input_grads, param_grads):
+    if evaluate and (input_grads or not param_grads):
+        raise ValueError("DesignStep.prepare: evaluate=True is the forward alone; it takes neither input_grads nor "
+                         "param_grads=False")
 
 
 class DesignStep:
@@ -352,6 +419,45 @@ class DesignStep:
                                   [p.detach() for p in self.gnn_params], save=False)
         pred, _ = self._head_forward(H, b, fmap.reshape(-1))
         return pred.squeeze(-1)
+
+    def evaluate(self, b):
+        """One evaluation step (validate(), train.py:137-291; test.py:124-318): the forward half of ``run``, laid out as
+        ``run`` lays it out -- the netlist branch on the current stream with the per-level kernels, the image branch on
+        the image stream, the head after the join -- followed by ONE ``tm_eval_metrics`` launch.  Returns ``(pred (T,),
+        metrics)``; ``metrics`` is an ``EvalMetrics`` (``.batch``, ``.design``, ``.level``, ``.to_host()``) against the
+        batch's labels, with the confusion counts when ``b.required`` / ``b.label`` are set.  Predictions are the same
+        bits as ``run(b)``'s.  Nothing of the model is touched except what ``forward`` touches: U-Net batch norm in train
+        mode updates its running statistics (the reference validates in train mode under ``no_grad``).  No ``.grad``, no
+        parameter, no gradient bucket, no collective.  Joined batches give every design's and every level's row;
+        ``prune`` does not apply (the cone of all endpoints is nearly the whole netlist)."""
+        m = self.model
+        dev = b.image.device
+        main = torch.cuda.current_stream()
+        if getattr(b, "dynamic", False):
+            for r in b.mask_rows_list:
+                r.rebuild()
+        seg_ptr, seg_idx, L = b.eval_segments()
+        side = self.image_stream if (self.overlap and self.image_stream is not None) else main
+        side.wait_stream(main)
+        sched = b.graph.schedule()
+        gp = [p.detach() for p in self.gnn_params]
+        T = int(b.endpoints.numel())
+        X = torch.empty(T, D + D + m.global_dim, dtype=torch.float32, device=dev)
+        H, _ = tm_ops.gnn_forward(sched, b.cell_feat, b.net_feat, gp, save=False,
+                                  impl=16 if side is not main and os.environ.get("TM_GNN_IMPL") is None else None)
+        img_cap = int(os.environ.get("TM_IMAGE_SM_CAP", "0")) if side is not main else 0
+        with torch.cuda.stream(side):
+            old_cap = tm_lib.lib().tm_tc_set_grid_cap(img_cap)
+            fmap, _ = self._image_forward(b.image, need_bwd=False)
+            tm_lib.lib().tm_tc_set_grid_cap(old_cap)
+            self._check_feature_map(fmap, b)
+            hs = self._head_image_side(b, fmap.reshape(-1), X)
+        main.wait_stream(side)
+        pred = self._head_netlist_side(H, b, hs).squeeze(-1)
+        table = tm_ops.eval_metrics(pred, b.arrival_time, seg_ptr, seg_idx, b.required, b.label)
+        # a tensor-core barrier timeout leaves garbage: the whole batch's mse becomes NaN (tm_lib.check_err_flags)
+        call("tm_poison_on_error", table, tm_lib.err_flag(dev), stream())
+        return pred, EvalMetrics(table, b.K, L)
 
     # ---------------------------------------------------------------- full step
     def run(self, b, grad_scale=1.0, input_grads=False, pred_grad=None, param_grads=True):
@@ -500,11 +606,26 @@ class DesignStep:
         if not param_grads and not input_grads:
             raise ValueError("DesignStep.capture: param_grads=False computes input gradients only; pass input_grads=True")
         opts = dict(input_grads=input_grads, pred_grad=pred_grad, param_grads=param_grads)
+
+        def rebind():
+            grads = [(p, p.grad) for p in list(self.model.parameters()) + list(self.cnn.parameters())
+                     if p.grad is not None] if param_grads else []
+            igrads = b.input_grads if input_grads else None
+
+            def after_replay():
+                for p, gr in grads:                      # several captured steps may coexist: re-point .grad
+                    p.grad = gr
+                if igrads is not None:
+                    b.input_grads = igrads
+            return after_replay
+
+        def fn():
+            return self.run(b, **opts)
         if self.world <= 1 or not param_grads or os.environ.get("TM_DP_GRAPH", "1") != "0":
-            return self._capture_local(b, warmup, pool, opts)
+            return self._capture_local(fn, warmup, pool, rebind)
         world, self.world = self.world, 1                  # no collectives inside the captured region
         try:
-            replay_local = self._capture_local(b, warmup, pool, opts)
+            replay_local = self._capture_local(fn, warmup, pool, rebind)
         finally:
             self.world = world
         params = [p for p in list(self.model.parameters()) + list(self.cnn.parameters())]
@@ -517,49 +638,60 @@ class DesignStep:
         replay.graph = replay_local.graph
         return replay
 
-    def _capture_local(self, b, warmup=2, pool=None, opts=None):
-        opts = opts or {}
+    def capture_evaluate(self, b, warmup=2, pool=None):
+        """Capture ``evaluate(b)`` into one CUDA graph.  Returns ``replay() -> (pred, metrics)``: the same tensors on every
+        replay, rewritten in place; refresh the batch's values (features, image, labels) in place in between.  The
+        metric rows follow the endpoint levels the batch had when this was called (``DesignBatch.eval_segments``), so a
+        dynamic batch, whose endpoints change between replays, is refused.  ``pool``: as in ``capture``."""
+        if getattr(b, "dynamic", False):
+            raise ValueError("DesignStep.capture_evaluate: a dynamic batch changes its endpoints between replays; "
+                             "evaluate a fixed endpoint set")
+        b.eval_segments()                                  # host work: before the capture
+        return self._capture_local(lambda: self.evaluate(b), warmup, pool)
+
+    def _capture_local(self, fn, warmup=2, pool=None, rebind=None):
+        """Capture ``fn()`` (warmed up ``warmup`` times on a side stream) into one CUDA graph; returns ``replay()``, which
+        replays it and returns what ``fn`` returned at capture.  ``rebind``: called once after the capture, it returns a
+        function that runs after every replay (re-pointing state the capture left, such as ``.grad``)."""
         cur = torch.cuda.current_stream()
         s = torch.cuda.Stream(priority=int(os.environ.get("TM_MAIN_PRIORITY", "0")))   # (a higher priority for the netlist branch was measured: no effect)
         s.wait_stream(cur)
         with torch.cuda.stream(s):
             for _ in range(warmup):
-                self.run(b, **opts)
+                fn()
         cur.wait_stream(s)
         torch.cuda.synchronize()
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, pool=pool):
-            loss, pred = self.run(b, **opts)
+            out = fn()
         self._graphs.append(g)
-        grads = [(p, p.grad) for p in list(self.model.parameters()) + list(self.cnn.parameters())
-                 if p.grad is not None] if opts.get("param_grads", True) else []
-        igrads = b.input_grads if opts.get("input_grads") else None
+        after_replay = rebind() if rebind is not None else None
 
         def replay():
             g.replay()
-            for p, gr in grads:                      # several captured steps may coexist: re-point .grad
-                p.grad = gr
-            if igrads is not None:
-                b.input_grads = igrads
-            return loss, pred
+            if after_replay is not None:
+                after_replay()
+            return out
         replay.graph = g
         return replay
 
-    def prepare(self, host, device, graph=None, pool=None, input_grads=False, param_grads=True):
+    def prepare(self, host, device, graph=None, pool=None, input_grads=False, param_grads=True, evaluate=False):
         """A design made resident for repeated steps: uploads everything once, builds the structure
         that depends only on the netlist and the endpoint batch (level schedule, CSRs, mask runs / CSC)
         and captures the step as a CUDA graph.  Returns a ``PreparedDesign``; its ``step(host)``
         refreshes the per-step VALUES (features, image, labels) from pinned host memory and replays.
         The structure (edges, endpoints, masks) must be the one given here.  ``input_grads``: every replay also
-        rewrites ``batch.input_grads`` (see ``run``); ``param_grads=False``: a frozen step (see ``run``)."""
-        return PreparedDesign(self, host, device, graph, pool, input_grads, param_grads)
+        rewrites ``batch.input_grads`` (see ``run``); ``param_grads=False``: a frozen step (see ``run``).
+        ``evaluate=True``: the captured step is ``evaluate`` (``capture_evaluate``) and ``step(host)`` returns ``(pred,
+        metrics)``; it takes neither ``input_grads`` nor ``param_grads=False`` (ValueError)."""
+        return PreparedDesign(self, host, device, graph, pool, input_grads, param_grads, evaluate)
 
-    def prepare_many(self, hosts, device, pool=None, input_grads=False, param_grads=True):
+    def prepare_many(self, hosts, device, pool=None, input_grads=False, param_grads=True, evaluate=False):
         """K designs made resident for repeated steps over all of them (``DesignBatch.concat``), captured as ONE CUDA
         graph.  Returns a ``PreparedDesigns``; its ``step(hosts)`` refreshes the per-step VALUES of all K from pinned
-        host memory and replays.  The structures must be the ones given here.  ``input_grads``, ``param_grads``: as in
-        ``prepare``."""
-        return PreparedDesigns(self, hosts, device, pool, input_grads, param_grads)
+        host memory and replays.  The structures must be the ones given here.  ``input_grads``, ``param_grads``,
+        ``evaluate``: as in ``prepare``."""
+        return PreparedDesigns(self, hosts, device, pool, input_grads, param_grads, evaluate)
 
     @staticmethod
     def _assign(pairs):

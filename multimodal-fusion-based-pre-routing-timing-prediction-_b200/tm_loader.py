@@ -218,6 +218,29 @@ class LoadedDesign:
         run.batch = b
         return run
 
+    def eval_batch(self, paths=None):
+        """-> (``tm_engine.DesignBatch``, path ids in prediction order) for ``DesignStep.evaluate``: ``paths`` (default:
+        the design's paths without the oversampled critical duplicates -- for ``usage="test"`` the validation split), with
+        the endpoints' required times and critical labels when the design has them."""
+        ids = self.order_batch(list(dict.fromkeys(self.paths)) if paths is None else paths)
+        b = self.batch(ids)
+        ep = b.endpoints.long()
+        if self.required is not None:
+            b.required = self.required[ep].contiguous()
+        if self.label is not None:
+            b.label = self.label[ep].to(torch.int64).contiguous()
+        return b, ids
+
+    def prepare_evaluate(self, step, paths=None):
+        """One CUDA-graph capture of ``step.evaluate`` over a fixed set of paths (validate(), train.py:137-291, or one
+        test design, test.py:124-318): returns ``run() -> (pred, metrics)`` that replays it; ``run.batch`` is the batch
+        and ``run.paths`` the path ids in prediction order.  Refresh values in place (``run.batch.cell_feat`` ...,
+        ``arrival_time``) between replays if they change; the paths and their levels are fixed."""
+        b, ids = self.eval_batch(paths)
+        run = step.capture_evaluate(b)
+        run.batch, run.paths = b, ids
+        return run
+
     def loader(self, batch_size=1350, shuffle=True, generator=None):
         """Batches like ``DataLoader(PathDataset(paths), batch_size, shuffle=True, drop_last=len(paths) > batch_size)``
         (train.py:468-472; the reference decides ``drop_last`` on ``len(path2level)``)."""
@@ -248,6 +271,24 @@ def prepare_many(designs, step, batch_size=1350):
             b.set_endpoints(*d.batch_tensors(ids), design=k)
         return replay()
     run.batch = b
+    return run
+
+
+def prepare_evaluate_many(designs, step, paths=None):
+    """``LoadedDesign.prepare_evaluate`` for K designs in ONE CUDA graph (``tm_engine.DesignBatch.concat``): a whole test
+    set per replay.  ``paths``: None (every design's default) or one path-id list per design.  Returns ``run() -> (pred,
+    metrics)``; ``metrics.design[k]`` / ``metrics.level[k]`` are design k's rows, ``run.paths[k]`` its path ids in
+    prediction order (its predictions are ``pred[run.batch.ep_off_h[k]:run.batch.ep_off_h[k + 1]]``)."""
+    import tm_engine
+    designs = list(designs)
+    if paths is None:
+        paths = [None] * len(designs)
+    if len(paths) != len(designs):
+        raise ValueError(f"prepare_evaluate_many: {len(paths)} path lists for {len(designs)} designs")
+    parts = [d.eval_batch(p) for d, p in zip(designs, paths)]
+    b = tm_engine.DesignBatch.concat([x[0] for x in parts])
+    run = step.capture_evaluate(b)
+    run.batch, run.paths = b, [x[1] for x in parts]
     return run
 
 

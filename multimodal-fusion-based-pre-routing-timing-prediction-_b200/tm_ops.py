@@ -563,6 +563,25 @@ def step_metrics(pred, arrival, required=None, label=None):
     return out
 
 
+EVAL_COLUMNS = ("mse", "r2", "correct", "tp", "fn", "tn", "fp", "count", "mape")
+
+
+def eval_metrics(pred, arrival, seg_ptr, seg_idx, required=None, label=None):
+    """``step_metrics`` per segment, one launch: segment s is the endpoints ``seg_idx[seg_ptr[s]:seg_ptr[s + 1]]``
+    (int32 device tensors).  Returns the (n_seg, 9) float32 device tensor whose columns are ``EVAL_COLUMNS``: the eight
+    of ``step_metrics`` (the last one the segment's endpoint count) and the mean absolute percentage error."""
+    pred, arrival = _f32c(pred.detach().reshape(-1)), _f32c(arrival.detach().reshape(-1))
+    tm_lib.require_cuda(pred, "pred")
+    if seg_ptr.dtype != torch.int32 or seg_idx.dtype != torch.int32:
+        raise ValueError("eval_metrics: seg_ptr and seg_idx must be int32")
+    n_seg = int(seg_ptr.numel()) - 1
+    out = torch.empty(max(n_seg, 0), len(EVAL_COLUMNS), dtype=torch.float32, device=pred.device)
+    req = None if required is None else _f32c(required.detach().reshape(-1))
+    lab = None if label is None else label.detach().reshape(-1).to(torch.int64).contiguous()
+    call("tm_eval_metrics", n_seg, seg_ptr.contiguous(), seg_idx.contiguous(), pred, arrival, req, lab, out, stream())
+    return out
+
+
 # --------------------------------------------------------------------------------------------
 # mask fusion
 # --------------------------------------------------------------------------------------------
