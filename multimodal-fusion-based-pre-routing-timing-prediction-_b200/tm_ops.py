@@ -32,8 +32,6 @@ BIAS, RELU, MASK, ACCUM = 1, 2, 4, 8
 #   "bf16" tcgen05 with plain bf16 operands (rtol 2e-2 class);
 #   "fp32" the CUDA-core FFMA kernels (tm_gemm_nn / tm_gemm_tn).
 MATH = os.environ.get("TM_MATH", "tf32x3")
-GEN_HIDDEN = os.environ.get("TM_GEN_HIDDEN", "1") != "0"  # generate Linear(<=2, hid) hidden layers instead of storing them
-FUSED_SELF_MLP = os.environ.get("TM_FUSED_SELF_MLP", "1") != "0"   # tm_selfmlp.cu for the 2 -> 256 -> 128 net-pin MLP
 FUSE_RUNS = os.environ.get("TM_FUSE_RUNS", "1") != "0"    # run-length / prefix-table mask fusion forward
 TC_MIN_N = 4           # Linear(hid, 1) (the head's last layer): a 128 x 32 tensor-core tile would be 97 % padding
 TC_MIN_K = 16          # contractions shorter than this stay on the CUDA-core kernel (K = 1, 2: pure bandwidth)
@@ -164,92 +162,94 @@ def colsum(X, R, C, ld, out=None, accumulate=0):
 # --------------------------------------------------------------------------------------------
 # two-layer MLP (model.py:10-24 with sizes (in, hid, out)):  y = W2 relu(W1 x + b1) + b2
 # --------------------------------------------------------------------------------------------
-def _recurrence_math():
-    """Arithmetic of the hoisted self-term MLPs, whose output S seeds the 101-level recurrence.  Round 1 kept
-    24-bit products ("tc6", six bf16 MMAs) here; measured on B200 (``profiles/diag_gemm_modes.py``) the default
-    3xTF32 contraction has the same error on these shapes (max 3.0e-6 against 2.4e-6 of the row scale: the fp32
-    accumulation dominates both) and every parity test -- including the full-size config 2 / 3 gradient checks -- is
-    unchanged, while the step is 0.09 ms shorter.  ``TM_RECURRENCE_MATH=tc6`` restores the round-1 choice."""
-    forced = os.environ.get("TM_RECURRENCE_MATH")
-    if forced:
-        return None if forced == "default" else forced
-    return None
+def _rows_aligned(t, ld):
+    """Every row of ``t`` (row stride ``ld`` floats) starts on a 16-byte boundary: the fused kernels' vector loads."""
+    return ld % 4 == 0 and t.data_ptr() % 16 == 0
 
 
-def mlp2_forward(x, ldx, rows, n_rows, w1, b1, w2, b2, out, ldo, out_rows=None, math=None):
-    """x rows (optionally gathered by ``rows``) -> out rows (optionally scattered by ``out_rows``).
-    Returns the hidden activations (n_rows, hid) needed by ``mlp2_backward``."""
+def mlp2_route(n_rows, kin, hid, nout, math=None, x_aligned=True, out_aligned=True, g_aligned=True, dx_aligned=True):
+    """The kernel that serves each product of the MLP kin -> hid -> nout over ``n_rows`` rows in arithmetic ``math``
+    (default ``MATH``), given whether the rows of the input x, of the output, of the output's gradient g and of the
+    input's gradient dx are 16-byte aligned.  Host logic only: ``mlp2_forward`` and ``mlp2_backward`` launch what it names.
+
+    Returns a dict.  "hidden" is "generated" -- a Linear(<=2, hid) first layer costs 2 FMAs per hidden activation, so
+    the kernels recompute the activations in their operand loaders and never store them -- or "stored".  The products:
+    "lin1" / "lin2" the two forward layers (one kernel for both when the hidden layer is generated), "dw2" (dW2, db2),
+    "dh" the hidden layer's gradient, "dw1" (dW1, db1), "dx" the data gradient next to the parameter gradients and
+    "dx_only" the data gradient alone.  "gemm" is ``gemm_nn`` / ``gemm_tn``; a ``tm_*`` name is that kernel, where
+    ``tm_selfmlp_gen_bwd1_dx`` is ``tm_selfmlp_gen_bwd1`` with dX in its epilogue.  The ``tm_selfmlp_*`` kernels
+    (tm_selfmlp.cu) serve the reference's sizes at tf32x3 on the fp16 two-term split: 256 hidden units, 128 outputs for
+    the second layer and its gradients, at most 48 inputs (a multiple of 4) for a stored first layer."""
+    prec = _precision(math)
+    split = prec == 3 and hid == 256
+    split_out = split and nout == 128
+    split_in = split and kin % 4 == 0 and kin <= 48
+    if kin <= 2 and prec is not None and n_rows > 0 and hid >= TC_MIN_K:
+        fwd = "tm_selfmlp_gen_forward" if split_out and out_aligned else "tm_tc_mlp2_smallk_forward"
+        if split_out and g_aligned:
+            return dict(hidden="generated", lin1=fwd, lin2=fwd, dw2="tm_selfmlp_gen_wgrad2", dh="tm_selfmlp_gen_bwd1",
+                        dw1="tm_selfmlp_gen_bwd1", dx="tm_selfmlp_gen_bwd1_dx", dx_only="tm_selfmlp_gen_bwd1_dx")
+        return dict(hidden="generated", lin1=fwd, lin2=fwd, dw2="tm_tc_mlp2_smallk_wgrad2", dh="gemm",
+                    dw1="tm_tc_mlp1_bwd_fused", dx="gemm", dx_only="gemm")
+    lin1 = "tm_selfmlp_lin1_relu" if split_in and n_rows > 0 and x_aligned else "gemm"
+    # the fused second layer scales each row by the row maximum tm_selfmlp_lin1_relu writes
+    lin2 = "tm_selfmlp_rows_forward" if lin1 != "gemm" and split_out and out_aligned else "gemm"
+    dh = "tm_selfmlp_rows_dh" if split_out and g_aligned else "gemm"
+    dx_only = "tm_selfmlp_rows_dx" if dh != "gemm" and split_in and dx_aligned else "gemm"
+    return dict(hidden="stored", lin1=lin1, lin2=lin2, dw2="gemm", dh=dh, dw1="gemm", dx="gemm", dx_only=dx_only)
+
+
+def mlp2_forward(x, ldx, rows, n_rows, w1, b1, w2, b2, out, ldo, out_rows=None):
+    """x rows (optionally gathered by ``rows``) -> out rows (optionally scattered by ``out_rows``), on the kernels
+    ``mlp2_route`` names.  Returns the hidden activations (n_rows, hid) needed by ``mlp2_backward``, or None when the
+    route generates them."""
     hid, kin = w1.shape
     nout = w2.shape[0]
-    prec = _precision(math)
-    if GEN_HIDDEN and kin <= 2 and prec is not None and n_rows > 0 and hid >= TC_MIN_K:
-        # Linear(<=2, hid) first layer: the hidden activations cost 2 FMAs each to recompute, so they are
-        # generated inside the GEMM's operand loader and never stored (returns None; mlp2_backward
-        # regenerates them the same way)
-        if FUSED_SELF_MLP and hid == 256 and nout == 128 and prec == 3 and ldo % 4 == 0 and out.data_ptr() % 16 == 0:
-            # the reference's sizes: fused kernel, fp16 two-term split operands generated in place (tm_selfmlp.cu)
-            nb = tm_lib.ws_bytes("tm_selfmlp_ws_bytes")
-            call("tm_selfmlp_gen_forward", n_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2), _f32c(b2), out, ldo,
-                 out_rows, tm_lib.workspace(nb, out.device), nb, stream())
-            return None
-        call("tm_tc_mlp2_smallk_forward", n_rows, hid, nout, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2), _f32c(b2),
-             out, ldo, out_rows, prec, tm_lib.err_flag(out.device), stream())
+    dev = out.device
+    r = mlp2_route(n_rows, kin, hid, nout, x_aligned=_rows_aligned(x, ldx), out_aligned=_rows_aligned(out, ldo))
+    if r["lin1"] == "tm_selfmlp_gen_forward":
+        nb = tm_lib.ws_bytes("tm_selfmlp_ws_bytes")
+        call("tm_selfmlp_gen_forward", n_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2), _f32c(b2), out, ldo,
+             out_rows, tm_lib.workspace(nb, dev), nb, stream())
         return None
-    h = torch.empty(n_rows, hid, dtype=torch.float32, device=out.device)
-    if (FUSED_SELF_MLP and hid == 256 and prec == 3 and kin % 4 == 0 and kin <= 48 and ldx % 4 == 0 and x.data_ptr() % 16 == 0
-            and n_rows > 0):
-        # fc_cell_self's first layer (36 inputs): output-bound, fp16 two-term split on tcgen05 (tm_selfmlp.cu)
+    if r["lin1"] == "tm_tc_mlp2_smallk_forward":
+        call("tm_tc_mlp2_smallk_forward", n_rows, hid, nout, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2), _f32c(b2),
+             out, ldo, out_rows, _precision(), tm_lib.err_flag(dev), stream())
+        return None
+    h = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
+    rowmax = None
+    if r["lin1"] == "tm_selfmlp_lin1_relu":
         nb = tm_lib.ws_bytes("tm_selfmlp_lin1_ws_bytes")
-        fuse2 = nout == 128 and ldo % 4 == 0 and out.data_ptr() % 16 == 0
-        rowmax = torch.empty(n_rows, dtype=torch.float32, device=out.device) if fuse2 else None
+        if r["lin2"] == "tm_selfmlp_rows_forward":
+            rowmax = torch.empty(n_rows, dtype=torch.float32, device=dev)
         call("tm_selfmlp_lin1_relu", n_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), h, hid, rowmax,
-             tm_lib.workspace(nb, out.device), nb, stream())
-        if fuse2:                                   # second layer on the same machinery, per-row scale from rowmax
-            nb = tm_lib.ws_bytes("tm_selfmlp_ws_bytes")
-            call("tm_selfmlp_rows_forward", n_rows, h, hid, None, rowmax, _f32c(w2), _f32c(b2), out, ldo, out_rows,
-                 tm_lib.workspace(nb, out.device), nb, stream())
-            return h
+             tm_lib.workspace(nb, dev), nb, stream())
     else:
-        gemm_nn(n_rows, hid, kin, x, ldx, _f32c(w1), kin, h, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True, math=math)
-    gemm_nn(n_rows, nout, hid, h, hid, _f32c(w2), hid, out, ldo, c_rows=out_rows, bias=b2, b_is_nk=True, math=math)
+        gemm_nn(n_rows, hid, kin, x, ldx, _f32c(w1), kin, h, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True)
+    if r["lin2"] == "tm_selfmlp_rows_forward":
+        nb = tm_lib.ws_bytes("tm_selfmlp_ws_bytes")
+        call("tm_selfmlp_rows_forward", n_rows, h, hid, None, rowmax, _f32c(w2), _f32c(b2), out, ldo, out_rows,
+             tm_lib.workspace(nb, dev), nb, stream())
+    else:
+        gemm_nn(n_rows, nout, hid, h, hid, _f32c(w2), hid, out, ldo, c_rows=out_rows, bias=b2, b_is_nk=True)
     return h
 
 
-def _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, h_rows, dh):
+def _hidden_grad(r, n_rows, g, ldg, g_rows, w2, h, h_rows, dh):
     """dh[r] = (g[g_rows] @ w2) * (h[r] > 0), r = h_rows or the row itself."""
-    if (FUSED_SELF_MLP and hid == 256 and nout == 128 and _precision() == 3 and ldg % 4 == 0 and g.data_ptr() % 16 == 0
-            and h.stride(0) % 4 == 0 and h.data_ptr() % 16 == 0 and dh.data_ptr() % 16 == 0):
-        # the reference's sizes: fp16 two-term split operands, W2 resident, tcgen05 (tm_selfmlp.cu)
+    nout, hid = w2.shape
+    if r["dh"] == "tm_selfmlp_rows_dh":
         nb = tm_lib.ws_bytes("tm_selfmlp_rows_dh_ws_bytes")
-        call("tm_selfmlp_rows_dh", n_rows, g, ldg, g_rows, _f32c(w2), h, h.stride(0), h_rows, dh, dh.stride(0),
+        call("tm_selfmlp_rows_dh", n_rows, g, ldg, g_rows, w2, h, h.stride(0), h_rows, dh, dh.stride(0),
              tm_lib.workspace(nb, dh.device), nb, stream())
-        return
-    gemm_nn(n_rows, hid, nout, g, ldg, _f32c(w2), hid, dh, hid, a_rows=g_rows, c_rows=h_rows, mask=h, ldmask=hid)
-
-
-def _rows_dx(n_rows, g, ldg, g_rows, w1, w2, h, dx_out, rows):
-    """Data gradient alone of an MLP whose hidden activations were stored: dx_out[rows[m]] = ((g[g_rows[m]] @ w2) *
-    (h[m] > 0)) @ w1.  The reference's sizes (256 hidden, 128 outputs, <= 48 inputs) run as one fused kernel
-    (``tm_selfmlp_rows_dx``: the hidden gradient never leaves the SM); others take the two GEMMs."""
-    hid, kin = w1.shape
-    nout = w2.shape[0]
-    w1c = _f32c(w1)
-    if (FUSED_SELF_MLP and hid == 256 and nout == 128 and _precision() == 3 and kin % 4 == 0 and kin <= 48
-            and ldg % 4 == 0 and g.data_ptr() % 16 == 0 and h.stride(0) % 4 == 0 and h.data_ptr() % 16 == 0
-            and dx_out.stride(0) % 4 == 0 and dx_out.data_ptr() % 16 == 0):
-        nb = tm_lib.ws_bytes("tm_selfmlp_rows_dh_ws_bytes")
-        call("tm_selfmlp_rows_dx", n_rows, g, ldg, g_rows, _f32c(w2), h, h.stride(0), None, w1c, kin, dx_out,
-             dx_out.stride(0), rows, tm_lib.workspace(nb, dx_out.device), nb, stream())
-        return
-    dh = torch.empty(n_rows, hid, dtype=torch.float32, device=g.device)
-    _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, None, dh)
-    gemm_nn(n_rows, kin, hid, dh, hid, w1c, kin, dx_out, dx_out.stride(0), c_rows=rows)
+    else:
+        gemm_nn(n_rows, hid, nout, g, ldg, w2, hid, dh, hid, a_rows=g_rows, c_rows=h_rows, mask=h, ldmask=hid)
 
 
 def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=False, b1=None, wgrad_stream=None,
                   h_rows=None, dx_out=None, need_wgrad=True):
-    """Gradients of a two-layer MLP.  ``g``: dLoss/d(out) rows (optionally gathered by ``g_rows``).
-    ``h``: the hidden activations mlp2_forward returned, or None when they were generated on the fly
+    """Gradients of a two-layer MLP, on the kernels ``mlp2_route`` names.  ``g``: dLoss/d(out) rows (optionally gathered
+    by ``g_rows``).  ``h``: the hidden activations mlp2_forward returned, or None when they were generated on the fly
     (then ``b1`` is required).  Returns (dw1, db1, dw2, db2, dx or None).
     ``wgrad_stream`` (with ``need_dx``): the data gradient is computed first on the current stream and the four
     parameter gradients on ``wgrad_stream`` (which waits for it); the caller joins that stream before reading them.
@@ -258,139 +258,103 @@ def mlp2_backward(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows=None, need_dx=
     ``dx_out`` (with ``need_dx``; required when ``rows`` gathers): the data gradient of MLP row i is written to row
     ``rows[i]`` of ``dx_out`` -- the row of ``x`` it read, so ``rows`` must be distinct -- and ``dx_out`` is returned as dx;
     its other rows are left as they are.  The parameter gradients are the same bits as without ``need_dx``.
-    ``need_wgrad=False`` (with ``need_dx``): the data gradient alone, no parameter-gradient work; returns
-    (None, None, None, None, dx).  dx is the same bits as with the parameter gradients, except for a stored hidden layer
-    of the reference's sizes (``fc_cell_self``), whose fused kernel sums the second product in another order."""
+    ``need_wgrad=False`` (with ``need_dx``): the data gradient alone, the same launches without the parameter-gradient
+    ones; returns (None, None, None, None, dx).  dx is the same bits as with the parameter gradients, except where the
+    route has a kernel for the data gradient alone (a stored hidden layer of the reference's sizes, ``fc_cell_self``:
+    ``tm_selfmlp_rows_dx`` sums the second product in another order)."""
     hid, kin = w1.shape
     nout = w2.shape[0]
     dev = g.device
-    if not need_wgrad:
-        if not need_dx or h_rows is not None:
-            raise RuntimeError("mlp2_backward: need_wgrad=False needs need_dx and no h_rows")
-        if dx_out is None:
-            if rows is not None:
-                raise RuntimeError("mlp2_backward: a data gradient of gathered rows needs dx_out")
-            dx_out = torch.empty(n_rows, kin, dtype=torch.float32, device=dev)
-        if n_rows > 0:
-            _mlp2_dx(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows, b1, dx_out, wgrad_stream is not None)
-        return None, None, None, None, dx_out
-    dw2 = torch.empty(nout, hid, dtype=torch.float32, device=dev)
-    db2 = torch.empty(nout, dtype=torch.float32, device=dev)
-    dw1 = torch.empty(hid, kin, dtype=torch.float32, device=dev)
-    db1 = torch.empty(hid, dtype=torch.float32, device=dev)
-    if need_dx and dx_out is None and rows is not None:
-        raise RuntimeError("mlp2_backward: a data gradient of gathered rows needs dx_out")
-    if n_rows == 0:
-        for t in (dw1, db1, dw2, db2):
-            t.zero_()
-        return dw1, db1, dw2, db2, dx_out if need_dx else None
+    if not need_wgrad and not need_dx:
+        raise RuntimeError("mlp2_backward: need_wgrad=False needs need_dx")
+    if need_dx and h_rows is not None:
+        raise RuntimeError("mlp2_backward: h_rows has no dx path")
     if need_dx and dx_out is None:
+        if rows is not None:
+            raise RuntimeError("mlp2_backward: a data gradient of gathered rows needs dx_out")
         dx_out = torch.empty(n_rows, kin, dtype=torch.float32, device=dev)
-    if h is None:                                            # generated hidden layer (kin <= 2)
+    dw1 = db1 = dw2 = db2 = None
+    if need_wgrad:
+        dw2 = torch.empty(nout, hid, dtype=torch.float32, device=dev)
+        db2 = torch.empty(nout, dtype=torch.float32, device=dev)
+        dw1 = torch.empty(hid, kin, dtype=torch.float32, device=dev)
+        db1 = torch.empty(hid, dtype=torch.float32, device=dev)
+    if n_rows == 0:
+        if need_wgrad:
+            for t in (dw1, db1, dw2, db2):
+                t.zero_()
+        return dw1, db1, dw2, db2, dx_out
+    r = mlp2_route(n_rows, kin, hid, nout, g_aligned=_rows_aligned(g, ldg),
+                   dx_aligned=need_dx and _rows_aligned(dx_out, dx_out.stride(0)))
+    if (h is None) != (r["hidden"] == "generated"):
+        raise RuntimeError(f"mlp2_backward: h is not what mlp2_forward returns for this MLP in {MATH} "
+                           f"(hidden layer {r['hidden']})")
+    w1, w2 = _f32c(w1), _f32c(w2)
+    if h is None:
         if b1 is None:
             raise RuntimeError("mlp2_backward: generated hidden activations need b1")
-        prec = _precision()
-        prec = 3 if prec is None else prec
-        fused = FUSED_SELF_MLP and hid == 256 and nout == 128 and prec == 3 and ldg % 4 == 0 and g.data_ptr() % 16 == 0
-        if fused:
-            # the reference's sizes: bias gradient and max |g| in one pass, then the fused weight-gradient kernel
-            # (hidden layer generated as a tcgen05 operand, accumulators resident in TMEM: tm_selfmlp.cu)
+        b1 = _f32c(b1)
+        if need_wgrad and r["dw2"] == "tm_selfmlp_gen_wgrad2":
+            # bias gradient and max |g| in one pass, then the fused weight-gradient kernel (hidden layer generated as
+            # a tcgen05 operand, accumulators resident in TMEM)
             gmax = torch.empty(1, dtype=torch.float32, device=dev)
             nbc = tm_lib.ws_bytes("tm_colsum_ws", n_rows, nout)
             call("tm_colsum_absmax", n_rows, nout, g, ldg, g_rows, db2, gmax, tm_lib.workspace(nbc, dev), nbc, stream())
             nb = tm_lib.ws_bytes("tm_selfmlp_wgrad2_ws_bytes")
-            call("tm_selfmlp_gen_wgrad2", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), gmax, dw2,
+            call("tm_selfmlp_gen_wgrad2", n_rows, g, ldg, g_rows, x, ldx, rows, kin, w1, b1, gmax, dw2,
                  tm_lib.workspace(nb, dev), nb, stream())
-        else:
+        elif need_wgrad:
             _Aux.run(lambda: _colsum(n_rows, nout, g, ldg, g_rows, db2, 0), g, db2, g_rows)
             nb = tm_lib.ws_bytes("tm_tc_gemm_tn_ws", nout, hid, n_rows)
-            call("tm_tc_mlp2_smallk_wgrad2", nout, hid, n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), dw2,
-                 prec, tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
-        if fused:
+            call("tm_tc_mlp2_smallk_wgrad2", nout, hid, n_rows, g, ldg, g_rows, x, ldx, rows, kin, w1, b1, dw2,
+                 _precision(), tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
+        if r["dw1"] == "tm_selfmlp_gen_bwd1":
             nb = tm_lib.ws_bytes("tm_selfmlp_bwd1_ws_bytes")
-            if need_dx:                                      # the same kernel with dX = dh W1 in its epilogue
-                call("tm_selfmlp_gen_bwd1_dx", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2),
+            if need_dx:                                      # dW1 / db1 NULL: the data gradient alone
+                call("tm_selfmlp_gen_bwd1_dx", n_rows, g, ldg, g_rows, x, ldx, rows, kin, w1, b1, w2,
                      dw1, db1, dx_out, dx_out.stride(0), tm_lib.workspace(nb, dev), nb, stream())
             else:
-                call("tm_selfmlp_gen_bwd1", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2),
+                call("tm_selfmlp_gen_bwd1", n_rows, g, ldg, g_rows, x, ldx, rows, kin, w1, b1, w2,
                      dw1, db1, tm_lib.workspace(nb, dev), nb, stream())
         else:
-            nb = tm_lib.ws_bytes("tm_tc_mlp1_bwd_ws", hid)
-            call("tm_tc_mlp1_bwd_fused", n_rows, hid, nout, g, ldg, g_rows, transpose(_f32c(w2)), None, 0, x, ldx, rows, kin,
-                 _f32c(w1), _f32c(b1), dw1, db1, tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
+            if need_wgrad:
+                nb = tm_lib.ws_bytes("tm_tc_mlp1_bwd_ws", hid)
+                call("tm_tc_mlp1_bwd_fused", n_rows, hid, nout, g, ldg, g_rows, transpose(w2), None, 0, x, ldx, rows, kin,
+                     w1, b1, dw1, db1, tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
             if need_dx:
-                # no fused data-gradient kernel in this precision: the hidden layer is materialised for the data
+                # no fused data-gradient kernel on this route: the hidden layer is materialised for the data
                 # gradient alone (the parameter gradients above are untouched)
                 hm = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
-                gemm_nn(n_rows, hid, kin, x, ldx, _f32c(w1), kin, hm, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True)
+                gemm_nn(n_rows, hid, kin, x, ldx, w1, kin, hm, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True)
                 dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
-                _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, hm, None, dh)
-                gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx_out, dx_out.stride(0), c_rows=rows)
+                _hidden_grad(r, n_rows, g, ldg, g_rows, w2, hm, None, dh)
+                gemm_nn(n_rows, kin, hid, dh, hid, w1, kin, dx_out, dx_out.stride(0), c_rows=rows)
         aux_join()
-        return dw1, db1, dw2, db2, dx_out if need_dx else None
-    if need_dx and wgrad_stream is not None:
-        dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
-        gemm_nn(n_rows, hid, nout, g, ldg, _f32c(w2), hid, dh, hid, a_rows=g_rows, mask=h, ldmask=hid)
-        dx = dx_out
-        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx, dx.stride(0), c_rows=rows)
+        return dw1, db1, dw2, db2, dx_out
+    if not need_wgrad and r["dx_only"] == "tm_selfmlp_rows_dx":
+        # one pass: the hidden layer's gradient never leaves the SM
+        nb = tm_lib.ws_bytes("tm_selfmlp_rows_dh_ws_bytes")
+        call("tm_selfmlp_rows_dx", n_rows, g, ldg, g_rows, w2, h, h.stride(0), None, w1, kin, dx_out,
+             dx_out.stride(0), rows, tm_lib.workspace(nb, dev), nb, stream())
+        return None, None, None, None, dx_out
+    on_side = need_dx and wgrad_stream is not None
+    if need_wgrad and not on_side:
+        gemm_tn(nout, hid, n_rows, g, ldg, h, hid, dw2, hid, a_rows=g_rows, b_rows=h_rows, colsum_a=db2)
+    # with h_rows, dh lives in the rows of h it belongs to, so the ReLU mask of the epilogue reads the matching row
+    dh = torch.empty(n_rows if h_rows is None else h.shape[0], hid, dtype=torch.float32, device=dev)
+    _hidden_grad(r, n_rows, g, ldg, g_rows, w2, h, h_rows, dh)
+    if need_wgrad and not on_side:
+        gemm_tn(hid, kin, n_rows, dh, hid, x, ldx, dw1, kin, a_rows=h_rows, b_rows=rows, colsum_a=db1)
+    if need_dx:
+        gemm_nn(n_rows, kin, hid, dh, hid, w1, kin, dx_out, dx_out.stride(0), c_rows=rows)
+    if need_wgrad and on_side:
         wgrad_stream.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(wgrad_stream):
             gemm_tn(nout, hid, n_rows, g, ldg, h, hid, dw2, hid, a_rows=g_rows, colsum_a=db2)
             gemm_tn(hid, kin, n_rows, dh, hid, x, ldx, dw1, kin, b_rows=rows, colsum_a=db1)
             aux_join()
-        return dw1, db1, dw2, db2, dx
-    gemm_tn(nout, hid, n_rows, g, ldg, h, hid, dw2, hid, a_rows=g_rows, b_rows=h_rows, colsum_a=db2)
-    if h_rows is not None:
-        if need_dx:
-            raise RuntimeError("mlp2_backward: h_rows has no dx path")
-        # dh lives in the rows of h it belongs to, so the ReLU mask of the epilogue reads the matching row
-        dh = torch.empty(h.shape[0], hid, dtype=torch.float32, device=dev)
-        _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, h_rows, dh)
-        gemm_tn(hid, kin, n_rows, dh, hid, x, ldx, dw1, kin, a_rows=h_rows, b_rows=rows, colsum_a=db1)
-        aux_join()
-        return dw1, db1, dw2, db2, None
-    if kin <= 2 and hid <= 256 and hid % 4 == 0 and not need_dx and _precision() == 3:
-        # Linear(<=2, hid) first layer: its whole backward (dW1, db1) is a reduction of the hidden
-        # gradient, fused into the data-gradient GEMM's epilogue -- dh is never written or re-read
-        nb = tm_lib.ws_bytes("tm_tc_mlp1_bwd_ws", hid)
-        call("tm_tc_mlp1_bwd_fused", n_rows, hid, nout, g, ldg, g_rows, transpose(_f32c(w2)), h, hid, x, ldx, rows, kin,
-             None, None, dw1, db1, tm_lib.workspace(nb, dev), nb, tm_lib.err_flag(dev), stream())
-        aux_join()
-        return dw1, db1, dw2, db2, None
-    dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
-    _hidden_grad(n_rows, hid, nout, g, ldg, g_rows, w2, h, None, dh)
-    gemm_tn(hid, kin, n_rows, dh, hid, x, ldx, dw1, kin, b_rows=rows, colsum_a=db1)
-    if need_dx:
-        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx_out, dx_out.stride(0), c_rows=rows)
     aux_join()
-    return dw1, db1, dw2, db2, dx_out if need_dx else None
-
-
-def _mlp2_dx(x, ldx, rows, n_rows, w1, w2, h, g, ldg, g_rows, b1, dx_out, head):
-    """``mlp2_backward(need_wgrad=False)``: the data-gradient launches of each route, without the weight-gradient ones."""
-    hid, kin = w1.shape
-    nout = w2.shape[0]
-    dev = g.device
-    if h is None:                                            # generated hidden layer (kin <= 2)
-        if b1 is None:
-            raise RuntimeError("mlp2_backward: generated hidden activations need b1")
-        prec = _precision()
-        prec = 3 if prec is None else prec
-        if FUSED_SELF_MLP and hid == 256 and nout == 128 and prec == 3 and ldg % 4 == 0 and g.data_ptr() % 16 == 0:
-            nb = tm_lib.ws_bytes("tm_selfmlp_bwd1_ws_bytes")
-            call("tm_selfmlp_gen_bwd1_dx", n_rows, g, ldg, g_rows, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2),
-                 None, None, dx_out, dx_out.stride(0), tm_lib.workspace(nb, dev), nb, stream())
-            return
-        hm = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
-        gemm_nn(n_rows, hid, kin, x, ldx, _f32c(w1), kin, hm, hid, a_rows=rows, bias=b1, flags=RELU, b_is_nk=True)
-        _rows_dx(n_rows, g, ldg, g_rows, w1, w2, hm, dx_out, rows)       # (kin <= 2: the two GEMMs)
-        return
-    if head:                                                 # the head's route (mlp2_backward with wgrad_stream)
-        dh = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
-        gemm_nn(n_rows, hid, nout, g, ldg, _f32c(w2), hid, dh, hid, a_rows=g_rows, mask=h, ldmask=hid)
-        gemm_nn(n_rows, kin, hid, dh, hid, _f32c(w1), kin, dx_out, dx_out.stride(0), c_rows=rows)
-        return
-    _rows_dx(n_rows, g, ldg, g_rows, w1, w2, h, dx_out, rows)
+    return dw1, db1, dw2, db2, dx_out
 
 
 # --------------------------------------------------------------------------------------------
@@ -424,10 +388,8 @@ def gnn_forward(sched, cell_feat, net_feat, params, save=True, impl=None, x_rows
     S = torch.empty(n, D, dtype=torch.float32, device=dev)
     nc, nn_ = int(sched.cell_class.numel()), int(sched.net_class.numel())
     xc, xn = x_rows if x_rows is not None else (sched.cell_class, sched.net_class)
-    hc = mlp2_forward(cell_feat, cell_feat.stride(0), xc, nc, cs1w, cs1b, cs2w, cs2b, S, D,
-                      out_rows=sched.cell_class, math=_recurrence_math())
-    hn = mlp2_forward(net_feat, net_feat.stride(0), xn, nn_, ns1w, ns1b, ns2w, ns2b, S, D,
-                      out_rows=sched.net_class, math=_recurrence_math())
+    hc = mlp2_forward(cell_feat, cell_feat.stride(0), xc, nc, cs1w, cs1b, cs2w, cs2b, S, D, out_rows=sched.cell_class)
+    hn = mlp2_forward(net_feat, net_feat.stride(0), xn, nn_, ns1w, ns1b, ns2w, ns2b, S, D, out_rows=sched.net_class)
     # every scheduled pin's row is written by its level's kernel: only pins outside the schedule need the zero fill
     # (170 MB = 42 us of the config-2 step when every pin is scheduled, as in the reference's designs)
     if sched.n_sched == n and os.environ.get("TM_H_FILL") != "1":
@@ -474,41 +436,30 @@ def gnn_backward(sched, saved, params, G, cone=None, need_dx=False, need_wgrad=T
     dev = G.device
     ncr = sched.n_cell_rows
     GA = torch.empty(max(ncr, 1), D, dtype=torch.float32, device=dev)
-    if not need_wgrad:
-        nb = tm_lib.ws_bytes("tm_gnn_ws_bytes")
-        call("tm_gnn_backward", sched.struct, saved["H"], G, cn1w, cn2w, saved["A"], saved["LSE"], saved["HID"],
-             GA, None, None, tm_lib.workspace(nb, dev), nb, stream())
-        cf, nf = saved["cell_feat"], saved["net_feat"]
-        cpins, npins = sched.cell_class, sched.net_class
-        xc, xn = saved.get("x_rows") or (cpins, npins)
-        dcf = torch.zeros(cf.shape, dtype=torch.float32, device=dev)
-        dnf = torch.zeros(nf.shape, dtype=torch.float32, device=dev)
-        mlp2_backward(cf, cf.stride(0), xc, int(cpins.numel()), cs1w, cs2w, saved["hc"], G, D, g_rows=cpins, b1=cs1b,
-                      need_dx=True, dx_out=dcf, need_wgrad=False)
-        mlp2_backward(nf, nf.stride(0), xn, int(npins.numel()), ns1w, ns2w, saved["hn"], G, D, g_rows=npins, b1=ns1b,
-                      need_dx=True, dx_out=dnf, need_wgrad=False)
-        return None, dcf, dnf
-    GHID = torch.empty(max(ncr, 1), 256, dtype=torch.float32, device=dev)
-    GZC = torch.empty(max(ncr, 1), D, dtype=torch.float32, device=dev)
+    GHID = GZC = None                                           # the fc_cell_neigh weight-gradient operands
+    if need_wgrad:
+        GHID = torch.empty(max(ncr, 1), 256, dtype=torch.float32, device=dev)
+        GZC = torch.empty(max(ncr, 1), D, dtype=torch.float32, device=dev)
     nb = tm_lib.ws_bytes("tm_gnn_ws_bytes")
     call("tm_gnn_backward", sched.struct, saved["H"], G, cn1w, cn2w, saved["A"], saved["LSE"], saved["HID"],
          GA, GHID, GZC, tm_lib.workspace(nb, dev), nb, stream())
-    dcn2w = torch.empty(D, 256, dtype=torch.float32, device=dev)
-    dcn2b = torch.empty(D, dtype=torch.float32, device=dev)
-    dcn1w = torch.empty(256, D, dtype=torch.float32, device=dev)
-    dcn1b = torch.empty(256, dtype=torch.float32, device=dev)
-    cr = cone.crows if cone is not None else None
-    if cr is not None:
-        ncr = int(cr.numel())
-    if ncr > 0:
-        gemm_tn(D, 256, ncr, GZC, D, saved["HID"], 256, dcn2w, 256, a_rows=cr, b_rows=cr, colsum_a=dcn2b)
-        gemm_tn(256, D, ncr, GHID, 256, saved["A"], D, dcn1w, D, a_rows=cr, b_rows=cr, colsum_a=dcn1b)
-        aux_join()
-    else:
-        for t in (dcn2w, dcn2b, dcn1w, dcn1b):
-            t.zero_()
+    if need_wgrad:
+        dcn2w = torch.empty(D, 256, dtype=torch.float32, device=dev)
+        dcn2b = torch.empty(D, dtype=torch.float32, device=dev)
+        dcn1w = torch.empty(256, D, dtype=torch.float32, device=dev)
+        dcn1b = torch.empty(256, dtype=torch.float32, device=dev)
+        cr = cone.crows if cone is not None else None
+        if cr is not None:
+            ncr = int(cr.numel())
+        if ncr > 0:
+            gemm_tn(D, 256, ncr, GZC, D, saved["HID"], 256, dcn2w, 256, a_rows=cr, b_rows=cr, colsum_a=dcn2b)
+            gemm_tn(256, D, ncr, GHID, 256, saved["A"], D, dcn1w, D, a_rows=cr, b_rows=cr, colsum_a=dcn1b)
+            aux_join()
+        else:
+            for t in (dcn2w, dcn2b, dcn1w, dcn1b):
+                t.zero_()
     cf, nf = saved["cell_feat"], saved["net_feat"]
-    cpins, npins, cpos = sched.cell_class, sched.net_class, None
+    cpins, npins, cpos, npos = sched.cell_class, sched.net_class, None, None
     xc, xn = saved.get("x_rows") or (cpins, npins)            # feature rows of the two classes
     if cone is not None:
         if saved.get("x_rows") is not None:
@@ -516,16 +467,17 @@ def gnn_backward(sched, saved, params, G, cone=None, need_dx=False, need_wgrad=T
         cpins, npins = cone.cell_pins, cone.net_pins
         xc, xn = cpins, npins
         cpos = cone.cell_pos if saved["hc"] is not None else None
-    nc, nn_ = int(cpins.numel()), int(npins.numel())
+        npos = cone.net_pos if saved["hn"] is not None else None
     dcf = torch.zeros(cf.shape, dtype=torch.float32, device=dev) if need_dx else None
     dnf = torch.zeros(nf.shape, dtype=torch.float32, device=dev) if need_dx else None
-    dcs1w, dcs1b, dcs2w, dcs2b, _ = mlp2_backward(cf, cf.stride(0), xc, nc, cs1w, cs2w,
-                                                  saved["hc"], G, D, g_rows=cpins, b1=cs1b, h_rows=cpos,
-                                                  need_dx=need_dx, dx_out=dcf)
-    dns1w, dns1b, dns2w, dns2b, _ = mlp2_backward(nf, nf.stride(0), xn, nn_, ns1w, ns2w,
-                                                  saved["hn"], G, D, g_rows=npins, b1=ns1b,
-                                                  h_rows=(cone.net_pos if cone is not None and saved["hn"] is not None else None),
-                                                  need_dx=need_dx, dx_out=dnf)
+    dcs1w, dcs1b, dcs2w, dcs2b, _ = mlp2_backward(cf, cf.stride(0), xc, int(cpins.numel()), cs1w, cs2w, saved["hc"], G, D,
+                                                  g_rows=cpins, b1=cs1b, h_rows=cpos, need_dx=need_dx, dx_out=dcf,
+                                                  need_wgrad=need_wgrad)
+    dns1w, dns1b, dns2w, dns2b, _ = mlp2_backward(nf, nf.stride(0), xn, int(npins.numel()), ns1w, ns2w, saved["hn"], G, D,
+                                                  g_rows=npins, b1=ns1b, h_rows=npos, need_dx=need_dx, dx_out=dnf,
+                                                  need_wgrad=need_wgrad)
+    if not need_wgrad:
+        return None, dcf, dnf
     grads = (dcs1w, dcs1b, dcs2w, dcs2b, dns1w, dns1b, dns2w, dns2b, dcn1w, dcn1b, dcn2w, dcn2b)
     return (grads, dcf, dnf) if need_dx else grads
 

@@ -32,12 +32,11 @@ def main():
     n = sched.n
     out = dict(n=n, nc=nc, nn=nn_, ncr=ncr)
     S = torch.empty(n, D, device=dev)
-    math = tm_ops._recurrence_math()
-    hc = tm_ops.mlp2_forward(cf, cf.stride(0), sched.cell_class, nc, cs1w, cs1b, cs2w, cs2b, S, D, out_rows=sched.cell_class, math=math)
+    hc = tm_ops.mlp2_forward(cf, cf.stride(0), sched.cell_class, nc, cs1w, cs1b, cs2w, cs2b, S, D, out_rows=sched.cell_class)
     out["fwd_cell_self_ms"] = timeit(lambda: tm_ops.mlp2_forward(cf, cf.stride(0), sched.cell_class, nc, cs1w, cs1b, cs2w, cs2b, S, D,
-                                                                 out_rows=sched.cell_class, math=math))
+                                                                 out_rows=sched.cell_class))
     out["fwd_net_self_ms"] = timeit(lambda: tm_ops.mlp2_forward(nf, nf.stride(0), sched.net_class, nn_, ns1w, ns1b, ns2w, ns2b, S, D,
-                                                                out_rows=sched.net_class, math=math))
+                                                                out_rows=sched.net_class))
     G = torch.randn(n, D, device=dev) * 1e-3
     GZC = torch.randn(ncr, D, device=dev) * 1e-3
     GHID = torch.randn(ncr, 256, device=dev) * 1e-3
