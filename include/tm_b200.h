@@ -107,6 +107,18 @@ int tm_schedule_edges(const tm_schedule* s, int64_t n_sched, int32_t* f_ptr, int
                       int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr,
                       int32_t* bc_row, void* ws, size_t ws_bytes, void* stream);
 
+size_t tm_forward_cone_ws(int64_t n);
+/* Forward cone of `n_seeds` seed pins (device int32; duplicates, pins outside the schedule and n_seeds = 0 are
+ * valid): every scheduled pin reachable from a scheduled seed along the in-edges the propagation reads (s->f_src),
+ * the seeds included -- the pins whose H row can change when the seeds' self terms S change.  Written as a
+ * sub-schedule into caller buffers sized by the parent: order[n_sched] (the stable subsequence of s->order),
+ * level_ptr[num_levels+1], f_ptr[n_sched+1] and f_src[len(s->f_src)] (the parent's in-edge lists of the cone's pins,
+ * in the parent's edge order), count (device int32: the cone's pin count).  No host synchronisation: one block
+ * sweeps the levels from the lowest seed's level on.  `s` needs order, level, level_ptr, f_ptr and f_src. */
+int tm_forward_cone(const tm_schedule* s, int64_t n_seeds, const int32_t* seeds, int32_t* order,
+                    int32_t* level_ptr, int32_t* f_ptr, int32_t* f_src, int32_t* count, void* ws,
+                    size_t ws_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * dense fp32 building blocks (replace the cuBLAS SGEMMs behind nn.Linear,
  * src/model.py:15,23 and every MLP call site model.py:104,141-142,151,272,280,292)
@@ -185,6 +197,14 @@ int tm_gnn_forward(const tm_schedule* s, int32_t level_begin, int32_t level_end,
 int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, const float* W1,
                     const float* W2, const float* A, const float* LSE, const float* HID,
                     float* GA, float* GHID, float* GZC, void* ws, size_t ws_bytes, void* stream);
+
+/* Forward over a sub-schedule built by tm_forward_cone (or any schedule with the device arrays order, f_ptr, f_src,
+ * level_ptr, cell_base): the persistent kernel over levels [0, num_levels), empty levels skipped on the device,
+ * nothing saved for a backward.  Never reads h_level_ptr.  H rows of the schedule's pins are rewritten, every other
+ * row is read only; a pin's row is the same bits tm_gnn_forward's persistent back end writes for the same inputs.
+ * ws: tm_gnn_ws_bytes(). */
+int tm_gnn_forward_cone(const tm_schedule* cone, float* H, const float* S, const float* W1t, const float* b1,
+                        const float* W2t, const float* b2, void* ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * G5  mask fusion (replaces  path_mask.to_dense()*feat_map  and  fcn(path_map),

@@ -934,3 +934,15 @@ extern "C" int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, c
   }
   return 0;
 }
+
+extern "C" int tm_gnn_forward_cone(const tm_schedule* cone, float* H, const float* S, const float* W1t, const float* b1,
+                                   const float* W2t, const float* b2, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(cone && cone->order && cone->f_ptr && cone->f_src && cone->level_ptr && cone->cell_base,
+             "tm_gnn_forward_cone: schedule lacks the device arrays (order, f_ptr, f_src, level_ptr, cell_base)");
+  TM_REQUIRE(cone->num_levels >= 0, "tm_gnn_forward_cone: bad level count");
+  TM_REQUIRE(H && S && W1t && b1 && W2t && b2, "tm_gnn_forward_cone: NULL operand");
+  TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_forward_cone: workspace too small (tm_gnn_ws_bytes)");
+  // the persistent kernel skips empty levels on the device, so the cone's sizes never reach the host
+  return tmk::gnn_persist_forward(cone, 0, cone->num_levels, H, S, W1t, b1, W2t, b2, nullptr, nullptr, nullptr, ws,
+                                  (cudaStream_t)stream);
+}

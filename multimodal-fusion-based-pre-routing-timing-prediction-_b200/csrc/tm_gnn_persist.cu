@@ -941,7 +941,6 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
 // ---------------------------------------------------------------------------------------------
 template <class Args>
 int launch_persist(void (*kern)(const Args), const Args& args, cudaStream_t st, const char* what) {
-  TM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
   cudaLaunchConfig_t cfg = {};
   cfg.blockDim = dim3(THREADS);
   cfg.dynamicSmemBytes = SMEM_BYTES;
@@ -957,7 +956,19 @@ int launch_persist(void (*kern)(const Args), const Args& args, cudaStream_t st, 
   // device can hold, one CTA per SM
   cfg.gridDim = dim3((unsigned)(sm_count() & ~1));
   int ncl = 0;
-  TM_CUDA(cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg));
+  // Inside a stream capture the attribute and occupancy calls are skipped when an eager launch on this device already
+  // made them (the attribute persists; the cluster count is cached): a captured launch then makes no driver query.
+  static std::atomic<int> ncl_cache[64];
+  int dev = 0;
+  TM_CUDA(cudaGetDevice(&dev));
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  TM_CUDA(cudaStreamIsCapturing(st, &cap));
+  if (cap != cudaStreamCaptureStatusNone && dev < 64) ncl = ncl_cache[dev].load(std::memory_order_relaxed);
+  if (ncl == 0) {
+    TM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES));
+    TM_CUDA(cudaOccupancyMaxActiveClusters(&ncl, kern, &cfg));
+    if (dev < 64 && ncl >= 1) ncl_cache[dev].store(ncl, std::memory_order_relaxed);
+  }
   TM_REQUIRE(ncl >= 1, "%s: no 2-CTA cluster with %u bytes of shared memory fits this device", what, SMEM_BYTES);
   cfg.gridDim = dim3((unsigned)(2 * std::min(ncl, sm_count() / 2)));
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args);

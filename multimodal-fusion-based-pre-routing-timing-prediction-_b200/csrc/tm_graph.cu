@@ -526,3 +526,180 @@ extern "C" int tm_schedule_edges(const tm_schedule* s, int64_t n_sched, int32_t*
   sched_edges_fill_kernel<<<blocks, 256, 0, st>>>(g, n_sched, f_ptr, f_src, bn_ptr, bn_dst, bn_w, bc_ptr, bc_row);
   return check_launch("sched_edges_fill");
 }
+
+// ------------------------------------------------------------------------------------------
+// forward cone: the sub-schedule of the pins whose H row can change after the self terms S of
+// some seed pins changed -- every scheduled pin reachable from a seed along the in-edges the
+// propagation reads (the f_ptr / f_src lists), the seeds included.
+//
+// ONE thread block sweeps the levels from the lowest seed's level upwards, PULLING: a pin is in
+// the cone when it is a seed or one of its f_src sources is.  Sources sit on earlier levels, so
+// a level depends only on the levels below it, and the level boundary is a __syncthreads, not a
+// grid-wide barrier (a whole-GPU barrier per level would cost about what the propagation over a
+// small cone does).  Membership is one bit per pin, in shared memory when it fits, else in the
+// workspace.  The same pass compacts the cone: a block scan of (in-cone, in-degree) per chunk of
+// positions gives each member its cone position and edge offset, so order / f_ptr / f_src are
+// written in the parent's order, and level_ptr and the count fall out of the running totals.
+// Work: every schedule position from the lowest seed's level on (one read of order / f_ptr /
+// f_src there), in L - lmin dependent steps; the next level's arrays are prefetched into L2 while
+// the current one is processed.
+//
+// The sweep itself only needs "is any source of this position marked", so a backward cone (the
+// pins an endpoint batch reads) is the same loop run downwards over out-edge lists.
+// ------------------------------------------------------------------------------------------
+namespace {
+constexpr int CONE_T = 1024;
+constexpr int CONE_V = 4;                          // consecutive schedule positions per thread per chunk
+constexpr int CONE_CHUNK = CONE_T * CONE_V;
+constexpr size_t CONE_SMEM_MAX = 192 * 1024;       // membership bitmap in shared memory up to 1.5M pins
+
+struct ConeArgs {
+  int n, L;
+  const int* level; const int* level_ptr; const int* order; const int* f_ptr; const int* f_src;
+  const int* seeds; int n_seeds;
+  uint32_t* gbits;                                 // NULL: the bitmap lives in dynamic shared memory
+  int* c_order; int* c_level_ptr; int* c_f_ptr; int* c_f_src; int* c_count;
+};
+
+__device__ __forceinline__ void pf_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+
+__device__ __forceinline__ bool cone_bit(const volatile uint32_t* bits, int v) {
+  return (bits[v >> 5] >> (v & 31)) & 1u;
+}
+
+__global__ void __launch_bounds__(CONE_T, 1) fwd_cone_kernel(const ConeArgs a) {
+  extern __shared__ uint32_t sbits[];
+  __shared__ int wsum_c[CONE_T / 32], wsum_e[CONE_T / 32];
+  __shared__ int s_lmin;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  uint32_t* bits = a.gbits ? a.gbits : sbits;      // generic: shared or global
+  const volatile uint32_t* vbits = bits;
+  if (!a.gbits)
+    for (int i = tid; i < ((a.n + 31) >> 5); i += CONE_T) sbits[i] = 0u;
+  if (tid == 0) s_lmin = a.L;
+  __syncthreads();
+  for (int i = tid; i < a.n_seeds; i += CONE_T) {
+    const int v = a.seeds[i];
+    if (v < 0 || v >= a.n) continue;
+    const int l = a.level[v];
+    if (l < 0 || l >= a.L) continue;               // outside the schedule: changes nothing
+    atomicOr(bits + (v >> 5), 1u << (v & 31));
+    atomicMin(&s_lmin, l);
+  }
+  __syncthreads();
+  const int lmin = s_lmin;
+  for (int l = tid; l < lmin; l += CONE_T) a.c_level_ptr[l] = 0;
+  int run_c = 0, run_e = 0;                        // cone pins / edges so far (block-uniform)
+  for (int l = lmin; l < a.L; ++l) {
+    const int p0 = __ldg(a.level_ptr + l), p1 = __ldg(a.level_ptr + l + 1);
+    if (tid == 0) a.c_level_ptr[l] = run_c;
+    int p2 = p1, fa = 0, fb = 0;
+    if (l + 1 < a.L) {
+      p2 = __ldg(a.level_ptr + l + 2);
+      fa = __ldg(a.f_ptr + p1);
+      fb = __ldg(a.f_ptr + p2);
+    }
+    for (int c0 = p0; c0 < p1; c0 += CONE_CHUNK) {
+      const int q = c0 + tid * CONE_V;
+      const int nq = max(0, min(CONE_V, p1 - q));
+      int ptr[CONE_V + 1], v[CONE_V];
+      bool in[CONE_V];
+#pragma unroll
+      for (int j = 0; j <= CONE_V; ++j) ptr[j] = (j <= nq && nq > 0) ? __ldg(a.f_ptr + q + j) : 0;
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) v[j] = j < nq ? __ldg(a.order + q + j) : 0;
+      if (c0 == p0) {                              // the next level's static arrays into L2
+        for (int i = p1 + tid * 32; i < p2; i += CONE_T * 32) {
+          pf_l2(a.order + i);
+          pf_l2(a.f_ptr + i);
+        }
+        for (int i = fa + tid * 32; i < fb; i += CONE_T * 32) pf_l2(a.f_src + i);
+      }
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) in[j] = j < nq && cone_bit(vbits, v[j]);
+      int e1 = ptr[0];                             // ptr[nq] without a dynamic register index
+#pragma unroll
+      for (int j = 1; j <= CONE_V; ++j) e1 = j == nq ? ptr[j] : e1;
+      const int e0 = ptr[0];
+      for (int e = e0; e < e1; e += 8) {
+        int src[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) src[u] = e + u < e1 ? __ldg(a.f_src + e + u) : -1;
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          if (src[u] >= 0 && cone_bit(vbits, src[u])) {
+#pragma unroll
+            for (int j = 0; j < CONE_V; ++j) in[j] |= (e + u >= ptr[j] && e + u < ptr[j + 1]);
+          }
+        }
+      }
+      int cnt = 0, edg = 0;
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j)
+        if (in[j]) { ++cnt; edg += ptr[j + 1] - ptr[j]; }
+      // block-wide exclusive scan of (cnt, edg)
+      int ic = cnt, ie = edg;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int yc = __shfl_up_sync(0xffffffffu, ic, o), ye = __shfl_up_sync(0xffffffffu, ie, o);
+        if (lane >= o) { ic += yc; ie += ye; }
+      }
+      if (lane == 31) { wsum_c[warp] = ic; wsum_e[warp] = ie; }
+      __syncthreads();
+      int oc = 0, oe = 0, tc = 0, te = 0;
+#pragma unroll 8
+      for (int w = 0; w < CONE_T / 32; ++w) {
+        const int xc = wsum_c[w], xe = wsum_e[w];
+        if (w < warp) { oc += xc; oe += xe; }
+        tc += xc;
+        te += xe;
+      }
+      int pos = run_c + oc + ic - cnt, eo = run_e + oe + ie - edg;
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) {
+        if (in[j]) {
+          a.c_order[pos] = v[j];
+          a.c_f_ptr[pos] = eo;
+          for (int e = ptr[j]; e < ptr[j + 1]; ++e) a.c_f_src[eo++] = __ldg(a.f_src + e);
+          ++pos;
+          atomicOr(bits + (v[j] >> 5), 1u << (v[j] & 31));
+        }
+      }
+      run_c += tc;
+      run_e += te;
+      __syncthreads();                             // bits of this level are set; wsum may be reused
+    }
+  }
+  if (tid == 0) {
+    a.c_level_ptr[a.L] = run_c;
+    a.c_f_ptr[run_c] = run_e;
+    *a.c_count = run_c;
+  }
+}
+}  // namespace
+
+extern "C" size_t tm_forward_cone_ws(int64_t n) { return (size_t)cdiv(n, 32) * sizeof(uint32_t) + 256; }
+
+extern "C" int tm_forward_cone(const tm_schedule* s, int64_t n_seeds, const int32_t* seeds, int32_t* order,
+                               int32_t* level_ptr, int32_t* f_ptr, int32_t* f_src, int32_t* count, void* ws,
+                               size_t ws_bytes, void* stream) {
+  TM_REQUIRE(s && s->order && s->level && s->level_ptr && s->f_ptr && s->f_src,
+             "tm_forward_cone: the parent schedule lacks its device arrays (order, level, level_ptr, f_ptr, f_src)");
+  TM_REQUIRE(s->n > 0 && s->n < INT32_MAX && s->num_levels > 0, "tm_forward_cone: bad schedule sizes");
+  TM_REQUIRE(n_seeds >= 0 && n_seeds < INT32_MAX && (n_seeds == 0 || seeds), "tm_forward_cone: bad seed list");
+  TM_REQUIRE(order && level_ptr && f_ptr && f_src && count, "tm_forward_cone: NULL output buffer");
+  TM_REQUIRE(ws && ws_bytes >= tm_forward_cone_ws(s->n), "tm_forward_cone: workspace too small (tm_forward_cone_ws)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t bit_bytes = (size_t)cdiv(s->n, 32) * sizeof(uint32_t);
+  const bool in_smem = bit_bytes <= CONE_SMEM_MAX;
+  uint32_t* gbits = nullptr;
+  if (!in_smem) {
+    gbits = reinterpret_cast<uint32_t*>(ws);
+    TM_CUDA(cudaMemsetAsync(gbits, 0, bit_bytes, st));
+  }
+  TM_CUDA(cudaFuncSetAttribute(fwd_cone_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONE_SMEM_MAX));
+  ConeArgs a{(int)s->n, s->num_levels, s->level, s->level_ptr, s->order, s->f_ptr, s->f_src, seeds, (int)n_seeds,
+             gbits, order, level_ptr, f_ptr, f_src, count};
+  fwd_cone_kernel<<<1, CONE_T, in_smem ? bit_bytes : 0, st>>>(a);
+  return check_launch("fwd_cone");
+}

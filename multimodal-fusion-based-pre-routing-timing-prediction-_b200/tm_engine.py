@@ -21,7 +21,7 @@ import tm_dp
 import tm_lib
 import tm_ops
 import tm_unet
-from tm_graph import ConeGraph, MaskCSR, TimingGraph
+from tm_graph import ConeGraph, ForwardCone, MaskCSR, TimingGraph
 from tm_lib import call, stream
 from tm_ops import D, RELU, gemm_nn, gemm_tn, transpose
 
@@ -391,14 +391,14 @@ class DesignStep:
                                  a2.bias.detach(), X[:, 2 * D:], width)
         return dict(X=X, wt=wt, ha=ha, lv=lv, width=width, tab=tab)
 
-    def _head_netlist_side(self, H, b, hs, endpoints=None):
-        """Endpoint rows of H into columns 0..D of X, then ``mlp_fuse``."""
+    def _head_netlist_side(self, H, b, hs, endpoints=None, out=None):
+        """Endpoint rows of H into columns 0..D of X, then ``mlp_fuse`` (into ``out`` when given)."""
         m = self.model
         T = int(b.endpoints.numel())
         X, width = hs["X"], hs["width"]
         call("tm_gather_cols", T, D, H, D, b.endpoints if endpoints is None else endpoints, X, width, 0, stream())
         f0, f2 = m.mlp_fuse.layers[0], m.mlp_fuse.layers[2]
-        pred = torch.empty(T, f2.weight.shape[0], dtype=torch.float32, device=H.device)
+        pred = out if out is not None else torch.empty(T, f2.weight.shape[0], dtype=torch.float32, device=H.device)
         hs["hf"] = tm_ops.mlp2_forward(X, width, None, T, f0.weight.detach(), f0.bias.detach(), f2.weight.detach(),
                                        f2.bias.detach(), pred, pred.shape[1])
         return pred
@@ -458,6 +458,11 @@ class DesignStep:
         # a tensor-core barrier timeout leaves garbage: the whole batch's mse becomes NaN (tm_lib.check_err_flags)
         call("tm_poison_on_error", table, tm_lib.err_flag(dev), stream())
         return pred, EvalMetrics(table, b.K, L)
+
+    def incremental(self, b):
+        """An ``IncrementalEvaluation`` of batch ``b``: one full forward now, then re-prediction after feature edits by
+        re-propagating only the edited pins' forward cone (see the class)."""
+        return IncrementalEvaluation(self, b)
 
     # ---------------------------------------------------------------- full step
     def run(self, b, grad_scale=1.0, input_grads=False, pred_grad=None, param_grads=True):
@@ -751,3 +756,141 @@ class DesignStep:
                                      torch.tensor(co, dtype=torch.int32, device=dev))
         call("tm_adam_multi", int(tab[2].numel()), tab[1], tab[2], tab[3], lr, betas[0], betas[1], eps, weight_decay,
              state["step"], 1.0, stream())
+
+
+class IncrementalEvaluation:
+    """Re-prediction of one batch after edits of its pin features, re-propagating only the edited pins' forward cone
+    (``DesignStep.incremental(batch)``)::
+
+        inc = step.incremental(batch)        # one full forward; keeps H, S and the head's image-side columns
+        batch.cell_feat[pins] = new_rows     # edit cell_feat and / or net_feat rows in place
+        pred = inc.update(pins)              # S rows of `pins`, cone build, cone propagation, head netlist side
+        replay = inc.capture_update(pins)    # one CUDA graph for a fixed pin set: edit rows in place, replay() -> pred
+        inc.refresh()                        # full recompute, after a parameter or image change
+        inc.cone_size()                      # pins re-propagated by the last update (one device read)
+
+    Predictions: ``pred`` (T,) and ``H`` (n, 128) are rewritten in place.  After any sequence of updates they are the
+    same bits as ``step.forward(batch)`` and ``tm_ops.gnn_forward`` on the persistent back end over the edited
+    features; against ``evaluate`` / ``run``, which propagate with the per-level kernels, they agree to fp32 class, as
+    ``forward`` does.  The baseline and every update run the persistent forward, whatever ``tm_gnn_set_impl`` /
+    ``TM_GNN_IMPL`` say.  The head's netlist side (endpoint gather + ``mlp_fuse`` over all T endpoints) reruns in
+    full: the same launches as ``forward``'s head.
+
+    The image branch runs once, in the constructor and in ``refresh()``; neither updates batch-norm running
+    statistics.  Nothing touches a ``.grad``, a parameter or a buffer, and no collective runs.  The state holds the
+    result of the weights and the image as they were at construction (or at the last ``refresh()``): call
+    ``refresh()`` after changing either -- this is documented, not detected (an in-place optimiser step such as
+    ``DesignStep.adam_step`` does not bump a tensor's version counter).
+
+    Pins: a host sequence (list, ndarray or CPU tensor) of pin ids of the batch's netlist; for a joined batch
+    (``DesignBatch.concat``) joined ids, design k owning ``pin_off_h[k]:pin_off_h[k + 1]``.  Duplicates are dropped;
+    pins outside the schedule are accepted and change nothing; an empty list launches nothing; ids out of range or not
+    integers raise ``ValueError``.  A dynamic batch raises ``ValueError``.  Memory: H and S (2 x n x 512 bytes, about
+    340 MB for a 331 819-pin design) plus cone buffers the size of the schedule."""
+
+    def __init__(self, step, b):
+        if getattr(b, "dynamic", False):
+            raise ValueError("DesignStep.incremental: a dynamic batch changes its endpoints between steps; "
+                             "incremental evaluation needs a fixed endpoint set")
+        self.step, self.b = step, b
+        sched = self.sched = b.graph.schedule()
+        dev = b.image.device
+        self.n = sched.n
+        self._level = sched.level.cpu().numpy()          # host copy: splits edited pins into cell / net class
+        T = int(b.endpoints.numel())
+        self.S = torch.empty(self.n, D, dtype=torch.float32, device=dev)
+        self.H = torch.zeros(self.n, D, dtype=torch.float32, device=dev)
+        self.X = torch.empty(T, D + D + step.model.global_dim, dtype=torch.float32, device=dev)
+        f2 = step.model.mlp_fuse.layers[2]
+        self._pred2 = torch.empty(T, f2.weight.shape[0], dtype=torch.float32, device=dev)
+        self.pred = self._pred2.squeeze(-1)
+        self.cone = ForwardCone(b.graph)
+        self._last = None                                 # None: full pass; 0: empty update; "cone": the cone's count
+        self.refresh()
+
+    def _params(self):
+        return [p.detach() for p in self.step.gnn_params]
+
+    def refresh(self):
+        """Full recompute of the image side, S, H and pred (in place), from the current parameters, image and
+        features.  Returns ``pred``."""
+        st, b, sched = self.step, self.b, self.sched
+        gp = self._params()
+        fmap, _ = st._image_forward(b.image, need_bwd=False, update_stats=False)
+        st._check_feature_map(fmap, b)
+        self._hs = st._head_image_side(b, fmap.reshape(-1), self.X)
+        tm_ops.gnn_self_terms(self.S, b.cell_feat, b.net_feat, gp, sched.cell_class, sched.net_class)
+        self.H.zero_()
+        tm_ops.gnn_forward_cone(sched, self.H, self.S, gp)
+        st._head_netlist_side(self.H, b, self._hs, out=self._pred2)
+        self._last = None
+        return self.pred
+
+    def _pins(self, pins):
+        """-> (device int32 [cell-class pins, net-class pins], n cell, n net) of the distinct scheduled pins, or None."""
+        if torch.is_tensor(pins):
+            if pins.device.type != "cpu":
+                raise ValueError("IncrementalEvaluation: pins must be a host sequence (list, ndarray or CPU tensor)")
+            pins = pins.numpy()
+        arr = np.asarray(pins)
+        if arr.size == 0:
+            return None
+        if not np.issubdtype(arr.dtype, np.integer):
+            raise ValueError(f"IncrementalEvaluation: pin ids must be integers, got {arr.dtype}")
+        arr = np.unique(arr.reshape(-1).astype(np.int64))
+        if arr[0] < 0 or arr[-1] >= self.n:
+            raise ValueError(f"IncrementalEvaluation: pin ids must lie in [0, {self.n}), got {arr[0]} .. {arr[-1]}")
+        lv = self._level[arr]
+        cell, net = arr[(lv >= 0) & (lv % 2 == 0)], arr[(lv >= 0) & (lv % 2 == 1)]
+        if cell.size + net.size == 0:
+            return None
+        idx = torch.from_numpy(np.concatenate([cell, net]).astype(np.int32)).to(self.H.device)
+        return idx, int(cell.size), int(net.size)
+
+    def _launch(self, sel):
+        idx, nc, nn_ = sel
+        gp = self._params()
+        tm_ops.gnn_self_terms(self.S, self.b.cell_feat, self.b.net_feat, gp, idx[:nc], idx[nc:])
+        self.cone.build(idx)
+        tm_ops.gnn_forward_cone(self.cone, self.H, self.S, gp)
+        self.step._head_netlist_side(self.H, self.b, self._hs, out=self._pred2)
+        return self.pred
+
+    def update(self, pins):
+        """Re-predict after the feature rows of ``pins`` were edited in place.  Returns ``pred`` (rewritten in place)."""
+        sel = self._pins(pins)
+        if sel is None:
+            self._last = 0
+            return self.pred
+        self._launch(sel)
+        self._last = "cone"
+        return self.pred
+
+    def capture_update(self, pins, pool=None):
+        """``update(pins)`` captured as one CUDA graph for this fixed pin set (run once eagerly first).  Returns
+        ``replay() -> pred``: edit the pins' feature rows in place, then replay.  Several captures coexist (they share
+        the cone buffers and are replayed one after the other on the stream)."""
+        sel = self._pins(pins)
+        if sel is None:
+            def replay_empty():
+                self._last = 0
+                return self.pred
+            return replay_empty
+        inner = self.step._capture_local(lambda: self._launch(sel), warmup=1, pool=pool)
+
+        def replay():
+            inner()
+            self._last = "cone"
+            return self.pred
+        replay.graph = inner.graph
+        replay.pins = sel[0]            # the graph reads this device pin list: it lives as long as the replay
+        return replay
+
+    def cone_size(self):
+        """Pins re-propagated by the last update: the schedule's size after a full pass, 0 after an empty update, else
+        the cone's pin count (one device read)."""
+        if self._last is None:
+            return self.sched.n_sched
+        if self._last == 0:
+            return 0
+        return self.cone.size()

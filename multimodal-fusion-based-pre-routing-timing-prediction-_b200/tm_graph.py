@@ -284,6 +284,52 @@ class BackwardCone:
         self.fraction = cur / max(n, 1)
 
 
+class ForwardCone:
+    """The forward cone of a set of seed pins as a device-side sub-schedule of ``graph.schedule()``: every scheduled pin
+    reachable from a scheduled seed along the in-edges the propagation reads, the seeds included -- the pins whose H
+    row can change when the seeds' self terms change.  ``build(seeds)`` enqueues ``tm_forward_cone`` (no host
+    synchronisation, so it can be captured) and returns ``.struct``, a ``tm_schedule`` that ``tm_gnn_forward_cone``
+    propagates over.  The buffers are allocated once, sized by the parent schedule, and rewritten by every build.
+
+    The struct has no host level offsets (``h_level_ptr`` NULL), so ``tm_gnn_forward`` / ``tm_gnn_backward`` refuse
+    it; it has no cell rows (``n_cell_rows`` 0, ``cell_base`` all zero) and no backward edge lists."""
+
+    def __init__(self, graph):
+        s = self.sched = graph.schedule()
+        dev = s.device
+        i32 = lambda k: torch.empty(max(int(k), 1), dtype=torch.int32, device=dev)      # noqa: E731
+        self.order = i32(s.n_sched)
+        self.level_ptr = i32(s.num_levels + 1)
+        self.f_ptr = i32(s.n_sched + 1)
+        self.f_src = i32(s.f_src.numel())
+        self.count = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.cell_base = torch.zeros(s.num_levels + 1, dtype=torch.int32, device=dev)
+        self.nb = tm_lib.ws_bytes("tm_forward_cone_ws", s.n)
+        self.ws = tm_lib.workspace(self.nb, dev)
+        p = s.struct
+        self.struct = tm_lib.tm_schedule(
+            n=s.n, num_levels=s.num_levels, n_cell_rows=0, h_level_ptr=None,
+            order=self.order.data_ptr(), level=p.level, crow=None,
+            net_iptr=p.net_iptr, net_isrc=p.net_isrc, cell_iptr=p.cell_iptr, cell_isrc=p.cell_isrc,
+            net_optr=p.net_optr, net_odst=p.net_odst, cell_optr=p.cell_optr, cell_odst=p.cell_odst,
+            f_ptr=self.f_ptr.data_ptr(), f_src=self.f_src.data_ptr(),
+            level_ptr=self.level_ptr.data_ptr(), cell_base=self.cell_base.data_ptr())
+
+    def build(self, seeds):
+        """Enqueue the cone of ``seeds`` (int32 pin ids on the device; duplicates and pins outside the schedule are
+        allowed) on the current stream.  Returns ``.struct``."""
+        if not (torch.is_tensor(seeds) and seeds.dtype == torch.int32 and seeds.device == self.sched.device):
+            raise ValueError(f"ForwardCone.build: seeds must be an int32 tensor on {self.sched.device}")
+        seeds = seeds.contiguous()
+        tm_lib.call("tm_forward_cone", self.sched.struct, int(seeds.numel()), seeds, self.order, self.level_ptr,
+                    self.f_ptr, self.f_src, self.count, self.ws, self.nb, tm_lib.stream())
+        return self.struct
+
+    def size(self):
+        """Pins in the last built cone (one device read: diagnostics only)."""
+        return int(self.count.item())
+
+
 def _reaches_endpoint(graph, endpoints):
     """int32 (n,): 1 for every pin from which one of ``endpoints`` is reachable along net / cell edges (the endpoints
     included).  ~num_levels scatter passes over the edge list, on the device."""

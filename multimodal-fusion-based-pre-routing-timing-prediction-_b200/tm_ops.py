@@ -415,6 +415,32 @@ def gnn_forward(sched, cell_feat, net_feat, params, save=True, impl=None, x_rows
     return H, saved
 
 
+def gnn_self_terms(S, cell_feat, net_feat, params, cell_pins, net_pins):
+    """Rewrite the rows of the hoisted self terms ``S`` (N, 128) of the given pins: ``cell_pins`` (int32 device, pins
+    on even levels) through ``fc_cell_self(cell_feat[pin])``, ``net_pins`` (odd levels) through
+    ``fc_net_self(net_feat[pin])`` -- the split of ``Schedule.cell_class`` / ``net_class``.  With those two class lists
+    these are exactly the launches ``gnn_forward`` makes; a pin's row does not depend on which other pins are listed
+    (every route of ``mlp2_route`` scales per row and tiles rows independently).  Other rows are left alone."""
+    (cs1w, cs1b, cs2w, cs2b, ns1w, ns1b, ns2w, ns2b) = [_f32c(p) for p in params[:8]]
+    cell_feat, net_feat = _rowmajor(cell_feat), _rowmajor(net_feat)
+    nc, nn_ = int(cell_pins.numel()), int(net_pins.numel())
+    if nc:
+        mlp2_forward(cell_feat, cell_feat.stride(0), cell_pins, nc, cs1w, cs1b, cs2w, cs2b, S, D, out_rows=cell_pins)
+    if nn_:
+        mlp2_forward(net_feat, net_feat.stride(0), net_pins, nn_, ns1w, ns1b, ns2w, ns2b, S, D, out_rows=net_pins)
+
+
+def gnn_forward_cone(cone, H, S, params):
+    """Re-propagate H (N, 128) in place over a sub-schedule -- ``cone`` a ``tm_graph.ForwardCone`` after ``build``, or a
+    whole ``Schedule`` -- from the self terms ``S``: the persistent forward kernel over the schedule's levels, whatever
+    ``tm_gnn_set_impl`` says, nothing saved.  Rows of the schedule's pins are rewritten (the same bits as the persistent
+    ``gnn_forward`` writes for them given the same sources), every other row is only read."""
+    cn1w, cn1b, cn2w, cn2b = [_f32c(p) for p in params[8:12]]
+    w1t, w2t = transpose(cn1w), transpose(cn2w)
+    nb = tm_lib.ws_bytes("tm_gnn_ws_bytes")
+    call("tm_gnn_forward_cone", cone.struct, H, S, w1t, cn1b, w2t, cn2b, tm_lib.workspace(nb, H.device), nb, stream())
+
+
 def gnn_backward(sched, saved, params, G, cone=None, need_dx=False, need_wgrad=True):
     """``G`` (N,128): dLoss/dH, consumed (overwritten with dLoss/d pre-activation).
     Returns the 12 parameter gradients in GNN_PARAM_NAMES order.
