@@ -119,6 +119,45 @@ int tm_forward_cone(const tm_schedule* s, int64_t n_seeds, const int32_t* seeds,
                     int32_t* level_ptr, int32_t* f_ptr, int32_t* f_src, int32_t* count, void* ws,
                     size_t ws_bytes, void* stream);
 
+size_t tm_forward_cones_ws(int64_t n, int32_t n_cand, int32_t num_levels);
+/* Forward cones of `n_cand` candidate edits, joined into ONE sub-schedule over private virtual rows, for scoring
+ * alternative edits of the same design without touching the rows of its pins (what-if evaluation).
+ *
+ * Candidate k's seeds are seeds[seed_ptr[k] : seed_ptr[k+1]] (seed_ptr: device int32 [n_cand+1]; seeds as in
+ * tm_forward_cone).  Its cone pins get the virtual rows n + row_base[k] + rank, rank = the pin's rank by id among the
+ * cone's pins, so H / S are (n + rows + 1)-row buffers; row n + rows is a sink row.  Candidates are admitted in index
+ * order while the running totals of cone pins fit in `rows` and of cone in-edges in `edge_cap`; the first that does
+ * not fit and every later one is not admitted (fitted[k] = 0) and writes nothing outside the buffers.
+ *
+ * Outputs (caller buffers): order[rows], level_ptr[num_levels+1], f_ptr[rows+1], f_src[edge_cap], count -- a
+ * sub-schedule for tm_gnn_forward_cone whose level l holds candidate 0's cone pins of level l, then candidate 1's, and
+ * so on (admitted candidates only), each in the parent's order, with order[pos] the virtual row and every in-edge
+ * source inside the candidate's cone replaced by its virtual row (sources outside it keep their pin id); vpin[rows]
+ * (the pin of each virtual row); S[virtual row] = S[pin] for every cone pin; seed_rows[seed_slot ? seed_slot[i] : i] =
+ * the virtual row of seed i, or the sink row for a seed outside the schedule or of a non-admitted candidate (where a
+ * caller writes the seeds' new self terms); head_rows[k * n_endpoints + t] = the virtual row of endpoints[t] when it
+ * is in candidate k's admitted cone, else endpoints[t]; fitted[n_cand] (1 = admitted), sizes[n_cand] (cone pins, also
+ * of non-admitted candidates), row_base[n_cand].
+ *
+ * Three launches, no host synchronisation (capturable): one 1024-thread block per candidate sweeps its levels pulling
+ * membership (bitmap in shared memory up to 1.5M pins, else in the workspace) and writes its bitmap, a rank directory
+ * and per-level pin / edge counts; one block admits and lays out the joined levels; blocks over (candidate, level)
+ * compact the cones into the joined arrays.  ws: tm_forward_cones_ws(s->n, n_cand, s->num_levels) -- two n/8-byte
+ * bitmaps per candidate plus 16 bytes per (candidate, level).  `s` needs order, level, level_ptr, f_ptr and f_src. */
+int tm_forward_cones(const tm_schedule* s, int32_t n_cand, const int32_t* seed_ptr, const int32_t* seeds,
+                     const int32_t* seed_slot, int64_t rows, int64_t edge_cap, int64_t n_endpoints,
+                     const int32_t* endpoints, float* S, int32_t* order, int32_t* level_ptr, int32_t* f_ptr,
+                     int32_t* f_src, int32_t* count, int32_t* vpin, int32_t* seed_rows, int32_t* head_rows,
+                     int32_t* fitted, int32_t* sizes, int32_t* row_base, void* ws, size_t ws_bytes, void* stream);
+
+/* Apply candidate k of a tm_forward_cones layout: H[vpin[r]] = H[n + r] and S[vpin[r]] = S[n + r] (128 floats a
+ * row) for r in [row_base[k], row_base[k] + sizes[k]); nothing when fitted[k] == 0. */
+int tm_what_if_commit(int64_t n, int32_t k, const int32_t* fitted, const int32_t* sizes, const int32_t* row_base,
+                      const int32_t* vpin, float* H, float* S, void* stream);
+
+/* pred[k * T + t] = NaN for every candidate k with fitted[k] == 0 (the rows of candidates not admitted). */
+int tm_what_if_mask(int32_t n_cand, int64_t T, const int32_t* fitted, float* pred, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * dense fp32 building blocks (replace the cuBLAS SGEMMs behind nn.Linear,
  * src/model.py:15,23 and every MLP call site model.py:104,141-142,151,272,280,292)

@@ -703,3 +703,413 @@ extern "C" int tm_forward_cone(const tm_schedule* s, int64_t n_seeds, const int3
   fwd_cone_kernel<<<1, CONE_T, in_smem ? bit_bytes : 0, st>>>(a);
   return check_launch("fwd_cone");
 }
+
+// ------------------------------------------------------------------------------------------
+// forward cones of K candidate edits, joined into one sub-schedule over private virtual rows
+// (what-if evaluation: score many alternative edits of one design in one propagation).
+//
+// mark:  grid K, one 1024-thread block per candidate.  fwd_cone_kernel's pull sweep from the
+//        candidate's lowest seed level, without compaction: a pin is in the cone when it is a seed
+//        or one of its f_src sources is.  Sources sit on earlier levels, so bits set during a level
+//        are never read in it and one block barrier per level suffices.  Per-level pin / edge
+//        counts are summed in shared memory (double-buffered by level parity).  At the end the
+//        block writes its bitmap to the workspace (when it lived in shared memory) and a rank
+//        directory: dir[w] = set bits in words < w, so rank(u) = dir[u>>5] + popc(lower bits).
+// plan:  one block.  Admission in index order, the joined level_ptr (level l = the admitted
+//        candidates' cone pins of level l, candidate by candidate), per-(candidate, level) pin and
+//        edge offsets inside the level, the edge offset of every level, the count.
+// emit:  blocks over (candidate, level); the extra level index L does the candidate's seed and
+//        endpoint rows.  A block scan of (in cone, in-degree) over the parent's level compacts the
+//        cone in the parent's order, as fwd_cone_kernel does; sources in the cone are remapped to
+//        their virtual rows; the cone pins' S rows are copied to their virtual rows, a warp a row.
+// ------------------------------------------------------------------------------------------
+namespace {
+constexpr int EMIT_T = 256;
+
+struct ConesArgs {
+  int n, L, K, R;
+  long long ecap;
+  int W;                                           // bitmap words per candidate
+  bool in_smem;                                    // mark keeps its bitmap in shared memory
+  const int* level; const int* level_ptr; const int* order; const int* f_ptr; const int* f_src;
+  const int* seed_ptr; const int* seeds; const int* seed_slot;
+  int T; const int* endpoints;
+  float* S;
+  int* c_order; int* c_level_ptr; int* c_f_ptr; int* c_f_src; int* c_count;
+  int* vpin; int* seed_rows; int* head_rows; int* fitted; int* sizes; int* row_base;
+  // workspace
+  uint32_t* bits; int* dir;                        // [K][W] each
+  int* cnt; int* edg; int* posoff; int* eoff;      // [K][L] each
+  int* lmin; int* etot;                            // [K]
+  int* lev_e;                                      // [L+1]: edges before level l in the joined schedule
+};
+
+// exclusive block scan of two ints; wsum: 64 ints of shared memory.  The caller syncs before wsum is reused.
+__device__ __forceinline__ void block_scan2(int& c, int& e, int& tc, int& te, int* wsum) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int ic = c, ie = e;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int yc = __shfl_up_sync(0xffffffffu, ic, o), ye = __shfl_up_sync(0xffffffffu, ie, o);
+    if (lane >= o) { ic += yc; ie += ye; }
+  }
+  if (lane == 31) { wsum[warp] = ic; wsum[32 + warp] = ie; }
+  __syncthreads();
+  int oc = 0, oe = 0;
+  tc = 0;
+  te = 0;
+  for (int w = 0; w < nw; ++w) {
+    const int xc = wsum[w], xe = wsum[32 + w];
+    if (w < warp) { oc += xc; oe += xe; }
+    tc += xc;
+    te += xe;
+  }
+  c = oc + ic - c;
+  e = oe + ie - e;
+}
+
+__device__ __forceinline__ int warp_sum(int x) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+  return x;
+}
+
+__global__ void __launch_bounds__(CONE_T, 1) cones_mark_kernel(const ConesArgs a) {
+  extern __shared__ uint32_t sbits[];
+  __shared__ int s_lmin, s_c[2], s_e[2];
+  __shared__ int wsum[64];
+  const int k = blockIdx.x, tid = threadIdx.x, lane = tid & 31;
+  uint32_t* gbits = a.bits + (size_t)k * a.W;
+  uint32_t* bits = a.in_smem ? sbits : gbits;
+  const volatile uint32_t* vbits = bits;
+  if (a.in_smem)
+    for (int i = tid; i < a.W; i += CONE_T) sbits[i] = 0u;
+  if (tid == 0) { s_lmin = a.L; s_c[0] = s_c[1] = 0; s_e[0] = s_e[1] = 0; }
+  __syncthreads();
+  const int s0 = __ldg(a.seed_ptr + k), s1 = __ldg(a.seed_ptr + k + 1);
+  for (int i = s0 + tid; i < s1; i += CONE_T) {
+    const int v = a.seeds[i];
+    if (v < 0 || v >= a.n) continue;
+    const int l = a.level[v];
+    if (l < 0 || l >= a.L) continue;               // outside the schedule: changes nothing
+    atomicOr(bits + (v >> 5), 1u << (v & 31));
+    atomicMin(&s_lmin, l);
+  }
+  __syncthreads();
+  const int lmin = s_lmin;
+  int* cnt = a.cnt + (size_t)k * a.L;
+  int* edg = a.edg + (size_t)k * a.L;
+  for (int l = tid; l < lmin; l += CONE_T) { cnt[l] = 0; edg[l] = 0; }
+  for (int l = lmin; l < a.L; ++l) {
+    const int p0 = __ldg(a.level_ptr + l), p1 = __ldg(a.level_ptr + l + 1);
+    int p2 = p1, fa = 0, fb = 0;
+    if (l + 1 < a.L) {
+      p2 = __ldg(a.level_ptr + l + 2);
+      fa = __ldg(a.f_ptr + p1);
+      fb = __ldg(a.f_ptr + p2);
+    }
+    for (int i = p1 + tid * 32; i < p2; i += CONE_T * 32) {   // the next level's static arrays into L2
+      pf_l2(a.order + i);
+      pf_l2(a.f_ptr + i);
+    }
+    for (int i = fa + tid * 32; i < fb; i += CONE_T * 32) pf_l2(a.f_src + i);
+    int my_c = 0, my_e = 0;
+    for (int c0 = p0; c0 < p1; c0 += CONE_CHUNK) {
+      const int q = c0 + tid * CONE_V;
+      const int nq = max(0, min(CONE_V, p1 - q));
+      if (nq == 0) continue;
+      int ptr[CONE_V + 1], v[CONE_V];
+      bool in[CONE_V];
+#pragma unroll
+      for (int j = 0; j <= CONE_V; ++j) ptr[j] = j <= nq ? __ldg(a.f_ptr + q + j) : 0;
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) v[j] = j < nq ? __ldg(a.order + q + j) : 0;
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) in[j] = j < nq && cone_bit(vbits, v[j]);
+      int e1 = ptr[0];                             // ptr[nq] without a dynamic register index
+#pragma unroll
+      for (int j = 1; j <= CONE_V; ++j) e1 = j == nq ? ptr[j] : e1;
+      for (int e = ptr[0]; e < e1; e += 8) {
+        int src[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) src[u] = e + u < e1 ? __ldg(a.f_src + e + u) : -1;
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          if (src[u] >= 0 && cone_bit(vbits, src[u])) {
+#pragma unroll
+            for (int j = 0; j < CONE_V; ++j) in[j] |= (e + u >= ptr[j] && e + u < ptr[j + 1]);
+          }
+        }
+      }
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) {
+        if (in[j]) {
+          ++my_c;
+          my_e += ptr[j + 1] - ptr[j];
+          atomicOr(bits + (v[j] >> 5), 1u << (v[j] & 31));
+        }
+      }
+    }
+    my_c = warp_sum(my_c);
+    my_e = warp_sum(my_e);
+    if (lane == 0 && (my_c | my_e)) { atomicAdd(&s_c[l & 1], my_c); atomicAdd(&s_e[l & 1], my_e); }
+    __syncthreads();                               // bits and counts of level l are complete
+    if (tid == 0) {
+      cnt[l] = s_c[l & 1];
+      edg[l] = s_e[l & 1];
+      s_c[l & 1] = 0;                              // reused by level l + 2, after the next barrier
+      s_e[l & 1] = 0;
+    }
+  }
+  if (a.in_smem) {
+    for (int i = tid; i < a.W; i += CONE_T) gbits[i] = sbits[i];
+  }
+  // rank directory: exclusive scan of the words' popcounts
+  int* dir = a.dir + (size_t)k * a.W;
+  int run = 0;
+  for (int w0 = 0; w0 < a.W; w0 += CONE_T) {
+    const int w = w0 + tid;
+    int c = w < a.W ? __popc(vbits[w]) : 0, e = 0, tc, te;
+    block_scan2(c, e, tc, te, wsum);
+    if (w < a.W) dir[w] = run + c;
+    run += tc;
+    __syncthreads();
+  }
+  if (tid == 0) {
+    a.sizes[k] = run;
+    a.lmin[k] = lmin;
+  }
+}
+
+__global__ void __launch_bounds__(CONE_T, 1) cones_plan_kernel(const ConesArgs a) {
+  __shared__ int wsum[64];
+  const int tid = threadIdx.x, K = a.K, L = a.L;
+  for (int k = tid; k < K; k += CONE_T) {
+    int e = 0;
+    for (int l = 0; l < L; ++l) e += a.edg[(size_t)k * L + l];
+    a.etot[k] = e;
+  }
+  __syncthreads();
+  if (tid == 0) {                                  // admission: the longest prefix that fits
+    long long rc = 0, re = 0;
+    bool open = true;
+    for (int k = 0; k < K; ++k) {
+      const int c = a.sizes[k], e = a.etot[k];
+      open = open && rc + c <= a.R && re + e <= a.ecap;
+      a.fitted[k] = open ? 1 : 0;
+      a.row_base[k] = open ? (int)rc : 0;
+      if (open) { rc += c; re += e; }
+    }
+  }
+  __syncthreads();
+  int run_c = 0, run_e = 0;
+  for (int l0 = 0; l0 < L; l0 += CONE_T) {
+    const int l = l0 + tid;
+    int c = 0, e = 0, tc, te;
+    if (l < L) {
+      for (int k = 0; k < K; ++k) {
+        if (!a.fitted[k]) break;                   // admitted candidates form a prefix
+        const size_t i = (size_t)k * L + l;
+        a.posoff[i] = c;
+        a.eoff[i] = e;
+        c += a.cnt[i];
+        e += a.edg[i];
+      }
+    }
+    block_scan2(c, e, tc, te, wsum);
+    if (l < L) {
+      a.c_level_ptr[l] = run_c + c;
+      a.lev_e[l] = run_e + e;
+    }
+    run_c += tc;
+    run_e += te;
+    __syncthreads();
+  }
+  if (tid == 0) {
+    a.c_level_ptr[L] = run_c;
+    a.lev_e[L] = run_e;
+    a.c_f_ptr[run_c] = run_e;
+    *a.c_count = run_c;
+  }
+}
+
+__device__ __forceinline__ int cone_vrow(const ConesArgs& a, const uint32_t* bits, const int* dir, int base, int u) {
+  return a.n + base + __ldg(dir + (u >> 5)) + __popc(__ldg(bits + (u >> 5)) & ((1u << (u & 31)) - 1u));
+}
+
+__global__ void __launch_bounds__(EMIT_T) cones_emit_kernel(const ConesArgs a) {
+  __shared__ int wsum[64];
+  __shared__ int s_vr[EMIT_T], s_pin[EMIT_T];
+  const int k = blockIdx.x, l = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t* bits = a.bits + (size_t)k * a.W;
+  const int* dir = a.dir + (size_t)k * a.W;
+  const bool admitted = a.fitted[k] != 0;
+  const int base = a.row_base[k];
+  auto in_cone = [&](int u) { return (__ldg(bits + (u >> 5)) >> (u & 31)) & 1u; };
+  if (l == a.L) {                                  // the candidate's seed rows and endpoint head rows
+    const int sink = a.n + a.R;
+    const int s0 = a.seed_ptr[k], s1 = a.seed_ptr[k + 1];
+    for (int i = s0 + tid; i < s1; i += EMIT_T) {
+      const int u = a.seeds[i];
+      int row = sink;
+      if (admitted && u >= 0 && u < a.n) {
+        const int lu = a.level[u];
+        if (lu >= 0 && lu < a.L) row = cone_vrow(a, bits, dir, base, u);
+      }
+      a.seed_rows[a.seed_slot ? a.seed_slot[i] : i] = row;
+    }
+    for (int t = tid; t < a.T; t += EMIT_T) {
+      const int u = a.endpoints[t];
+      a.head_rows[(size_t)k * a.T + t] = (admitted && in_cone(u)) ? cone_vrow(a, bits, dir, base, u) : u;
+    }
+    return;
+  }
+  if (!admitted || l < a.lmin[k]) return;
+  const size_t kl = (size_t)k * a.L + l;
+  if (a.cnt[kl] == 0) return;
+  int pos = a.c_level_ptr[l] + a.posoff[kl];
+  int eo = a.lev_e[l] + a.eoff[kl];
+  const int p0 = __ldg(a.level_ptr + l), p1 = __ldg(a.level_ptr + l + 1);
+  for (int c0 = p0; c0 < p1; c0 += EMIT_T) {
+    const int p = c0 + tid;
+    int v = 0, e0 = 0, e1 = 0;
+    bool in = false;
+    if (p < p1) {
+      v = __ldg(a.order + p);
+      in = in_cone(v);
+      if (in) { e0 = __ldg(a.f_ptr + p); e1 = __ldg(a.f_ptr + p + 1); }
+    }
+    int oc = in ? 1 : 0, oe = e1 - e0, tc, te;
+    block_scan2(oc, oe, tc, te, wsum);
+    if (in) {
+      const int vr = cone_vrow(a, bits, dir, base, v);
+      a.c_order[pos + oc] = vr;
+      a.c_f_ptr[pos + oc] = eo + oe;
+      int o = eo + oe;
+      for (int e = e0; e < e1; ++e) {
+        const int src = __ldg(a.f_src + e);
+        a.c_f_src[o++] = in_cone(src) ? cone_vrow(a, bits, dir, base, src) : src;
+      }
+      a.vpin[vr - a.n] = v;
+      s_vr[oc] = vr;
+      s_pin[oc] = v;
+    }
+    __syncthreads();
+    for (int i = warp; i < tc; i += EMIT_T / 32) {  // S[virtual row] = S[pin], a warp a 512-byte row
+      const float4* src = reinterpret_cast<const float4*>(a.S + (size_t)s_pin[i] * 128);
+      float4* dst = reinterpret_cast<float4*>(a.S + (size_t)s_vr[i] * 128);
+      dst[lane] = src[lane];
+    }
+    pos += tc;
+    eo += te;
+    __syncthreads();                               // wsum / s_vr / s_pin are reused
+  }
+}
+
+__global__ void what_if_commit_kernel(int n, int k, const int* fitted, const int* sizes, const int* row_base,
+                                      const int* vpin, float4* H, float4* S) {
+  if (!fitted[k]) return;
+  const int r0 = row_base[k], cnt = sizes[k];
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (int64_t)cnt * 32;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    const int r = r0 + (int)(i >> 5), c = (int)(i & 31);
+    const int64_t from = (int64_t)(n + r) * 32 + c, to = (int64_t)vpin[r] * 32 + c;
+    H[to] = H[from];
+    S[to] = S[from];
+  }
+}
+
+__global__ void what_if_mask_kernel(int K, int64_t T, const int* fitted, float* pred) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < (int64_t)K * T && !fitted[i / T]) pred[i] = __int_as_float(0x7fc00000);
+}
+
+struct ConesWs {
+  size_t bits, dir, kl, k, lev, total;
+};
+ConesWs cones_ws_layout(int64_t n, int64_t K, int64_t L) {
+  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  ConesWs w{};
+  w.bits = up((size_t)K * cdiv(n, 32) * sizeof(uint32_t));
+  w.dir = w.bits;
+  w.kl = up((size_t)K * L * sizeof(int));
+  w.k = up((size_t)K * sizeof(int));
+  w.lev = up((size_t)(L + 1) * sizeof(int));
+  w.total = w.bits + w.dir + 4 * w.kl + 2 * w.k + w.lev;
+  return w;
+}
+}  // namespace
+
+extern "C" size_t tm_forward_cones_ws(int64_t n, int32_t n_cand, int32_t num_levels) {
+  return cones_ws_layout(n, n_cand > 0 ? n_cand : 1, num_levels > 0 ? num_levels : 1).total;
+}
+
+extern "C" int tm_forward_cones(const tm_schedule* s, int32_t n_cand, const int32_t* seed_ptr, const int32_t* seeds,
+                                const int32_t* seed_slot, int64_t rows, int64_t edge_cap, int64_t n_endpoints,
+                                const int32_t* endpoints, float* S, int32_t* order, int32_t* level_ptr, int32_t* f_ptr,
+                                int32_t* f_src, int32_t* count, int32_t* vpin, int32_t* seed_rows, int32_t* head_rows,
+                                int32_t* fitted, int32_t* sizes, int32_t* row_base, void* ws, size_t ws_bytes,
+                                void* stream) {
+  TM_REQUIRE(s && s->order && s->level && s->level_ptr && s->f_ptr && s->f_src,
+             "tm_forward_cones: the parent schedule lacks its device arrays (order, level, level_ptr, f_ptr, f_src)");
+  TM_REQUIRE(s->n > 0 && s->num_levels > 0 && s->num_levels < 65535, "tm_forward_cones: bad schedule sizes");
+  TM_REQUIRE(n_cand > 0 && n_cand < 65536 && seed_ptr, "tm_forward_cones: bad candidate list");
+  TM_REQUIRE(rows > 0 && s->n + rows + 1 < INT32_MAX && edge_cap >= 0 && edge_cap < INT32_MAX,
+             "tm_forward_cones: bad capacity (rows, edge_cap)");
+  TM_REQUIRE(n_endpoints >= 0 && (int64_t)n_cand * n_endpoints < INT32_MAX && (n_endpoints == 0 || endpoints),
+             "tm_forward_cones: bad endpoint list");
+  TM_REQUIRE(S && order && level_ptr && f_ptr && f_src && count && vpin && seed_rows && head_rows && fitted && sizes &&
+                 row_base,
+             "tm_forward_cones: NULL output buffer");
+  TM_REQUIRE(ws && ws_bytes >= tm_forward_cones_ws(s->n, n_cand, s->num_levels),
+             "tm_forward_cones: workspace too small (tm_forward_cones_ws)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int K = n_cand, L = s->num_levels;
+  const ConesWs w = cones_ws_layout(s->n, K, L);
+  uint8_t* p = reinterpret_cast<uint8_t*>(ws);
+  ConesArgs a{};
+  a.n = (int)s->n; a.L = L; a.K = K; a.R = (int)rows; a.ecap = edge_cap;
+  a.W = (int)cdiv(s->n, 32);
+  const size_t bit_bytes = (size_t)a.W * sizeof(uint32_t);
+  a.in_smem = bit_bytes <= CONE_SMEM_MAX;
+  a.level = s->level; a.level_ptr = s->level_ptr; a.order = s->order; a.f_ptr = s->f_ptr; a.f_src = s->f_src;
+  a.seed_ptr = seed_ptr; a.seeds = seeds; a.seed_slot = seed_slot;
+  a.T = (int)n_endpoints; a.endpoints = endpoints; a.S = S;
+  a.c_order = order; a.c_level_ptr = level_ptr; a.c_f_ptr = f_ptr; a.c_f_src = f_src; a.c_count = count;
+  a.vpin = vpin; a.seed_rows = seed_rows; a.head_rows = head_rows; a.fitted = fitted; a.sizes = sizes;
+  a.row_base = row_base;
+  a.bits = reinterpret_cast<uint32_t*>(p); p += w.bits;
+  a.dir = reinterpret_cast<int*>(p); p += w.dir;
+  a.cnt = reinterpret_cast<int*>(p); p += w.kl;
+  a.edg = reinterpret_cast<int*>(p); p += w.kl;
+  a.posoff = reinterpret_cast<int*>(p); p += w.kl;
+  a.eoff = reinterpret_cast<int*>(p); p += w.kl;
+  a.lmin = reinterpret_cast<int*>(p); p += w.k;
+  a.etot = reinterpret_cast<int*>(p); p += w.k;
+  a.lev_e = reinterpret_cast<int*>(p);
+  if (!a.in_smem) TM_CUDA(cudaMemsetAsync(a.bits, 0, (size_t)K * bit_bytes, st));
+  TM_CUDA(cudaFuncSetAttribute(cones_mark_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONE_SMEM_MAX));
+  cones_mark_kernel<<<K, CONE_T, a.in_smem ? bit_bytes : 0, st>>>(a);
+  if (int rc = check_launch("cones_mark")) return rc;
+  cones_plan_kernel<<<1, CONE_T, 0, st>>>(a);
+  if (int rc = check_launch("cones_plan")) return rc;
+  cones_emit_kernel<<<dim3((unsigned)K, (unsigned)(L + 1)), EMIT_T, 0, st>>>(a);
+  return check_launch("cones_emit");
+}
+
+extern "C" int tm_what_if_commit(int64_t n, int32_t k, const int32_t* fitted, const int32_t* sizes,
+                                 const int32_t* row_base, const int32_t* vpin, float* H, float* S, void* stream) {
+  TM_REQUIRE(n > 0 && n < INT32_MAX && k >= 0, "tm_what_if_commit: bad sizes");
+  TM_REQUIRE(fitted && sizes && row_base && vpin && H && S, "tm_what_if_commit: NULL operand");
+  what_if_commit_kernel<<<296, 256, 0, (cudaStream_t)stream>>>((int)n, k, fitted, sizes, row_base, vpin,
+                                                              reinterpret_cast<float4*>(H), reinterpret_cast<float4*>(S));
+  return check_launch("what_if_commit");
+}
+
+extern "C" int tm_what_if_mask(int32_t n_cand, int64_t T, const int32_t* fitted, float* pred, void* stream) {
+  TM_REQUIRE(n_cand >= 0 && T >= 0 && (n_cand == 0 || T == 0 || (fitted && pred)), "tm_what_if_mask: bad operands");
+  const int64_t m = (int64_t)n_cand * T;
+  if (m == 0) return 0;
+  what_if_mask_kernel<<<(unsigned)cdiv(m, 256), 256, 0, (cudaStream_t)stream>>>(n_cand, T, fitted, pred);
+  return check_launch("what_if_mask");
+}

@@ -21,7 +21,7 @@ import tm_dp
 import tm_lib
 import tm_ops
 import tm_unet
-from tm_graph import ConeGraph, ForwardCone, MaskCSR, TimingGraph
+from tm_graph import ConeGraph, ForwardCone, ForwardCones, MaskCSR, TimingGraph
 from tm_lib import call, stream
 from tm_ops import D, RELU, gemm_nn, gemm_tn, transpose
 
@@ -459,10 +459,11 @@ class DesignStep:
         call("tm_poison_on_error", table, tm_lib.err_flag(dev), stream())
         return pred, EvalMetrics(table, b.K, L)
 
-    def incremental(self, b):
+    def incremental(self, b, what_if_rows=0):
         """An ``IncrementalEvaluation`` of batch ``b``: one full forward now, then re-prediction after feature edits by
-        re-propagating only the edited pins' forward cone (see the class)."""
-        return IncrementalEvaluation(self, b)
+        re-propagating only the edited pins' forward cone (see the class).  ``what_if_rows`` (default 0): rows reserved
+        for ``what_if`` candidates' cone pins (see ``WhatIf``); 0 allocates nothing extra."""
+        return IncrementalEvaluation(self, b, what_if_rows)
 
     # ---------------------------------------------------------------- full step
     def run(self, b, grad_scale=1.0, input_grads=False, pred_grad=None, param_grads=True):
@@ -786,20 +787,38 @@ class IncrementalEvaluation:
     (``DesignBatch.concat``) joined ids, design k owning ``pin_off_h[k]:pin_off_h[k + 1]``.  Duplicates are dropped;
     pins outside the schedule are accepted and change nothing; an empty list launches nothing; ids out of range or not
     integers raise ``ValueError``.  A dynamic batch raises ``ValueError``.  Memory: H and S (2 x n x 512 bytes, about
-    340 MB for a 331 819-pin design) plus cone buffers the size of the schedule."""
+    340 MB for a 331 819-pin design) plus cone buffers the size of the schedule.
 
-    def __init__(self, step, b):
+    ``what_if_rows=R`` > 0 makes ``H`` / ``S`` the first n rows of (n + R + 1)-row buffers, whose rows n.. hold the
+    cone pins of ``what_if`` candidates (see ``WhatIf``): R x 1 KB more.  ``generation`` counts the changes of the
+    base state (``update``, a replayed ``capture_update``, ``refresh``, ``WhatIf.commit``)."""
+
+    def __init__(self, step, b, what_if_rows=0):
         if getattr(b, "dynamic", False):
             raise ValueError("DesignStep.incremental: a dynamic batch changes its endpoints between steps; "
                              "incremental evaluation needs a fixed endpoint set")
+        if isinstance(what_if_rows, bool) or not isinstance(what_if_rows, (int, np.integer)) or what_if_rows < 0:
+            raise ValueError(f"DesignStep.incremental: what_if_rows must be a non-negative integer, got {what_if_rows!r}")
         self.step, self.b = step, b
         sched = self.sched = b.graph.schedule()
         dev = b.image.device
         self.n = sched.n
+        self.R = int(what_if_rows)
+        if self.n + self.R + 1 >= 2 ** 31:
+            raise ValueError(f"DesignStep.incremental: what_if_rows={self.R} exceeds the int32 row range")
         self._level = sched.level.cpu().numpy()          # host copy: splits edited pins into cell / net class
         T = int(b.endpoints.numel())
-        self.S = torch.empty(self.n, D, dtype=torch.float32, device=dev)
-        self.H = torch.zeros(self.n, D, dtype=torch.float32, device=dev)
+        if self.R:
+            # rows n .. n+R-1: what-if candidates' virtual rows; row n+R: the sink of rows that are not admitted
+            self.S_ext = torch.empty(self.n + self.R + 1, D, dtype=torch.float32, device=dev)
+            self.H_ext = torch.zeros(self.n + self.R + 1, D, dtype=torch.float32, device=dev)
+            self.S, self.H = self.S_ext[:self.n], self.H_ext[:self.n]
+        else:
+            self.S = torch.empty(self.n, D, dtype=torch.float32, device=dev)
+            self.H = torch.zeros(self.n, D, dtype=torch.float32, device=dev)
+        self.generation = 0
+        self._overlay = None                              # the WhatIf whose candidates the rows n.. hold
+        self._max_in_degree = None
         self.X = torch.empty(T, D + D + step.model.global_dim, dtype=torch.float32, device=dev)
         f2 = step.model.mlp_fuse.layers[2]
         self._pred2 = torch.empty(T, f2.weight.shape[0], dtype=torch.float32, device=dev)
@@ -824,22 +843,30 @@ class IncrementalEvaluation:
         tm_ops.gnn_forward_cone(sched, self.H, self.S, gp)
         st._head_netlist_side(self.H, b, self._hs, out=self._pred2)
         self._last = None
+        self.generation += 1
         return self.pred
 
-    def _pins(self, pins):
-        """-> (device int32 [cell-class pins, net-class pins], n cell, n net) of the distinct scheduled pins, or None."""
+    def _distinct(self, pins):
+        """-> int64 ndarray of the distinct pin ids (sorted), validated; empty for an empty sequence."""
         if torch.is_tensor(pins):
             if pins.device.type != "cpu":
                 raise ValueError("IncrementalEvaluation: pins must be a host sequence (list, ndarray or CPU tensor)")
             pins = pins.numpy()
         arr = np.asarray(pins)
         if arr.size == 0:
-            return None
+            return np.zeros(0, np.int64)
         if not np.issubdtype(arr.dtype, np.integer):
             raise ValueError(f"IncrementalEvaluation: pin ids must be integers, got {arr.dtype}")
         arr = np.unique(arr.reshape(-1).astype(np.int64))
         if arr[0] < 0 or arr[-1] >= self.n:
             raise ValueError(f"IncrementalEvaluation: pin ids must lie in [0, {self.n}), got {arr[0]} .. {arr[-1]}")
+        return arr
+
+    def _pins(self, pins):
+        """-> (device int32 [cell-class pins, net-class pins], n cell, n net) of the distinct scheduled pins, or None."""
+        arr = self._distinct(pins)
+        if arr.size == 0:
+            return None
         lv = self._level[arr]
         cell, net = arr[(lv >= 0) & (lv % 2 == 0)], arr[(lv >= 0) & (lv % 2 == 1)]
         if cell.size + net.size == 0:
@@ -859,6 +886,7 @@ class IncrementalEvaluation:
     def update(self, pins):
         """Re-predict after the feature rows of ``pins`` were edited in place.  Returns ``pred`` (rewritten in place)."""
         sel = self._pins(pins)
+        self.generation += 1
         if sel is None:
             self._last = 0
             return self.pred
@@ -874,13 +902,16 @@ class IncrementalEvaluation:
         if sel is None:
             def replay_empty():
                 self._last = 0
+                self.generation += 1
                 return self.pred
             return replay_empty
         inner = self.step._capture_local(lambda: self._launch(sel), warmup=1, pool=pool)
+        self.generation += 1                             # the warm-up ran an update
 
         def replay():
             inner()
             self._last = "cone"
+            self.generation += 1
             return self.pred
         replay.graph = inner.graph
         replay.pins = sel[0]            # the graph reads this device pin list: it lives as long as the replay
@@ -893,4 +924,172 @@ class IncrementalEvaluation:
             return self.sched.n_sched
         if self._last == 0:
             return 0
+        if isinstance(self._last, tuple):                # ("what_if", wi, k): a committed candidate
+            return int(self._last[1].cone_sizes()[self._last[2]])
         return self.cone.size()
+
+    def what_if(self, pin_sets):
+        """A ``WhatIf`` over the candidate edits ``pin_sets`` (a sequence of K pin sequences, validated as ``update``
+        validates its pins).  Needs ``what_if_rows`` > 0 at construction."""
+        return WhatIf(self, pin_sets)
+
+    def max_in_degree(self):
+        """The largest in-edge count of a scheduled pin (one device read, cached)."""
+        if self._max_in_degree is None:
+            fp = self.sched.f_ptr
+            self._max_in_degree = int((fp[1:] - fp[:-1]).max()) if self.sched.n_sched else 0
+        return self._max_in_degree
+
+
+class WhatIf:
+    """Score K alternative feature edits of one design in one call, without changing it
+    (``IncrementalEvaluation.what_if(pin_sets)``)::
+
+        inc = step.incremental(batch, what_if_rows=R)
+        wi = inc.what_if(pin_sets)           # K host pin lists (joined ids for a joined batch)
+        wi.cell_feat, wi.net_feat            # (P, 36) / (P, 2) candidate rows, from the batch's rows at creation
+        wi.rows(k)                           # (pins, cell_feat, net_feat) of candidate k: views into the two above
+        pred = wi.run()                      # (K, T): row k = the predictions with candidate k's rows alone
+        replay = wi.capture()                # one CUDA graph: edit wi.cell_feat / net_feat in place, replay() -> (K, T)
+        wi.commit(k)                         # apply candidate k to the batch and the incremental state
+        wi.fitted(), wi.cone_sizes()         # (K,) admitted / cone pins (one device read each)
+
+    Row k of ``run()`` is the same bits as ``step.forward(batch)`` with candidate k's rows written into the batch (and
+    no other candidate's), i.e. as ``inc.pred`` after writing them and ``inc.update(pins)``.  Each candidate's cone
+    pins propagate in private virtual rows n.. of ``inc``'s extended H / S (``tm_forward_cones``): one cone build of
+    three launches, the edited pins' self terms, ONE persistent propagation over the joined cone levels, and the head
+    over K x T rows, whose image-side columns are read from ``inc`` at run time.  Nothing the committed state owns is
+    written: ``inc.H``, ``inc.S``, ``inc.pred``, the batch's features, parameters, buffers and ``.grad``.  So a
+    ``WhatIf`` stays valid across ``inc.update`` / ``refresh`` / ``commit`` and always predicts against the current base.
+
+    Pin sets: duplicates are dropped, pins outside the schedule are accepted and change nothing, an empty set predicts
+    the base (cone 0), bad ids raise ``ValueError``; a pin may be in several sets, each with its own rows.  Capacity:
+    candidates are admitted in index order while their cone pins fit in ``what_if_rows`` and their cone in-edges in
+    ``what_if_rows`` x the schedule's largest in-degree; from the first that does not fit on, a candidate's row of the
+    result is NaN and ``fitted()`` False.  Memory beyond ``inc``'s rows: two n/8-byte bitmaps per candidate, the joined
+    schedule's arrays (sized by ``what_if_rows``), and the (K x T, 288) head matrix.
+
+    ``commit(k)`` propagates nothing: it copies candidate k's virtual H / S rows back to their pins, its feature rows
+    into the batch and its predictions into ``inc.pred`` -- the state ``inc.update`` leaves.  It raises ``ValueError``
+    when the base changed since this object's last run / replay, when another ``WhatIf`` of ``inc`` ran since, or when
+    candidate k was not admitted."""
+
+    def __init__(self, inc, pin_sets):
+        if inc.R == 0:
+            raise ValueError("IncrementalEvaluation.what_if: built with what_if_rows=0; pass what_if_rows > 0 to "
+                             "DesignStep.incremental")
+        if torch.is_tensor(pin_sets) or isinstance(pin_sets, (str, bytes)):
+            raise ValueError("IncrementalEvaluation.what_if: pin_sets must be a sequence of pin sequences")
+        sets = [inc._distinct(p) for p in pin_sets]
+        if not sets:
+            raise ValueError("IncrementalEvaluation.what_if: no candidate")
+        self.inc, b = inc, inc.b
+        dev = inc.H.device
+        K, T = len(sets), int(b.endpoints.numel())
+        self.K, self.T = K, T
+        self._off = np.concatenate([[0], np.cumsum([s.size for s in sets])]).astype(np.int64)
+        self._pins = np.concatenate(sets).astype(np.int64)
+        P = int(self._off[-1])
+        idx = torch.from_numpy(self._pins).to(dev)
+        self._pin_idx = idx
+        self.cell_feat = b.cell_feat.index_select(0, idx).contiguous()
+        self.net_feat = b.net_feat.index_select(0, idx).contiguous()
+        # seeds: each candidate's scheduled pins (candidate by candidate); self-term slots: cell class first
+        lv = inc._level[self._pins] if P else np.zeros(0, np.int32)
+        loc = np.nonzero(lv >= 0)[0]
+        is_cell = lv[loc] % 2 == 0
+        cand = np.searchsorted(self._off, loc, side="right") - 1
+        seed_ptr = np.concatenate([[0], np.cumsum(np.bincount(cand, minlength=K))]).astype(np.int32)
+        slot = np.empty(loc.size, np.int64)
+        nc = int(is_cell.sum())
+        slot[is_cell] = np.arange(nc)
+        slot[~is_cell] = nc + np.arange(loc.size - nc)
+        i32 = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.int32)).to(dev)    # noqa: E731
+        self._seed_ptr, self._seeds, self._seed_slot = i32(seed_ptr), i32(self._pins[loc]), i32(slot)
+        self._x_cell, self._x_net = i32(loc[is_cell]), i32(loc[~is_cell])
+        self._nc = nc
+        self.cones = ForwardCones(b.graph, K, inc.R, inc.R * max(inc.max_in_degree(), 1), b.endpoints, loc.size)
+        self._img_rows = i32(np.tile(np.arange(T), K))
+        width = inc.X.shape[1]
+        self._Xw = torch.empty(K * T, width, dtype=torch.float32, device=dev)
+        self._pred2 = torch.empty(K * T, inc._pred2.shape[1], dtype=torch.float32, device=dev)
+        self.pred = self._pred2.view(K, T)
+        self._gen = None                                  # inc.generation at the last run / replay
+
+    def rows(self, k):
+        """(pins int64 ndarray, cell_feat rows, net_feat rows) of candidate k: views into ``cell_feat`` / ``net_feat``."""
+        if not 0 <= k < self.K:
+            raise ValueError(f"WhatIf.rows: candidate {k} out of range [0, {self.K})")
+        s, e = int(self._off[k]), int(self._off[k + 1])
+        return self._pins[s:e], self.cell_feat[s:e], self.net_feat[s:e]
+
+    def _launch(self):
+        inc, c, st = self.inc, self.cones, self.inc.step
+        gp = inc._params()
+        c.build(self._seed_ptr, self._seeds, self._seed_slot, inc.S_ext)
+        nc = self._nc
+        tm_ops.gnn_self_terms(inc.S_ext, self.cell_feat, self.net_feat, gp, self._x_cell, self._x_net,
+                              cell_out=c.seed_rows[:nc], net_out=c.seed_rows[nc:])
+        tm_ops.gnn_forward_cone(c, inc.H_ext, inc.S_ext, gp)
+        KT, Xw = self.K * self.T, self._Xw
+        width = Xw.shape[1]
+        call("tm_gather_cols", KT, D, inc.H_ext, D, c.head_rows, Xw, width, 0, stream())
+        call("tm_gather_cols", KT, width - D, inc.X[:, D:], width, self._img_rows, Xw, width, D, stream())
+        f0, f2 = st.model.mlp_fuse.layers[0], st.model.mlp_fuse.layers[2]
+        tm_ops.mlp2_forward(Xw, width, None, KT, f0.weight.detach(), f0.bias.detach(), f2.weight.detach(),
+                            f2.bias.detach(), self._pred2, self._pred2.shape[1])
+        call("tm_what_if_mask", self.K, self.T, c.fitted, self._pred2, stream())
+        return self.pred
+
+    def _ran(self):
+        self._gen = self.inc.generation
+        self.inc._overlay = self
+
+    def run(self):
+        """Every candidate's predictions against the current base: (K, T) device tensor, rewritten by every run /
+        replay."""
+        self._launch()
+        self._ran()
+        return self.pred
+
+    def capture(self, pool=None):
+        """``run()`` captured as one CUDA graph (run once eagerly first).  Returns ``replay() -> (K, T)``: edit
+        ``cell_feat`` / ``net_feat`` in place, then replay."""
+        inner = self.inc.step._capture_local(self._launch, warmup=1, pool=pool)
+        self._ran()
+
+        def replay():
+            inner()
+            self._ran()
+            return self.pred
+        replay.graph = inner.graph
+        return replay
+
+    def commit(self, k):
+        """Apply candidate k: the batch's feature rows, ``inc.H``, ``inc.S`` and ``inc.pred`` as ``inc.update`` leaves
+        them, without a propagation."""
+        inc = self.inc
+        if self._gen is None or self._gen != inc.generation or inc._overlay is not self:
+            raise ValueError("WhatIf.commit: the base changed (or another what-if ran) since this object's last run / "
+                             "replay; run it again first")
+        if not isinstance(k, (int, np.integer)) or not 0 <= k < self.K:
+            raise ValueError(f"WhatIf.commit: candidate {k!r} out of range [0, {self.K})")
+        c = self.cones
+        if not bool(c.fitted[k].item()):
+            raise ValueError(f"WhatIf.commit: candidate {k} was not admitted (what_if_rows too small)")
+        call("tm_what_if_commit", inc.n, int(k), c.fitted, c.sizes, c.row_base, c.vpin, inc.H_ext, inc.S_ext, stream())
+        s, e = int(self._off[k]), int(self._off[k + 1])
+        if e > s:
+            inc.b.cell_feat.index_copy_(0, self._pin_idx[s:e], self.cell_feat[s:e])
+            inc.b.net_feat.index_copy_(0, self._pin_idx[s:e], self.net_feat[s:e])
+        inc._pred2.copy_(self._pred2[k * self.T:(k + 1) * self.T])
+        inc.generation += 1
+        inc._last = ("what_if", self, int(k))
+
+    def fitted(self):
+        """(K,) bool host array: the candidates admitted by the last run / replay (one device read)."""
+        return self.cones.fitted.cpu().numpy().astype(bool)
+
+    def cone_sizes(self):
+        """(K,) int host array: each candidate's cone pins in the last run / replay (one device read)."""
+        return self.cones.sizes.cpu().numpy().astype(np.int64)

@@ -330,6 +330,56 @@ class ForwardCone:
         return int(self.count.item())
 
 
+class ForwardCones:
+    """The forward cones of ``n_cand`` candidate edits of one design, joined into one device-side sub-schedule over
+    private virtual rows (``tm_forward_cones``): candidate k's cone pins get the rows ``n + row_base[k] + rank`` of
+    (n + rows + 1)-row H / S buffers, so K alternative edits propagate side by side in one ``tm_gnn_forward_cone``
+    without touching the rows of the design's pins.  Row ``n + rows`` is a sink row.  Candidates are admitted in index
+    order while their cone pins fit in ``rows`` and their cone in-edges in ``edge_cap``; ``fitted`` marks them.
+
+    ``build(seed_ptr, seeds, seed_slot, S)`` enqueues the build (no host synchronisation, so it can be captured),
+    copies every cone pin's S row to its virtual row and returns ``.struct``.  It also fills ``seed_rows`` (the
+    virtual row of every seed, or the sink row), ``head_rows`` (K x T: each endpoint's row per candidate), ``vpin``,
+    ``fitted``, ``sizes`` and ``row_base``.  The buffers are allocated once: the joined arrays sized by ``rows`` and
+    ``edge_cap``, two n/8-byte bitmaps per candidate in the workspace."""
+
+    def __init__(self, graph, n_cand, rows, edge_cap, endpoints, n_seeds):
+        s = self.sched = graph.schedule()
+        dev = s.device
+        i32 = lambda k: torch.empty(max(int(k), 1), dtype=torch.int32, device=dev)      # noqa: E731
+        self.K, self.rows, self.edge_cap, self.T = int(n_cand), int(rows), int(edge_cap), int(endpoints.numel())
+        self.endpoints = endpoints
+        self.order = i32(rows)
+        self.level_ptr = i32(s.num_levels + 1)
+        self.f_ptr = i32(rows + 1)
+        self.f_src = i32(edge_cap)
+        self.count = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.vpin = i32(rows)
+        self.seed_rows = i32(n_seeds)
+        self.head_rows = i32(self.K * self.T)
+        self.fitted = torch.zeros(self.K, dtype=torch.int32, device=dev)
+        self.sizes = torch.zeros(self.K, dtype=torch.int32, device=dev)
+        self.row_base = torch.zeros(self.K, dtype=torch.int32, device=dev)
+        self.cell_base = torch.zeros(s.num_levels + 1, dtype=torch.int32, device=dev)
+        self.nb = tm_lib.ws_bytes("tm_forward_cones_ws", s.n, self.K, s.num_levels)
+        self.ws = tm_lib.workspace(self.nb, dev)
+        # only what tm_gnn_forward_cone reads: the joined order / level_ptr / f_ptr / f_src over n + rows + 1 rows
+        self.struct = tm_lib.tm_schedule(
+            n=s.n + rows + 1, num_levels=s.num_levels, n_cell_rows=0, h_level_ptr=None,
+            order=self.order.data_ptr(), f_ptr=self.f_ptr.data_ptr(), f_src=self.f_src.data_ptr(),
+            level_ptr=self.level_ptr.data_ptr(), cell_base=self.cell_base.data_ptr())
+
+    def build(self, seed_ptr, seeds, seed_slot, S):
+        """Enqueue the joined cones of the candidates' seeds (int32 device CSR ``seed_ptr`` (K+1) / ``seeds``; seed i's
+        row goes to ``seed_rows[seed_slot[i]]``) on the current stream, with S the (n + rows + 1, 128) self terms.
+        Returns ``.struct``."""
+        tm_lib.call("tm_forward_cones", self.sched.struct, self.K, seed_ptr, seeds, seed_slot, self.rows, self.edge_cap,
+                    self.T, self.endpoints, S, self.order, self.level_ptr, self.f_ptr, self.f_src, self.count,
+                    self.vpin, self.seed_rows, self.head_rows, self.fitted, self.sizes, self.row_base, self.ws,
+                    self.nb, tm_lib.stream())
+        return self.struct
+
+
 def _reaches_endpoint(graph, endpoints):
     """int32 (n,): 1 for every pin from which one of ``endpoints`` is reachable along net / cell edges (the endpoints
     included).  ~num_levels scatter passes over the edge list, on the device."""

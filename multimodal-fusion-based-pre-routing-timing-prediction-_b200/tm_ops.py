@@ -415,19 +415,23 @@ def gnn_forward(sched, cell_feat, net_feat, params, save=True, impl=None, x_rows
     return H, saved
 
 
-def gnn_self_terms(S, cell_feat, net_feat, params, cell_pins, net_pins):
+def gnn_self_terms(S, cell_feat, net_feat, params, cell_pins, net_pins, cell_out=None, net_out=None):
     """Rewrite the rows of the hoisted self terms ``S`` (N, 128) of the given pins: ``cell_pins`` (int32 device, pins
     on even levels) through ``fc_cell_self(cell_feat[pin])``, ``net_pins`` (odd levels) through
     ``fc_net_self(net_feat[pin])`` -- the split of ``Schedule.cell_class`` / ``net_class``.  With those two class lists
     these are exactly the launches ``gnn_forward`` makes; a pin's row does not depend on which other pins are listed
-    (every route of ``mlp2_route`` scales per row and tiles rows independently).  Other rows are left alone."""
+    (every route of ``mlp2_route`` scales per row and tiles rows independently).  Other rows are left alone.
+    ``cell_out`` / ``net_out`` (int32 device, as long as the pin lists): write row i to ``S[cell_out[i]]`` instead
+    of ``S[cell_pins[i]]`` (what-if evaluation: candidate rows into their virtual rows)."""
     (cs1w, cs1b, cs2w, cs2b, ns1w, ns1b, ns2w, ns2b) = [_f32c(p) for p in params[:8]]
     cell_feat, net_feat = _rowmajor(cell_feat), _rowmajor(net_feat)
     nc, nn_ = int(cell_pins.numel()), int(net_pins.numel())
     if nc:
-        mlp2_forward(cell_feat, cell_feat.stride(0), cell_pins, nc, cs1w, cs1b, cs2w, cs2b, S, D, out_rows=cell_pins)
+        mlp2_forward(cell_feat, cell_feat.stride(0), cell_pins, nc, cs1w, cs1b, cs2w, cs2b, S, D,
+                     out_rows=cell_pins if cell_out is None else cell_out)
     if nn_:
-        mlp2_forward(net_feat, net_feat.stride(0), net_pins, nn_, ns1w, ns1b, ns2w, ns2b, S, D, out_rows=net_pins)
+        mlp2_forward(net_feat, net_feat.stride(0), net_pins, nn_, ns1w, ns1b, ns2w, ns2b, S, D,
+                     out_rows=net_pins if net_out is None else net_out)
 
 
 def gnn_forward_cone(cone, H, S, params):
