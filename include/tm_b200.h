@@ -119,6 +119,26 @@ int tm_forward_cone(const tm_schedule* s, int64_t n_seeds, const int32_t* seeds,
                     int32_t* level_ptr, int32_t* f_ptr, int32_t* f_src, int32_t* count, void* ws,
                     size_t ws_bytes, void* stream);
 
+size_t tm_fanin_cone_ws(int64_t n, int32_t n_cell_rows);
+/* Fan-in cone of the endpoints whose seed is non-zero (endpoints: device int32 [n_endpoints], seed: device float32
+ * [n_endpoints], both read on the device; duplicates and endpoints outside the schedule are valid): every scheduled
+ * pin from which a seeded endpoint is reachable along the out-edges a backward pass reads (s->bn_dst and the cell
+ * out-edges s->bc_row), the seeded endpoints included -- the pins whose gradient can be non-zero.  Written as a
+ * sub-schedule for tm_gnn_save_cone / tm_gnn_backward_cone into caller buffers sized by the parent, laid out from their
+ * END: positions [n_sched - count, n_sched) of order[n_sched] (the stable subsequence of s->order), level_ptr and
+ * cell_base [num_levels+1] (cell rows [n_cell_rows - cone cell rows, n_cell_rows), one per cone pin on an even level
+ * > 0, in schedule order), f_ptr / bn_ptr / bc_ptr [n_sched+1] with f_src [len(s->f_src)] (the parent's in-edge lists,
+ * unchanged), bn_dst / bn_w [len(s->bn_dst)] and bc_row [len(s->bc_row)] (out-edges whose destination is in the
+ * cone, in the parent's order, bc_row as cone cell rows).  cell_pins / net_pins (capacity: the pins on even / odd
+ * levels) list the cone's pins on even / odd levels from index 0; counts (device int32 [3]) = cone pins, cell_pins
+ * entries, net_pins entries.  No host synchronisation: one block sweeps from the highest seeded level down.  ws:
+ * tm_fanin_cone_ws(s->n, s->n_cell_rows) -- the membership bitmap when it exceeds shared memory (over 1.5M pins) and
+ * one int per cell row. */
+int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints, const float* seed,
+                  int32_t* order, int32_t* level_ptr, int32_t* cell_base, int32_t* f_ptr, int32_t* f_src,
+                  int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr, int32_t* bc_row, int32_t* cell_pins,
+                  int32_t* net_pins, int32_t* counts, void* ws, size_t ws_bytes, void* stream);
+
 size_t tm_forward_cones_ws(int64_t n, int32_t n_cand, int32_t num_levels);
 /* Forward cones of `n_cand` candidate edits, joined into ONE sub-schedule over private virtual rows, for scoring
  * alternative edits of the same design without touching the rows of its pins (what-if evaluation).
@@ -244,6 +264,21 @@ int tm_gnn_backward(const tm_schedule* s, const float* H, float* G, const float*
  * ws: tm_gnn_ws_bytes(). */
 int tm_gnn_forward_cone(const tm_schedule* cone, float* H, const float* S, const float* W1t, const float* b1,
                         const float* W2t, const float* b2, void* ws, size_t ws_bytes, void* stream);
+
+/* What tm_gnn_forward saves for the backward (A, LSE, HID), recomputed over the cell levels of a sub-schedule built by
+ * tm_fanin_cone whose in-edge sources are all final in H: per cell pin the gather's online softmax and the first
+ * fc_cell_neigh product with its per-pin scale, written at the sub-schedule's cell rows (cell_base).  No second product,
+ * no H store, no grid barrier.  The rows are the same bits tm_gnn_forward's persistent back end saves for those pins.
+ * Never reads h_level_ptr.  ws: tm_gnn_ws_bytes(). */
+int tm_gnn_save_cone(const tm_schedule* cone, const float* H, const float* W1t, const float* b1, const float* W2t,
+                     float* A, float* LSE, float* HID, void* ws, size_t ws_bytes, void* stream);
+/* tm_gnn_backward's data-gradient sweep (GHID = GZC = NULL) on the persistent back end over a sub-schedule built by
+ * tm_fanin_cone, empty levels skipped on the device: G rows of the sub-schedule's pins are read (the head's gradient)
+ * and rewritten with dLoss/dS; A / LSE / HID / GA are indexed by the sub-schedule's cell rows (tm_gnn_save_cone).  Never
+ * reads h_level_ptr.  ws: tm_gnn_ws_bytes(). */
+int tm_gnn_backward_cone(const tm_schedule* cone, const float* H, float* G, const float* W1, const float* W2,
+                         const float* A, const float* LSE, const float* HID, float* GA, void* ws, size_t ws_bytes,
+                         void* stream);
 
 /* ------------------------------------------------------------------------------------
  * G5  mask fusion (replaces  path_mask.to_dense()*feat_map  and  fcn(path_map),
@@ -570,6 +605,21 @@ int tm_selfmlp_rows_dh(int64_t M, const float* G, int64_t ldg, const int32_t* g_
 int tm_selfmlp_rows_dx(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* W2, const float* H,
                        int64_t ldh, const int32_t* h_rows, const float* W1, int64_t kin, float* dX, int64_t lddx,
                        const int32_t* x_rows, void* ws, size_t ws_bytes, void* stream);
+/* tm_selfmlp_lin1_relu (without rowmax), tm_selfmlp_rows_dx and tm_selfmlp_gen_bwd1_dx (dW1 = db1 = NULL) over a row
+ * count that exists only on the device: m_dev (device int32) holds it, at most `cap`, the host capacity the grid is sized
+ * by; CTAs past the count do nothing.  Row m's results are the same bits as with the host count (a fan-in cone's class
+ * lists, tm_fanin_cone). */
+int tm_selfmlp_lin1_relu_dcount(int64_t cap, const int32_t* m_dev, const float* X, int64_t ldx, const int32_t* x_rows,
+                                int64_t kin, const float* W1, const float* b1, float* HID, int64_t ldh, void* ws,
+                                size_t ws_bytes, void* stream);
+int tm_selfmlp_rows_dx_dcount(int64_t cap, const int32_t* m_dev, const float* G, int64_t ldg, const int32_t* g_rows,
+                              const float* W2, const float* H, int64_t ldh, const int32_t* h_rows, const float* W1,
+                              int64_t kin, float* dX, int64_t lddx, const int32_t* x_rows, void* ws, size_t ws_bytes,
+                              void* stream);
+int tm_selfmlp_gen_bwd1_dx_dcount(int64_t cap, const int32_t* m_dev, const float* G, int64_t ldg, const int32_t* g_rows,
+                                  const float* X, int64_t ldx, const int32_t* x_rows, int64_t kx, const float* W1,
+                                  const float* b1, const float* W2, float* dX, int64_t lddx, void* ws, size_t ws_bytes,
+                                  void* stream);
 size_t tm_selfmlp_wgrad2_ws_bytes(void);
 int tm_selfmlp_gen_wgrad2(int64_t M, const float* G, int64_t ldg, const int32_t* g_rows, const float* X, int64_t ldx,
                           const int32_t* x_rows, int64_t kx, const float* W1, const float* b1, const float* gmax,

@@ -797,6 +797,8 @@ int gnn_persist_forward(const tm_schedule* s, int lb, int le, float* H, const fl
 int gnn_persist_backward(const tm_schedule* s, const float* H, float* G, const float* W1, const float* W2, const float* A,
                          const float* LSE, const float* HIDb, float* GA, float* GHID, float* GZC, void* ws, cudaStream_t st,
                          int lb, int le);
+int gnn_persist_save(const tm_schedule* s, const float* H, const float* W1t, const float* b1, const float* W2t, float* A,
+                     float* LSE, float* HIDb, void* ws, cudaStream_t st);
 }  // namespace tmk
 
 namespace {
@@ -945,4 +947,30 @@ extern "C" int tm_gnn_forward_cone(const tm_schedule* cone, float* H, const floa
   // the persistent kernel skips empty levels on the device, so the cone's sizes never reach the host
   return tmk::gnn_persist_forward(cone, 0, cone->num_levels, H, S, W1t, b1, W2t, b2, nullptr, nullptr, nullptr, ws,
                                   (cudaStream_t)stream);
+}
+
+extern "C" int tm_gnn_save_cone(const tm_schedule* cone, const float* H, const float* W1t, const float* b1,
+                                const float* W2t, float* A, float* LSE, float* HID, void* ws, size_t ws_bytes,
+                                void* stream) {
+  TM_REQUIRE(cone && cone->order && cone->f_ptr && cone->f_src && cone->level_ptr && cone->cell_base,
+             "tm_gnn_save_cone: schedule lacks the device arrays (order, f_ptr, f_src, level_ptr, cell_base)");
+  TM_REQUIRE(cone->num_levels >= 0, "tm_gnn_save_cone: bad level count");
+  TM_REQUIRE(H && W1t && b1 && W2t && A && LSE && HID, "tm_gnn_save_cone: NULL operand");
+  TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_save_cone: workspace too small (tm_gnn_ws_bytes)");
+  return tmk::gnn_persist_save(cone, H, W1t, b1, W2t, A, LSE, HID, ws, (cudaStream_t)stream);
+}
+
+extern "C" int tm_gnn_backward_cone(const tm_schedule* cone, const float* H, float* G, const float* W1, const float* W2,
+                                    const float* A, const float* LSE, const float* HID, float* GA, void* ws,
+                                    size_t ws_bytes, void* stream) {
+  TM_REQUIRE(cone && cone->order && cone->level_ptr && cone->cell_base && cone->bn_ptr && cone->bn_dst && cone->bn_w &&
+                 cone->bc_ptr && cone->bc_row,
+             "tm_gnn_backward_cone: schedule lacks the device arrays (order, level_ptr, cell_base, bn_ptr, bn_dst, "
+             "bn_w, bc_ptr, bc_row)");
+  TM_REQUIRE(cone->num_levels >= 0, "tm_gnn_backward_cone: bad level count");
+  TM_REQUIRE(H && G && W1 && W2 && A && LSE && HID && GA, "tm_gnn_backward_cone: NULL operand");
+  TM_REQUIRE(ws && ws_bytes >= tm_gnn_ws_bytes(), "tm_gnn_backward_cone: workspace too small (tm_gnn_ws_bytes)");
+  // the persistent sweep skips empty levels on the device, so the cone's sizes never reach the host
+  return tmk::gnn_persist_backward(cone, H, G, W1, W2, A, LSE, HID, GA, nullptr, nullptr, ws, (cudaStream_t)stream, 0,
+                                   cone->num_levels);
 }

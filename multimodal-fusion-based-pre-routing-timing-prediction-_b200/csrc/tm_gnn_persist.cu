@@ -936,6 +936,142 @@ __global__ void __launch_bounds__(THREADS, 1) gnn_persist_bwd_kernel(const BwdAr
   ctx_teardown(c);
 }
 
+// =============================================================================================
+// save-only forward (tm_gnn_save_cone): what the forward saves for the backward -- A, LSE and HID -- recomputed over the
+// cell levels of a sub-schedule whose in-edge sources are all final in H.  Per tile: the gather's online softmax and
+// MMA 1 with its per-pin scale; no MMA 2, no exchange, no H store.  No level waits for another, so there is no grid
+// barrier and the tiles of all levels are dealt to the clusters round-robin.  The gather and epilogue 1 repeat
+// gnn_persist_fwd_kernel's expressions one for one: a pin's rows depend only on its own sources, its scale and the
+// weights (not on the tile it shares), so they are the same bits the full forward saves.
+// =============================================================================================
+struct SaveArgs {
+  const int* level_ptr; const int* cell_base; const int* order; const int* f_ptr; const int* f_src;
+  const float* H;
+  const uint8_t* planes; const float* b1;                                 // packed fc_cell_neigh weights
+  float* A; float* LSE; float* HIDb;
+  long long* prof;
+  int L;
+};
+
+__global__ void __launch_bounds__(THREADS, 1) gnn_persist_save_kernel(const SaveArgs a) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  Ctx c;
+  ctx_setup(c, smem, a.planes, a.prof);
+  const int cluster_id = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
+  const int qd = warp & 3, cg = warp >> 2, m = qd * 32 + lane;
+  const float b1m = __ldg(a.b1 + c.rank * 128 + qd * 32 + lane);
+  const uint32_t sW = smem_u32(c.smem + OFF_W), sB = smem_u32(c.smem + OFF_B);
+  const uint32_t tl = c.tmem + ((uint32_t)(qd * 32) << 16);
+  int dealt = 0;                                             // tiles of the levels before this one
+  for (int l = 2; l < a.L; l += 2) {
+    const int p0 = __ldg(a.level_ptr + l), cnt = __ldg(a.level_ptr + l + 1) - p0;
+    if (cnt <= 0) continue;
+    const int crow0 = __ldg(a.cell_base + l);
+    const int N = tile_width(cnt, nclusters), ntiles = (cnt + N - 1) / N;
+    const int PPW = N >> 4, nper = N >> 2;
+    const int first = (cluster_id - dealt % nclusters + nclusters) % nclusters;
+    dealt += ntiles;
+    for (int tile = first; tile < ntiles; tile += nclusters) {
+      const int t0 = tile * N;
+      const int r0 = warp * PPW;
+      const int npin = min(PPW, cnt - (t0 + r0));
+      const int pb = p0 + t0 + r0;
+      const bool owner = ((uint32_t)(warp >> 3) == c.rank);
+      int ptrs = 0, vv = -1;
+      if (npin > 0) {
+        if (lane <= npin) ptrs = __ldg(a.f_ptr + pb + lane);
+        if (lane < npin) vv = __ldg(a.order + pb + lane);
+      }
+      const int E0 = __shfl_sync(0xffffffffu, ptrs, 0), E1 = __shfl_sync(0xffffffffu, ptrs, max(npin, 0));
+      int idx = (E0 + (lane & 7) < E1) ? __ldg(a.f_src + E0 + (lane & 7)) : 0;
+      tc_fence_before();
+      __syncthreads();                                       // the previous tile's epilogue still reads the scales
+      c.stamp(PH_CPRE);
+
+      int q = 0;
+      float mx[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+      float sm[4] = {0.f, 0.f, 0.f, 0.f}, tw[4] = {0.f, 0.f, 0.f, 0.f};
+      auto finish_pin = [&]() {
+        float4 av = f4zero(), lse = av;
+        if (sm[0] > 0.f) {
+          av = make_float4(__fdividef(tw[0], sm[0]), __fdividef(tw[1], sm[1]), __fdividef(tw[2], sm[2]), __fdividef(tw[3], sm[3]));
+          lse = make_float4(mx[0] + __logf(sm[0]), mx[1] + __logf(sm[1]), mx[2] + __logf(sm[2]), mx[3] + __logf(sm[3]));
+        }
+        if (owner) {
+          const int64_t o = (int64_t)(crow0 + t0 + r0 + q) * D + lane * 4;
+          *reinterpret_cast<float4*>(a.A + o) = av;
+          *reinterpret_cast<float4*>(a.LSE + o) = lse;
+        }
+        store_pin_row(smem, r0 + q, lane, av, -4, __shfl_sync(0xffffffffu, vv, q));
+#pragma unroll
+        for (int ch = 0; ch < 4; ++ch) { mx[ch] = -INFINITY; sm[ch] = 0.f; tw[ch] = 0.f; }
+        ++q;
+      };
+      if (npin > 0) {
+        int bnd = __shfl_sync(0xffffffffu, ptrs, 1);
+        for (int i = E0; i < E1; i += 8) {
+          if (i > E0) idx = (i + (lane & 7) < E1) ? __ldg(a.f_src + i + (lane & 7)) : 0;
+          float4 mv8[8];
+#pragma unroll
+          for (int u = 0; u < 8; ++u) {
+            const int src = __shfl_sync(0xffffffffu, idx, u);
+            mv8[u] = (i + u < E1) ? ldcg4(a.H + (int64_t)src * D + lane * 4) : f4zero();
+          }
+#pragma unroll
+          for (int u = 0; u < 8; ++u) {
+            if (i + u < E1) {
+              while (i + u >= bnd) { finish_pin(); bnd = __shfl_sync(0xffffffffu, ptrs, q + 1); }
+              const float mv[4] = {mv8[u].x, mv8[u].y, mv8[u].z, mv8[u].w};
+#pragma unroll
+              for (int ch = 0; ch < 4; ++ch) {
+                const float nm = fmaxf(mx[ch], mv[ch]);
+                const float sc = __expf(mx[ch] - nm);
+                const float ex = __expf(mv[ch] - nm);
+                sm[ch] = sm[ch] * sc + ex;
+                tw[ch] = tw[ch] * sc + mv[ch] * ex;
+                mx[ch] = nm;
+              }
+            }
+          }
+        }
+        while (q < npin) finish_pin();
+      }
+      for (int r = max(npin, 0); r < PPW; ++r) store_pin_row(smem, r0 + r, lane, f4zero(), -4, -1);
+
+      // MMA 1 and its epilogue: hidden = relu(W1 a + b1), stored unscaled
+      fence_async_smem();
+      tc_fence_before();
+      __syncthreads();
+      c.stamp(PH_GATHER);
+      if (tid == 0) {
+        tc_fence_after();
+        issue_gemm(sW, sW + W_PLANE, sB, sB + B_PLANE, c.tmem + TM_MAIN1, c.tmem + TM_CORR1, make_idesc(Fmt::F16, N), c.mbar);
+      }
+      mbar_wait_trap<MBAR_SPINS>(c.mbar, c.mphase);
+      c.mphase ^= 1u;
+      tc_fence_after();
+      c.stamp(PH_MMA1);
+#pragma unroll
+      for (int cc = 0; cc < NMAX / 4 / 8; ++cc) {
+        if (cc * 8 < nper) {
+          const int n0 = cg * nper + cc * 8;
+          float vm[8], vc[8];
+          tmem_ld8(tl + TM_MAIN1 + n0, vm);
+          tmem_ld8(tl + TM_CORR1 + n0, vc);
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const float hv = fmaxf(fmaf(vc[j], LO_INV, vm[j]) + b1m * c.scale_s[n0 + j], 0.f);
+            if (t0 + n0 + j < cnt) a.HIDb[(int64_t)(crow0 + t0 + n0 + j) * HID + c.rank * 128 + m] = hv * c.inv_s[n0 + j];
+          }
+        }
+      }
+      c.stamp(PH_EPI1);
+    }
+  }
+  ctx_teardown(c);
+}
+
 // ---------------------------------------------------------------------------------------------
 // host
 // ---------------------------------------------------------------------------------------------
@@ -1014,5 +1150,13 @@ int gnn_persist_backward(const tm_schedule* s, const float* H, float* G, const f
             A, LSE, HIDb, GA, GHID, GZC, ws_bar(ws), g_prof, lb, le};
   if (GHID) return launch_persist(gnn_persist_bwd_kernel<true>, a, st, "gnn_persist_bwd");
   return launch_persist(gnn_persist_bwd_kernel<false>, a, st, "gnn_persist_bwd");
+}
+
+int gnn_persist_save(const tm_schedule* s, const float* H, const float* W1t, const float* b1, const float* W2t, float* A,
+                     float* LSE, float* HIDb, void* ws, cudaStream_t st) {
+  TM_TRY(gnn_persist_begin(s, W1t, W2t, ws, st));
+  SaveArgs a{s->level_ptr, s->cell_base, s->order, s->f_ptr, s->f_src, H, ws_planes(ws), b1, A, LSE, HIDb, g_prof,
+             s->num_levels};
+  return launch_persist(gnn_persist_save_kernel, a, st, "gnn_persist_save");
 }
 }  // namespace tmk

@@ -705,6 +705,274 @@ extern "C" int tm_forward_cone(const tm_schedule* s, int64_t n_seeds, const int3
 }
 
 // ------------------------------------------------------------------------------------------
+// fan-in cone: the sub-schedule a backward pass seeded on some endpoints reads -- every scheduled pin from which a
+// seeded endpoint is reachable along the out-edges that carry gradient (bn_dst, and the cell out-edges bc_row), the
+// seeded endpoints included.  Every other pin's gradient is exactly zero in the full backward, so the edges into such
+// pins are dropped: no sum changes except possibly the sign of a zero.  Every in-edge source of a cone pin is in the
+// cone (the source's out-edge to it carries gradient), so the in-edge lists are copied unchanged.
+//
+// fwd_cone_kernel's loop run downwards: ONE block sweeps from the highest seeded level to level 0, and a position is in
+// the cone when its pin is a seeded endpoint or one of its carrying out-edges leads into the cone.  Destinations sit on
+// later levels, so a level depends only on the levels above it.  Pins are marked in the same bitmap; a cell out-edge
+// names its destination's compact cell row, so row_map[row] (-1 outside the cone) is both the membership test of that
+// destination and its cone row.
+// The cone is laid out from the END of the buffers (positions, edges and cell rows): each chunk of positions takes the
+// block just below what the chunks above it took, and the chunks of a level are visited from the top, so the layout is
+// the parent's order with ascending levels, and no second pass is needed.  The class lists (fc_cell_self /
+// fc_net_self rows of the self-MLP data gradients) start at index 0 in the sweep's (descending) order.
+// ------------------------------------------------------------------------------------------
+namespace {
+struct FaninArgs {
+  int n, L, T;
+  const int* level; const int* level_ptr; const int* cell_base; const int* order; const int* f_ptr; const int* f_src;
+  const int* bn_ptr; const int* bn_dst; const float* bn_w; const int* bc_ptr; const int* bc_row;
+  const int* endpoints; const float* seed;
+  uint32_t* gbits;                                 // NULL: the bitmap lives in dynamic shared memory
+  int* row_map;                                    // parent cell row -> cone cell row, -1 outside the cone
+  int* c_order; int* c_level_ptr; int* c_cell_base; int* c_f_ptr; int* c_f_src;
+  int* c_bn_ptr; int* c_bn_dst; float* c_bn_w; int* c_bc_ptr; int* c_bc_row;
+  int* c_cell_pins; int* c_net_pins; int* c_counts;
+};
+
+// exclusive block scan of four ints over CONE_T threads; tot receives the block totals.  The caller syncs before wsum
+// is reused.
+__device__ __forceinline__ void block_scan4(int (&x)[4], int (&tot)[4], int (*wsum)[32]) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int inc[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) inc[k] = x[k];
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int y = __shfl_up_sync(0xffffffffu, inc[k], o);
+      if (lane >= o) inc[k] += y;
+    }
+  }
+  if (lane == 31) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) wsum[k][warp] = inc[k];
+  }
+  __syncthreads();
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    int off = 0, t = 0;
+#pragma unroll 8
+    for (int w = 0; w < CONE_T / 32; ++w) {
+      const int xv = wsum[k][w];
+      if (w < warp) off += xv;
+      t += xv;
+    }
+    x[k] = off + inc[k] - x[k];
+    tot[k] = t;
+  }
+}
+
+__global__ void __launch_bounds__(CONE_T, 1) fanin_cone_kernel(const FaninArgs a) {
+  extern __shared__ uint32_t sbits[];
+  __shared__ int wsum[4][32];
+  __shared__ int s_lmax;
+  const int tid = threadIdx.x;
+  uint32_t* bits = a.gbits ? a.gbits : sbits;      // generic: shared or global
+  const volatile uint32_t* vbits = bits;
+  const volatile int* vrow = a.row_map;            // written by this block on the levels above
+  if (!a.gbits)
+    for (int i = tid; i < ((a.n + 31) >> 5); i += CONE_T) sbits[i] = 0u;
+  if (tid == 0) s_lmax = -1;
+  __syncthreads();
+  for (int t = tid; t < a.T; t += CONE_T) {
+    if (a.seed[t] == 0.f) continue;                // an unseeded endpoint: its gradient is exactly zero
+    const int v = a.endpoints[t];
+    if (v < 0 || v >= a.n) continue;
+    const int l = a.level[v];
+    if (l < 0 || l >= a.L) continue;               // outside the schedule: reads nothing
+    atomicOr(bits + (v >> 5), 1u << (v & 31));
+    atomicMax(&s_lmax, l);
+  }
+  __syncthreads();
+  const int lmax = s_lmax;
+  const int ns = __ldg(a.level_ptr + a.L);
+  int top = ns, ftop = __ldg(a.f_ptr + ns), ntop = __ldg(a.bn_ptr + ns), ctop = __ldg(a.bc_ptr + ns);
+  int rtop = __ldg(a.cell_base + a.L), ncell = 0, nnet = 0;   // block-uniform running totals
+  for (int l = lmax + 1 + tid; l <= a.L; l += CONE_T) {
+    a.c_level_ptr[l] = ns;
+    a.c_cell_base[l] = rtop;
+  }
+  if (tid == 0) {
+    a.c_f_ptr[ns] = ftop;
+    a.c_bn_ptr[ns] = ntop;
+    a.c_bc_ptr[ns] = ctop;
+  }
+  for (int l = lmax; l >= 0; --l) {
+    const int p0 = __ldg(a.level_ptr + l), p1 = __ldg(a.level_ptr + l + 1);
+    const bool cell_rows = l > 0 && !(l & 1);
+    const int crow0 = cell_rows ? __ldg(a.cell_base + l) : 0;
+    if (l > 0) {                                   // the next level's static arrays into L2
+      const int pm = __ldg(a.level_ptr + l - 1);
+      for (int i = pm + tid * 32; i < p0; i += CONE_T * 32) {
+        pf_l2(a.order + i);
+        pf_l2(a.bn_ptr + i);
+        pf_l2(a.bc_ptr + i);
+      }
+      for (int i = __ldg(a.bn_ptr + pm) + tid * 32; i < __ldg(a.bn_ptr + p0); i += CONE_T * 32) pf_l2(a.bn_dst + i);
+      for (int i = __ldg(a.bc_ptr + pm) + tid * 32; i < __ldg(a.bc_ptr + p0); i += CONE_T * 32) pf_l2(a.bc_row + i);
+    }
+    for (int c0 = p1 > p0 ? p0 + (p1 - p0 - 1) / CONE_CHUNK * CONE_CHUNK : p0 - 1; c0 >= p0; c0 -= CONE_CHUNK) {
+      const int q = c0 + tid * CONE_V;
+      const int nq = max(0, min(CONE_V, p1 - q));
+      int nptr[CONE_V + 1], cptr[CONE_V + 1], v[CONE_V];
+      bool in[CONE_V];
+      // pins, in-edges, net out-edges kept, cell out-edges kept; a pin outside the cone has no kept out-edge, so the
+      // kept edges are counted over all of the thread's positions
+      int x[4] = {0, 0, 0, 0}, tot[4];
+#pragma unroll
+      for (int j = 0; j <= CONE_V; ++j) {
+        nptr[j] = (j <= nq && nq > 0) ? __ldg(a.bn_ptr + q + j) : 0;
+        cptr[j] = (j <= nq && nq > 0) ? __ldg(a.bc_ptr + q + j) : 0;
+      }
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) {
+        v[j] = j < nq ? __ldg(a.order + q + j) : 0;
+        in[j] = false;
+      }
+      int ne1 = nptr[0], ce1 = cptr[0];            // ptr[nq] without a dynamic register index
+#pragma unroll
+      for (int j = 1; j <= CONE_V; ++j) {
+        ne1 = j == nq ? nptr[j] : ne1;
+        ce1 = j == nq ? cptr[j] : ce1;
+      }
+      for (int e = nptr[0]; e < ne1; e += 8) {     // net out-edges into the cone
+        int dst[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) dst[u] = e + u < ne1 ? __ldg(a.bn_dst + e + u) : -1;
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          if (dst[u] >= 0 && cone_bit(vbits, dst[u])) {
+            ++x[2];
+#pragma unroll
+            for (int j = 0; j < CONE_V; ++j) in[j] |= (e + u >= nptr[j] && e + u < nptr[j + 1]);
+          }
+        }
+      }
+      for (int e = cptr[0]; e < ce1; e += 8) {     // cell out-edges into the cone
+        int row[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) row[u] = e + u < ce1 ? __ldg(a.bc_row + e + u) : -1;
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          if (row[u] >= 0 && vrow[row[u]] >= 0) {
+            ++x[3];
+#pragma unroll
+            for (int j = 0; j < CONE_V; ++j) in[j] |= (e + u >= cptr[j] && e + u < cptr[j + 1]);
+          }
+        }
+      }
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) {
+        in[j] = j < nq && (in[j] || cone_bit(vbits, v[j]));
+        if (in[j]) {
+          ++x[0];
+          x[1] += __ldg(a.f_ptr + q + j + 1) - __ldg(a.f_ptr + q + j);
+        }
+      }
+      block_scan4(x, tot, wsum);
+      int rank = x[0];                             // cone pins of this chunk before this thread's first
+      int pos = top - tot[0] + x[0], fo = ftop - tot[1] + x[1], no = ntop - tot[2] + x[2], co = ctop - tot[3] + x[3];
+#pragma unroll
+      for (int j = 0; j < CONE_V; ++j) {
+        if (in[j]) {
+          a.c_order[pos] = v[j];
+          a.c_f_ptr[pos] = fo;
+          for (int e = __ldg(a.f_ptr + q + j); e < __ldg(a.f_ptr + q + j + 1); ++e) a.c_f_src[fo++] = __ldg(a.f_src + e);
+          a.c_bn_ptr[pos] = no;
+          for (int e = nptr[j]; e < nptr[j + 1]; ++e) {
+            const int u = __ldg(a.bn_dst + e);
+            if (cone_bit(vbits, u)) {
+              a.c_bn_dst[no] = u;
+              a.c_bn_w[no] = __ldg(a.bn_w + e);
+              ++no;
+            }
+          }
+          a.c_bc_ptr[pos] = co;
+          for (int e = cptr[j]; e < cptr[j + 1]; ++e) {
+            const int r = vrow[__ldg(a.bc_row + e)];
+            if (r >= 0) a.c_bc_row[co++] = r;
+          }
+          if (cell_rows) a.row_map[crow0 + (q + j - p0)] = rtop - tot[0] + rank;
+          if (l & 1) a.c_net_pins[nnet + tot[0] - 1 - rank] = v[j];
+          else a.c_cell_pins[ncell + tot[0] - 1 - rank] = v[j];
+          atomicOr(bits + (v[j] >> 5), 1u << (v[j] & 31));
+          ++pos;
+          ++rank;
+        }
+      }
+      top -= tot[0];
+      ftop -= tot[1];
+      ntop -= tot[2];
+      ctop -= tot[3];
+      if (cell_rows) rtop -= tot[0];
+      if (l & 1) nnet += tot[0];
+      else ncell += tot[0];
+      __syncthreads();                             // bits / row_map of this chunk are set; wsum may be reused
+    }
+    if (tid == 0) {
+      a.c_level_ptr[l] = top;
+      a.c_cell_base[l] = rtop;
+    }
+  }
+  if (tid == 0) {
+    a.c_counts[0] = ns - top;
+    a.c_counts[1] = ncell;
+    a.c_counts[2] = nnet;
+  }
+}
+
+size_t fanin_bits_bytes(int64_t n) { return ((size_t)cdiv(n, 32) * sizeof(uint32_t) + 255) & ~(size_t)255; }
+}  // namespace
+
+extern "C" size_t tm_fanin_cone_ws(int64_t n, int32_t n_cell_rows) {
+  return fanin_bits_bytes(n) + (size_t)(n_cell_rows > 0 ? n_cell_rows : 0) * sizeof(int) + 256;
+}
+
+extern "C" int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints, const float* seed,
+                             int32_t* order, int32_t* level_ptr, int32_t* cell_base, int32_t* f_ptr, int32_t* f_src,
+                             int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr, int32_t* bc_row,
+                             int32_t* cell_pins, int32_t* net_pins, int32_t* counts, void* ws, size_t ws_bytes,
+                             void* stream) {
+  TM_REQUIRE(s && s->order && s->level && s->level_ptr && s->cell_base && s->f_ptr && s->f_src && s->bn_ptr &&
+                 s->bn_dst && s->bn_w && s->bc_ptr && s->bc_row,
+             "tm_fanin_cone: the parent schedule lacks its device arrays (order, level, level_ptr, cell_base, f_ptr, "
+             "f_src, bn_ptr, bn_dst, bn_w, bc_ptr, bc_row)");
+  TM_REQUIRE(s->n > 0 && s->n < INT32_MAX && s->num_levels > 0 && s->n_cell_rows >= 0,
+             "tm_fanin_cone: bad schedule sizes");
+  TM_REQUIRE(n_endpoints >= 0 && n_endpoints < INT32_MAX && (n_endpoints == 0 || (endpoints && seed)),
+             "tm_fanin_cone: bad endpoint list or seed");
+  TM_REQUIRE(order && level_ptr && cell_base && f_ptr && f_src && bn_ptr && bn_dst && bn_w && bc_ptr && bc_row &&
+                 cell_pins && net_pins && counts,
+             "tm_fanin_cone: NULL output buffer");
+  TM_REQUIRE(ws && ws_bytes >= tm_fanin_cone_ws(s->n, s->n_cell_rows),
+             "tm_fanin_cone: workspace too small (tm_fanin_cone_ws)");
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t bit_bytes = (size_t)cdiv(s->n, 32) * sizeof(uint32_t);
+  const bool in_smem = bit_bytes <= CONE_SMEM_MAX;
+  uint8_t* p = reinterpret_cast<uint8_t*>(ws);
+  uint32_t* gbits = nullptr;
+  if (!in_smem) {
+    gbits = reinterpret_cast<uint32_t*>(p);
+    TM_CUDA(cudaMemsetAsync(gbits, 0, bit_bytes, st));
+  }
+  int* row_map = reinterpret_cast<int*>(p + fanin_bits_bytes(s->n));
+  if (s->n_cell_rows > 0) TM_CUDA(cudaMemsetAsync(row_map, 0xff, (size_t)s->n_cell_rows * sizeof(int), st));
+  TM_CUDA(cudaFuncSetAttribute(fanin_cone_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CONE_SMEM_MAX));
+  FaninArgs a{(int)s->n, s->num_levels, (int)n_endpoints, s->level, s->level_ptr, s->cell_base, s->order, s->f_ptr,
+              s->f_src, s->bn_ptr, s->bn_dst, s->bn_w, s->bc_ptr, s->bc_row, endpoints, seed, gbits, row_map,
+              order, level_ptr, cell_base, f_ptr, f_src, bn_ptr, bn_dst, bn_w, bc_ptr, bc_row, cell_pins, net_pins,
+              counts};
+  fanin_cone_kernel<<<1, CONE_T, in_smem ? bit_bytes : 0, st>>>(a);
+  return check_launch("fanin_cone");
+}
+
+// ------------------------------------------------------------------------------------------
 // forward cones of K candidate edits, joined into one sub-schedule over private virtual rows
 // (what-if evaluation: score many alternative edits of one design in one propagation).
 //

@@ -668,6 +668,7 @@ struct B1Args {
   // forward read (x_rows)
   float* dX;
   int64_t lddx;
+  const int* m_dev;       // DEVM: device row count; M is then the capacity the grid was sized for
 };
 
 // STORE == false: first-layer gradients of the generated MLP (above); DX adds the data gradient dX = dh W1, two FMAs per
@@ -675,8 +676,10 @@ struct B1Args {
 // gradients and leaves dX the same bits.  STORE == true: the same product with the epilogue of the general MLP
 // backward -- dh = (G W2) * (H > 0) written to DH (fc_cell_self: 36 inputs, the hidden layer is stored); with DX, dh is
 // not written but multiplied into dX = dh W1 (kx <= 48 inputs) in the lane that owns the row, in hidden-unit order.
-template <bool STORE, bool DX, bool WG = true>
+// DEVM: the row count is *m_dev (at most M), read on the device; CTAs past it have no tile.
+template <bool STORE, bool DX, bool WG = true, bool DEVM = false>
 __global__ void __launch_bounds__(THREADS, 1) selfmlp_gen_bwd1_kernel(B1Args a) {
+  if constexpr (DEVM) a.M = max((int64_t)0, min(a.M, (int64_t)*a.m_dev));
   extern __shared__ __align__(1024) uint8_t smem[];
   float* w0_s = reinterpret_cast<float*>(smem + B1_OFF_P);
   float* w1_s = w0_s + HIDF;
@@ -1014,9 +1017,13 @@ struct L1Args {
   float* out;
   int64_t ldo;
   float* rowmax;          // optional: max over the row's 256 outputs (the scale of tm_selfmlp_rows_forward)
+  const int* m_dev;       // DEVM: device row count; M is then the capacity the grid was sized for
 };
 
+// DEVM: the row count is *m_dev (at most M), read on the device; CTAs past it have no tile.
+template <bool DEVM = false>
 __global__ void __launch_bounds__(THREADS, 1) selfmlp_lin1_kernel(L1Args a) {
+  if constexpr (DEVM) a.M = max((int64_t)0, min(a.M, (int64_t)*a.m_dev));
   extern __shared__ __align__(1024) uint8_t smem[];
   float* b1_s = reinterpret_cast<float*>(smem + L1_OFF_B);
   float* inv_s = reinterpret_cast<float*>(smem + L1_OFF_INV);
@@ -1340,11 +1347,11 @@ extern "C" int tm_selfmlp_lin1_relu(int64_t M, const float* X, int64_t ldx, cons
   uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
   selfmlp_pack_w1_kernel<<<(HIDF * L1_K + 255) / 256, 256, 0, st>>>(W1, (int)kin, planes);
   TM_TRY(check_launch("selfmlp_pack_w1"));
-  TM_CUDA(cudaFuncSetAttribute(selfmlp_lin1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L1_SMEM + 1024));
+  TM_CUDA(cudaFuncSetAttribute(selfmlp_lin1_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L1_SMEM + 1024));
   const int64_t ntiles = (M + TM - 1) / TM;
   const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
   L1Args a{M, X, ldx, x_rows, (int)kin, b1, planes, HID, ldh, rowmax};
-  selfmlp_lin1_kernel<<<grid, THREADS, L1_SMEM + 1024, st>>>(a);
+  selfmlp_lin1_kernel<false><<<grid, THREADS, L1_SMEM + 1024, st>>>(a);
   return check_launch("selfmlp_lin1");
 }
 
@@ -1368,4 +1375,77 @@ extern "C" int tm_selfmlp_rows_forward(int64_t M, const float* H, int64_t ldh, c
   const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
   selfmlp_gen_fwd_kernel<true><<<grid, THREADS, SMEM_BYTES + 1024, st>>>(a);
   return check_launch("selfmlp_rows_fwd");
+}
+
+// ------------------------------------------------------------------------------------------
+// The same data-gradient products over a row count that exists only on the device (*m_dev, at most `cap`): the grid is
+// sized by the capacity and the kernels read the count (a fan-in cone's class lists, tm_fanin_cone).  Each is its own
+// template instance, so the entry points above compile as before.
+// ------------------------------------------------------------------------------------------
+extern "C" int tm_selfmlp_lin1_relu_dcount(int64_t cap, const int32_t* m_dev, const float* X, int64_t ldx,
+                                           const int32_t* x_rows, int64_t kin, const float* W1, const float* b1, float* HID,
+                                           int64_t ldh, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(m_dev && X && x_rows && W1 && b1 && HID, "tm_selfmlp_lin1_relu_dcount: NULL operand");
+  TM_REQUIRE(kin > 0 && kin <= L1_K && (kin & 3) == 0, "tm_selfmlp_lin1_relu_dcount: kin must be a multiple of 4, <= 48");
+  TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_lin1_ws_bytes(), "tm_selfmlp_lin1_relu_dcount: workspace too small (tm_selfmlp_lin1_ws_bytes)");
+  TM_REQUIRE((ldx & 3) == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0 && (ldh & 3) == 0 && (reinterpret_cast<uintptr_t>(HID) & 15) == 0,
+             "tm_selfmlp_lin1_relu_dcount: X and HID rows must be 16-byte aligned");
+  if (cap <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  selfmlp_pack_w1_kernel<<<(HIDF * L1_K + 255) / 256, 256, 0, st>>>(W1, (int)kin, planes);
+  TM_TRY(check_launch("selfmlp_pack_w1"));
+  TM_CUDA(cudaFuncSetAttribute(selfmlp_lin1_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L1_SMEM + 1024));
+  const int64_t ntiles = (cap + TM - 1) / TM;
+  const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
+  L1Args a{cap, X, ldx, x_rows, (int)kin, b1, planes, HID, ldh, nullptr, m_dev};
+  selfmlp_lin1_kernel<true><<<grid, THREADS, L1_SMEM + 1024, st>>>(a);
+  return check_launch("selfmlp_lin1(device count)");
+}
+
+extern "C" int tm_selfmlp_rows_dx_dcount(int64_t cap, const int32_t* m_dev, const float* G, int64_t ldg,
+                                         const int32_t* g_rows, const float* W2, const float* H, int64_t ldh,
+                                         const int32_t* h_rows, const float* W1, int64_t kin, float* dX, int64_t lddx,
+                                         const int32_t* x_rows, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(m_dev && G && W2 && H && W1 && dX, "tm_selfmlp_rows_dx_dcount: NULL operand");
+  TM_REQUIRE(kin > 0 && kin <= 48 && (kin & 3) == 0, "tm_selfmlp_rows_dx_dcount: kin must be a multiple of 4, <= 48");
+  TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_rows_dh_ws_bytes(), "tm_selfmlp_rows_dx_dcount: workspace too small (tm_selfmlp_rows_dh_ws_bytes)");
+  TM_REQUIRE((ldg & 3) == 0 && (reinterpret_cast<uintptr_t>(G) & 15) == 0 && (ldh & 3) == 0 && (reinterpret_cast<uintptr_t>(H) & 15) == 0 &&
+                 (lddx & 3) == 0 && lddx >= kin && (reinterpret_cast<uintptr_t>(dX) & 15) == 0 && (reinterpret_cast<uintptr_t>(W1) & 15) == 0,
+             "tm_selfmlp_rows_dx_dcount: G, H, W1 and dX rows must be 16-byte aligned (lddx >= kin)");
+  if (cap <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  selfmlp_pack_t_kernel<<<(NOUT * HIDF + 255) / 256, 256, 0, st>>>(W2, planes);
+  TM_TRY(check_launch("selfmlp_pack_t"));
+  TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+  const int64_t ntiles = (cap + TM - 1) / TM;
+  const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
+  B1Args a{cap, G, ldg, g_rows, nullptr, 0, x_rows, (int)kin, W1, nullptr, planes, nullptr, H, ldh, h_rows, nullptr, 0, dX, lddx,
+           m_dev};
+  selfmlp_gen_bwd1_kernel<true, true, false, true><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+  return check_launch("selfmlp_rows_dx(device count)");
+}
+
+extern "C" int tm_selfmlp_gen_bwd1_dx_dcount(int64_t cap, const int32_t* m_dev, const float* G, int64_t ldg,
+                                             const int32_t* g_rows, const float* X, int64_t ldx, const int32_t* x_rows,
+                                             int64_t kx, const float* W1, const float* b1, const float* W2, float* dX,
+                                             int64_t lddx, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(m_dev && G && X && W1 && b1 && W2 && dX, "tm_selfmlp_gen_bwd1_dx_dcount: NULL operand");
+  TM_REQUIRE(kx == 1 || kx == 2, "tm_selfmlp_gen_bwd1_dx_dcount: the first layer must have 1 or 2 inputs");
+  TM_REQUIRE(lddx >= kx, "tm_selfmlp_gen_bwd1_dx_dcount: dX row stride lddx < kx");
+  TM_REQUIRE(ws && ws_bytes >= tm_selfmlp_bwd1_ws_bytes(), "tm_selfmlp_gen_bwd1_dx_dcount: workspace too small (tm_selfmlp_bwd1_ws_bytes)");
+  TM_REQUIRE((ldg & 3) == 0 && (reinterpret_cast<uintptr_t>(G) & 15) == 0, "tm_selfmlp_gen_bwd1_dx_dcount: G rows must be 16-byte aligned");
+  if (cap <= 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* planes = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
+  selfmlp_pack_t_kernel<<<(NOUT * HIDF + 255) / 256, 256, 0, st>>>(W2, planes);
+  TM_TRY(check_launch("selfmlp_pack_t"));
+  TM_CUDA(cudaFuncSetAttribute(selfmlp_gen_bwd1_kernel<false, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B1_SMEM + 1024));
+  const int64_t ntiles = (cap + TM - 1) / TM;
+  const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
+  B1Args a{cap, G, ldg, g_rows, X, ldx, x_rows, (int)kx, W1, b1, planes, nullptr, nullptr, 0, nullptr, nullptr, 0, dX, lddx,
+           m_dev};
+  selfmlp_gen_bwd1_kernel<false, true, false, true><<<grid, THREADS, B1_SMEM + 1024, st>>>(a);
+  return check_launch("selfmlp_gen_bwd1_dx(device count)");
 }

@@ -21,7 +21,7 @@ import tm_dp
 import tm_lib
 import tm_ops
 import tm_unet
-from tm_graph import ConeGraph, ForwardCone, ForwardCones, MaskCSR, TimingGraph
+from tm_graph import ConeGraph, FaninCone, ForwardCone, ForwardCones, MaskCSR, TimingGraph
 from tm_lib import call, stream
 from tm_ops import D, RELU, gemm_nn, gemm_tn, transpose
 
@@ -391,8 +391,9 @@ class DesignStep:
                                  a2.bias.detach(), X[:, 2 * D:], width)
         return dict(X=X, wt=wt, ha=ha, lv=lv, width=width, tab=tab)
 
-    def _head_netlist_side(self, H, b, hs, endpoints=None, out=None):
-        """Endpoint rows of H into columns 0..D of X, then ``mlp_fuse`` (into ``out`` when given)."""
+    def _head_netlist_side(self, H, b, hs, endpoints=None, out=None, hf_out=None):
+        """Endpoint rows of H into columns 0..D of X, then ``mlp_fuse`` (into ``out`` when given; its hidden rows into
+        ``hf_out`` when given)."""
         m = self.model
         T = int(b.endpoints.numel())
         X, width = hs["X"], hs["width"]
@@ -400,7 +401,7 @@ class DesignStep:
         f0, f2 = m.mlp_fuse.layers[0], m.mlp_fuse.layers[2]
         pred = out if out is not None else torch.empty(T, f2.weight.shape[0], dtype=torch.float32, device=H.device)
         hs["hf"] = tm_ops.mlp2_forward(X, width, None, T, f0.weight.detach(), f0.bias.detach(), f2.weight.detach(),
-                                       f2.bias.detach(), pred, pred.shape[1])
+                                       f2.bias.detach(), pred, pred.shape[1], h_out=hf_out)
         return pred
 
     def _head_forward(self, H, b, feat):
@@ -769,6 +770,7 @@ class IncrementalEvaluation:
         replay = inc.capture_update(pins)    # one CUDA graph for a fixed pin set: edit rows in place, replay() -> pred
         inc.refresh()                        # full recompute, after a parameter or image change
         inc.cone_size()                      # pins re-propagated by the last update (one device read)
+        g = inc.input_grads(seed)            # d(seed . pred)/d features through the seeded endpoints' fan-in cone
 
     Predictions: ``pred`` (T,) and ``H`` (n, 128) are rewritten in place.  After any sequence of updates they are the
     same bits as ``step.forward(batch)`` and ``tm_ops.gnn_forward`` on the persistent back end over the edited
@@ -820,11 +822,14 @@ class IncrementalEvaluation:
         self._overlay = None                              # the WhatIf whose candidates the rows n.. hold
         self._max_in_degree = None
         self.X = torch.empty(T, D + D + step.model.global_dim, dtype=torch.float32, device=dev)
-        f2 = step.model.mlp_fuse.layers[2]
+        f0, f2 = step.model.mlp_fuse.layers[0], step.model.mlp_fuse.layers[2]
         self._pred2 = torch.empty(T, f2.weight.shape[0], dtype=torch.float32, device=dev)
+        # the head's hidden rows live as long as inc: captured updates and gradients read and write this one buffer
+        self._hf = torch.empty(T, f0.weight.shape[0], dtype=torch.float32, device=dev)
         self.pred = self._pred2.squeeze(-1)
         self.cone = ForwardCone(b.graph)
         self._last = None                                 # None: full pass; 0: empty update; "cone": the cone's count
+        self._grad = None                                 # input_grads' cone, scratch and results (first call)
         self.refresh()
 
     def _params(self):
@@ -841,7 +846,7 @@ class IncrementalEvaluation:
         tm_ops.gnn_self_terms(self.S, b.cell_feat, b.net_feat, gp, sched.cell_class, sched.net_class)
         self.H.zero_()
         tm_ops.gnn_forward_cone(sched, self.H, self.S, gp)
-        st._head_netlist_side(self.H, b, self._hs, out=self._pred2)
+        st._head_netlist_side(self.H, b, self._hs, out=self._pred2, hf_out=self._hf)
         self._last = None
         self.generation += 1
         return self.pred
@@ -880,7 +885,7 @@ class IncrementalEvaluation:
         tm_ops.gnn_self_terms(self.S, self.b.cell_feat, self.b.net_feat, gp, idx[:nc], idx[nc:])
         self.cone.build(idx)
         tm_ops.gnn_forward_cone(self.cone, self.H, self.S, gp)
-        self.step._head_netlist_side(self.H, self.b, self._hs, out=self._pred2)
+        self.step._head_netlist_side(self.H, self.b, self._hs, out=self._pred2, hf_out=self._hf)
         return self.pred
 
     def update(self, pins):
@@ -928,6 +933,89 @@ class IncrementalEvaluation:
             return int(self._last[1].cone_sizes()[self._last[2]])
         return self.cone.size()
 
+    # ---------------------------------------------------------------- input gradients
+    def _check_seed(self, seed, what):
+        T, dev = int(self.b.endpoints.numel()), self.b.endpoints.device
+        if (not torch.is_tensor(seed) or seed.shape != (T,) or seed.dtype != torch.float32 or not seed.is_contiguous()
+                or seed.device != dev):
+            got = (f"{seed.dtype} {tuple(seed.shape)} on {seed.device}" if torch.is_tensor(seed) else type(seed).__name__)
+            raise ValueError(f"IncrementalEvaluation.{what}: seed must be a contiguous float32 ({T},) tensor on {dev}, "
+                             f"got {got}")
+
+    def _grad_state(self):
+        if self._grad is None:
+            b, dev = self.b, self.H.device
+            self._grad = dict(cone=FaninCone(b.graph), G=torch.empty(self.n, D, dtype=torch.float32, device=dev),
+                              scratch=tm_ops.gnn_cone_scratch(self.sched, dev),
+                              out={"cell_feat": torch.empty(b.cell_feat.shape, dtype=torch.float32, device=dev),
+                                   "net_feat": torch.empty(b.net_feat.shape, dtype=torch.float32, device=dev)})
+        return self._grad
+
+    def _grad_launch(self, seed, mark=None):
+        gs, b, st = self._grad_state(), self.b, self.step
+        T, width = int(b.endpoints.numel()), self.X.shape[1]
+        cone, G, out = gs["cone"], gs["G"], gs["out"]
+        cone.build(b.endpoints, seed)
+        if mark:
+            mark("cone")
+        f0, f2 = st.model.mlp_fuse.layers[0], st.model.mlp_fuse.layers[2]
+        dX = tm_ops.mlp2_backward(self.X, width, None, T, f0.weight.detach(), f2.weight.detach(), self._hf,
+                                  seed.reshape(T, 1), 1, need_dx=True, need_wgrad=False)[4]
+        if mark:
+            mark("head")
+        # all of G is zeroed (one memset) rather than the cone's rows: the cone's size is known only on the device
+        G.zero_()
+        call("tm_scatter_add_cols", T, D, dX, width, 0, b.endpoints, G, D, stream())
+        out["cell_feat"].zero_()
+        out["net_feat"].zero_()
+        if mark:
+            mark("zero_scatter")
+        tm_ops.gnn_backward_cone(cone, self.H, G, self._params(), b.cell_feat, b.net_feat, out["cell_feat"],
+                                 out["net_feat"], gs["scratch"], mark=mark)
+        return out
+
+    def input_grads(self, seed):
+        """The gradient of ``sum_t seed[t] * pred[t]`` with respect to the batch's ``cell_feat`` and ``net_feat`` at the
+        current state (after every ``update``, replayed ``capture_update`` and ``WhatIf.commit``), backpropagated
+        through only the fan-in cone of the endpoints whose seed is non-zero.  ``seed``: contiguous float32 (T,) on the
+        batch's device, dObjective/dpred, taken as given as ``run(..., pred_grad=seed)`` takes it.  Returns the dict
+        {"cell_feat", "net_feat"}, shaped like the features and rewritten by every call.  Rows outside the cone are
+        exactly zero, and so are the rows the propagation never reads (net-class pins in "cell_feat", cell-class pins in
+        "net_feat", unscheduled pins), as in ``batch.input_grads``.
+
+        There is no image gradient: the image branch is frozen inside this object (use the frozen step,
+        ``step.run(batch, input_grads=True, pred_grad=seed, param_grads=False)``, for it).  Device work only, no host
+        synchronisation: the head's data gradient over the T endpoints (``mlp_fuse`` from X and its hidden rows), the
+        cone build (``tm_fanin_cone``), A / LSE / HID of the cone's cell pins recomputed from ``H``, the persistent
+        backward sweep over the cone, and the self-MLP data gradients of the cone's pins.  The rows are the same bits
+        as the persistent full backward's (``tm_ops.gnn_backward(..., need_dx=True, need_wgrad=False)`` after
+        ``gnn_forward`` on the persistent back end).  Nothing the committed state owns is written (``H``, ``S``,
+        ``pred``, ``X``, the batch, what-if rows, parameters, buffers, ``.grad``), no collective runs and
+        ``generation`` is unchanged.  Needs the tf32x3 arithmetic (``TM_MATH``), whose self-MLP kernels take a device
+        row count.  Memory, on the first call: G (n x 512 bytes), four buffers per cell row (2.5 KB; the fc_cell_self
+        hidden rows reuse one of them), the cone's buffers (the size of the schedule) and the two results."""
+        self._check_seed(seed, "input_grads")
+        return self._grad_launch(seed)
+
+    def capture_input_grads(self, seed, pool=None):
+        """``input_grads(seed)`` captured as one CUDA graph (run once eagerly first), with ``seed`` a static input.
+        Returns ``replay() -> {"cell_feat", "net_feat"}``: edit ``seed`` in place -- other endpoints may be seeded,
+        the cone is rebuilt on the device -- and the features / updates as usual, then replay."""
+        self._check_seed(seed, "capture_input_grads")
+        self._grad_state()              # allocated outside the graph's pool
+        inner = self.step._capture_local(lambda: self._grad_launch(seed), warmup=1, pool=pool)
+
+        def replay():
+            inner()
+            return self._grad["out"]
+        replay.graph = inner.graph
+        replay.seed = seed              # the graph reads this tensor: it lives as long as the replay
+        return replay
+
+    def grad_cone_size(self):
+        """Pins of the last ``input_grads`` cone (one device read, diagnostics); 0 before the first call."""
+        return self._grad["cone"].size() if self._grad is not None else 0
+
     def what_if(self, pin_sets):
         """A ``WhatIf`` over the candidate edits ``pin_sets`` (a sequence of K pin sequences, validated as ``update``
         validates its pins).  Needs ``what_if_rows`` > 0 at construction."""
@@ -969,8 +1057,9 @@ class WhatIf:
     result is NaN and ``fitted()`` False.  Memory beyond ``inc``'s rows: two n/8-byte bitmaps per candidate, the joined
     schedule's arrays (sized by ``what_if_rows``), and the (K x T, 288) head matrix.
 
-    ``commit(k)`` propagates nothing: it copies candidate k's virtual H / S rows back to their pins, its feature rows
-    into the batch and its predictions into ``inc.pred`` -- the state ``inc.update`` leaves.  It raises ``ValueError``
+    ``commit(k)`` propagates nothing: it copies candidate k's virtual H / S rows back to their pins and its feature rows
+    into the batch, then reruns the head over the committed H (``inc.pred`` gets candidate k's predictions, the same
+    bits, and ``inc.X`` / the head's hidden rows follow) -- the state ``inc.update`` leaves.  It raises ``ValueError``
     when the base changed since this object's last run / replay, when another ``WhatIf`` of ``inc`` ran since, or when
     candidate k was not admitted."""
 
@@ -1066,8 +1155,8 @@ class WhatIf:
         return replay
 
     def commit(self, k):
-        """Apply candidate k: the batch's feature rows, ``inc.H``, ``inc.S`` and ``inc.pred`` as ``inc.update`` leaves
-        them, without a propagation."""
+        """Apply candidate k: the batch's feature rows, ``inc.H``, ``inc.S``, ``inc.pred`` and the head's inputs as
+        ``inc.update`` leaves them, without a propagation."""
         inc = self.inc
         if self._gen is None or self._gen != inc.generation or inc._overlay is not self:
             raise ValueError("WhatIf.commit: the base changed (or another what-if ran) since this object's last run / "
@@ -1082,7 +1171,8 @@ class WhatIf:
         if e > s:
             inc.b.cell_feat.index_copy_(0, self._pin_idx[s:e], self.cell_feat[s:e])
             inc.b.net_feat.index_copy_(0, self._pin_idx[s:e], self.net_feat[s:e])
-        inc._pred2.copy_(self._pred2[k * self.T:(k + 1) * self.T])
+        # the head over the committed H: candidate k's predictions (the same bits) and the head's X / hidden rows
+        inc.step._head_netlist_side(inc.H, inc.b, inc._hs, out=inc._pred2, hf_out=inc._hf)
         inc.generation += 1
         inc._last = ("what_if", self, int(k))
 

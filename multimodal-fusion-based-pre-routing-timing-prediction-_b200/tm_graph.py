@@ -330,6 +330,66 @@ class ForwardCone:
         return int(self.count.item())
 
 
+class FaninCone:
+    """The fan-in cone of the endpoints a backward pass is seeded on, as a device-side sub-schedule of
+    ``graph.schedule()``: every scheduled pin from which an endpoint with a non-zero seed is reachable along the out-edges
+    the backward reads, those endpoints included -- the pins whose gradient can be non-zero.  ``build(endpoints, seed)``
+    enqueues ``tm_fanin_cone``, which reads both on the device (no host synchronisation, so it can be captured with the
+    seed as a static input), and returns ``.struct``: the sub-schedule ``tm_gnn_save_cone`` / ``tm_gnn_backward_cone``
+    run over, laid out at the end of the buffers (see the header), with the backward edge lists filtered to the cone and
+    cone cell rows.  ``cell_pins`` / ``net_pins`` list the cone's pins on even / odd levels (the rows of the two
+    self-term MLPs), ``counts`` (device int32 [3]) the cone's pins and the two lists' lengths.  The buffers are
+    allocated once, sized by the parent schedule, and rewritten by every build.
+
+    Not ``BackwardCone``: that one is built on the host for the weight-gradient contractions of a training step."""
+
+    def __init__(self, graph):
+        s = self.sched = graph.schedule()
+        dev = s.device
+        i32 = lambda k: torch.empty(max(int(k), 1), dtype=torch.int32, device=dev)      # noqa: E731
+        self.order = i32(s.n_sched)
+        self.level_ptr = i32(s.num_levels + 1)
+        self.cell_base = i32(s.num_levels + 1)
+        self.f_ptr, self.f_src = i32(s.n_sched + 1), i32(s.f_src.numel())
+        self.bn_ptr, self.bn_dst = i32(s.n_sched + 1), i32(s.bn_dst.numel())
+        self.bn_w = torch.empty(max(int(s.bn_w.numel()), 1), dtype=torch.float32, device=dev)
+        self.bc_ptr, self.bc_row = i32(s.n_sched + 1), i32(s.bc_row.numel())
+        self.n_cell_cap, self.n_net_cap = int(s.cell_class.numel()), int(s.net_class.numel())
+        self.cell_pins, self.net_pins = i32(self.n_cell_cap), i32(self.n_net_cap)
+        self.counts = torch.zeros(3, dtype=torch.int32, device=dev)
+        self.nb = tm_lib.ws_bytes("tm_fanin_cone_ws", s.n, s.n_cell_rows)
+        self.ws = tm_lib.workspace(self.nb, dev)
+        p = s.struct
+        self.struct = tm_lib.tm_schedule(
+            n=s.n, num_levels=s.num_levels, n_cell_rows=s.n_cell_rows, h_level_ptr=None,
+            order=self.order.data_ptr(), level=p.level, crow=None,
+            net_iptr=p.net_iptr, net_isrc=p.net_isrc, cell_iptr=p.cell_iptr, cell_isrc=p.cell_isrc,
+            net_optr=p.net_optr, net_odst=p.net_odst, cell_optr=p.cell_optr, cell_odst=p.cell_odst,
+            f_ptr=self.f_ptr.data_ptr(), f_src=self.f_src.data_ptr(),
+            bn_ptr=self.bn_ptr.data_ptr(), bn_dst=self.bn_dst.data_ptr(), bn_w=self.bn_w.data_ptr(),
+            bc_ptr=self.bc_ptr.data_ptr(), bc_row=self.bc_row.data_ptr(),
+            level_ptr=self.level_ptr.data_ptr(), cell_base=self.cell_base.data_ptr())
+
+    def build(self, endpoints, seed):
+        """Enqueue the cone of the ``endpoints`` (int32 pin ids on the device) whose ``seed`` (float32, as long) is
+        non-zero, on the current stream.  Returns ``.struct``."""
+        dev = self.sched.device
+        if not (torch.is_tensor(endpoints) and endpoints.dtype == torch.int32 and endpoints.device == dev
+                and torch.is_tensor(seed) and seed.dtype == torch.float32 and seed.device == dev
+                and seed.shape == endpoints.shape and endpoints.is_contiguous() and seed.is_contiguous()):
+            raise ValueError(f"FaninCone.build: endpoints (int32) and seed (float32) must be contiguous tensors of one "
+                             f"shape on {dev}")
+        tm_lib.call("tm_fanin_cone", self.sched.struct, int(endpoints.numel()), endpoints, seed, self.order,
+                    self.level_ptr, self.cell_base, self.f_ptr, self.f_src, self.bn_ptr, self.bn_dst, self.bn_w,
+                    self.bc_ptr, self.bc_row, self.cell_pins, self.net_pins, self.counts, self.ws, self.nb,
+                    tm_lib.stream())
+        return self.struct
+
+    def size(self):
+        """Pins in the last built cone (one device read: diagnostics only)."""
+        return int(self.counts[0].item())
+
+
 class ForwardCones:
     """The forward cones of ``n_cand`` candidate edits of one design, joined into one device-side sub-schedule over
     private virtual rows (``tm_forward_cones``): candidate k's cone pins get the rows ``n + row_base[k] + rank`` of

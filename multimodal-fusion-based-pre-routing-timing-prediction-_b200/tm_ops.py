@@ -199,10 +199,11 @@ def mlp2_route(n_rows, kin, hid, nout, math=None, x_aligned=True, out_aligned=Tr
     return dict(hidden="stored", lin1=lin1, lin2=lin2, dw2="gemm", dh=dh, dw1="gemm", dx="gemm", dx_only=dx_only)
 
 
-def mlp2_forward(x, ldx, rows, n_rows, w1, b1, w2, b2, out, ldo, out_rows=None):
+def mlp2_forward(x, ldx, rows, n_rows, w1, b1, w2, b2, out, ldo, out_rows=None, h_out=None):
     """x rows (optionally gathered by ``rows``) -> out rows (optionally scattered by ``out_rows``), on the kernels
     ``mlp2_route`` names.  Returns the hidden activations (n_rows, hid) needed by ``mlp2_backward``, or None when the
-    route generates them."""
+    route generates them.  ``h_out``: a contiguous (n_rows, hid) float32 tensor the stored hidden activations are
+    written to (and returned) instead of a new one."""
     hid, kin = w1.shape
     nout = w2.shape[0]
     dev = out.device
@@ -216,7 +217,7 @@ def mlp2_forward(x, ldx, rows, n_rows, w1, b1, w2, b2, out, ldo, out_rows=None):
         call("tm_tc_mlp2_smallk_forward", n_rows, hid, nout, x, ldx, rows, kin, _f32c(w1), _f32c(b1), _f32c(w2), _f32c(b2),
              out, ldo, out_rows, _precision(), tm_lib.err_flag(dev), stream())
         return None
-    h = torch.empty(n_rows, hid, dtype=torch.float32, device=dev)
+    h = torch.empty(n_rows, hid, dtype=torch.float32, device=dev) if h_out is None else h_out
     rowmax = None
     if r["lin1"] == "tm_selfmlp_lin1_relu":
         nb = tm_lib.ws_bytes("tm_selfmlp_lin1_ws_bytes")
@@ -510,6 +511,71 @@ def gnn_backward(sched, saved, params, G, cone=None, need_dx=False, need_wgrad=T
         return None, dcf, dnf
     grads = (dcs1w, dcs1b, dcs2w, dcs2b, dns1w, dns1b, dns2w, dns2b, dcn1w, dcn1b, dcn2w, dcn2b)
     return (grads, dcf, dnf) if need_dx else grads
+
+
+def gnn_cone_scratch(sched, device):
+    """The buffers ``gnn_backward_cone`` works in, sized by the parent ``sched``: A / LSE / GA (n_cell_rows, 128) and HID
+    (max(n_cell_rows, pins on even levels), 256), which after the sweep holds the ``fc_cell_self`` hidden rows."""
+    ncr = max(sched.n_cell_rows, 1)
+    hid_rows = max(ncr, int(sched.cell_class.numel()))
+    f32 = lambda r, c: torch.empty(r, c, dtype=torch.float32, device=device)     # noqa: E731
+    return dict(A=f32(ncr, D), LSE=f32(ncr, D), GA=f32(ncr, D), HID=f32(hid_rows, 256))
+
+
+def gnn_backward_cone(cone, H, G, params, cell_feat, net_feat, dcell, dnet, scratch, mark=None):
+    """The feature gradients of ``gnn_backward(..., need_dx=True, need_wgrad=False)`` over a ``tm_graph.FaninCone``
+    after ``build``, from the final ``H`` of a forward (every source of a cone pin is final there):
+
+    1. ``tm_gnn_save_cone``: A / LSE / HID of the cone's cell pins recomputed from H (what the forward would have saved);
+    2. ``tm_gnn_backward_cone``: the persistent data-gradient sweep over the cone; ``G`` (n, 128) holds dLoss/dH on the
+       cone's pins on entry (the head's gradient; zero elsewhere in the cone) and dLoss/dS on exit;
+    3. the self-MLP data gradients over the cone's class lists, with device row counts: ``fc_cell_self``'s hidden rows
+       recomputed (``tm_selfmlp_lin1_relu_dcount``) then ``tm_selfmlp_rows_dx_dcount``; ``fc_net_self`` through
+       ``tm_selfmlp_gen_bwd1_dx_dcount``.  Those are the routes ``mlp2_route`` gives the full backward (they depend on
+       the row count only through ``n_rows > 0``); in another arithmetic than tf32x3 there is no device-count kernel
+       and this raises.
+
+    Rows of ``dcell`` / ``dnet`` (shaped like the features) of the cone's pins are written; the caller zeroes the rest.
+    Every row written is the same bits as the full backward's.  ``scratch``: ``gnn_cone_scratch``.  ``mark(phase)``,
+    when given, is called after each of the three stages ("recompute", "backward", "self_dx": diagnostics)."""
+    (cs1w, cs1b, cs2w, cs2b, ns1w, ns1b, ns2w, ns2b, cn1w, cn1b, cn2w, cn2b) = [_f32c(p) for p in params]
+    cell_feat, net_feat = _rowmajor(cell_feat), _rowmajor(net_feat)
+    cap_c, cap_n = cone.n_cell_cap, cone.n_net_cap
+    rc = mlp2_route(cap_c, cs1w.shape[1], cs1w.shape[0], cs2w.shape[0], x_aligned=_rows_aligned(cell_feat, cell_feat.stride(0)),
+                    dx_aligned=_rows_aligned(dcell, dcell.stride(0)))
+    rn = mlp2_route(cap_n, ns1w.shape[1], ns1w.shape[0], ns2w.shape[0], g_aligned=_rows_aligned(G, D),
+                    dx_aligned=_rows_aligned(dnet, dnet.stride(0)))
+    if (cap_c and (rc["lin1"], rc["dx_only"]) != ("tm_selfmlp_lin1_relu", "tm_selfmlp_rows_dx")) or \
+            (cap_n and rn["dx_only"] != "tm_selfmlp_gen_bwd1_dx"):
+        raise RuntimeError(f"gnn_backward_cone: the self-term MLPs route to {rc['dx_only']} / {rn['dx_only']} in {MATH}; "
+                           "only the fused tf32x3 kernels take a device row count")
+    dev = H.device
+    nb = tm_lib.ws_bytes("tm_gnn_ws_bytes")
+    ws = tm_lib.workspace(nb, dev)
+    call("tm_gnn_save_cone", cone.struct, H, transpose(cn1w), cn1b, transpose(cn2w), scratch["A"], scratch["LSE"],
+         scratch["HID"], ws, nb, stream())
+    if mark:
+        mark("recompute")
+    call("tm_gnn_backward_cone", cone.struct, H, G, cn1w, cn2w, scratch["A"], scratch["LSE"], scratch["HID"],
+         scratch["GA"], ws, nb, stream())
+    if mark:
+        mark("backward")
+    hc = scratch["HID"]                                        # free after the sweep: fc_cell_self's hidden rows
+    counts = cone.counts
+    if cap_c:
+        nb = tm_lib.ws_bytes("tm_selfmlp_lin1_ws_bytes")
+        call("tm_selfmlp_lin1_relu_dcount", cap_c, counts[1:], cell_feat, cell_feat.stride(0), cone.cell_pins,
+             cs1w.shape[1], cs1w, cs1b, hc, 256, tm_lib.workspace(nb, dev), nb, stream())
+        nb = tm_lib.ws_bytes("tm_selfmlp_rows_dh_ws_bytes")
+        call("tm_selfmlp_rows_dx_dcount", cap_c, counts[1:], G, D, cone.cell_pins, cs2w, hc, 256, None, cs1w,
+             cs1w.shape[1], dcell, dcell.stride(0), cone.cell_pins, tm_lib.workspace(nb, dev), nb, stream())
+    if cap_n:
+        nb = tm_lib.ws_bytes("tm_selfmlp_bwd1_ws_bytes")
+        call("tm_selfmlp_gen_bwd1_dx_dcount", cap_n, counts[2:], G, D, cone.net_pins, net_feat, net_feat.stride(0),
+             cone.net_pins, ns1w.shape[1], ns1w, ns1b, ns2w, dnet, dnet.stride(0), tm_lib.workspace(nb, dev), nb,
+             stream())
+    if mark:
+        mark("self_dx")
 
 
 class GnnPropagateFn(torch.autograd.Function):
