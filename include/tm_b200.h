@@ -139,6 +139,15 @@ int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const int32_t* endp
                   int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr, int32_t* bc_row, int32_t* cell_pins,
                   int32_t* net_pins, int32_t* counts, void* ws, size_t ws_bytes, void* stream);
 
+/* tm_fanin_cone that also keeps the cone's membership bitmap: bits[ceil(n/32)] (device, caller's), bit v of word
+ * v / 32 set for every cone pin.  The same kernel, with the bitmap in bits instead of shared memory; ws as for
+ * tm_fanin_cone.  For tm_forward_cones_within. */
+int tm_fanin_cone_bits(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints, const float* seed,
+                       int32_t* order, int32_t* level_ptr, int32_t* cell_base, int32_t* f_ptr, int32_t* f_src,
+                       int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr, int32_t* bc_row,
+                       int32_t* cell_pins, int32_t* net_pins, int32_t* counts, uint32_t* bits, void* ws,
+                       size_t ws_bytes, void* stream);
+
 size_t tm_forward_cones_ws(int64_t n, int32_t n_cand, int32_t num_levels);
 /* Forward cones of `n_cand` candidate edits, joined into ONE sub-schedule over private virtual rows, for scoring
  * alternative edits of the same design without touching the rows of its pins (what-if evaluation).
@@ -169,6 +178,22 @@ int tm_forward_cones(const tm_schedule* s, int32_t n_cand, const int32_t* seed_p
                      const int32_t* endpoints, float* S, int32_t* order, int32_t* level_ptr, int32_t* f_ptr,
                      int32_t* f_src, int32_t* count, int32_t* vpin, int32_t* seed_rows, int32_t* head_rows,
                      int32_t* fitted, int32_t* sizes, int32_t* row_base, void* ws, size_t ws_bytes, void* stream);
+
+size_t tm_forward_cones_within_ws(int64_t n, int32_t n_cand, int32_t num_levels, int64_t n_seeds);
+/* tm_forward_cones restricted to a fan-in cone R(E) (what-if evaluation of an objective that reads only the endpoints
+ * E): `s` is R(E)'s sub-schedule as tm_fanin_cone_bits wrote it and `within` its bitmap.  Candidate k's cone is its
+ * forward cone intersected with R(E), exactly: every in-edge source of a pin of R(E) is in R(E), so the pins of R(E)
+ * that candidate k can change are reached from its seeds inside R(E) through R(E) only.  A seed outside R(E) is
+ * treated as one outside the schedule: not marked, not counted, the sink row in seed_rows.  The outputs are those of
+ * tm_forward_cones (the endpoints passed are normally E).  seeds[n_seeds] with seed_ptr[n_cand] <= n_seeds.  One more
+ * launch than tm_forward_cones (the seed filter), no host synchronisation.  ws: tm_forward_cones_within_ws(s->n, n_cand,
+ * s->num_levels, n_seeds). */
+int tm_forward_cones_within(const tm_schedule* s, const uint32_t* within, int32_t n_cand, const int32_t* seed_ptr,
+                            const int32_t* seeds, const int32_t* seed_slot, int64_t n_seeds, int64_t rows,
+                            int64_t edge_cap, int64_t n_endpoints, const int32_t* endpoints, float* S, int32_t* order,
+                            int32_t* level_ptr, int32_t* f_ptr, int32_t* f_src, int32_t* count, int32_t* vpin,
+                            int32_t* seed_rows, int32_t* head_rows, int32_t* fitted, int32_t* sizes,
+                            int32_t* row_base, void* ws, size_t ws_bytes, void* stream);
 
 /* Apply candidate k of a tm_forward_cones layout: H[vpin[r]] = H[n + r] and S[vpin[r]] = S[n + r] (128 floats a
  * row) for r in [row_base[k], row_base[k] + sizes[k]); nothing when fitted[k] == 0. */

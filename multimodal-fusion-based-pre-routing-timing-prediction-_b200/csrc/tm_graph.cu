@@ -934,11 +934,13 @@ extern "C" size_t tm_fanin_cone_ws(int64_t n, int32_t n_cell_rows) {
   return fanin_bits_bytes(n) + (size_t)(n_cell_rows > 0 ? n_cell_rows : 0) * sizeof(int) + 256;
 }
 
-extern "C" int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints, const float* seed,
+// bits_out NULL: the bitmap lives in shared memory (or the workspace over 1.5M pins) and dies with the build; else the
+// same kernel keeps it in bits_out, which outlives the build (tm_fanin_cone_bits)
+static int fanin_cone_launch(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints, const float* seed,
                              int32_t* order, int32_t* level_ptr, int32_t* cell_base, int32_t* f_ptr, int32_t* f_src,
                              int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr, int32_t* bc_row,
-                             int32_t* cell_pins, int32_t* net_pins, int32_t* counts, void* ws, size_t ws_bytes,
-                             void* stream) {
+                             int32_t* cell_pins, int32_t* net_pins, int32_t* counts, uint32_t* bits_out, void* ws,
+                             size_t ws_bytes, void* stream) {
   TM_REQUIRE(s && s->order && s->level && s->level_ptr && s->cell_base && s->f_ptr && s->f_src && s->bn_ptr &&
                  s->bn_dst && s->bn_w && s->bc_ptr && s->bc_row,
              "tm_fanin_cone: the parent schedule lacks its device arrays (order, level, level_ptr, cell_base, f_ptr, "
@@ -954,11 +956,11 @@ extern "C" int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const in
              "tm_fanin_cone: workspace too small (tm_fanin_cone_ws)");
   cudaStream_t st = (cudaStream_t)stream;
   const size_t bit_bytes = (size_t)cdiv(s->n, 32) * sizeof(uint32_t);
-  const bool in_smem = bit_bytes <= CONE_SMEM_MAX;
+  const bool in_smem = !bits_out && bit_bytes <= CONE_SMEM_MAX;
   uint8_t* p = reinterpret_cast<uint8_t*>(ws);
   uint32_t* gbits = nullptr;
   if (!in_smem) {
-    gbits = reinterpret_cast<uint32_t*>(p);
+    gbits = bits_out ? bits_out : reinterpret_cast<uint32_t*>(p);
     TM_CUDA(cudaMemsetAsync(gbits, 0, bit_bytes, st));
   }
   int* row_map = reinterpret_cast<int*>(p + fanin_bits_bytes(s->n));
@@ -970,6 +972,25 @@ extern "C" int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const in
               counts};
   fanin_cone_kernel<<<1, CONE_T, in_smem ? bit_bytes : 0, st>>>(a);
   return check_launch("fanin_cone");
+}
+
+extern "C" int tm_fanin_cone(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints, const float* seed,
+                             int32_t* order, int32_t* level_ptr, int32_t* cell_base, int32_t* f_ptr, int32_t* f_src,
+                             int32_t* bn_ptr, int32_t* bn_dst, float* bn_w, int32_t* bc_ptr, int32_t* bc_row,
+                             int32_t* cell_pins, int32_t* net_pins, int32_t* counts, void* ws, size_t ws_bytes,
+                             void* stream) {
+  return fanin_cone_launch(s, n_endpoints, endpoints, seed, order, level_ptr, cell_base, f_ptr, f_src, bn_ptr, bn_dst,
+                           bn_w, bc_ptr, bc_row, cell_pins, net_pins, counts, nullptr, ws, ws_bytes, stream);
+}
+
+extern "C" int tm_fanin_cone_bits(const tm_schedule* s, int64_t n_endpoints, const int32_t* endpoints,
+                                  const float* seed, int32_t* order, int32_t* level_ptr, int32_t* cell_base,
+                                  int32_t* f_ptr, int32_t* f_src, int32_t* bn_ptr, int32_t* bn_dst, float* bn_w,
+                                  int32_t* bc_ptr, int32_t* bc_row, int32_t* cell_pins, int32_t* net_pins,
+                                  int32_t* counts, uint32_t* bits, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(bits, "tm_fanin_cone_bits: NULL bitmap");
+  return fanin_cone_launch(s, n_endpoints, endpoints, seed, order, level_ptr, cell_base, f_ptr, f_src, bn_ptr, bn_dst,
+                           bn_w, bc_ptr, bc_row, cell_pins, net_pins, counts, bits, ws, ws_bytes, stream);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1292,6 +1313,14 @@ __global__ void what_if_mask_kernel(int K, int64_t T, const int* fitted, float* 
   if (i < (int64_t)K * T && !fitted[i / T]) pred[i] = __int_as_float(0x7fc00000);
 }
 
+// a seed outside the restriction becomes -1, which the mark and emit kernels treat as a seed outside the schedule
+__global__ void seeds_within_kernel(int n, int m, const int* seeds, const uint32_t* within, int* out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const int v = seeds[i];
+  out[i] = (v >= 0 && v < n && ((within[v >> 5] >> (v & 31)) & 1u)) ? v : -1;
+}
+
 struct ConesWs {
   size_t bits, dir, kl, k, lev, total;
 };
@@ -1363,6 +1392,38 @@ extern "C" int tm_forward_cones(const tm_schedule* s, int32_t n_cand, const int3
   if (int rc = check_launch("cones_plan")) return rc;
   cones_emit_kernel<<<dim3((unsigned)K, (unsigned)(L + 1)), EMIT_T, 0, st>>>(a);
   return check_launch("cones_emit");
+}
+
+// The cones restricted to a fan-in cone R(E): the same three kernels over R(E)'s sub-schedule (their sweeps only walk
+// level_ptr / order / f_ptr / f_src), after the seeds outside R(E) are replaced by -1.  R(E) holds every in-edge
+// source of its pins, so a candidate's restricted cone is exactly its forward cone intersected with R(E).
+extern "C" size_t tm_forward_cones_within_ws(int64_t n, int32_t n_cand, int32_t num_levels, int64_t n_seeds) {
+  return tm_forward_cones_ws(n, n_cand, num_levels) + (((size_t)(n_seeds > 0 ? n_seeds : 0) * sizeof(int) + 255) &
+                                                       ~(size_t)255);
+}
+
+extern "C" int tm_forward_cones_within(const tm_schedule* s, const uint32_t* within, int32_t n_cand,
+                                       const int32_t* seed_ptr, const int32_t* seeds, const int32_t* seed_slot,
+                                       int64_t n_seeds, int64_t rows, int64_t edge_cap, int64_t n_endpoints,
+                                       const int32_t* endpoints, float* S, int32_t* order, int32_t* level_ptr,
+                                       int32_t* f_ptr, int32_t* f_src, int32_t* count, int32_t* vpin,
+                                       int32_t* seed_rows, int32_t* head_rows, int32_t* fitted, int32_t* sizes,
+                                       int32_t* row_base, void* ws, size_t ws_bytes, void* stream) {
+  TM_REQUIRE(s && s->n > 0 && s->num_levels > 0 && within, "tm_forward_cones_within: bad schedule or bitmap");
+  TM_REQUIRE(n_seeds >= 0 && n_seeds < INT32_MAX && (n_seeds == 0 || seeds),
+             "tm_forward_cones_within: bad seed list");
+  TM_REQUIRE(ws && ws_bytes >= tm_forward_cones_within_ws(s->n, n_cand, s->num_levels, n_seeds),
+             "tm_forward_cones_within: workspace too small (tm_forward_cones_within_ws)");
+  const size_t cones_bytes = tm_forward_cones_ws(s->n, n_cand, s->num_levels);
+  int* kept = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(ws) + cones_bytes);
+  if (n_seeds > 0) {
+    seeds_within_kernel<<<(unsigned)cdiv(n_seeds, 256), 256, 0, (cudaStream_t)stream>>>((int)s->n, (int)n_seeds, seeds,
+                                                                                         within, kept);
+    if (int rc = check_launch("seeds_within")) return rc;
+  }
+  return tm_forward_cones(s, n_cand, seed_ptr, n_seeds > 0 ? kept : seeds, seed_slot, rows, edge_cap, n_endpoints,
+                          endpoints, S, order, level_ptr, f_ptr, f_src, count, vpin, seed_rows, head_rows, fitted,
+                          sizes, row_base, ws, cones_bytes, stream);
 }
 
 extern "C" int tm_what_if_commit(int64_t n, int32_t k, const int32_t* fitted, const int32_t* sizes,

@@ -1016,10 +1016,12 @@ class IncrementalEvaluation:
         """Pins of the last ``input_grads`` cone (one device read, diagnostics); 0 before the first call."""
         return self._grad["cone"].size() if self._grad is not None else 0
 
-    def what_if(self, pin_sets):
+    def what_if(self, pin_sets, endpoints=None):
         """A ``WhatIf`` over the candidate edits ``pin_sets`` (a sequence of K pin sequences, validated as ``update``
-        validates its pins).  Needs ``what_if_rows`` > 0 at construction."""
-        return WhatIf(self, pin_sets)
+        validates its pins).  ``endpoints``: a host sequence of endpoint positions (indices into ``pred``) to predict
+        only those, propagating each candidate through only the pins that reach them; None predicts all T.  Needs
+        ``what_if_rows`` > 0 at construction."""
+        return WhatIf(self, pin_sets, endpoints)
 
     def max_in_degree(self):
         """The largest in-edge count of a scheduled pin (one device read, cached)."""
@@ -1061,9 +1063,23 @@ class WhatIf:
     into the batch, then reruns the head over the committed H (``inc.pred`` gets candidate k's predictions, the same
     bits, and ``inc.X`` / the head's hidden rows follow) -- the state ``inc.update`` leaves.  It raises ``ValueError``
     when the base changed since this object's last run / replay, when another ``WhatIf`` of ``inc`` ran since, or when
-    candidate k was not admitted."""
+    candidate k was not admitted.
 
-    def __init__(self, inc, pin_sets):
+    ``inc.what_if(pin_sets, endpoints=E)`` predicts only the endpoint positions E (indices into ``inc.pred``, joined
+    positions for a joined batch; validated as pins are, against [0, T), and kept sorted in ``endpoints``).  Only pins
+    from which an endpoint of E is reachable -- E's fan-in cone R(E), built once here (``within_size()``) -- can change
+    an H row E reads, so each candidate propagates through its forward cone intersected with R(E)
+    (``tm_forward_cones_within``), and the head runs over K x T_E rows.  ``run()`` / ``capture()`` return (K, T_E):
+    row k is the same bits as ``step.forward`` with candidate k's rows alone at ``endpoints``, and as the unrestricted
+    ``run()[k, endpoints]``.  A candidate's pins outside R(E) change nothing (an all-outside candidate has cone 0 and
+    predicts the base), and admission counts restricted cones, so many more candidates fit in ``what_if_rows``.  Memory
+    beyond the unrestricted form's: R(E)'s sub-schedule (the size of the schedule) and its n/8-byte bitmap.
+    ``commit(k)`` of a restricted ``WhatIf`` has the same preconditions and errors, but the rest of candidate k's cone
+    was never computed: it writes candidate k's feature rows into the batch and runs ``inc.update`` over its pins, so it
+    propagates, and leaves exactly the state ``update`` leaves (``H``, ``S``, ``pred``, the batch, ``generation``,
+    ``cone_size()``)."""
+
+    def __init__(self, inc, pin_sets, endpoints=None):
         if inc.R == 0:
             raise ValueError("IncrementalEvaluation.what_if: built with what_if_rows=0; pass what_if_rows > 0 to "
                              "DesignStep.incremental")
@@ -1074,7 +1090,9 @@ class WhatIf:
             raise ValueError("IncrementalEvaluation.what_if: no candidate")
         self.inc, b = inc, inc.b
         dev = inc.H.device
-        K, T = len(sets), int(b.endpoints.numel())
+        K, T_all = len(sets), int(b.endpoints.numel())
+        self.endpoints = None if endpoints is None else self._positions(endpoints, T_all)
+        T = T_all if self.endpoints is None else int(self.endpoints.size)
         self.K, self.T = K, T
         self._off = np.concatenate([[0], np.cumsum([s.size for s in sets])]).astype(np.int64)
         self._pins = np.concatenate(sets).astype(np.int64)
@@ -1097,13 +1115,43 @@ class WhatIf:
         self._seed_ptr, self._seeds, self._seed_slot = i32(seed_ptr), i32(self._pins[loc]), i32(slot)
         self._x_cell, self._x_net = i32(loc[is_cell]), i32(loc[~is_cell])
         self._nc = nc
-        self.cones = ForwardCones(b.graph, K, inc.R, inc.R * max(inc.max_in_degree(), 1), b.endpoints, loc.size)
-        self._img_rows = i32(np.tile(np.arange(T), K))
+        edge_cap = inc.R * max(inc.max_in_degree(), 1)
+        if self.endpoints is None:
+            self._fanin = None
+            self.cones = ForwardCones(b.graph, K, inc.R, edge_cap, b.endpoints, loc.size)
+            img = np.arange(T)
+        else:
+            # R(E): built once, E and the structure are fixed for this object's life
+            ep = b.endpoints.index_select(0, torch.from_numpy(self.endpoints).to(dev)).contiguous()
+            self._fanin = FaninCone(b.graph, keep_bits=True)
+            self._fanin.build(ep, torch.ones(T, dtype=torch.float32, device=dev))
+            self.cones = ForwardCones(b.graph, K, inc.R, edge_cap, ep, loc.size, within=self._fanin)
+            img = self.endpoints
+        self._img_rows = i32(np.tile(img, K))
         width = inc.X.shape[1]
         self._Xw = torch.empty(K * T, width, dtype=torch.float32, device=dev)
         self._pred2 = torch.empty(K * T, inc._pred2.shape[1], dtype=torch.float32, device=dev)
         self.pred = self._pred2.view(K, T)
         self._gen = None                                  # inc.generation at the last run / replay
+
+    @staticmethod
+    def _positions(endpoints, T):
+        """-> int64 ndarray of the distinct endpoint positions (sorted), validated against [0, T)."""
+        if torch.is_tensor(endpoints):
+            if endpoints.device.type != "cpu":
+                raise ValueError("IncrementalEvaluation.what_if: endpoints must be a host sequence (list, ndarray or "
+                                 "CPU tensor)")
+            endpoints = endpoints.numpy()
+        arr = np.asarray(endpoints)
+        if arr.size == 0:
+            raise ValueError("IncrementalEvaluation.what_if: no endpoint")
+        if not np.issubdtype(arr.dtype, np.integer):
+            raise ValueError(f"IncrementalEvaluation.what_if: endpoint positions must be integers, got {arr.dtype}")
+        arr = np.unique(arr.reshape(-1).astype(np.int64))
+        if arr[0] < 0 or arr[-1] >= T:
+            raise ValueError(f"IncrementalEvaluation.what_if: endpoint positions must lie in [0, {T}), got "
+                             f"{arr[0]} .. {arr[-1]}")
+        return arr
 
     def rows(self, k):
         """(pins int64 ndarray, cell_feat rows, net_feat rows) of candidate k: views into ``cell_feat`` / ``net_feat``."""
@@ -1156,7 +1204,9 @@ class WhatIf:
 
     def commit(self, k):
         """Apply candidate k: the batch's feature rows, ``inc.H``, ``inc.S``, ``inc.pred`` and the head's inputs as
-        ``inc.update`` leaves them, without a propagation."""
+        ``inc.update`` leaves them, without a propagation.  With ``endpoints`` the run computed only the part of the
+        cone inside R(E): candidate k's feature rows are written into the batch and ``inc.update(pins)`` propagates
+        them, so the state is exactly the one ``update`` leaves."""
         inc = self.inc
         if self._gen is None or self._gen != inc.generation or inc._overlay is not self:
             raise ValueError("WhatIf.commit: the base changed (or another what-if ran) since this object's last run / "
@@ -1166,8 +1216,14 @@ class WhatIf:
         c = self.cones
         if not bool(c.fitted[k].item()):
             raise ValueError(f"WhatIf.commit: candidate {k} was not admitted (what_if_rows too small)")
-        call("tm_what_if_commit", inc.n, int(k), c.fitted, c.sizes, c.row_base, c.vpin, inc.H_ext, inc.S_ext, stream())
         s, e = int(self._off[k]), int(self._off[k + 1])
+        if self._fanin is not None:                      # restricted: only the part of the cone inside R(E) ran
+            if e > s:
+                inc.b.cell_feat.index_copy_(0, self._pin_idx[s:e], self.cell_feat[s:e])
+                inc.b.net_feat.index_copy_(0, self._pin_idx[s:e], self.net_feat[s:e])
+            inc.update(self._pins[s:e])
+            return
+        call("tm_what_if_commit", inc.n, int(k), c.fitted, c.sizes, c.row_base, c.vpin, inc.H_ext, inc.S_ext, stream())
         if e > s:
             inc.b.cell_feat.index_copy_(0, self._pin_idx[s:e], self.cell_feat[s:e])
             inc.b.net_feat.index_copy_(0, self._pin_idx[s:e], self.net_feat[s:e])
@@ -1181,5 +1237,11 @@ class WhatIf:
         return self.cones.fitted.cpu().numpy().astype(bool)
 
     def cone_sizes(self):
-        """(K,) int host array: each candidate's cone pins in the last run / replay (one device read)."""
+        """(K,) int host array: each candidate's cone pins in the last run / replay (one device read); with
+        ``endpoints``, the pins of its cone inside R(E)."""
         return self.cones.sizes.cpu().numpy().astype(np.int64)
+
+    def within_size(self):
+        """|R(E)|, the pins of the endpoints' fan-in cone (one device read, diagnostics only); the schedule's pin count
+        without ``endpoints``."""
+        return self._fanin.size() if self._fanin is not None else self.inc.sched.n_sched

@@ -341,12 +341,16 @@ class FaninCone:
     self-term MLPs), ``counts`` (device int32 [3]) the cone's pins and the two lists' lengths.  The buffers are
     allocated once, sized by the parent schedule, and rewritten by every build.
 
+    ``keep_bits=True`` keeps the cone's membership bitmap in ``bits`` (device int32 [ceil(n / 32)], bit v of word
+    v // 32 for pin v; ``tm_fanin_cone_bits``): the restriction ``ForwardCones(..., within=cone)`` reads it.
+
     Not ``BackwardCone``: that one is built on the host for the weight-gradient contractions of a training step."""
 
-    def __init__(self, graph):
+    def __init__(self, graph, keep_bits=False):
         s = self.sched = graph.schedule()
         dev = s.device
         i32 = lambda k: torch.empty(max(int(k), 1), dtype=torch.int32, device=dev)      # noqa: E731
+        self.bits = i32((s.n + 31) // 32) if keep_bits else None
         self.order = i32(s.n_sched)
         self.level_ptr = i32(s.num_levels + 1)
         self.cell_base = i32(s.num_levels + 1)
@@ -379,10 +383,13 @@ class FaninCone:
                 and seed.shape == endpoints.shape and endpoints.is_contiguous() and seed.is_contiguous()):
             raise ValueError(f"FaninCone.build: endpoints (int32) and seed (float32) must be contiguous tensors of one "
                              f"shape on {dev}")
-        tm_lib.call("tm_fanin_cone", self.sched.struct, int(endpoints.numel()), endpoints, seed, self.order,
-                    self.level_ptr, self.cell_base, self.f_ptr, self.f_src, self.bn_ptr, self.bn_dst, self.bn_w,
-                    self.bc_ptr, self.bc_row, self.cell_pins, self.net_pins, self.counts, self.ws, self.nb,
-                    tm_lib.stream())
+        args = (self.sched.struct, int(endpoints.numel()), endpoints, seed, self.order, self.level_ptr, self.cell_base,
+                self.f_ptr, self.f_src, self.bn_ptr, self.bn_dst, self.bn_w, self.bc_ptr, self.bc_row, self.cell_pins,
+                self.net_pins, self.counts)
+        if self.bits is None:
+            tm_lib.call("tm_fanin_cone", *args, self.ws, self.nb, tm_lib.stream())
+        else:
+            tm_lib.call("tm_fanin_cone_bits", *args, self.bits, self.ws, self.nb, tm_lib.stream())
         return self.struct
 
     def size(self):
@@ -401,11 +408,20 @@ class ForwardCones:
     copies every cone pin's S row to its virtual row and returns ``.struct``.  It also fills ``seed_rows`` (the
     virtual row of every seed, or the sink row), ``head_rows`` (K x T: each endpoint's row per candidate), ``vpin``,
     ``fitted``, ``sizes`` and ``row_base``.  The buffers are allocated once: the joined arrays sized by ``rows`` and
-    ``edge_cap``, two n/8-byte bitmaps per candidate in the workspace."""
+    ``edge_cap``, two n/8-byte bitmaps per candidate in the workspace.
 
-    def __init__(self, graph, n_cand, rows, edge_cap, endpoints, n_seeds):
+    ``within``: a built ``FaninCone(graph, keep_bits=True)`` of endpoints E restricts every cone to E's fan-in cone
+    R(E) (``tm_forward_cones_within``): candidate k's cone is its forward cone intersected with R(E), the sweeps walk
+    R(E)'s sub-schedule instead of the whole schedule, and seeds outside R(E) are treated as seeds outside the schedule.
+    Exact for the predictions of E: R(E) holds every in-edge source of its pins.  The fan-in cone must not be rebuilt
+    for other endpoints while this object is in use."""
+
+    def __init__(self, graph, n_cand, rows, edge_cap, endpoints, n_seeds, within=None):
         s = self.sched = graph.schedule()
         dev = s.device
+        if within is not None and within.bits is None:
+            raise ValueError("ForwardCones: the restriction needs a FaninCone built with keep_bits=True")
+        self.within, self.n_seeds = within, int(n_seeds)
         i32 = lambda k: torch.empty(max(int(k), 1), dtype=torch.int32, device=dev)      # noqa: E731
         self.K, self.rows, self.edge_cap, self.T = int(n_cand), int(rows), int(edge_cap), int(endpoints.numel())
         self.endpoints = endpoints
@@ -421,7 +437,10 @@ class ForwardCones:
         self.sizes = torch.zeros(self.K, dtype=torch.int32, device=dev)
         self.row_base = torch.zeros(self.K, dtype=torch.int32, device=dev)
         self.cell_base = torch.zeros(s.num_levels + 1, dtype=torch.int32, device=dev)
-        self.nb = tm_lib.ws_bytes("tm_forward_cones_ws", s.n, self.K, s.num_levels)
+        if within is None:
+            self.nb = tm_lib.ws_bytes("tm_forward_cones_ws", s.n, self.K, s.num_levels)
+        else:
+            self.nb = tm_lib.ws_bytes("tm_forward_cones_within_ws", s.n, self.K, s.num_levels, self.n_seeds)
         self.ws = tm_lib.workspace(self.nb, dev)
         # only what tm_gnn_forward_cone reads: the joined order / level_ptr / f_ptr / f_src over n + rows + 1 rows
         self.struct = tm_lib.tm_schedule(
@@ -433,10 +452,16 @@ class ForwardCones:
         """Enqueue the joined cones of the candidates' seeds (int32 device CSR ``seed_ptr`` (K+1) / ``seeds``; seed i's
         row goes to ``seed_rows[seed_slot[i]]``) on the current stream, with S the (n + rows + 1, 128) self terms.
         Returns ``.struct``."""
-        tm_lib.call("tm_forward_cones", self.sched.struct, self.K, seed_ptr, seeds, seed_slot, self.rows, self.edge_cap,
-                    self.T, self.endpoints, S, self.order, self.level_ptr, self.f_ptr, self.f_src, self.count,
-                    self.vpin, self.seed_rows, self.head_rows, self.fitted, self.sizes, self.row_base, self.ws,
-                    self.nb, tm_lib.stream())
+        out = (self.rows, self.edge_cap, self.T, self.endpoints, S, self.order, self.level_ptr, self.f_ptr, self.f_src,
+               self.count, self.vpin, self.seed_rows, self.head_rows, self.fitted, self.sizes, self.row_base, self.ws,
+               self.nb, tm_lib.stream())
+        if self.within is None:
+            tm_lib.call("tm_forward_cones", self.sched.struct, self.K, seed_ptr, seeds, seed_slot, *out)
+        else:
+            if int(seeds.numel()) > self.n_seeds:
+                raise ValueError(f"ForwardCones.build: {int(seeds.numel())} seeds, sized for {self.n_seeds}")
+            tm_lib.call("tm_forward_cones_within", self.within.struct, self.within.bits, self.K, seed_ptr, seeds,
+                        seed_slot, int(seeds.numel()), *out)
         return self.struct
 
 
